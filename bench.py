@@ -4,6 +4,7 @@
     python bench.py --gpus N --steps K --warmup W            (ours; torchrun for N > 1)
     python bench.py --impl reference --gpus N --steps K ...   (the reference's CPU path)
     python bench.py --config c3|c4|c5 ...                     (the other BASELINE configurations)
+    python bench.py ... --dump-outputs DIR                    (also write the last timed step's run to DIR/*.npy)
 
 A step is one pass of the whole counting path over one batch of synthetic reads:
 reads -> super-window records -> per-bin count -> distinct records in key order
@@ -37,6 +38,8 @@ if ROOT not in sys.path:
 METRIC = "k-mers counted/s at k=31"          # BASELINE.json's metric; a line run with another k says so (metric_for)
 UNIT = "kmers/s"
 REF_CHUNK = 89364           # reads per chunk at the reference's defaults (KMerCounter.cpp:193-212, SURVEY 3.1)
+DUMP_BYTES = 48 << 20       # --dump-outputs writes at most this much; larger runs are sampled at seeded record indices
+DUMP_SEED = 20261020
 
 # BASELINE.json configs[0..4] (SURVEY.md 8(d) "Synthetic inputs"); reads are per GPU
 CONFIGS = {
@@ -77,7 +80,14 @@ def parse_args():
     ap.add_argument("--occ", type=int, default=0, help="k-mer occurrences per minimizer bin (0 = library default)")
     ap.add_argument("--bench", default="count", choices=["count", "merge"],
                     help="merge: time kc_merge_runs (GPU KMerFileMerger) over --runs runs of --reads reads each")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the run the last step computed to DIR as float64 .npy files "
+                         "(a seeded sample of its records beyond %d MB)" % (DUMP_BYTES >> 20))
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl == "reference":
+        ap.error("--dump-outputs writes what this project's GPU path computed; the reference arm computes on the host")
     cfg = dict(CONFIGS[a.config or "c2"])
     changed = []
     for key in ("reads", "k", "genome", "sub_rate", "n_rate", "seed", "zipf_loci", "runs"):
@@ -342,6 +352,30 @@ def run_reference(a, rank):
 
 
 # ------------------------------------------------------------------- our arm
+def dump_run(run, out_dir, device, budget, suffix=""):
+    """--dump-outputs: the records of a device-resident run as float64 .npy files in out_dir --
+    keys[m, 2W] (every key word as its high and low 32 bits, exact in float64), counts[m], record_index[m]
+    (the records' positions in the run) and run_summary = [records, sum of counts]. A run whose m = n
+    records do not fit `budget` bytes is sampled at seeded, sorted record indices."""
+    import numpy as np
+    import torch
+    from kmer_counter_b200.multigpu import run_as_tensors
+    keys, counts = run_as_tensors(run, device)
+    n, W = keys.shape
+    cap = budget // (8 * (2 * W + 2))
+    idx = np.arange(n) if n <= cap else np.unique(np.random.default_rng(DUMP_SEED).integers(0, n, size=cap))
+    sel = torch.from_numpy(idx).to(device)
+    k = keys.index_select(0, sel).cpu().numpy().view(np.uint64)
+    c = counts.index_select(0, sel).cpu().numpy().view(np.uint32)
+    halves = np.empty((len(idx), 2 * W), dtype=np.float64)
+    halves[:, 0::2] = k >> np.uint64(32)
+    halves[:, 1::2] = k & np.uint64(0xFFFFFFFF)
+    total = int((counts.to(torch.int64) & 0xFFFFFFFF).sum().item())
+    os.makedirs(out_dir, exist_ok=True)
+    for name, arr in (("keys", halves), ("counts", c), ("record_index", idx), ("run_summary", [n, total])):
+        np.save(os.path.join(out_dir, name + suffix + ".npy"), np.asarray(arr, dtype=np.float64))
+
+
 class Job:
     """One rank's share of the workload and the path it is counted through."""
 
@@ -386,6 +420,7 @@ class Job:
             self.counter.accum_begin(per_run + 4096)          # (pieces are whole multiples of 16 reads: the last one is a little longer)
         self.per_run = per_run
         self.d_reads = None
+        self.last_run = None
         self.acc = self.new_acc()
 
     @staticmethod
@@ -445,10 +480,14 @@ class Job:
             stack.append((lv + 1, m))
         return stack[0][1]
 
-    def step(self):
+    def step(self, keep=False):
+        """One pass over this rank's reads -> records in its run; keep=True holds the run in last_run."""
         run = self.count(self.d_reads.data_ptr(), self.R)
         n = len(run)
-        run.free()
+        if keep:
+            self.last_run = run
+        else:
+            run.free()
         return n
 
 
@@ -543,8 +582,8 @@ def run_ours(a, rank, world, local_rank):
         ev0.record(stream)
         t0 = time.perf_counter()
         distinct = 0
-        for _ in range(a.steps):
-            distinct = job.step()
+        for i in range(a.steps):
+            distinct = job.step(keep=a.dump_outputs is not None and i == a.steps - 1)
         ev1.record(stream)
         barrier()
         wall = time.perf_counter() - t0
@@ -586,6 +625,11 @@ def run_ours(a, rank, world, local_rank):
                   "achieved_gbs_over_step": x.item() / (ms_per_step * 1e-3) / 1e9, "peak": 900, "measured_peer_copy": 770,
                   "note": "both exchanges are the load side of the consuming kernels (peer loads over NVLink/NVSwitch), "
                           "spread over the step: the rate is bytes over the whole step time, not a link saturation figure"}
+
+    if job.last_run is not None:
+        dump_run(job.last_run, a.dump_outputs, dev, DUMP_BYTES // world, "_rank%d" % rank if world > 1 else "")
+        job.last_run.free()
+        job.last_run = None
 
     # ---- end to end through the host-buffer API (pinned in, pinned out)
     e2e = None
@@ -828,13 +872,17 @@ def run_merge_bench(a):
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     with ClockSampler(0) as clk:
         ev0.record(stream)
-        for _ in range(a.steps):
+        for i in range(a.steps):
             m = counter.merge(parts)
             U = len(m)
-            m.free()
+            if a.dump_outputs is None or i + 1 < a.steps:
+                m.free()
         ev1.record(stream)
         torch.cuda.synchronize()
     ms = ev0.elapsed_time(ev1) / a.steps
+    if a.dump_outputs is not None:
+        dump_run(m, a.dump_outputs, dev, DUMP_BYTES)
+        m.free()
     peak, peak_src = measured_peak_gbs()
     # bytes of the tree: every level reads its inputs and writes its outputs once
     sizes, tree_bytes = [len(p) for p in parts], 0

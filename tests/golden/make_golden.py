@@ -65,4 +65,31 @@ with tempfile.TemporaryDirectory() as d:
     open(os.path.join(HERE, "small_k31.records"), "wb").write(open(out, "rb").read())
     oracle.ref_count_packed(reads, 60, 40, 64, 1, d, out)
     open(os.path.join(HERE, "small_k40.records"), "wb").write(open(out, "rb").read())
+
+# sha256 of the reference's outputs on the inputs of test_oracle.py's reference comparisons
+sys.path.insert(0, os.path.dirname(HERE))
+import test_oracle  # noqa: E402
+
+sha = lambda b: hashlib.sha256(bytes(b)).hexdigest()
+dig = {"source": "reference build via oracle/_ref (ref_process_chunk, ref_count_packed, ref_read_fastq_dir)",
+       "chunks": {}, "random_shapes": []}
+for (R, L, k, G, e, n) in test_oracle.REFERENCE_CASES:
+    reads = oracle.gen_reads(R, L, G, e, n, seed=1000 + R + k)
+    with tempfile.TemporaryDirectory() as d:
+        out = os.path.join(d, "out.bin")
+        oracle.ref_count_packed(reads, L, k, max(1, R // 5), 2, d, out)
+        art = open(out, "rb").read()
+    dig["chunks"][test_oracle.case_key(R, L, k, G, e, n)] = {
+        "reads_sha256": sha(reads), "sorted_sha256": sha(oracle.ref_process_chunk(reads, L, k, True)),
+        "unsorted_sha256": sha(oracle.ref_process_chunk(reads, L, k, False)), "artefact_sha256": sha(art)}
+for L, k, R, reads in test_oracle.random_shapes():
+    dig["random_shapes"].append({"L": L, "k": k, "R": R, "reads_sha256": sha(reads),
+                                 "sorted_sha256": sha(oracle.ref_process_chunk(reads, L, k, True)),
+                                 "unsorted_sha256": sha(oracle.ref_process_chunk(reads, L, k, False))})
+fq = oracle.gen_fastq(50, 100, 5000, 0.01, 0.01, seed=3)
+with tempfile.TemporaryDirectory() as d:
+    open(os.path.join(d, "a.fastq"), "wb").write(fq)
+    data, L = oracle.ref_read_fastq_dir(d)
+dig["fastq_reader"] = {"fastq_sha256": sha(fq), "L": L, "sha256": sha(data)}
+json.dump(dig, open(os.path.join(HERE, "reference_digests.json"), "w"), indent=1)
 print("golden vectors written to", HERE)

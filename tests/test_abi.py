@@ -3,6 +3,8 @@ declares, fails loudly without a device, and the host-side helpers behave."""
 import ctypes as C
 import os
 import re
+import subprocess
+import sys
 
 import numpy as np
 import pytest
@@ -45,14 +47,14 @@ def test_config_struct_layout_matches_header():
 
 
 def test_no_cpu_fallback():
-    """Without a CUDA device the product path must fail loudly, not compute on the CPU."""
-    import torch
-    import kmer_counter_b200 as kc
-    if torch.cuda.is_available():
-        pytest.skip("a GPU is present")
-    with pytest.raises(kc.KcError) as ei:
-        kc.Counter(31, 100)
-    assert ei.value.code == -2
+    """Without a CUDA device the product path must fail loudly, not compute on the CPU. The check
+    runs in a child process that sees no device, so it runs on GPU machines too."""
+    code = ("import kmer_counter_b200 as kc\n"
+            "try:\n    kc.Counter(31, 100)\nexcept kc.KcError as e:\n    print('code', e.code)\n")
+    r = subprocess.run([sys.executable, "-c", code], cwd=ROOT, env=dict(os.environ, CUDA_VISIBLE_DEVICES=""),
+                       capture_output=True, text=True, timeout=300)
+    assert r.returncode == 0, r.stderr[-2000:]
+    assert r.stdout.split() == ["code", "-2"], r.stdout
 
 
 def test_bad_arguments_are_rejected_before_touching_the_device():

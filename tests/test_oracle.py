@@ -1,7 +1,6 @@
 """CPU tests: the oracle (oracle/kc_oracle.c) against the golden vectors produced by the
-reference's own code (tests/golden, made by make_golden.py from oracle/_ref), against
-SURVEY.md Appendix A.4's known answers, and -- where oracle/_ref is present -- against the
-reference build directly."""
+reference's own code (tests/golden, made by make_golden.py from oracle/_ref) and against
+SURVEY.md Appendix A.4's known answers."""
 import hashlib
 import json
 import os
@@ -13,10 +12,51 @@ import oracle
 
 GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
+# shapes of the comparisons with the reference build (tests/golden/reference_digests.json)
+REFERENCE_CASES = [(1500, 100, 31, 20000, 0.01, 0.003), (600, 70, 63, 5000, 0.0, 0.002),
+                   (300, 150, 96, 2000, 0.01, 0.01), (300, 150, 128, 2000, 0.01, 0.01),
+                   (400, 45, 5, 0, 0.0, 0.02), (900, 100, 28, 9000, 0.0, 0.0),
+                   (400, 133, 100, 3000, 0.001, 0.001), (500, 41, 33, 0, 0.0, 0.01),
+                   (300, 37, 29, 0, 0.0, 0.0), (300, 100, 64, 4000, 0.0, 0.004)]
+
 
 def _hexkeys(data, k):
     keys, counts = oracle.records_to_arrays(data, k)
     return [[["%016x" % int(w) for w in row], int(c)] for row, c in zip(keys, counts)]
+
+
+def _sha(data):
+    return hashlib.sha256(bytes(data)).hexdigest()
+
+
+def _reference_digests():
+    with open(os.path.join(GOLD, "reference_digests.json")) as f:
+        return json.load(f)
+
+
+def case_key(R, L, k, G, e, n):
+    return "R=%d L=%d k=%d G=%d e=%r n=%r" % (R, L, k, G, e, n)
+
+
+def random_shapes():
+    """60 random shapes (k 1..128, L up to 200, L % 32 != 0) over a hostile alphabet -- lower case,
+    N, IUPAC letters, digits, bytes >= 0x80 -- so that validity runs start and stop everywhere.
+    Yields (L, k, R, reads)."""
+    rng = np.random.default_rng(20261018)
+    alphabet = np.frombuffer(b"ACGT" * 12 + b"acgtNnRYKM-.*0" + bytes([0, 127, 128, 255]), dtype=np.uint8)
+    done = 0
+    while done < 60:
+        L = int(rng.integers(10, 201))
+        if L % 32 == 0 or 2 + 8 * ((L + 31) // 32) > L:            # shapes the reference corrupts (SURVEY F8)
+            continue
+        k = int(rng.integers(1, min(L, 128) + 1))
+        R = int(rng.integers(1, 60))
+        reads = alphabet[rng.integers(0, alphabet.size, size=R * L)]
+        if done % 3 == 0:                                           # mostly valid reads with a few bad letters
+            reads = np.frombuffer(b"ACGT", dtype=np.uint8)[rng.integers(0, 4, size=R * L)].copy()
+            reads[rng.integers(0, R * L, size=max(1, R * L // 50))] = ord("N")
+        yield L, k, R, np.ascontiguousarray(reads)
+        done += 1
 
 
 def test_survey_appendix_a4_known_answers():
@@ -81,46 +121,32 @@ def test_golden_small_artefacts_bytes():
         assert order == sorted(order) and len(set(order)) == len(order)           # strictly ascending
 
 
-@pytest.mark.skipif(not oracle.ref_available(), reason="oracle/_ref not built")
-@pytest.mark.parametrize("R,L,k,G,e,n", [(1500, 100, 31, 20000, 0.01, 0.003), (600, 70, 63, 5000, 0.0, 0.002),
-                                         (300, 150, 96, 2000, 0.01, 0.01), (300, 150, 128, 2000, 0.01, 0.01),
-                                         (400, 45, 5, 0, 0.0, 0.02), (900, 100, 28, 9000, 0.0, 0.0),
-                                         (400, 133, 100, 3000, 0.001, 0.001), (500, 41, 33, 0, 0.0, 0.01),
-                                         (300, 37, 29, 0, 0.0, 0.0), (300, 100, 64, 4000, 0.0, 0.004)])
-def test_oracle_equals_reference_build(R, L, k, G, e, n, tmp_path):
+@pytest.mark.parametrize("R,L,k,G,e,n", REFERENCE_CASES)
+def test_oracle_equals_reference_build(R, L, k, G, e, n):
+    """The chunk artefact (sorted and unsorted) and Pipeline B's merged file against the reference
+    build's on the same reads (sha256, tests/golden/reference_digests.json)."""
+    want = _reference_digests()["chunks"][case_key(R, L, k, G, e, n)]
     reads = oracle.gen_reads(R, L, G, e, n, seed=1000 + R + k)
-    for do_sort in (True, False):
-        assert oracle.process_chunk(reads, L, k, do_sort) == oracle.ref_process_chunk(reads, L, k, do_sort)
-    out = str(tmp_path / "out.bin")
-    oracle.ref_count_packed(reads, L, k, max(1, R // 5), 2, str(tmp_path), out)
-    want = open(out, "rb").read()
-    assert oracle.count(reads, L, k, chunk_reads=max(1, R // 5), threads=2) == want
-    assert oracle.naive_count(reads, L, k) == want
+    assert _sha(reads) == want["reads_sha256"], "generator drifted"
+    assert _sha(oracle.process_chunk(reads, L, k, True)) == want["sorted_sha256"]
+    assert _sha(oracle.process_chunk(reads, L, k, False)) == want["unsorted_sha256"]
+    art = oracle.count(reads, L, k, chunk_reads=max(1, R // 5), threads=2)
+    assert _sha(art) == want["artefact_sha256"]
+    assert oracle.naive_count(reads, L, k) == art
 
 
-@pytest.mark.skipif(not oracle.ref_available(), reason="oracle/_ref not built")
 def test_random_shapes_and_alphabets_three_way():
-    """60 random shapes (k 1..128, L up to 200, L % 32 != 0) over a hostile alphabet -- lower case,
-    N, IUPAC letters, digits, bytes >= 0x80 -- so that validity runs start and stop everywhere:
-    restatement == reference build == independent window model, sorted and unsorted."""
-    rng = np.random.default_rng(20261018)
-    alphabet = np.frombuffer(b"ACGT" * 12 + b"acgtNnRYKM-.*0" + bytes([0, 127, 128, 255]), dtype=np.uint8)
+    """random_shapes(): restatement == reference build (sha256 of its output, sorted and unsorted)
+    == independent window model."""
+    want = _reference_digests()["random_shapes"]
     done = 0
-    while done < 60:
-        L = int(rng.integers(10, 201))
-        if L % 32 == 0 or 2 + 8 * ((L + 31) // 32) > L:            # shapes the reference corrupts (SURVEY F8)
-            continue
-        k = int(rng.integers(1, min(L, 128) + 1))
-        R = int(rng.integers(1, 60))
-        reads = alphabet[rng.integers(0, alphabet.size, size=R * L)]
-        if done % 3 == 0:                                           # mostly valid reads with a few bad letters
-            reads = np.frombuffer(b"ACGT", dtype=np.uint8)[rng.integers(0, 4, size=R * L)].copy()
-            reads[rng.integers(0, R * L, size=max(1, R * L // 50))] = ord("N")
-        reads = np.ascontiguousarray(reads)
-        for do_sort in (True, False):
-            assert oracle.process_chunk(reads, L, k, do_sort) == oracle.ref_process_chunk(reads, L, k, do_sort), (L, k, R)
+    for (L, k, R, reads), w in zip(random_shapes(), want):
+        assert (L, k, R, _sha(reads)) == (w["L"], w["k"], w["R"], w["reads_sha256"]), "shape generator drifted"
+        assert _sha(oracle.process_chunk(reads, L, k, True)) == w["sorted_sha256"], (L, k, R)
+        assert _sha(oracle.process_chunk(reads, L, k, False)) == w["unsorted_sha256"], (L, k, R)
         assert oracle.count(reads, L, k, chunk_reads=7) == oracle.naive_count(reads, L, k), (L, k, R)
         done += 1
+    assert done == len(want) == 60
 
 
 def test_merge_semantics():
@@ -142,19 +168,16 @@ def test_unsupported_shapes_are_rejected():
         oracle.process_chunk(oracle.gen_reads(4, 20, 0, 0, 0, seed=1), 20, 31)     # k > L
 
 
-def test_fastq_parser_restatement(tmp_path):
+def test_fastq_parser_restatement():
     fq = oracle.gen_fastq(50, 100, 5000, 0.01, 0.01, seed=3)
     packed = oracle.parse_fastq(fq)
     assert packed == oracle.gen_reads(50, 100, 5000, 0.01, 0.01, seed=3).tobytes()
+    # what the reference's reader (FASTQFileReader / InputFileHandler) made of the same file
+    want = _reference_digests()["fastq_reader"]
+    assert (want["fastq_sha256"], want["L"], want["sha256"]) == (_sha(fq), 100, _sha(packed))
     # a quality line that starts with '+' is harmless; lower-case bases survive the reader
     txt = b"@r1\nACGTACGTAC\n+\n+IIIIIIIII\n@r2\nacgtNNACGT\n+\nIIIIIIIIII\n"
     assert oracle.parse_fastq(txt) == b"ACGTACGTACacgtNNACGT"
-    if oracle.ref_available():
-        d = tmp_path / "fq"
-        d.mkdir()
-        (d / "a.fastq").write_bytes(fq)
-        data, L = oracle.ref_read_fastq_dir(str(d))
-        assert L == 100 and data == packed
 
 
 def test_printer_restatement():
