@@ -45,6 +45,15 @@ extern "C" {
                                      unmasked tail window at k%32 in {29,30,31} and the
                                      zero-count key-0 record (SURVEY.md F4, F7)           */
 #define KC_COMPAT_STRICT    0x1u  /* true k-mers: tail always masked to k bases, no phantom */
+#define KC_CANONICAL        0x2u  /* canonical k-mers (implies KC_COMPAT_STRICT): a k-mer x and its reverse
+                                     complement rc(x) -- the complemented bases (code ^ 3 under A0 C1 G2 T3)
+                                     in reverse order, stored like any key -- are counted under one key,
+                                     min(x, rc(x)) in record order (words as unsigned 64-bit, word 0 first).
+                                     Its count = occurrences of x or rc(x); a palindrome counts once per
+                                     occurrence; windows with a non-ACGT byte are dropped. Every method, k
+                                     1..128, the accumulating mode and the exchange. The records have the same
+                                     format, but a run does not say which keys it holds: never merge canonical
+                                     and forward runs, and create every rank of an exchange with the same flags */
 
 /* kc_config.method: how occurrences are counted inside one chunk */
 #define KC_COUNT_AUTO       0u
@@ -75,7 +84,7 @@ typedef struct kc_config {
     uint32_t k;                /* kmerLength= (main.cpp:33), 1..128                        */
     uint32_t read_len;         /* lineLength (FASTQFileReader.cpp:30-35), k..4096          */
     int32_t  device;           /* CUDA device ordinal                                      */
-    uint32_t flags;            /* KC_COMPAT_*                                              */
+    uint32_t flags;            /* KC_COMPAT_* | KC_CANONICAL                               */
     uint32_t method;           /* KC_COUNT_*                                               */
     uint32_t n_slots;          /* pinned input slots (the reference's 8 GPUStreams,
                                   KMerCounter.cpp:117); 0 -> 2                             */
@@ -205,8 +214,11 @@ int  kc_accum_flush(kc_ctx *ctx, kc_run **run);
  *   n_ranks x 1024 buffer -> kc_xchg_group_local -> B -> kc_xchg_pull -> B -> kc_xchg_finish. */
 int  kc_xchg_begin(kc_ctx *ctx, uint32_t rank, uint32_t n_ranks, uint64_t expected_reads);
 int  kc_xchg_export(kc_ctx *ctx, void *handle64);                       /* CUDA IPC handle of this rank's workspace */
-int  kc_xchg_import(kc_ctx *ctx, uint32_t peer, const void *handle64);  /* a peer in another process               */
-int  kc_xchg_set_peer(kc_ctx *ctx, uint32_t peer, kc_ctx *peer_ctx);    /* a peer in this process                  */
+/* a peer in another process: every rank must be created with the same k, read_len and flags (the
+ * handle carries no plan, so a peer counting other keys is not detected here) */
+int  kc_xchg_import(kc_ctx *ctx, uint32_t peer, const void *handle64);
+/* a peer in this process: refused (KC_ERR_ARG) if it was planned differently or counts other keys */
+int  kc_xchg_set_peer(kc_ctx *ctx, uint32_t peer, kc_ctx *peer_ctx);
 int  kc_xchg_count_local(kc_ctx *ctx);
 int  kc_xchg_hist(kc_ctx *ctx, void **d_hist, void **d_all_hist);
 int  kc_xchg_group_local(kc_ctx *ctx);

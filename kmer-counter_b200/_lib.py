@@ -13,6 +13,7 @@ CSRC_DIR = os.path.join(_PKG_DIR, "csrc")
 
 KC_OK = 0
 KC_COMPAT_REF, KC_COMPAT_STRICT = 0, 1
+KC_CANONICAL = 0x2          # count a k-mer and its reverse complement under min(x, rc(x)); implies strict
 KC_COUNT_AUTO, KC_COUNT_SORT, KC_COUNT_HASH, KC_COUNT_HASH_GLOBAL, KC_COUNT_SUPER, KC_COUNT_PLACE = 0, 1, 2, 3, 4, 5
 METHODS = {"auto": KC_COUNT_AUTO, "sort": KC_COUNT_SORT, "hash": KC_COUNT_HASH, "hash_global": KC_COUNT_HASH_GLOBAL,
            "super": KC_COUNT_SUPER, "place": KC_COUNT_PLACE}

@@ -17,6 +17,8 @@
 #include "../../include/kc_api.h"
 #include "kc_internal.h"
 
+static_assert(kc::kPlanStrict == KC_COMPAT_STRICT && kc::kPlanCanonical == KC_CANONICAL, "plan flags are kc_config.flags bits");
+
 using namespace kc;
 
 struct kc_run {
@@ -76,7 +78,8 @@ struct Slot {
 struct kc_ctx {
     kc_config cfg{};
     int W = 1, S = 12;
-    bool strict = false;
+    bool strict = false;         // KC_COMPAT_STRICT, also set by KC_CANONICAL
+    uint32_t key_flags = 0;      // kPlanStrict | kPlanCanonical: the key semantics every plan is made for
     int n_sms = 148;
     cudaStream_t stream = nullptr;
     bool own_stream = false;
@@ -286,7 +289,7 @@ constexpr uint64_t kMaxSortKeys = (1ull << 30) - 1;
 // the super-window path takes 64/128-bit keys whose windows span at least 22 bases
 bool super_ok(const kc_ctx *c) {
     SuperPlan pl;
-    return c->W <= 2 && super_plan(c->cfg.k, c->cfg.read_len, c->strict, 1, 0, &pl) && super_supported(pl);
+    return c->W <= 2 && super_plan(c->cfg.k, c->cfg.read_len, c->key_flags, 1, 0, &pl) && super_supported(pl);
 }
 
 uint32_t pick_method(const kc_ctx *c) {
@@ -331,17 +334,17 @@ int count_enqueue_impl(kc_ctx *c, Pending &p, const void *d_reads, uint64_t n_by
     if (p.n_slots > kMaxSortKeys) return c->set_error(KC_ERR_ARG, "chunk too large: %llu k-mer slots (max %llu)",
                                                       (unsigned long long)p.n_slots, (unsigned long long)kMaxSortKeys);
     ExtractParams ep;
-    if (!extract_plan(d_reads, p.n_reads, L, k, c->strict, &p.d_scal[SC_INVALID], &ep))
+    if (!extract_plan(d_reads, p.n_reads, L, k, c->key_flags, &p.d_scal[SC_INVALID], &ep))
         return c->set_error(KC_ERR_ARG, "unsupported shape k=%u read_len=%u", k, L);
 
     if (method == KC_COUNT_SUPER) {
         // super-window records binned by minimizer, counted in shared memory (kc_super.cu)
-        if (!super_plan(k, L, c->strict, p.n_slots, (uint32_t)c->cfg.table_slots, &p.splan))
+        if (!super_plan(k, L, c->key_flags, p.n_slots, (uint32_t)c->cfg.table_slots, &p.splan))
             return c->set_error(KC_ERR_ARG, "unsupported shape k=%u read_len=%u", k, L);
         KC_TRY(arena_reserve(c, p, arena_round(p.splan.ws_bytes), s));
         p.ws_super = arena_take(p, p.splan.ws_bytes);
         KC_CUDA_TRY(c, super_reset(p.splan, p.ws_super, p.d_scal, s));
-        KC_CUDA_TRY(c, super_scatter(p.splan, d_reads, p.n_reads, c->strict, p.ws_super, p.d_scal, c->n_sms, s));
+        KC_CUDA_TRY(c, super_scatter(p.splan, d_reads, p.n_reads, p.ws_super, p.d_scal, c->n_sms, s));
         KC_CUDA_TRY(c, cudaEventRecord(p.ev[1], s));
         KC_CUDA_TRY(c, super_count(p.splan, !c->strict, p.ws_super, p.d_scal, c->n_sms, s, &p.ev[2]));
         p.n_ev = 6;
@@ -366,7 +369,7 @@ int count_enqueue_impl(kc_ctx *c, Pending &p, const void *d_reads, uint64_t n_by
         ExtractParams ep64;
         static int pa_stage = -1;               // KC_PA_STAGE (development knob): bytes of reads per PA tile
         if (pa_stage < 0) { const char *v = getenv("KC_PA_STAGE"); pa_stage = v ? atoi(v) : 6400; }
-        if (!extract_plan(d_reads, p.n_reads, L, k, c->strict, &p.d_scal[SC_INVALID], &ep64, (uint32_t)pa_stage))
+        if (!extract_plan(d_reads, p.n_reads, L, k, c->key_flags, &p.d_scal[SC_INVALID], &ep64, (uint32_t)pa_stage))
             return c->set_error(KC_ERR_ARG, "unsupported shape k=%u read_len=%u", k, L);
         const uint64_t kb = p.n_slots * 8 * W + 64, cb = (p.n_slots + 2) * 4, wb = partition_workspace_bytes(p.n_slots);
         KC_TRY(arena_reserve(c, p, 2 * arena_round(kb) + arena_round(cb) + arena_round(wb), s));
@@ -842,7 +845,10 @@ int kc_create(const kc_config *cfg, kc_ctx **out) {
     c->cfg = c0;
     c->W = (int)kc_key_words(c0.k);
     c->S = (int)kc_record_size(c0.k);
-    c->strict = (c0.flags & KC_COMPAT_STRICT) != 0;
+    // a canonical key is exactly k bases: KC_CANONICAL implies KC_COMPAT_STRICT
+    if (c0.flags & KC_CANONICAL) c->cfg.flags |= KC_COMPAT_STRICT;
+    c->strict = (c->cfg.flags & KC_COMPAT_STRICT) != 0;
+    c->key_flags = c->cfg.flags & (KC_COMPAT_STRICT | KC_CANONICAL);
     cudaDeviceGetAttribute(&c->n_sms, cudaDevAttrMultiProcessorCount, c0.device);
     if (c->n_sms <= 0) c->n_sms = 148;
     // keep freed blocks in the stream-ordered pool: chunk after chunk reuses the same arena
@@ -1158,7 +1164,7 @@ int accum_finish(kc_ctx *c, bool force_dup, kc_run **out, kc_run *pre_run, bool 
         const uint32_t have = (uint32_t)((a.max_windows + a.pl.n_bins - 1) / a.pl.n_bins);
         if (want < have * 0.75 || want > have * 1.5) {
             SuperPlan np;
-            if (super_plan(c->cfg.k, c->cfg.read_len, c->strict, a.max_windows, want, &np, 0.0, c->cfg.distinct_hint, true)) {
+            if (super_plan(c->cfg.k, c->cfg.read_len, c->key_flags, a.max_windows, want, &np, 0.0, c->cfg.distinct_hint, true)) {
                 bool ok = true;
                 if (np.ws_bytes > a.ws_bytes) {
                     KC_CUDA_TRY(c, cudaStreamSynchronize(s));
@@ -1222,7 +1228,7 @@ int accum_scatter(kc_ctx *c, const void *d_reads, uint64_t n_reads, cudaStream_t
         a.sc_ev.push_back(e);
     }
     KC_CUDA_TRY(c, cudaEventRecord(a.sc_ev[2 * a.n_scatter], s));
-    KC_CUDA_TRY(c, super_scatter(a.pl, d_reads, n_reads, c->strict, a.ws, a.d_sc, c->n_sms, s));
+    KC_CUDA_TRY(c, super_scatter(a.pl, d_reads, n_reads, a.ws, a.d_sc, c->n_sms, s));
     KC_CUDA_TRY(c, cudaEventRecord(a.sc_ev[2 * a.n_scatter + 1], s));
     const uint64_t nk = c->cfg.read_len - c->cfg.k + 1;
     a.fresh = false;
@@ -1260,7 +1266,7 @@ static int accum_begin_impl(kc_ctx *c, uint64_t expected_reads, bool exchange, u
     // exchange: a bin collects what ALL ranks put into it, so each rank plans bins 1/n_ranks the size
     uint32_t occ = (uint32_t)c->cfg.table_slots;
     if (exchange && n_ranks > 1) occ = (occ ? occ : 8192u) / n_ranks;
-    if (!super_plan(c->cfg.k, c->cfg.read_len, c->strict, windows, occ, &pl, exchange ? 0.25 : 0.0, c->cfg.distinct_hint, !exchange))
+    if (!super_plan(c->cfg.k, c->cfg.read_len, c->key_flags, windows, occ, &pl, exchange ? 0.25 : 0.0, c->cfg.distinct_hint, !exchange))
         return c->set_error(KC_ERR_ARG, "unsupported shape k=%u read_len=%u", c->cfg.k, c->cfg.read_len);
     if (!a.h_sc) {
         KC_CUDA_TRY(c, cudaMallocHost((void **)&a.h_sc, SC_COUNT * 8));
@@ -1438,6 +1444,8 @@ int kc_xchg_set_peer(kc_ctx *c, uint32_t peer, kc_ctx *peer_ctx) {
     if (!peer_ctx || !a.xchg || !peer_ctx->acc.xchg || peer >= a.n_ranks)
         return c->set_error(KC_ERR_ARG, "kc_xchg_set_peer: bad peer");
     if (peer_ctx->acc.pl.ws_bytes != a.pl.ws_bytes) return c->set_error(KC_ERR_ARG, "kc_xchg_set_peer: the ranks were planned differently");
+    if (peer_ctx->key_flags != c->key_flags)
+        return c->set_error(KC_ERR_ARG, "kc_xchg_set_peer: the ranks count different keys (KC_COMPAT_STRICT / KC_CANONICAL)");
     cudaSetDevice(c->cfg.device);
     if (peer_ctx->cfg.device != c->cfg.device) {
         cudaError_t e = cudaDeviceEnablePeerAccess(peer_ctx->cfg.device, 0);

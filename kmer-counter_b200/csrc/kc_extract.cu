@@ -15,9 +15,11 @@ struct StoreSink : SinkBase {
     }
 };
 
-bool extract_plan(const void *d_reads, uint64_t n_reads, uint32_t L, uint32_t k, bool strict,
+bool extract_plan(const void *d_reads, uint64_t n_reads, uint32_t L, uint32_t k, uint32_t flags,
                   unsigned long long *d_n_invalid, ExtractParams *out, uint32_t stage_bytes_target) {
     if (k == 0 || k > 128 || L < k || L > 4096) return false;
+    if (flags & kPlanCanonical) flags |= kPlanStrict;      // a canonical key is exactly k bases
+    const bool strict = (flags & kPlanStrict) != 0;
     ExtractParams p{};
     p.reads = static_cast<const uint8_t *>(d_reads);
     p.n_reads = n_reads;
@@ -36,7 +38,7 @@ bool extract_plan(const void *d_reads, uint64_t n_reads, uint32_t L, uint32_t k,
     uint32_t m = k % 32;
     bool masked = strict ? (m != 0) : (m >= 1 && m <= 28);   // SURVEY F4
     p.last_mask = masked ? (~0ull << (64 - 2 * m)) : ~0ull;
-    p.last_mask_strict = strict ? 1u : 0u;
+    p.plan_flags = flags & (kPlanStrict | kPlanCanonical);
     p.n_invalid = d_n_invalid;
     extract_smem_layout(p);
     if (p.smem_total > 200 * 1024) return false;
@@ -47,7 +49,7 @@ bool extract_plan(const void *d_reads, uint64_t n_reads, uint32_t L, uint32_t k,
 template <int W, class Sink>
 static cudaError_t launch_extract(const ExtractParams &p, Sink sink, int n_sms, cudaStream_t s) {
     if (p.n_tiles == 0) return cudaSuccess;
-    auto kern = extract_kernel<W, Sink>;
+    auto kern = extract_kernel_for<W, Sink>(p);
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p.smem_total);
     if (e != cudaSuccess) return e;
     int per_sm = 1;

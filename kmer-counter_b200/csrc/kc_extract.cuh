@@ -13,6 +13,10 @@
 // reference's missing tail mask, F4) and k otherwise; positions past the read end
 // contribute 0; non-ACGT letters contribute 3 and invalidate every k-mer [p,p+k)
 // that contains them.  The span is carried by Params::last_mask.
+//
+// Canonical keys (KC_CANONICAL, always with the strict span k): the key handed to the sink is
+// min(x, rc(x)) in record order, rc = the complemented bases of x in reverse order, left-aligned.
+// It is a template parameter of the kernel, so the forward instantiations are untouched.
 #pragma once
 
 #include "kc_common.cuh"
@@ -32,7 +36,7 @@ struct ExtractParams {
     uint32_t nb4_magic;      // floor(2^32 / nb4) + 1
     uint32_t segs_per_read, seg_len;   // rolling walk: a read's nk positions in segs_per_read runs of seg_len
     uint64_t last_mask;      // applied to key word W-1
-    uint32_t last_mask_strict;   // the plan was made for KC_COMPAT_STRICT (kept so that a plan can be re-made)
+    uint32_t plan_flags;     // kPlanStrict | kPlanCanonical the plan was made for (kept so that a plan can be re-made)
     unsigned long long *n_invalid;  // += slots that hold no k-mer (the phantom of SURVEY F7)
     uint32_t stage_bytes, enc_off, bad_off, flag_off, bar_off, smem_total;  // shared-memory layout
 };
@@ -45,6 +49,9 @@ inline void extract_smem_layout(ExtractParams &p) {
     p.bar_off = (p.flag_off + p.tile_reads + 15u) & ~15u;
     p.smem_total = p.bar_off + 16;
 }
+
+// extract_plan's flags: the KC_COMPAT_STRICT and KC_CANONICAL bits of kc_config.flags
+constexpr uint32_t kPlanStrict = 0x1u, kPlanCanonical = 0x2u;
 
 constexpr int kExtractThreads = 256;
 constexpr uint32_t kMaxSegLen = 18;      // positions a thread walks in the sliding-window mode (plan: seg_len <= 18)
@@ -117,6 +124,28 @@ __device__ __forceinline__ void encode_tile(const ExtractParams &p, const uint8_
     }
 }
 
+// Reverse complement of a 64-bit word of 32 bases: base order reversed, code ^ 3 (A0 C1 G2 T3).
+__device__ __forceinline__ uint64_t word_revcomp(uint64_t x) {
+    x = __brevll(x);                                                         // bits reversed ...
+    x = ((x >> 1) & 0x5555555555555555ull) | ((x & 0x5555555555555555ull) << 1);   // ... bases back in bit order
+    return ~x;
+}
+// The canonical key of a strict key x (k bases left-aligned, low bits zero): min(x, rc(x)) in record
+// order. rc_sh = 2 (32 W - k) = the zero tail of word W-1, always < 64.
+template <int W>
+__device__ __forceinline__ Key<W> key_canonical(const Key<W> &x, uint32_t rc_sh) {
+    uint64_t r[W + 1];
+#pragma unroll
+    for (int q = 0; q < W; q++) r[q] = word_revcomp(x.w[W - 1 - q]);
+    r[W] = 0;
+    Key<W> rc;
+#pragma unroll
+    for (int q = 0; q < W; q++) rc.w[q] = rc_sh ? ((r[q] << rc_sh) | (r[q + 1] >> (64 - rc_sh))) : r[q];
+    return key_lt<W>(rc, x) ? rc : x;
+}
+// rc_sh of a plan: the bits last_mask clears
+__device__ __forceinline__ uint32_t rc_shift_of(uint64_t last_mask) { return (uint32_t)__ffsll((long long)last_mask) - 1u; }
+
 // rare path: any bad base inside [pos, pos+k) kills the k-mer (bad4 row of the read)
 __device__ __forceinline__ bool kmer_window_valid(const uint8_t *bn, uint32_t pos, uint32_t k) {
     const uint32_t lo = pos, hi = pos + k;  // [lo, hi)
@@ -130,7 +159,7 @@ __device__ __forceinline__ bool kmer_window_valid(const uint8_t *bn, uint32_t po
     return true;
 }
 
-template <int W, class Sink>
+template <int W, class Sink, bool CANON = false>
 __global__ void __launch_bounds__(kExtractThreads) extract_kernel(ExtractParams p, Sink sink) {
     extern __shared__ __align__(128) uint8_t smem[];
     const uint32_t stage_bytes = p.stage_bytes;
@@ -142,6 +171,7 @@ __global__ void __launch_bounds__(kExtractThreads) extract_kernel(ExtractParams 
     uint8_t *flag = smem + p.flag_off;
     uint64_t *bars = reinterpret_cast<uint64_t *>(smem + p.bar_off);
     const uint32_t tid = threadIdx.x, lane = tid & 31;
+    [[maybe_unused]] const uint32_t rc_sh = CANON ? rc_shift_of(p.last_mask) : 0u;
 
     if (tid == 0) {
         mbar_init(&bars[0], 1);
@@ -237,9 +267,10 @@ __global__ void __launch_bounds__(kExtractThreads) extract_kernel(ExtractParams 
 #pragma unroll
                     for (int q = 0; q <= W; q++) win[q] = sh ? ((ew[q] << sh) | (ew[q + 1] >> (64 - sh))) : ew[q];
                     const bool check = flag[r] != 0;
-                    if (Sink::kTopOnlySweep0 && sw == 0) {
+                    if (Sink::kTopOnlySweep0 && !CANON && sw == 0) {
                         // the sink only wants leading key bits here (a digit histogram): they all come
-                        // from the 64-bit window at p0, one constant funnel shift per position
+                        // from the 64-bit window at p0, one constant funnel shift per position (not so for
+                        // canonical keys, whose leading bits depend on the whole k-mer)
                         const uint64_t x = win[0];
 #pragma unroll
                         for (uint32_t i = 0; i < kMaxSegLen; i++) {
@@ -257,6 +288,7 @@ __global__ void __launch_bounds__(kExtractThreads) extract_kernel(ExtractParams 
 #pragma unroll
                         for (int q = 0; q < W; q++) key.w[q] = win[q];
                         key.w[W - 1] &= p.last_mask;
+                        if constexpr (CANON) key = key_canonical<W>(key, rc_sh);
                         const bool valid = check ? kmer_valid(r, pos) : true;
                         if (sw == 0 && !valid) invalid_local++;
                         sink(sw, slot0 + r * p.nk + pos, key, valid);
@@ -282,6 +314,7 @@ __global__ void __launch_bounds__(kExtractThreads) extract_kernel(ExtractParams 
                         a = b;
                     }
                     key.w[W - 1] &= p.last_mask;
+                    if constexpr (CANON) key = key_canonical<W>(key, rc_sh);
                     const bool valid = flag[r] ? kmer_valid(r, pos) : true;
                     if (sw == 0 && !valid) invalid_local++;
                     sink(sw, slot0 + s, key, valid);
@@ -300,6 +333,12 @@ __global__ void __launch_bounds__(kExtractThreads) extract_kernel(ExtractParams 
     for (int o = 16; o > 0; o >>= 1) invalid_local += __shfl_xor_sync(0xffffffffu, invalid_local, o);
     if (lane == 0 && invalid_local) atomicAdd(p.n_invalid, invalid_local);
     sink.finish();
+}
+
+// the instantiation a plan asks for (kPlanCanonical: canonical keys)
+template <int W, class Sink>
+inline auto extract_kernel_for(const ExtractParams &p) {
+    return (p.plan_flags & kPlanCanonical) ? extract_kernel<W, Sink, true> : extract_kernel<W, Sink, false>;
 }
 
 }  // namespace kc

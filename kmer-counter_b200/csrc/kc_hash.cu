@@ -116,7 +116,7 @@ cudaError_t hash_clear(HashTable t, cudaStream_t s) {
 
 cudaError_t launch_extract_hash(const ExtractParams &p, HashTable t, int n_sms, cudaStream_t s) {
     if (p.n_tiles == 0) return cudaSuccess;
-    auto kern = extract_kernel<1, HashSink>;
+    auto kern = extract_kernel_for<1, HashSink>(p);
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p.smem_total);
     if (e != cudaSuccess) return e;
     int per_sm = 1;

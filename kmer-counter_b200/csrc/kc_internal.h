@@ -10,9 +10,10 @@
 namespace kc {
 
 // ---- extraction (kc_extract.cu)
-// Fills every field of ExtractParams for (reads, n_reads, L, k); strict selects
-// KC_COMPAT_STRICT masking. Returns false for unsupported shapes.
-bool extract_plan(const void *d_reads, uint64_t n_reads, uint32_t L, uint32_t k, bool strict,
+// Fills every field of ExtractParams for (reads, n_reads, L, k); flags: kPlanStrict selects
+// KC_COMPAT_STRICT masking, kPlanCanonical canonical keys (implies strict). Returns false for
+// unsupported shapes.
+bool extract_plan(const void *d_reads, uint64_t n_reads, uint32_t L, uint32_t k, uint32_t flags,
                   unsigned long long *d_n_invalid, ExtractParams *out, uint32_t stage_bytes_target = 12800);
 // keys[slot] for every slot r*(L-k+1)+p; slots without a k-mer get key 0
 cudaError_t launch_extract_store(const ExtractParams &p, int W, uint64_t *d_keys, int n_sms, cudaStream_t s);

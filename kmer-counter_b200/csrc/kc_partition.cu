@@ -967,11 +967,11 @@ static cudaError_t partition_count_w(const ExtractParams &ep_in, uint64_t n_slot
         ExtractParams ep = ep_in;
         static int p0_stage = -1;               // KC_P0_STAGE (development knob): bytes of reads per P0 tile
         if (p0_stage < 0) { const char *v = getenv("KC_P0_STAGE"); p0_stage = v ? atoi(v) : 12800; }
-        if (!extract_plan(ep_in.reads, ep_in.n_reads, ep_in.L, ep_in.k, ep_in.last_mask_strict != 0, d_scratch_invalid, &ep,
+        if (!extract_plan(ep_in.reads, ep_in.n_reads, ep_in.L, ep_in.k, ep_in.plan_flags, d_scratch_invalid, &ep,
                           (uint32_t)p0_stage))
             ep = ep_in;
         ep.n_invalid = d_scratch_invalid;
-        auto kern = extract_kernel<W, Hist1Sink<W>>;
+        auto kern = extract_kernel_for<W, Hist1Sink<W>>(ep_in);
         const uint32_t smem = ep.smem_total + kMaxBins * 4;
         if ((e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)) != cudaSuccess) return e;
         int per_sm = 1;
@@ -988,7 +988,7 @@ static cudaError_t partition_count_w(const ExtractParams &ep_in, uint64_t n_slot
     if (evs) cudaEventRecord(evs[0], s);
     // PA: keys grouped by level-1 digit
     {
-        auto kern = extract_kernel<W, Scatter1Sink<W>>;
+        auto kern = extract_kernel_for<W, Scatter1Sink<W>>(ep_in);
         const uint32_t max_tile_keys = ep_in.tile_reads * ep_in.nk;
         const uint32_t smem = ep_in.smem_total + Scatter1Sink<W>::smem_bytes(max_tile_keys);
         if ((e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)) != cudaSuccess) return e;

@@ -50,7 +50,7 @@ struct SwScatterParams {
     unsigned long long *sc;
 };
 
-template <int W>
+template <int W, bool CANON>
 __global__ void __launch_bounds__(kSwThreads) sw_scatter_kernel(SwScatterParams q) {
     const ExtractParams &p = q.ep;
     extern __shared__ __align__(128) uint8_t smem[];
@@ -135,9 +135,21 @@ __global__ void __launch_bounds__(kSwThreads) sw_scatter_kernel(SwScatterParams 
             const uint64_t b = wi + 1 <= p.nw ? e[wi + 1] : 0ull;
             const uint64_t x = sh ? ((a << sh) | (b >> (64 - sh))) : a;
             uint32_t *row = hh + r * q.nh_stride + j0;
+            if constexpr (CANON) {
+                // canonical m-mer min(mm, rc(mm)): the m-mers of rc(x) are the reverse complements of
+                // x's, so the window's minimizer (its bin, its owner rank) is the same on both strands
 #pragma unroll
-            for (uint32_t i = 0; i < 8; i++)
-                if (j0 + i < q.nh) row[i] = mmer_hash((uint32_t)(x >> (mshift - 2 * i)) & mmask);
+                for (uint32_t i = 0; i < 8; i++) {
+                    const uint32_t mm = (uint32_t)(x >> (mshift - 2 * i)) & mmask;
+                    uint32_t r = __brev(mm);
+                    r = ((r >> 1) & 0x55555555u) | ((r & 0x55555555u) << 1);
+                    if (j0 + i < q.nh) row[i] = mmer_hash(min(mm, (r >> (32 - 2 * q.m)) ^ mmask));
+                }
+            } else {
+#pragma unroll
+                for (uint32_t i = 0; i < 8; i++)
+                    if (j0 + i < q.nh) row[i] = mmer_hash((uint32_t)(x >> (mshift - 2 * i)) & mmask);
+            }
         }
         __syncthreads();
 
@@ -366,7 +378,8 @@ struct SwCountParams {
 // wait for each other. A unit with more distinct keys than the table takes is redone in 2, 4, ...
 // passes, pass v counting the keys whose pass hash starts with v: the records a unit emits are
 // always key-distinct.
-template <int W, int THREADS, int TSLOTS, int RPT>
+// CANON: every window's key is min(forward, rc) (the records still hold forward bases).
+template <int W, int THREADS, int TSLOTS, int RPT, bool CANON = false>
 __global__ void __launch_bounds__(THREADS) sw_count_kernel(SwCountParams p) {
     constexpr int RB = THREADS * RPT;                                       // records per round
     extern __shared__ __align__(16) uint8_t cs_smem[];
@@ -390,6 +403,7 @@ __global__ void __launch_bounds__(THREADS) sw_count_kernel(SwCountParams p) {
     const uint32_t tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     constexpr uint32_t kLimit = TSLOTS / 4 * 3;
     constexpr uint32_t hshift = 32 - ILog2<(uint32_t)TSLOTS>::v;
+    [[maybe_unused]] const uint32_t rc_sh = CANON ? rc_shift_of(p.last_mask) : 0u;
 
     {
         Key<W> empty;
@@ -750,6 +764,7 @@ __global__ void __launch_bounds__(THREADS) sw_count_kernel(SwCountParams p) {
 #pragma unroll
                             for (int t = 0; t < W; t++) key.w[t] = rw[t];
                             key.w[W - 1] &= p.last_mask;
+                            if constexpr (CANON) key = key_canonical<W>(key, rc_sh);
                             in_rec--;
                             rem--;
 #pragma unroll
@@ -1723,10 +1738,13 @@ constexpr int kFinCapWide = 1024;                           // ... of 192/256-bi
 // ------------------------------------------------------------------------ host
 static void plan_layout(SuperPlan &pl, bool ext_e);
 
-bool super_plan(uint32_t k, uint32_t L, bool strict, uint64_t max_windows, uint32_t occ_per_bin, SuperPlan *out,
+bool super_plan(uint32_t k, uint32_t L, uint32_t flags, uint64_t max_windows, uint32_t occ_per_bin, SuperPlan *out,
                 double record_headroom, uint64_t distinct_hint, bool ext_e) {
     if (k == 0 || k > 64 || L < k || L > 4096) return false;
+    if (flags & kPlanCanonical) flags |= kPlanStrict;                  // a canonical key is exactly k bases
+    const bool strict = (flags & kPlanStrict) != 0;
     SuperPlan pl{};
+    pl.flags = flags & (kPlanStrict | kPlanCanonical);
     pl.W = (int)((k + 31) / 32);
     pl.k = k;
     pl.L = L;
@@ -1879,12 +1897,12 @@ cudaError_t super_reset(const SuperPlan &pl, void *ws, unsigned long long *d_sc,
 }
 
 template <int W>
-static cudaError_t super_scatter_w(const SuperPlan &pl, const void *d_reads, uint64_t n_reads, bool strict, void *ws,
+static cudaError_t super_scatter_w(const SuperPlan &pl, const void *d_reads, uint64_t n_reads, void *ws,
                                    unsigned long long *d_sc, int n_sms, cudaStream_t s) {
     static int tile_bytes = -1;                 // KC_SW_STAGE (development knob): bytes of reads per S1 tile
     if (tile_bytes < 0) { const char *v = getenv("KC_SW_STAGE"); tile_bytes = v ? atoi(v) : 4800; }   // 3200: 3.82 ms, 4800: 3.60, 6400: 4.0, 9600: 4.28 at C2
     SwScatterParams q{};
-    if (!extract_plan(d_reads, n_reads, pl.L, pl.k, strict, &d_sc[SW_INVALID], &q.ep, (uint32_t)tile_bytes))
+    if (!extract_plan(d_reads, n_reads, pl.L, pl.k, pl.flags, &d_sc[SW_INVALID], &q.ep, (uint32_t)tile_bytes))
         return cudaErrorInvalidValue;
     if (q.ep.n_tiles == 0) return cudaSuccess;
     q.m = pl.m; q.w = pl.w; q.nh = pl.nh; q.nh_stride = pl.nh_stride;
@@ -1899,7 +1917,7 @@ static cudaError_t super_scatter_w(const SuperPlan &pl, const void *d_reads, uin
     q.bins = at<uint8_t>(ws, pl.off_bins);
     q.ovf = at<uint8_t>(ws, pl.off_ovf);
     q.sc = d_sc;
-    auto kern = sw_scatter_kernel<W>;
+    auto kern = (pl.flags & kPlanCanonical) ? sw_scatter_kernel<W, true> : sw_scatter_kernel<W, false>;
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
     int per_sm = 1;
@@ -1914,25 +1932,25 @@ static cudaError_t super_scatter_w(const SuperPlan &pl, const void *d_reads, uin
 // false when the shared-memory tile of S1 cannot hold even 16 reads of this length
 static bool super_scatter_fits(const SuperPlan &pl) {
     ExtractParams ep;
-    if (!extract_plan(nullptr, 16, pl.L, pl.k, false, nullptr, &ep, 6400)) return false;
+    if (!extract_plan(nullptr, 16, pl.L, pl.k, 0u, nullptr, &ep, 6400)) return false;
     const uint64_t smem = ((ep.smem_total + 15u) & ~15u) + (uint64_t)ep.tile_reads * pl.nh_stride * 4 +
                           (uint64_t)ep.tile_reads * pl.nk * 4 + 2ull * ep.tile_reads * pl.segs_per_read * 4;
     return smem <= 200 * 1024;
 }
 
-cudaError_t super_scatter(const SuperPlan &pl, const void *d_reads, uint64_t n_reads, bool strict, void *ws,
+cudaError_t super_scatter(const SuperPlan &pl, const void *d_reads, uint64_t n_reads, void *ws,
                           unsigned long long *d_sc, int n_sms, cudaStream_t s) {
-    if (pl.W == 1) return super_scatter_w<1>(pl, d_reads, n_reads, strict, ws, d_sc, n_sms, s);
-    if (pl.W == 2) return super_scatter_w<2>(pl, d_reads, n_reads, strict, ws, d_sc, n_sms, s);
+    if (pl.W == 1) return super_scatter_w<1>(pl, d_reads, n_reads, ws, d_sc, n_sms, s);
+    if (pl.W == 2) return super_scatter_w<2>(pl, d_reads, n_reads, ws, d_sc, n_sms, s);
     return cudaErrorInvalidValue;
 }
 
-template <int W, int THREADS, int TSLOTS, int RPT = 2>
+template <int W, int THREADS, int TSLOTS, int RPT = 2, bool CANON = false>
 static cudaError_t launch_count(const SwCountParams &cp, int n_sms, cudaStream_t s) {
     const uint32_t RB = THREADS * RPT, RT = W == 1 ? (RPT > 1 ? RB : 2 * RB) : 1;
     const uint32_t smem = TSLOTS * (8 * W + 4) + RB * 16 * W + (RB + 8) * 4 + kNb1Max * 4 +
                           (THREADS / 32) * (RPT > 1 ? 64 : 96) * (8 * W + 4) + RT * 20 + RB * 4 + 64;
-    auto kern = sw_count_kernel<W, THREADS, TSLOTS, RPT>;
+    auto kern = sw_count_kernel<W, THREADS, TSLOTS, RPT, CANON>;
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
     int per_sm = 1;
@@ -1966,6 +1984,9 @@ static cudaError_t super_count_bins_w(const SuperPlan &pl, bool add_phantom, voi
     cp.hist1 = at<uint32_t>(ws, pl.off_hist1); cp.shift1 = 64 - pl.b1; cp.nb1 = 1 << pl.b1;
     cp.add_phantom = add_phantom ? 1 : 0;
     cp.sc = d_sc;
+    // canonical keys: the default shapes only (the KC_SW_COUNT variants below are forward-only)
+    if (pl.flags & kPlanCanonical) return W == 1 ? launch_count<1, 512, 4096, 2, true>(cp, n_sms, s)
+                                                 : launch_count<2, 512, 4096, 1, true>(cp, n_sms, s);
     static int variant = -1;                    // KC_SW_COUNT (development knob): CTA / table shape of S2
     if (variant < 0) { const char *v = getenv("KC_SW_COUNT"); variant = v ? atoi(v) : 0; }
     if constexpr (W == 1) {

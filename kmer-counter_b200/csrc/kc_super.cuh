@@ -86,20 +86,23 @@ struct SuperPlan {
     bool ext_e;
     uint64_t *ext_ek;
     uint32_t *ext_ec;
+    uint32_t flags;             // kPlanStrict | kPlanCanonical; canonical: keys are min(x, rc(x)), S1 bins
+                                // windows by their canonical minimizer so that x and rc(x) share a bin
 };
 
 constexpr uint32_t kSuperMaxSub = 1u << 20;
 
 // Plans a pipeline for up to max_windows k-mer slots (one chunk, or everything that will be
-// accumulated before the count). occ_per_bin = 0 -> default. Returns false for shapes the path
-// does not take (W > 2, span < 22, reads too long for the shared-memory tile).
-bool super_plan(uint32_t k, uint32_t L, bool strict, uint64_t max_windows, uint32_t occ_per_bin, SuperPlan *out,
+// accumulated before the count). flags: kPlanStrict / kPlanCanonical (as extract_plan).
+// occ_per_bin = 0 -> default. Returns false for shapes the path does not take (W > 2, span < 22,
+// reads too long for the shared-memory tile).
+bool super_plan(uint32_t k, uint32_t L, uint32_t flags, uint64_t max_windows, uint32_t occ_per_bin, SuperPlan *out,
                 double record_headroom = 0.0, uint64_t distinct_hint = 0, bool ext_e = false);
 
 // zero cursors, histograms and scalars: once before the first super_scatter of a pipeline
 cudaError_t super_reset(const SuperPlan &pl, void *ws, unsigned long long *d_sc, cudaStream_t s);
-// S1: append the super-window records of (reads, n_reads) to the bins
-cudaError_t super_scatter(const SuperPlan &pl, const void *d_reads, uint64_t n_reads, bool strict, void *ws,
+// S1: append the super-window records of (reads, n_reads) to the bins (key semantics of the plan)
+cudaError_t super_scatter(const SuperPlan &pl, const void *d_reads, uint64_t n_reads, void *ws,
                           unsigned long long *d_sc, int n_sms, cudaStream_t s);
 // S2 .. S3b: count the bins, place the distinct records into sub-buckets. evs (may be NULL):
 // events recorded after S2, S3a, H2, S3b.

@@ -4,7 +4,7 @@ import ctypes as C
 import numpy as np
 
 from . import _lib
-from ._lib import KcConfig, KcStats, METHODS, METHOD_NAMES, KC_COMPAT_REF, KC_COMPAT_STRICT
+from ._lib import KcConfig, KcStats, METHODS, METHOD_NAMES, KC_COMPAT_REF, KC_COMPAT_STRICT, KC_CANONICAL
 
 
 STAGE_NAMES = {
@@ -125,12 +125,16 @@ class Counter:
     """One kc_ctx: the replacement for PrepareGPU's GPUStream array (GPUHandler.cu:479-509)."""
 
     def __init__(self, k, read_len, device=0, method="auto", compat="ref", n_slots=2, max_chunk_bytes=0,
-                 table_slots=0, stream=None, distinct_hint=0):
+                 table_slots=0, stream=None, distinct_hint=0, canonical=False):
+        """canonical=True counts every k-mer with its reverse complement under min(x, rc(x))
+        (KC_CANONICAL; implies compat="strict"). Its runs must not be merged with forward runs."""
         self._lib = _lib.load()
         cfg = KcConfig()
         cfg.struct_size = C.sizeof(KcConfig)
         cfg.k, cfg.read_len, cfg.device = k, read_len, device
         cfg.flags = KC_COMPAT_STRICT if compat == "strict" else KC_COMPAT_REF
+        if canonical:
+            cfg.flags |= KC_CANONICAL | KC_COMPAT_STRICT
         cfg.method = METHODS[method] if isinstance(method, str) else int(method)
         cfg.n_slots, cfg.max_chunk_bytes, cfg.table_slots = n_slots, max_chunk_bytes, table_slots
         cfg.stream = stream
@@ -141,6 +145,7 @@ class Counter:
             raise KcError(rc, (self._lib.kc_last_error(None) or b"").decode())
         self._ctx = ctx
         self.k, self.read_len, self.device = k, read_len, device
+        self.canonical = bool(canonical)
         self.words = self._lib.kc_key_words(k)
         self.record_size = self._lib.kc_record_size(k)
         self.max_chunk_bytes = max_chunk_bytes

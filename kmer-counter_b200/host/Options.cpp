@@ -23,6 +23,7 @@ Options Options::parse(int argc, char **argv) {
         else if (take(argv[i], "noOfMergeThreads=", &v)) o.noOfMergeThreads = (uint32_t)atoi(v);
         else if (take(argv[i], "method=", &v)) o.method = v;
         else if (take(argv[i], "compat=", &v)) o.compat = v;
+        else if (take(argv[i], "canonical=", &v)) o.canonical = atoi(v) != 0;
         else if (take(argv[i], "device=", &v)) o.device = atoi(v);
         else if (take(argv[i], "keepRuns=", &v)) o.keepRuns = atoi(v) != 0;
         else if (take(argv[i], "parser=", &v)) o.parser = v;

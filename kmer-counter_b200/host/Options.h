@@ -17,6 +17,8 @@ struct Options {
     // additions
     std::string method = "auto";              // method=auto|sort|hash
     std::string compat = "ref";               // compat=ref|strict
+    bool canonical = false;                   // canonical=1: count each k-mer with its reverse complement under
+                                              // min(x, rc(x)) (KC_CANONICAL, implies compat=strict)
     int device = 0;                           // device=
     bool keepRuns = false;                    // keepRuns=1: also write every chunk's run to tempFileLocation/<id>
     int64_t runBudget = 0;                    // runBudget=BYTES: a merged run larger than this is spilled to pinned host

@@ -2,7 +2,7 @@
 //
 //   kmer_counter_b200 kmerLength=31 inputFileLocation=<dir> outputFile=<file> [gpuMemoryLimit=..]
 //                     [tempFileLocation=..] [noOfMergersAtOnce=..] [noOfMergeThreads=..]
-//                     [method=auto|sort|hash] [compat=ref|strict] [device=N] [keepRuns=1] [parser=gpu|host]
+//                     [method=auto|sort|hash] [compat=ref|strict] [canonical=1] [device=N] [keepRuns=1] [parser=gpu|host]
 //                     [runBudget=BYTES] [gpus=N] [mode=auto|accumulate|runs] [expectedReads=N]
 //   kmer_counter_b200 print <record file> <ignored> <k>       (KMerPrinter, main.cpp:78-82)
 //
@@ -76,7 +76,7 @@ static int run_accumulate(const Options &opt, FastqChunker &reader, int64_t L, i
         cfg.k = (uint32_t)opt.kmerLength;
         cfg.read_len = (uint32_t)L;
         cfg.device = getenv("KC_CLI_SAME_DEVICE") ? opt.device : opt.device + g;   // (test knob: all ranks on one device)
-        cfg.flags = opt.compat == "strict" ? KC_COMPAT_STRICT : KC_COMPAT_REF;
+        cfg.flags = (opt.compat == "strict" ? KC_COMPAT_STRICT : KC_COMPAT_REF) | (opt.canonical ? KC_CANONICAL : 0u);
         cfg.method = method;
         cfg.n_slots = 2;
         cfg.max_chunk_bytes = (uint64_t)chunk;
@@ -207,7 +207,7 @@ int main(int argc, char **argv) {
     if (argc == 5 && strncmp(argv[1], "print", 5) == 0) return print_records(argv[2], strtoull(argv[4], nullptr, 10));
     Options opt = Options::parse(argc, argv);
     if (opt.inputFileDirectory.empty()) {
-        fprintf(stderr, "usage: %s kmerLength=K inputFileLocation=DIR outputFile=FILE [gpuMemoryLimit=BYTES] ...\n", argv[0]);
+        fprintf(stderr, "usage: %s kmerLength=K inputFileLocation=DIR outputFile=FILE [gpuMemoryLimit=BYTES] [canonical=1] ...\n", argv[0]);
         return 2;
     }
     FastqChunker reader(opt.inputFileDirectory);
@@ -235,7 +235,7 @@ int main(int argc, char **argv) {
     cfg.k = (uint32_t)opt.kmerLength;
     cfg.read_len = (uint32_t)L;
     cfg.device = opt.device;
-    cfg.flags = opt.compat == "strict" ? KC_COMPAT_STRICT : KC_COMPAT_REF;
+    cfg.flags = (opt.compat == "strict" ? KC_COMPAT_STRICT : KC_COMPAT_REF) | (opt.canonical ? KC_CANONICAL : 0u);
     cfg.method = method_of(opt.method);
     cfg.n_slots = 2;
     cfg.max_chunk_bytes = (uint64_t)chunk;

@@ -52,8 +52,10 @@ class Exchange:
         self.world, self.rank = dist.get_world_size(group), dist.get_rank(group)
         counter.xchg_begin(self.rank, self.world, expected_reads)
         everyone = [None] * self.world
-        dist.all_gather_object(everyone, counter.xchg_export(), group=group)
-        for r, h in enumerate(everyone):
+        dist.all_gather_object(everyone, (counter.xchg_export(), counter.canonical), group=group)
+        if any(c != counter.canonical for _, c in everyone):
+            raise ValueError("multigpu.Exchange: every rank's Counter must have the same canonical setting")
+        for r, (h, _) in enumerate(everyone):
             if r != self.rank:
                 counter.xchg_import(r, h)           # the peer's workspace, mapped into this process (CUDA IPC)
         hp, ap = counter.xchg_hist()
