@@ -276,6 +276,20 @@ int  kc_run_write(kc_ctx *ctx, const kc_run *run, const char *path, int append);
 int  kc_run_split(kc_ctx *ctx, const kc_run *run, const uint64_t *splitters, uint32_t n_splitters,
                   uint64_t *offsets);
 
+/* ---- count spectrum and filtering: what `jellyfish histo` / `kmc_tools histogram` and the count
+ * cut-offs of KMC (-ci/-cx) and Jellyfish (-L/-U) give, computed on the device from a finished run ---- */
+/* hist[c] = records of the run with count exactly c, for c < n_bins - 1; hist[n_bins - 1] = records
+ * with count >= n_bins - 1 (the "high" bin). 2 <= n_bins <= 1 << 24; hist is host memory, overwritten.
+ * hist[0] holds zero-count records: under KC_COMPAT_REF the phantom key-0 record (SURVEY F7), and any
+ * count that wrapped at 2^32. Records hidden by the run's strict-mode skip are not counted. */
+int  kc_run_histogram(kc_ctx *ctx, const kc_run *run, uint64_t *hist, uint32_t n_bins);
+/* A new run with the records whose count c satisfies min_count <= c <= max_count, in the same order
+ * (so it is sorted and key-unique). The input run is unchanged. The output is sized exactly and has
+ * no partition structure (kc_run_parts: n_sub == 0). min_count > max_count -> KC_ERR_ARG.
+ * Filter only a run whose counts are final: filtering one chunk's run before it is merged with the
+ * others would drop k-mers whose total count is in range. */
+int  kc_run_filter(kc_ctx *ctx, const kc_run *run, uint32_t min_count, uint32_t max_count, kc_run **out);
+
 /* Runs produced by KC_COUNT_HASH also carry their partition structure: the key space is cut
  * into n_sub equal ranges on the leading prefix_bits of the key and d_offsets[j] (uint32,
  * n_sub + 1 entries, device memory owned by the run) is the first record of range j. n_sub == 0

@@ -92,6 +92,8 @@ SYMBOLS = {
     "kc_run_from_device": (_i, [_vp, _vp, _vp, _u64, _pp]),
     "kc_run_write": (_i, [_vp, _vp, C.c_char_p, _i]),
     "kc_run_split": (_i, [_vp, _vp, _pu64, _u32, _pu64]),
+    "kc_run_histogram": (_i, [_vp, _vp, _pu64, _u32]),
+    "kc_run_filter": (_i, [_vp, _vp, _u32, _u32, _pp]),
     "kc_merge_runs": (_i, [_vp, _pp, _u32, _pp]),
     "kc_place_next_run": (_i, [_vp, _vp, _vp, _vp, _u64, _u32]),
     "kc_peer_alloc": (_i, [_vp, _u64, C.POINTER(_vp), _vp]),

@@ -2110,6 +2110,73 @@ int kc_run_split(kc_ctx *c, const kc_run *r, const uint64_t *splitters, uint32_t
     return KC_OK;
 }
 
+// ------------------------------------------------------- count spectrum and filtering
+int kc_run_histogram(kc_ctx *c, const kc_run *r, uint64_t *hist, uint32_t n_bins) {
+    KC_TRY(check_ctx(c));
+    if (!r || !hist) return c->set_error(KC_ERR_ARG, "null argument");
+    if (n_bins < 2 || n_bins > (1u << 24)) return c->set_error(KC_ERR_ARG, "kc_run_histogram: n_bins %u is not in 2..2^24", n_bins);
+    std::lock_guard<std::recursive_mutex> dg(c->direct_mu);
+    const uint64_t n = r->n - r->skip;
+    memset(hist, 0, (uint64_t)n_bins * 8);
+    if (n == 0) return KC_OK;
+    cudaSetDevice(c->cfg.device);
+    cudaStream_t s = c->stream;
+    void *d_hist = nullptr;
+    KC_TRY(dev_alloc(c, s, (uint64_t)n_bins * 8, &d_hist));
+    int launches = 0;
+    cudaError_t e = run_histogram(r->d_counts + r->skip, n, n_bins, static_cast<unsigned long long *>(d_hist), c->n_sms,
+                                  s, &launches);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(hist, d_hist, (uint64_t)n_bins * 8, cudaMemcpyDeviceToHost, s);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(s);
+    dev_free(s, d_hist);
+    if (e != cudaSuccess) return c->set_error(KC_ERR_CUDA, "kc_run_histogram: %s", cudaGetErrorString(e));
+    std::lock_guard<std::mutex> g(c->mu);
+    c->stats.launches += launches;
+    c->stats.d2h_bytes += (uint64_t)n_bins * 8;
+    return KC_OK;
+}
+
+int kc_run_filter(kc_ctx *c, const kc_run *r, uint32_t min_count, uint32_t max_count, kc_run **out) {
+    KC_TRY(check_ctx(c));
+    if (!r || !out) return c->set_error(KC_ERR_ARG, "null argument");
+    if (min_count > max_count) return c->set_error(KC_ERR_ARG, "kc_run_filter: min_count %u > max_count %u", min_count, max_count);
+    std::lock_guard<std::recursive_mutex> dg(c->direct_mu);
+    cudaSetDevice(c->cfg.device);
+    cudaStream_t s = c->stream;
+    const uint64_t n = r->n - r->skip;
+    if (n == 0) return make_run(c, s, 0, out);
+    const uint64_t *keys = r->d_keys + r->skip * r->W;
+    const uint32_t *counts = r->d_counts + r->skip;
+    void *ws = nullptr, *d_total = nullptr;
+    kc_run *f = nullptr;
+    unsigned long long total = 0;
+    int launches = 0;
+    auto body = [&]() -> int {
+        KC_TRY(dev_alloc(c, s, filter_workspace_bytes(n), &ws));
+        KC_TRY(dev_alloc(c, s, 8, &d_total));
+        KC_CUDA_TRY(c, filter_count(counts, n, min_count, max_count, ws, static_cast<unsigned long long *>(d_total), s, &launches));
+        KC_CUDA_TRY(c, cudaMemcpyAsync(&total, d_total, 8, cudaMemcpyDeviceToHost, s));
+        KC_CUDA_TRY(c, cudaStreamSynchronize(s));
+        KC_TRY(make_run(c, s, total, &f));
+        KC_CUDA_TRY(c, filter_write(keys, counts, n, r->W, min_count, max_count, ws, f->d_keys, f->d_counts, s, &launches));
+        KC_CUDA_TRY(c, cudaStreamSynchronize(s));
+        return KC_OK;
+    };
+    const int rc = body();
+    dev_free(s, ws); dev_free(s, d_total);
+    if (rc != KC_OK) {
+        if (f) kc_run_free(c, f);
+        return rc;
+    }
+    {
+        std::lock_guard<std::mutex> g(c->mu);
+        c->stats.launches += launches;
+        c->stats.d2h_bytes += 8;
+    }
+    *out = f;
+    return KC_OK;
+}
+
 // ------------------------------------------------------------------------- merge
 int kc_merge_runs(kc_ctx *c, kc_run *const *runs, uint32_t n, kc_run **out) {
     KC_TRY(check_ctx(c));

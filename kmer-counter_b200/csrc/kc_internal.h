@@ -60,6 +60,18 @@ cudaError_t fold_sorted_pairs(const uint64_t *keys, const uint32_t *counts, uint
 cudaError_t lower_bounds(const uint64_t *keys, uint64_t n, int W, const uint64_t *d_queries, uint32_t n_q,
                          unsigned long long *d_out, cudaStream_t s);
 
+// ---- count spectrum and count-range filter of a run (kc_spectrum.cu)
+// d_hist[min(c, n_bins - 1)] += 1 for every count c (d_hist: n_bins uint64, cleared here); n_bins >= 2
+cudaError_t run_histogram(const uint32_t *counts, uint64_t n, uint32_t n_bins, unsigned long long *d_hist, int n_sms,
+                          cudaStream_t s, int *n_launches);
+// survivors (lo <= count <= hi) per tile, scanned into tile offsets in ws; *d_total = survivors
+uint64_t filter_workspace_bytes(uint64_t n);
+cudaError_t filter_count(const uint32_t *counts, uint64_t n, uint32_t lo, uint32_t hi, void *ws,
+                         unsigned long long *d_total, cudaStream_t s, int *n_launches);
+// then the survivors in order into out_keys / out_counts (capacity *d_total), same ws
+cudaError_t filter_write(const uint64_t *keys, const uint32_t *counts, uint64_t n, int W, uint32_t lo, uint32_t hi,
+                         const void *ws, uint64_t *out_keys, uint32_t *out_counts, cudaStream_t s, int *n_launches);
+
 // ---- merge path (kc_merge.cu)
 uint64_t merge_workspace_bytes(uint64_t na, uint64_t nb);
 // two sorted unique runs -> one, equal keys summed (uint32 wrap); *d_num_out = records

@@ -109,6 +109,22 @@ class Run:
             off.ctypes.data_as(C.POINTER(C.c_uint64))))
         return off
 
+    def histogram(self, n_bins=10001) -> np.ndarray:
+        """Count spectrum, computed on the device (kc_run_histogram): uint64[n_bins], where h[c] = records
+        with count c and h[n_bins - 1] = records with count >= n_bins - 1. The default matches
+        Jellyfish's histo: counts up to 10,000 get their own bins."""
+        h = np.zeros(max(int(n_bins), 1), dtype=np.uint64)
+        self._c._check(self._c._lib.kc_run_histogram(self._c._ctx, self._h, h.ctypes.data_as(C.POINTER(C.c_uint64)),
+                                                     int(n_bins)))
+        return h
+
+    def filter(self, min_count=0, max_count=2**32 - 1) -> "Run":
+        """A new run with the records whose count is in [min_count, max_count], in order (kc_run_filter).
+        Filter only final counts: a chunk's run filtered before a merge loses k-mers."""
+        h = C.c_void_p()
+        self._c._check(self._c._lib.kc_run_filter(self._c._ctx, self._h, int(min_count), int(max_count), C.byref(h)))
+        return Run(self._c, h)
+
     def free(self):
         if self._h and self._c._ctx:
             self._c._lib.kc_run_free(self._c._ctx, self._h)

@@ -31,10 +31,16 @@ Options Options::parse(int argc, char **argv) {
         else if (take(argv[i], "mode=", &v)) o.mode = v;
         else if (take(argv[i], "expectedReads=", &v)) o.expectedReads = strtoll(v, nullptr, 10);
         else if (take(argv[i], "runBudget=", &v)) o.runBudget = strtoll(v, nullptr, 10);
+        else if (take(argv[i], "minCount=", &v)) o.minCount = strtoll(v, nullptr, 10);
+        else if (take(argv[i], "maxCount=", &v)) o.maxCount = strtoll(v, nullptr, 10);
+        else if (take(argv[i], "histoFile=", &v)) o.histoFile = v;
+        else if (take(argv[i], "histoMax=", &v)) o.histoMax = strtoll(v, nullptr, 10);
     }
     if (o.noOfMergersAtOnce < 2) o.noOfMergersAtOnce = 2;
     if (o.gpus < 1) o.gpus = 1;
     if (o.gpus > 8) o.gpus = 8;
+    if (o.histoMax < 1) o.histoMax = 1;
+    if (o.histoMax > (1 << 24) - 1) o.histoMax = (1 << 24) - 1;
     return o;
 }
 

@@ -32,9 +32,15 @@ struct Options {
     int64_t expectedReads = 0;                // expectedReads=: plan the accumulator for this many reads (0 = from file sizes)
     std::string parser = "gpu";               // parser=gpu|host: where FASTQ text is parsed (gpu falls back to host
                                               // for input that is not plain 4-line fixed-length FASTQ)
+    int64_t minCount = -1;                    // minCount=N / maxCount=N: the artefact keeps only k-mers whose final
+    int64_t maxCount = -1;                    // count is in [minCount, maxCount] (KMC -ci/-cx, Jellyfish -L/-U); -1 = no bound
+    std::string histoFile;                    // histoFile=PATH: the count spectrum of the final (unfiltered) counts as
+                                              // "c n" lines, c = 1..histoMax with n > 0; the histoMax line means >= histoMax
+    int64_t histoMax = 10000;                 // histoMax=N (Jellyfish's default high)
 
     // Same prefix matching as the reference. Unknown tokens are ignored, as there.
     static Options parse(int argc, char **argv);
+    bool filtering() const { return minCount >= 0 || maxCount >= 0; }
     // KMerCounter::GetChunkSize (KMerCounter.cpp:193-212): bytes of reads per chunk
     int64_t chunkSize(int64_t lineLength) const;
 };

@@ -19,6 +19,11 @@
 // whose records fit the budget, and range by range the matching slice of every spilled run
 // is uploaded (kc_run_upload), merged (kc_merge_runs) and appended to the output file --
 // ranges are key-disjoint and ascending, so the file is the sorted unique artefact.
+//
+// An optional hook sees every final run just before it is written (or handed out by InputComplete):
+// the one merged run, or each range's merged run of the out-of-core merge. Its counts are final
+// there, so it may replace the run (a count filter) or read it (the count spectrum). Chunk runs and
+// intermediate merges never reach it.
 #pragma once
 
 #include <stdint.h>
@@ -27,6 +32,7 @@
 #include <algorithm>
 #include <condition_variable>
 #include <deque>
+#include <functional>
 #include <mutex>
 #include <thread>
 #include <vector>
@@ -65,7 +71,8 @@ public:
         if ((rc = mergeAll()) != KC_OK) return rc;
         if (!_spilled.empty()) return KC_ERR_STATE;
         kc_run *last = takeOnly();
-        if (!last) return kc_merge_runs(_ctx, nullptr, 0, out);
+        if (!last && (rc = kc_merge_runs(_ctx, nullptr, 0, &last)) != KC_OK) return rc;
+        if ((rc = finalRun(&last)) != KC_OK) return rc;
         *out = last;
         return KC_OK;
     }
@@ -87,6 +94,8 @@ public:
         if (last && (rc = spill(last)) != KC_OK) return rc;
         return mergeOutOfCore(path, n_records);
     }
+    // hook(&run): may replace *run (freeing the old one) or leave it; a non-KC_OK result aborts the merge
+    void SetFinalHook(std::function<int(kc_run **)> hook) { _final = std::move(hook); }
     uint64_t merges() const { return _merges; }
     uint64_t spills() const { return _spills; }
     uint64_t ranges() const { return _ranges; }
@@ -100,6 +109,12 @@ private:
         uint64_t w[4];
     };
 
+    int finalRun(kc_run **run) {
+        if (!_final) return KC_OK;
+        const int rc = _final(run);
+        if (rc != KC_OK && *run) { kc_run_free(_ctx, *run); *run = nullptr; }
+        return rc;
+    }
     // ---- background merging
     void workerLoop() {
         for (;;) {
@@ -244,6 +259,7 @@ private:
             if (rc == KC_OK && !parts.empty()) {
                 kc_run *out = nullptr;
                 rc = kc_merge_runs(_ctx, parts.data(), (uint32_t)parts.size(), &out);
+                if (rc == KC_OK) rc = finalRun(&out);
                 if (rc == KC_OK) {
                     rc = kc_run_write(_ctx, out, path, first ? 0 : 1);
                     written += kc_run_records(out);
@@ -280,4 +296,5 @@ private:
     std::deque<kc_run *> _queue;
     bool _stop = false, _busy = false;
     int _rc = KC_OK;
+    std::function<int(kc_run **)> _final;
 };

@@ -4,7 +4,16 @@
 //                     [tempFileLocation=..] [noOfMergersAtOnce=..] [noOfMergeThreads=..]
 //                     [method=auto|sort|hash] [compat=ref|strict] [canonical=1] [device=N] [keepRuns=1] [parser=gpu|host]
 //                     [runBudget=BYTES] [gpus=N] [mode=auto|accumulate|runs] [expectedReads=N]
+//                     [minCount=N] [maxCount=N] [histoFile=PATH] [histoMax=N]
 //   kmer_counter_b200 print <record file> <ignored> <k>       (KMerPrinter, main.cpp:78-82)
+//   kmer_counter_b200 histo <record file> <out|-> <k> [histoMax]
+//                     the count spectrum of a record file, computed on the GPU (histoFile's format)
+//
+// minCount= / maxCount= keep only the k-mers whose final count is in range (KMC -ci/-cx, Jellyfish
+// -L/-U); histoFile= writes the spectrum of the final counts before that filter: one line "c n" per
+// count c = 1..histoMax that n k-mers have, the histoMax line counting every k-mer seen >= histoMax
+// times (Jellyfish's histo format). Both run on the device, on the final runs only, so records that
+// are filtered out never cross PCIe.
 //
 // What KMerCounter::Start does (KMerCounter.cpp:108-191), on the B200 path: read fixed
 // length reads into pinned chunks, count each chunk on the GPU into a sorted run
@@ -50,12 +59,82 @@ static int print_records(const char *path, uint64_t k) {
 
 #include <sys/stat.h>
 
+// "c n" for c = 1..hist.size()-1 with n > 0; the last bin holds every count >= its index
+static int write_histo(const char *path, const std::vector<uint64_t> &hist) {
+    FILE *f = strcmp(path, "-") == 0 ? stdout : fopen(path, "w");
+    if (!f) { fprintf(stderr, "cannot open %s\n", path); return KC_ERR_IO; }
+    bool ok = true;
+    for (size_t c = 1; c < hist.size() && ok; c++)
+        if (hist[c]) ok = fprintf(f, "%zu %" PRIu64 "\n", c, hist[c]) > 0;
+    if (f == stdout) ok = fflush(f) == 0 && ok;
+    else ok = fclose(f) == 0 && ok;
+    if (!ok) { fprintf(stderr, "short write to %s\n", path); return KC_ERR_IO; }
+    return KC_OK;
+}
+
+// minCount= / maxCount= / histoFile=: applied to every final run just before it is written (every
+// rank's key range, the one merged run, or each range of the out-of-core merge); the spectra add up
+struct FinalRuns {
+    const Options &opt;
+    std::vector<uint64_t> hist;                 // histoMax + 1 bins when histoFile= is given
+    uint64_t dropped = 0;
+    explicit FinalRuns(const Options &o) : opt(o), hist(o.histoFile.empty() ? 0 : (size_t)o.histoMax + 1, 0) {}
+    bool active() const { return opt.filtering() || !hist.empty(); }
+    int apply(kc_ctx *ctx, kc_run **run) {
+        int rc = KC_OK;
+        if (!hist.empty()) {
+            std::vector<uint64_t> h(hist.size());
+            if ((rc = kc_run_histogram(ctx, *run, h.data(), (uint32_t)h.size())) != KC_OK) return rc;
+            for (size_t c = 0; c < h.size(); c++) hist[c] += h[c];
+        }
+        if (opt.filtering()) {
+            const auto bound = [](int64_t v, uint32_t none) { return v < 0 ? none : v > 0xffffffffll ? 0xffffffffu : (uint32_t)v; };
+            kc_run *kept = nullptr;
+            if ((rc = kc_run_filter(ctx, *run, bound(opt.minCount, 0), bound(opt.maxCount, 0xffffffffu), &kept)) != KC_OK) return rc;
+            dropped += kc_run_records(*run) - kc_run_records(kept);
+            kc_run_free(ctx, *run);
+            *run = kept;
+        }
+        return rc;
+    }
+};
+
+// `histo <record file> <out|-> <k> [histoMax]`: the file is uploaded piece by piece and each piece's
+// spectrum is computed on the GPU; a record file is key-unique, so the pieces' spectra add up
+static int histo_records(const char *path, const char *out, uint32_t k, int64_t histo_max) {
+    if (histo_max < 1 || histo_max > (1 << 24) - 1) { fprintf(stderr, "histoMax must be 1..%d\n", (1 << 24) - 1); return 2; }
+    FILE *f = fopen(path, "rb");
+    if (!f) { fprintf(stderr, "cannot open %s\n", path); return 1; }
+    kc_config cfg = {};
+    cfg.struct_size = sizeof cfg;
+    cfg.k = k;
+    cfg.read_len = k;
+    kc_ctx *ctx = nullptr;
+    if (kc_create(&cfg, &ctx) != KC_OK) { fprintf(stderr, "kc_create: %s\n", kc_last_error(nullptr)); fclose(f); return 1; }
+    const uint64_t S = kc_record_size(k), piece = ((64ull << 20) / S) * S;
+    std::vector<unsigned char> buf(piece);
+    std::vector<uint64_t> hist((size_t)histo_max + 1, 0), h(hist.size());
+    int rc = KC_OK;
+    size_t n;
+    while (rc == KC_OK && (n = fread(buf.data(), 1, piece, f)) >= S) {
+        kc_run *run = nullptr;
+        if ((rc = kc_run_upload(ctx, buf.data(), n, &run)) == KC_OK) rc = kc_run_histogram(ctx, run, h.data(), (uint32_t)h.size());
+        if (run) kc_run_free(ctx, run);
+        for (size_t c = 0; c < h.size() && rc == KC_OK; c++) hist[c] += h[c];
+    }
+    fclose(f);
+    if (rc != KC_OK) fprintf(stderr, "kmer_counter_b200 histo: %s\n", kc_last_error(ctx));
+    kc_destroy(ctx);
+    if (rc == KC_OK) rc = write_histo(out, hist);
+    return rc == KC_OK ? 0 : 1;
+}
+
 // mode=accumulate: every chunk is only packed into super-window records (kc_accum_*); the count
 // happens once, over everything -- on one GPU, or on gpus=N with the two exchanges fused into the
 // counting kernels (kc_xchg_*). Returns 1 if this input / shape is not for this mode (the caller
 // then counts chunk by chunk into runs), 0 on success, -1 on error.
 static int run_accumulate(const Options &opt, FastqChunker &reader, int64_t L, int64_t chunk, uint32_t method,
-                          uint64_t *n_records_out) {
+                          FinalRuns &fin, uint64_t *n_records_out) {
     const int G = opt.gpus;
     // reads to plan for: a FASTQ record is 2L + header + '+' line + newlines
     uint64_t expected = opt.expectedReads > 0 ? (uint64_t)opt.expectedReads : 0;
@@ -151,7 +230,7 @@ static int run_accumulate(const Options &opt, FastqChunker &reader, int64_t L, i
             Options o2 = opt;
             o2.parser = "host";
             FastqChunker again(opt.inputFileDirectory);
-            return run_accumulate(o2, again, L, chunk, method, n_records_out);
+            return run_accumulate(o2, again, L, chunk, method, fin, n_records_out);
         }
     } else {
         while (rc == KC_OK) {
@@ -175,6 +254,7 @@ static int run_accumulate(const Options &opt, FastqChunker &reader, int64_t L, i
     if (rc == KC_OK) rc = G > 1 ? kc_xchg_run_all(ctx.data(), (uint32_t)G, runs.data()) : kc_accum_flush(ctx[0], &runs[0]);
     uint64_t n_records = 0;
     for (int g = 0; g < G && rc == KC_OK; g++) {
+        if (fin.active() && (rc = fin.apply(ctx[g], &runs[g])) != KC_OK) break;
         rc = kc_run_write(ctx[g], runs[g], opt.outputFile.c_str(), g == 0 ? 0 : 1);      // truncates, then appends
         n_records += kc_run_records(runs[g]);
     }
@@ -184,9 +264,11 @@ static int run_accumulate(const Options &opt, FastqChunker &reader, int64_t L, i
         kc_stats st;
         kc_stats_get(ctx[0], &st);
         for (int g = 1; g < G; g++) { kc_stats sg; kc_stats_get(ctx[g], &sg); st.reads += sg.reads; }
-        fprintf(stderr, "mode=accumulate gpus=%d parser=%s reads=%llu skipped=%llu chunks=%llu records=%llu\n", G,
+        fprintf(stderr, "mode=accumulate gpus=%d parser=%s reads=%llu skipped=%llu chunks=%llu records=%llu", G,
                 opt.parser != "host" ? "gpu" : "host", (unsigned long long)(opt.parser != "host" ? st.reads : reader.totalReads()),
                 (unsigned long long)reader.skippedReads(), (unsigned long long)n_chunks, (unsigned long long)n_records);
+        if (opt.filtering()) fprintf(stderr, " filtered=%llu", (unsigned long long)fin.dropped);
+        fprintf(stderr, "\n");
     }
     for (int g = 0; g < G; g++) if (runs[g]) kc_run_free(ctx[g], runs[g]);
     destroy_all();
@@ -205,7 +287,10 @@ static uint32_t method_of(const std::string &m) {
 
 int main(int argc, char **argv) {
     if (argc == 5 && strncmp(argv[1], "print", 5) == 0) return print_records(argv[2], strtoull(argv[4], nullptr, 10));
+    if ((argc == 5 || argc == 6) && strcmp(argv[1], "histo") == 0)
+        return histo_records(argv[2], argv[3], (uint32_t)strtoul(argv[4], nullptr, 10), argc == 6 ? strtoll(argv[5], nullptr, 10) : 10000);
     Options opt = Options::parse(argc, argv);
+    FinalRuns fin(opt);
     if (opt.inputFileDirectory.empty()) {
         fprintf(stderr, "usage: %s kmerLength=K inputFileLocation=DIR outputFile=FILE [gpuMemoryLimit=BYTES] [canonical=1] ...\n", argv[0]);
         return 2;
@@ -223,7 +308,8 @@ int main(int argc, char **argv) {
                            (opt.mode == "auto" && (method_of(opt.method) != KC_COUNT_AUTO && method_of(opt.method) != KC_COUNT_SUPER));
     if (!want_runs || opt.gpus > 1) {
         uint64_t n_rec = 0;
-        const int r = run_accumulate(opt, reader, L, chunk, method_of(opt.method), &n_rec);
+        const int r = run_accumulate(opt, reader, L, chunk, method_of(opt.method), fin, &n_rec);
+        if (r == 0 && !opt.histoFile.empty() && write_histo(opt.histoFile.c_str(), fin.hist) != KC_OK) return 1;
         if (r == 0) { fprintf(stderr, "records=%" PRIu64 " -> %s\n", n_rec, opt.outputFile.c_str()); return 0; }
         if (r < 0) return 1;
         if (opt.gpus > 1) { fprintf(stderr, "gpus=%d needs k <= 64 with windows of at least 22 bases\n", opt.gpus); return 1; }
@@ -251,6 +337,7 @@ int main(int argc, char **argv) {
     for (int attempt = opt.parser == "host" ? 1 : 0; attempt < 2; attempt++) {
         RunMerger merger(ctx, opt.noOfMergersAtOnce, (uint32_t)opt.kmerLength, opt.runBudget > 0 ? (uint64_t)opt.runBudget : 0,
                          opt.noOfMergeThreads);
+        if (fin.active()) merger.SetFinalHook([&](kc_run **run) { return fin.apply(ctx, run); });
         bool busy[2] = {false, false};
         bool refused = false;
         chunk_id = 0;
@@ -338,9 +425,12 @@ int main(int argc, char **argv) {
             kc_stats st;
             kc_stats_get(ctx, &st);
             fprintf(stderr, "parser=%s reads=%" PRIu64 " skipped=%" PRIu64 " kmers=%" PRIu64 " chunks=%" PRIu64
-                            " merges=%" PRIu64 " spills=%" PRIu64 " ranges=%" PRIu64 "\n",
+                            " merges=%" PRIu64 " spills=%" PRIu64 " ranges=%" PRIu64,
                     attempt == 0 ? "gpu" : "host", attempt == 0 ? st.reads : reader.totalReads(), reader.skippedReads(),
                     st.kmers_valid, st.chunks, merger.merges(), merger.spills(), merger.ranges());
+            if (opt.filtering()) fprintf(stderr, " filtered=%" PRIu64, fin.dropped);
+            fprintf(stderr, "\n");
+            if (!opt.histoFile.empty()) rc = write_histo(opt.histoFile.c_str(), fin.hist);
         }
         break;
     }

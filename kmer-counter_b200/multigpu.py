@@ -101,6 +101,24 @@ def count_shard(counter, d_reads_ptr, n_bytes, device, group=None, exchange=None
     return exchange_and_combine(counter, local, device, group)
 
 
+def histogram(run, n_bins=10001, group=None):
+    """Count spectrum of the whole distributed artefact: every rank's Run.histogram summed by one
+    all-reduce; every rank gets the same uint64[n_bins]. Collective.
+
+    After the exchange (Exchange.finish, or exchange_and_combine for k > 64) rank r holds key range r
+    with its final counts, so this sum is the spectrum of the concatenated artefact. For the same
+    reason Run.filter may be applied rank by rank: the concatenation of the filtered runs in rank
+    order is the filtered artefact."""
+    import torch
+    import torch.distributed as dist
+    h = run.histogram(n_bins)
+    t = torch.from_numpy(h.view(np.int64).copy())             # sums stay far below 2^63
+    if dist.get_backend(group) == "nccl":                     # NCCL reduces device tensors: the run's device
+        t = t.to(torch.device("cuda", run._c.device))
+    dist.all_reduce(t, group=group)
+    return t.cpu().numpy().view(np.uint64)
+
+
 # ------------------------------------------------------------------ ownership
 def range_splitters(world, words):
     """P-1 ascending splitter keys cutting the key space into P equal-width ranges
