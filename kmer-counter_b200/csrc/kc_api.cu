@@ -10,6 +10,8 @@
 #include <string.h>
 
 #include <algorithm>
+#include <atomic>
+#include <memory>
 #include <mutex>
 #include <string>
 #include <vector>
@@ -34,6 +36,14 @@ struct kc_run {
 };
 
 namespace {
+
+// A run this scope owns: kc_run_free'd when the scope ends unless released to the caller. make_run
+// fills one; a run reaches a caller of the ABI only through release() on success.
+struct RunFree {
+    kc_ctx *c = nullptr;
+    void operator()(kc_run *r) const { kc_run_free(c, r); }
+};
+using RunPtr = std::unique_ptr<kc_run, RunFree>;
 
 thread_local std::string g_create_error;
 
@@ -101,7 +111,7 @@ struct kc_ctx {
         uint64_t windows = 0, reads = 0;     // accumulated since the last reset
         uint64_t max_windows = 0;            // what the plan was made for
         uint64_t ovf_reserved = 0;           // overflow records that chunks queued so far may still produce
-        std::vector<kc_run *> parts;         // runs of earlier automatic flushes
+        std::vector<RunPtr> parts;           // runs of earlier automatic flushes
         cudaEvent_t ev[8] = {};
         bool fresh = true;                   // bins are empty
         // multi-GPU exchange (kc_xchg_*): this context is rank `rank` of `n_ranks`
@@ -122,6 +132,8 @@ struct kc_ctx {
     unsigned long long last_scal[SC_COUNT] = {0};   // device scalars of the most recent chunk (kc_debug_scalars)
     int last_code = 0;
     char err[512] = {0};
+    uint64_t fail_alloc_at = 0;           // KC_TEST_FAIL_ALLOC
+    std::atomic<uint64_t> n_alloc_calls{0};
 
     int set_error(int code, const char *fmt, ...) {
         va_list ap;
@@ -149,6 +161,9 @@ std::vector<void *> g_plain;
 
 int dev_alloc(kc_ctx *c, cudaStream_t s, uint64_t bytes, void **out) {
     *out = nullptr;
+    // KC_TEST_FAIL_ALLOC=n (test knob, read in kc_create): the context's n-th call fails once, before allocating anything
+    if (c->fail_alloc_at && ++c->n_alloc_calls == c->fail_alloc_at)
+        return c->set_error(KC_ERR_NOMEM, "device allocation of %llu bytes failed (KC_TEST_FAIL_ALLOC)", (unsigned long long)bytes);
     if (bytes == 0) bytes = 16;
     const bool dbg = getenv("KC_DEBUG_PLAN") != nullptr;
     if (dbg && bytes > (1ull << 30)) {
@@ -199,6 +214,28 @@ void dev_free(cudaStream_t s, void *p) {
     }
     cudaFreeAsync(p, s);
 }
+
+// Short-lived device scratch from dev_alloc, given back on its stream when the scope ends unless released.
+class DevBuf {
+  public:
+    explicit DevBuf(cudaStream_t s) : s_(s) {}
+    DevBuf(DevBuf &&o) noexcept : s_(o.s_), p_(o.release()) {}
+    DevBuf(const DevBuf &) = delete;
+    DevBuf &operator=(const DevBuf &) = delete;
+    ~DevBuf() { reset(); }
+    int alloc(kc_ctx *c, uint64_t bytes) { return dev_alloc(c, s_, bytes, &p_); }
+    template <class T = void> T *get() const { return static_cast<T *>(p_); }
+    template <class T = void> T *release() {
+        T *p = get<T>();
+        p_ = nullptr;
+        return p;
+    }
+    void reset() { dev_free(s_, release()); }
+
+  private:
+    cudaStream_t s_;
+    void *p_ = nullptr;
+};
 
 int pending_init(kc_ctx *c, Pending &p) {
     if (p.d_scal) return KC_OK;
@@ -432,19 +469,23 @@ int count_enqueue_impl(kc_ctx *c, Pending &p, const void *d_reads, uint64_t n_by
     return KC_OK;
 }
 
-int make_run(kc_ctx *c, cudaStream_t s, uint64_t n, kc_run **out) {
-    kc_run *r = new kc_run();
+int make_run(kc_ctx *c, cudaStream_t s, uint64_t n, RunPtr *out) {
+    DevBuf keys(s), counts(s);
+    KC_TRY(keys.alloc(c, n * c->W * 8));
+    KC_TRY(counts.alloc(c, n * 4));
+    RunPtr r(new kc_run(), RunFree{c});
     r->W = c->W;
     r->n = n;
-    void *mem = nullptr;
-    int rc = dev_alloc(c, s, n * c->W * 8, &mem);
-    if (rc != KC_OK) { delete r; return rc; }
-    r->d_keys = static_cast<uint64_t *>(mem);
-    rc = dev_alloc(c, s, n * 4, &mem);
-    if (rc != KC_OK) { dev_free(s, r->d_keys); delete r; return rc; }
-    r->d_counts = static_cast<uint32_t *>(mem);
-    *out = r;
+    r->d_keys = keys.release<uint64_t>();
+    r->d_counts = counts.release<uint32_t>();
+    *out = std::move(r);
     return KC_OK;
+}
+// kc_merge_runs of runs the caller owns (they are freed with the vector)
+int merge_owned(kc_ctx *c, const std::vector<RunPtr> &parts, kc_run **out) {
+    std::vector<kc_run *> in;
+    for (const RunPtr &p : parts) in.push_back(p.get());
+    return kc_merge_runs(c, in.data(), (uint32_t)in.size(), out);
 }
 
 // Super-window path: sub-buckets S3c left out because they exceed its shared memory (skewed input:
@@ -457,88 +498,115 @@ int super_finish_big(kc_ctx *c, const SuperPlan &pl, void *ws, unsigned long lon
     if (n_big_records > kMaxSortKeys) return c->set_error(KC_ERR_CAPACITY, "%llu records in oversized key ranges", (unsigned long long)n_big_records);
     const int W = c->W;
     const uint64_t kb = n_big_records * W * 8, cb = n_big_records * 4, wsb = sort_workspace_bytes(n_big_records, W);
-    void *ka = nullptr, *kb2 = nullptr, *ca = nullptr, *cb2 = nullptr, *sw = nullptr;
-    int rc = dev_alloc(c, s, kb, &ka);
-    if (rc == KC_OK) rc = dev_alloc(c, s, kb, &kb2);
-    if (rc == KC_OK) rc = dev_alloc(c, s, cb, &ca);
-    if (rc == KC_OK) rc = dev_alloc(c, s, cb, &cb2);
-    if (rc == KC_OK) rc = dev_alloc(c, s, wsb, &sw);
-    cudaError_t e = cudaSuccess;
+    DevBuf ka(s), kb2(s), ca(s), cb2(s), sw(s);
+    KC_TRY(ka.alloc(c, kb));
+    KC_TRY(kb2.alloc(c, kb));
+    KC_TRY(ca.alloc(c, cb));
+    KC_TRY(cb2.alloc(c, cb));
+    KC_TRY(sw.alloc(c, wsb));
     int launches = 0;
-    if (rc == KC_OK) {
-        uint64_t *sk = nullptr;
-        uint32_t *sv = nullptr;
-        e = super_big_gather(pl, ws, static_cast<uint64_t *>(ka), static_cast<uint32_t *>(ca), c->n_sms, s);
-        if (e == cudaSuccess)
-            e = radix_sort(static_cast<uint64_t *>(ka), static_cast<uint64_t *>(kb2), static_cast<uint32_t *>(ca),
-                           static_cast<uint32_t *>(cb2), n_big_records, W, static_zero_bits(c), SortWorkspace{sw, wsb}, s, &sk,
-                           &sv, &launches, nullptr, nullptr);
-        if (e == cudaSuccess) e = super_big_place(pl, dup, ws, d_sc, sk, sv, out_keys, out_counts, c->n_sms, s);
-    }
-    dev_free(s, ka); dev_free(s, kb2); dev_free(s, ca); dev_free(s, cb2); dev_free(s, sw);
-    if (rc != KC_OK) return rc;
-    if (e != cudaSuccess) return c->set_error(KC_ERR_CUDA, "oversized key ranges: %s", cudaGetErrorString(e));
+    uint64_t *sk = nullptr;
+    uint32_t *sv = nullptr;
+    KC_CUDA_TRY(c, super_big_gather(pl, ws, ka.get<uint64_t>(), ca.get<uint32_t>(), c->n_sms, s));
+    KC_CUDA_TRY(c, radix_sort(ka.get<uint64_t>(), kb2.get<uint64_t>(), ca.get<uint32_t>(), cb2.get<uint32_t>(), n_big_records, W,
+                              static_zero_bits(c), SortWorkspace{sw.get(), wsb}, s, &sk, &sv, &launches, nullptr, nullptr));
+    KC_CUDA_TRY(c, super_big_place(pl, dup, ws, d_sc, sk, sv, out_keys, out_counts, c->n_sms, s));
     std::lock_guard<std::mutex> g(c->mu);
     c->stats.launches += launches + 3;
     return KC_OK;
 }
 
-int count_finish_sort(kc_ctx *c, Pending &p, cudaStream_t s, kc_run **out);
-int count_finish_hash_global(kc_ctx *c, Pending &p, cudaStream_t s, kc_run **out);
-int count_finish_partition(kc_ctx *c, Pending &p, cudaStream_t s, kc_run **out);
-int count_finish_super(kc_ctx *c, Pending &p, cudaStream_t s, kc_run **out, bool *failed);
-int count_finish_place(kc_ctx *c, Pending &p, cudaStream_t s, kc_run **out, bool *failed);
-int strict_hide_zero(kc_ctx *c, Pending &p, kc_run *r, cudaStream_t s);
+// S3c, the last stage of the super-window and key-placement paths, once S3a/S3b are queued: every
+// sub-bucket is sorted in shared memory, straight into the run of n_d records, or -- if records may
+// repeat (dup) -- folded into a temporary that a gather compacts into a run of the survivors.
+// fpl is the plan whose S3c variant runs, h_sc the host mirror of the scalars d_sc. *run may come
+// allocated (!dup: its arrays were the second record buffer E of S3a/S3b). ext_e (dup only): E is
+// the caller's own allocation {keys, counts}, and the temporary: the survivors are gathered into D,
+// E is given back and only then the run is allocated, so that both are never held next to the
+// workspace. h_sc[SW_FAIL] set on return: the records did not fit, *run is no count.
+int super_emit(kc_ctx *c, const SuperPlan &pl, const SuperPlan &fpl, void *ws, unsigned long long *d_sc,
+               unsigned long long *h_sc, bool dup, uint64_t n_d, cudaStream_t s, RunPtr *run, DevBuf *ext_e = nullptr) {
+    auto read_back = [&]() {
+        cudaError_t e = cudaMemcpyAsync(h_sc, d_sc, SC_COUNT * 8, cudaMemcpyDeviceToHost, s);
+        return e == cudaSuccess ? cudaStreamSynchronize(s) : e;
+    };
+    if (!dup) {
+        if (!*run) KC_TRY(make_run(c, s, n_d, run));
+        if (n_d) {                                  // (nothing ran otherwise: the scalars are the ones the caller holds)
+            KC_CUDA_TRY(c, super_finish(fpl, false, ws, d_sc, (*run)->d_keys, (*run)->d_counts, c->n_sms, s));
+            KC_CUDA_TRY(c, read_back());
+        }
+        if (!h_sc[SW_FAIL] && h_sc[SW_BIG])
+            KC_TRY(super_finish_big(c, pl, ws, d_sc, false, h_sc[SW_BIG_RECORDS], (*run)->d_keys, (*run)->d_counts, s));
+        return KC_OK;
+    }
+    uint64_t *tk = nullptr;
+    uint32_t *tc = nullptr;
+    super_tmp_buffers(pl, ws, &tk, &tc);
+    KC_CUDA_TRY(c, super_finish(fpl, true, ws, d_sc, tk, tc, c->n_sms, s));
+    KC_CUDA_TRY(c, read_back());
+    if (!h_sc[SW_FAIL] && h_sc[SW_BIG]) KC_TRY(super_finish_big(c, pl, ws, d_sc, true, h_sc[SW_BIG_RECORDS], tk, tc, s));
+    KC_CUDA_TRY(c, super_fold_offsets(pl, ws, d_sc, s));
+    KC_CUDA_TRY(c, read_back());
+    if (h_sc[SW_FAIL]) return KC_OK;
+    const uint64_t n_out = h_sc[SW_OUT];
+    if (!ext_e) {
+        KC_TRY(make_run(c, s, n_out, run));
+        if (n_out) KC_CUDA_TRY(c, super_gather(pl, ws, tk, tc, (*run)->d_keys, (*run)->d_counts, c->n_sms, s));
+        return KC_OK;
+    }
+    uint64_t *dk = reinterpret_cast<uint64_t *>(static_cast<uint8_t *>(ws) + pl.off_dk);
+    uint32_t *dc = reinterpret_cast<uint32_t *>(static_cast<uint8_t *>(ws) + pl.off_dc);
+    if (n_out) KC_CUDA_TRY(c, super_gather(pl, ws, tk, tc, dk, dc, c->n_sms, s));
+    ext_e[0].reset();
+    ext_e[1].reset();
+    KC_TRY(make_run(c, s, n_out, run));
+    if (n_out) {
+        KC_CUDA_TRY(c, cudaMemcpyAsync((*run)->d_keys, dk, n_out * c->W * 8, cudaMemcpyDeviceToDevice, s));
+        KC_CUDA_TRY(c, cudaMemcpyAsync((*run)->d_counts, dc, n_out * 4, cudaMemcpyDeviceToDevice, s));
+    }
+    return KC_OK;
+}
+
+// kc_stats' per-stage fields of a count whose stage i took ms[i], moving bytes[i] in launches[i]
+// kernels; the dominant stage is the slowest of stages 0 .. n_dom - 1. st.ms_total is set already.
+void stage_stats(kc_stats &st, int n_stages, const float *ms, const uint64_t *bytes, const uint32_t *launches, int n_dom) {
+    st.n_stages = (uint32_t)n_stages;
+    for (int i = 0; i < 8; i++) { st.ms_stage[i] = ms[i]; st.stage_bytes[i] = bytes[i]; st.stage_launches[i] = launches[i]; }
+    int dom = 0;
+    for (int i = 1; i < n_dom; i++)
+        if (st.ms_stage[i] > st.ms_stage[dom]) dom = i;
+    st.dominant_stage = (uint32_t)dom;
+    st.ms_dominant = st.ms_stage[dom];
+    st.dominant_bytes = st.stage_bytes[dom];
+    st.dominant_launches = st.stage_launches[dom] ? st.stage_launches[dom] : 1;
+    st.ms_extract = st.ms_stage[0];
+    st.ms_emit = n_stages ? st.ms_stage[n_stages - 1] : 0;
+    st.ms_count = st.ms_total - st.ms_extract - st.ms_emit;
+}
+
+// What a chunk is re-counted with when method m could not take it (input far from the plan's
+// assumptions): the super-window path's lists or sub-buckets overflowed -> the partitioned path,
+// which sizes everything from exact histograms; a sub-bucket arrangement the placement path cannot
+// take, or a full hash table -> sort + run-length.
+uint32_t fallback(const kc_ctx *c, uint32_t m) {
+    return m == KC_COUNT_SUPER && c->W <= 2 ? KC_COUNT_HASH : KC_COUNT_SORT;
+}
+
+int count_finish_method(kc_ctx *c, Pending &p, cudaStream_t s, RunPtr *out);
 
 // Wait for the queued kernels, build the run, record stage timings.
-int count_finish(kc_ctx *c, Pending &p, const void *d_reads, uint64_t n_bytes, cudaStream_t s, kc_run **out) {
-    *out = nullptr;
-    if (!p.active) return c->set_error(KC_ERR_STATE, "no chunk queued");
+int count_finish_impl(kc_ctx *c, Pending &p, const void *d_reads, uint64_t n_bytes, cudaStream_t s, RunPtr *out) {
     KC_CUDA_TRY(c, cudaStreamSynchronize(s));
-    int rc;
-    uint32_t used = p.method;
     memcpy(c->last_scal, p.h_scal, sizeof c->last_scal);
-    if (p.n_slots && p.method == KC_COUNT_SUPER) {
-        // a list or a sub-bucket overflowed (input far from the plan's assumptions): the chunk is
-        // re-counted by the partitioned path, which sizes everything from exact histograms
-        bool failed = false;
-        rc = count_finish_super(c, p, s, out, &failed);
-        if (rc != KC_OK) { pending_release(s, p); return rc; }
-        if (failed) {
-            if (*out) { kc_run_free(c, *out); *out = nullptr; }
-            pending_release(s, p);
-            used = c->W <= 2 ? KC_COUNT_HASH : KC_COUNT_SORT;
-            KC_TRY(count_enqueue(c, p, d_reads, n_bytes, s, used));
-            KC_CUDA_TRY(c, cudaStreamSynchronize(s));
-        }
-    }
-    if (p.n_slots && p.method == KC_COUNT_PLACE) {
-        // a sub-bucket arrangement the path cannot take: the chunk is re-counted by sort + run-length
-        bool failed = false;
-        rc = count_finish_place(c, p, s, out, &failed);
-        if (rc != KC_OK) { pending_release(s, p); return rc; }
-        if (failed) {
-            if (*out) { kc_run_free(c, *out); *out = nullptr; }
-            pending_release(s, p);
-            used = KC_COUNT_SORT;
-            KC_TRY(count_enqueue(c, p, d_reads, n_bytes, s, used));
-            KC_CUDA_TRY(c, cudaStreamSynchronize(s));
-        }
-    }
-    const bool overflow = p.n_slots && (used == KC_COUNT_HASH || used == KC_COUNT_HASH_GLOBAL) &&
-                          p.h_scal[SC_SIDE + 1];
-    if (overflow) {                               // table(s) full: redo this chunk with sort + run-length
+    while (true) {                                // until the path the chunk was counted by gives a run
+        KC_TRY(count_finish_method(c, p, s, out));
+        if (*out) break;
         pending_release(s, p);
-        KC_TRY(count_enqueue(c, p, d_reads, n_bytes, s, KC_COUNT_SORT));
+        KC_TRY(count_enqueue(c, p, d_reads, n_bytes, s, fallback(c, p.method)));
         KC_CUDA_TRY(c, cudaStreamSynchronize(s));
-        used = KC_COUNT_SORT;
     }
-    if ((used == KC_COUNT_SUPER || used == KC_COUNT_PLACE) && p.n_slots) rc = KC_OK;     // the run was built above
-    else if (p.n_slots == 0) rc = make_run(c, s, 0, out);
-    else if (used == KC_COUNT_HASH) rc = count_finish_partition(c, p, s, out);
-    else if (used == KC_COUNT_HASH_GLOBAL) rc = count_finish_hash_global(c, p, s, out);
-    else rc = count_finish_sort(c, p, s, out);
-    if (rc != KC_OK) { pending_release(s, p); return rc; }
+    const uint32_t used = p.method;
     if (used != KC_COUNT_HASH) {                  // kc_place_next_run is one-shot: a chunk that took another path disarms it too
         std::lock_guard<std::mutex> g(c->mu);
         c->place.set = false;
@@ -546,162 +614,87 @@ int count_finish(kc_ctx *c, Pending &p, const void *d_reads, uint64_t n_bytes, c
     const int n_stages = p.n_ev;                  // the last stage (emit) ends at the event recorded now
     KC_CUDA_TRY(c, cudaEventRecord(p.ev[p.n_ev], s));
     KC_CUDA_TRY(c, cudaEventSynchronize(p.ev[p.n_ev]));
-    {
-        std::lock_guard<std::mutex> g(c->mu);
-        kc_stats &st = c->stats;
-        st.chunks++;
-        st.reads += p.n_reads;
-        st.kmer_slots += p.n_slots;
-        const uint64_t invalid = p.h_scal[SC_INVALID];
-        const uint64_t nv = p.n_slots - invalid, U = (*out)->n;
-        const uint64_t in_bytes = p.n_reads * c->cfg.read_len, Kb = 8ull * c->W;
-        st.kmers_valid += nv;
-        st.distinct_last = (*out)->n - (*out)->skip;
-        st.method_used = used;
-        st.n_stages = (uint32_t)n_stages;
-        for (int i = 0; i < 8; i++) { st.ms_stage[i] = 0; st.stage_bytes[i] = 0; st.stage_launches[i] = 0; }
-        for (int i = 0; i < n_stages; i++) cudaEventElapsedTime(&st.ms_stage[i], p.ev[i], p.ev[i + 1]);
-        cudaEventElapsedTime(&st.ms_total, p.ev[0], p.ev[n_stages]);
-        // algorithmic bytes per stage: what the stage must read and write once
-        if (used == KC_COUNT_SORT && p.n_slots) {
-            const uint64_t N = p.n_slots;
-            st.stage_bytes[0] = in_bytes + Kb * N;                         st.stage_launches[0] = 1;
-            st.stage_bytes[1] = Kb * N;                                    st.stage_launches[1] = 2;
-            st.stage_bytes[2] = (uint64_t)p.n_passes * 2 * Kb * N;         st.stage_launches[2] = (uint32_t)p.n_passes;
-            st.stage_bytes[3] = Kb * N + U * (Kb + 4);                     st.stage_launches[3] = 1;
-            st.stage_bytes[4] = U * (2 * Kb + 8);                          st.stage_launches[4] = 1;
-        } else if (used == KC_COUNT_HASH && p.n_slots) {
-            st.stage_bytes[0] = in_bytes;                                  st.stage_launches[0] = 1;   // + a one-block scan
-            st.stage_bytes[1] = in_bytes + Kb * nv;                        st.stage_launches[1] = 1;
-            st.stage_bytes[2] = Kb * nv;                                   st.stage_launches[2] = 1;   // + a one-block scan
-            st.stage_bytes[3] = 2 * Kb * nv;                               st.stage_launches[3] = 1;
-            st.stage_bytes[4] = Kb * nv + (Kb + 4) * U;                    st.stage_launches[4] = 1;   // + a one-block scan
-            st.stage_bytes[5] = 2 * (Kb + 4) * U;                          st.stage_launches[5] = 1;
-        } else if (used == KC_COUNT_SUPER && p.n_slots) {
-            const uint64_t rec = c->last_scal[SW_RECORDS] * 16ull * c->W, ub = U * (Kb + 4);
-            st.stage_bytes[0] = in_bytes + rec;                            st.stage_launches[0] = 1;   // S1 scatter
-            st.stage_bytes[1] = rec + ub;                                  st.stage_launches[1] = 1;   // S2 count
-            st.stage_bytes[2] = 2 * ub;                                    st.stage_launches[2] = 1;   // S3a (+ plan)
-            st.stage_bytes[3] = U * Kb;                                    st.stage_launches[3] = 1;   // level-2 histogram (+ scan)
-            st.stage_bytes[4] = 2 * ub;                                    st.stage_launches[4] = 1;   // S3b
-            st.stage_bytes[5] = 2 * ub;                                    st.stage_launches[5] = 1;   // S3c
-        } else if (used == KC_COUNT_PLACE && p.n_slots) {
-            const uint64_t N = p.n_slots, nb = N * (Kb + 4), ub = U * (Kb + 4);
-            st.stage_bytes[0] = in_bytes + Kb * N;                         st.stage_launches[0] = 1;   // extract: a key per slot
-            st.stage_bytes[1] = 8 * N + 4 * N;                             st.stage_launches[1] = 1;   // leading word in, count out
-            st.stage_bytes[2] = 2 * nb;                                    st.stage_launches[2] = 1;   // S3a (+ plan)
-            st.stage_bytes[3] = 8 * N;                                     st.stage_launches[3] = 1;   // level-2 histogram (+ scan)
-            st.stage_bytes[4] = 2 * nb;                                    st.stage_launches[4] = 1;   // S3b
-            st.stage_bytes[5] = nb + 3 * ub;                               st.stage_launches[5] = 3;   // S3c fold, offsets, gather
-        } else if (used == KC_COUNT_HASH_GLOBAL && p.n_slots) {
-            st.stage_bytes[0] = p.table.capacity * 16;                     st.stage_launches[0] = 1;
-            st.stage_bytes[1] = in_bytes + nv * 16;                        st.stage_launches[1] = 1;   // SURVEY 8(d) terms
-            st.stage_bytes[2] = p.table.capacity * 16 + U * 12 * 17;       st.stage_launches[2] = 10;
-        }
-        int dom = 0;
-        if (used == KC_COUNT_SUPER || used == KC_COUNT_PLACE) {             // every stage is a kernel of the path
-            for (int i = 1; i < n_stages; i++)
-                if (st.ms_stage[i] > st.ms_stage[dom]) dom = i;
-        } else {
-            for (int i = 1; i + 1 < n_stages; i++)
-                if (st.ms_stage[i] > st.ms_stage[dom]) dom = i;
-        }
-        st.dominant_stage = (uint32_t)dom;
-        st.ms_dominant = st.ms_stage[dom];
-        st.dominant_bytes = st.stage_bytes[dom];
-        st.dominant_launches = st.stage_launches[dom] ? st.stage_launches[dom] : 1;
-        st.ms_extract = st.ms_stage[0];
-        st.ms_emit = n_stages ? st.ms_stage[n_stages - 1] : 0;
-        st.ms_count = st.ms_total - st.ms_extract - st.ms_emit;
+    std::lock_guard<std::mutex> g(c->mu);
+    kc_stats &st = c->stats;
+    st.chunks++;
+    st.reads += p.n_reads;
+    st.kmer_slots += p.n_slots;
+    const uint64_t invalid = p.h_scal[SC_INVALID];
+    const uint64_t nv = p.n_slots - invalid, U = (*out)->n;
+    const uint64_t in_bytes = p.n_reads * c->cfg.read_len, Kb = 8ull * c->W;
+    st.kmers_valid += nv;
+    st.distinct_last = (*out)->n - (*out)->skip;
+    st.method_used = used;
+    float ms[8] = {0};
+    uint64_t b[8] = {0};
+    uint32_t l[8] = {0};
+    for (int i = 0; i < n_stages; i++) cudaEventElapsedTime(&ms[i], p.ev[i], p.ev[i + 1]);
+    cudaEventElapsedTime(&st.ms_total, p.ev[0], p.ev[n_stages]);
+    // algorithmic bytes per stage: what the stage must read and write once
+    if (used == KC_COUNT_SORT && p.n_slots) {
+        const uint64_t N = p.n_slots;
+        b[0] = in_bytes + Kb * N;                         l[0] = 1;
+        b[1] = Kb * N;                                    l[1] = 2;
+        b[2] = (uint64_t)p.n_passes * 2 * Kb * N;         l[2] = (uint32_t)p.n_passes;
+        b[3] = Kb * N + U * (Kb + 4);                     l[3] = 1;
+        b[4] = U * (2 * Kb + 8);                          l[4] = 1;
+    } else if (used == KC_COUNT_HASH && p.n_slots) {
+        b[0] = in_bytes;                                  l[0] = 1;   // + a one-block scan
+        b[1] = in_bytes + Kb * nv;                        l[1] = 1;
+        b[2] = Kb * nv;                                   l[2] = 1;   // + a one-block scan
+        b[3] = 2 * Kb * nv;                               l[3] = 1;
+        b[4] = Kb * nv + (Kb + 4) * U;                    l[4] = 1;   // + a one-block scan
+        b[5] = 2 * (Kb + 4) * U;                          l[5] = 1;
+    } else if (used == KC_COUNT_SUPER && p.n_slots) {
+        const uint64_t rec = c->last_scal[SW_RECORDS] * 16ull * c->W, ub = U * (Kb + 4);
+        b[0] = in_bytes + rec;                            l[0] = 1;   // S1 scatter
+        b[1] = rec + ub;                                  l[1] = 1;   // S2 count
+        b[2] = 2 * ub;                                    l[2] = 1;   // S3a (+ plan)
+        b[3] = U * Kb;                                    l[3] = 1;   // level-2 histogram (+ scan)
+        b[4] = 2 * ub;                                    l[4] = 1;   // S3b
+        b[5] = 2 * ub;                                    l[5] = 1;   // S3c
+    } else if (used == KC_COUNT_PLACE && p.n_slots) {
+        const uint64_t N = p.n_slots, nb = N * (Kb + 4), ub = U * (Kb + 4);
+        b[0] = in_bytes + Kb * N;                         l[0] = 1;   // extract: a key per slot
+        b[1] = 8 * N + 4 * N;                             l[1] = 1;   // leading word in, count out
+        b[2] = 2 * nb;                                    l[2] = 1;   // S3a (+ plan)
+        b[3] = 8 * N;                                     l[3] = 1;   // level-2 histogram (+ scan)
+        b[4] = 2 * nb;                                    l[4] = 1;   // S3b
+        b[5] = nb + 3 * ub;                               l[5] = 3;   // S3c fold, offsets, gather
+    } else if (used == KC_COUNT_HASH_GLOBAL && p.n_slots) {
+        b[0] = p.table.capacity * 16;                     l[0] = 1;
+        b[1] = in_bytes + nv * 16;                        l[1] = 1;   // SURVEY 8(d) terms
+        b[2] = p.table.capacity * 16 + U * 12 * 17;       l[2] = 10;
     }
-    pending_release(s, p);
+    // every stage of the super-window and placement paths is a kernel of the path; elsewhere the emit stage is not
+    const bool all_kernels = used == KC_COUNT_SUPER || used == KC_COUNT_PLACE;
+    stage_stats(st, n_stages, ms, b, l, all_kernels ? n_stages : n_stages - 1);
     return KC_OK;
 }
 
-// Super-window path, after S1..S3b have drained: the host knows |D| now, allocates the run and
-// lets S3c sort every sub-bucket straight into it. If records may repeat (overflow list in use)
-// S3c folds them into a temporary and a gather closes the gaps.
-int count_finish_super(kc_ctx *c, Pending &p, cudaStream_t s, kc_run **out, bool *failed) {
-    *failed = false;
+int count_finish(kc_ctx *c, Pending &p, const void *d_reads, uint64_t n_bytes, cudaStream_t s, kc_run **out) {
     *out = nullptr;
-    const SuperPlan &pl = p.splan;
-    if (p.h_scal[SW_FAIL]) { *failed = true; return KC_OK; }
-    const uint64_t n_d = p.h_scal[SW_D];
+    if (!p.active) return c->set_error(KC_ERR_STATE, "no chunk queued");
+    RunPtr r;
+    const int rc = count_finish_impl(c, p, d_reads, n_bytes, s, &r);
+    pending_release(s, p);
+    if (rc == KC_OK) *out = r.release();
+    return rc;
+}
+
+// Super-window path, after S1..S3b have drained: the host knows |D| now, and S3c writes the run.
+// h_scal[SW_FAIL] set on return: a list or a sub-bucket overflowed, no run.
+int count_finish_super(kc_ctx *c, Pending &p, cudaStream_t s, RunPtr *out) {
+    if (p.h_scal[SW_FAIL]) return KC_OK;
     const bool dup = p.h_scal[SW_OVF] != 0 || env_force_dup();
-    kc_run *r = nullptr;
-    if (!dup) {
-        KC_TRY(make_run(c, s, n_d, &r));
-        if (n_d) {
-            KC_CUDA_TRY(c, super_finish(pl, false, p.ws_super, p.d_scal, r->d_keys, r->d_counts, c->n_sms, s));
-            KC_CUDA_TRY(c, cudaMemcpyAsync(p.h_scal, p.d_scal, SC_COUNT * 8, cudaMemcpyDeviceToHost, s));
-            KC_CUDA_TRY(c, cudaStreamSynchronize(s));
-            if (!p.h_scal[SW_FAIL] && p.h_scal[SW_BIG]) {
-                const int rc = super_finish_big(c, pl, p.ws_super, p.d_scal, false, p.h_scal[SW_BIG_RECORDS], r->d_keys, r->d_counts, s);
-                if (rc != KC_OK) { kc_run_free(c, r); return rc; }
-            }
-        }
-    } else {
-        uint64_t *tk = nullptr;
-        uint32_t *tc = nullptr;
-        super_tmp_buffers(pl, p.ws_super, &tk, &tc);
-        KC_CUDA_TRY(c, super_finish(pl, true, p.ws_super, p.d_scal, tk, tc, c->n_sms, s));
-        KC_CUDA_TRY(c, cudaMemcpyAsync(p.h_scal, p.d_scal, SC_COUNT * 8, cudaMemcpyDeviceToHost, s));
-        KC_CUDA_TRY(c, cudaStreamSynchronize(s));
-        if (!p.h_scal[SW_FAIL] && p.h_scal[SW_BIG])
-            KC_TRY(super_finish_big(c, pl, p.ws_super, p.d_scal, true, p.h_scal[SW_BIG_RECORDS], tk, tc, s));
-        KC_CUDA_TRY(c, super_fold_offsets(pl, p.ws_super, p.d_scal, s));
-        KC_CUDA_TRY(c, cudaMemcpyAsync(p.h_scal, p.d_scal, SC_COUNT * 8, cudaMemcpyDeviceToHost, s));
-        KC_CUDA_TRY(c, cudaStreamSynchronize(s));
-        if (!p.h_scal[SW_FAIL]) {
-            KC_TRY(make_run(c, s, p.h_scal[SW_OUT], &r));
-            if (r->n) KC_CUDA_TRY(c, super_gather(pl, p.ws_super, tk, tc, r->d_keys, r->d_counts, c->n_sms, s));
-        }
-    }
+    RunPtr r;
+    KC_TRY(super_emit(c, p.splan, p.splan, p.ws_super, p.d_scal, p.h_scal, dup, p.h_scal[SW_D], s, &r));
     memcpy(c->last_scal, p.h_scal, sizeof c->last_scal);
     {
         std::lock_guard<std::mutex> g(c->mu);
         c->stats.launches += dup ? 3 : 1;
     }
-    if (p.h_scal[SW_FAIL]) { *failed = true; if (r) kc_run_free(c, r); return KC_OK; }
-    *out = r;
-    return KC_OK;
-}
-
-// Key-placement path, after the extraction and S3a..S3b have drained: S3c sorts and folds every
-// sub-bucket into the level-1 buffer (dead by now), a scan gives the survivors' offsets, a gather
-// writes the run. Empty slots were placed as key 0 and are taken off that record's count.
-int count_finish_place(kc_ctx *c, Pending &p, cudaStream_t s, kc_run **out, bool *failed) {
-    *failed = false;
-    *out = nullptr;
-    const SuperPlan &pl = p.splan;
-    if (p.h_scal[SW_FAIL]) { *failed = true; return KC_OK; }
-    uint64_t *tk = nullptr;
-    uint32_t *tc = nullptr;
-    super_tmp_buffers(pl, p.ws_super, &tk, &tc);
-    KC_CUDA_TRY(c, super_finish(pl, true, p.ws_super, p.d_scal, tk, tc, c->n_sms, s));
-    KC_CUDA_TRY(c, cudaMemcpyAsync(p.h_scal, p.d_scal, SC_COUNT * 8, cudaMemcpyDeviceToHost, s));
-    KC_CUDA_TRY(c, cudaStreamSynchronize(s));
-    if (!p.h_scal[SW_FAIL] && p.h_scal[SW_BIG])
-        KC_TRY(super_finish_big(c, pl, p.ws_super, p.d_scal, true, p.h_scal[SW_BIG_RECORDS], tk, tc, s));
-    KC_CUDA_TRY(c, super_fold_offsets(pl, p.ws_super, p.d_scal, s));
-    KC_CUDA_TRY(c, cudaMemcpyAsync(p.h_scal, p.d_scal, SC_COUNT * 8, cudaMemcpyDeviceToHost, s));
-    KC_CUDA_TRY(c, cudaStreamSynchronize(s));
-    memcpy(c->last_scal, p.h_scal, sizeof c->last_scal);
-    if (p.h_scal[SW_FAIL]) { *failed = true; return KC_OK; }
-    kc_run *r = nullptr;
-    KC_TRY(make_run(c, s, p.h_scal[SW_OUT], &r));
-    if (r->n) {
-        KC_CUDA_TRY(c, super_gather(pl, p.ws_super, tk, tc, r->d_keys, r->d_counts, c->n_sms, s));
-        if (p.h_scal[SC_INVALID])
-            KC_CUDA_TRY(c, place_fix_zero(c->W, r->d_keys, r->d_counts, &p.d_scal[SC_INVALID], s));
-    }
-    {
-        std::lock_guard<std::mutex> g(c->mu);
-        c->stats.launches += 4;
-    }
-    const int rc = strict_hide_zero(c, p, r, s);
-    if (rc != KC_OK) { kc_run_free(c, r); return rc; }
-    *out = r;
+    if (!p.h_scal[SW_FAIL]) *out = std::move(r);
     return KC_OK;
 }
 
@@ -719,41 +712,53 @@ int strict_hide_zero(kc_ctx *c, Pending &p, kc_run *r, cudaStream_t s) {
     return KC_OK;
 }
 
-int count_finish_partition(kc_ctx *c, Pending &p, cudaStream_t s, kc_run **out) {
+// Key-placement path, after the extraction and S3a..S3b have drained: S3c sorts and folds every
+// sub-bucket into the level-1 buffer (dead by now), a scan gives the survivors' offsets, a gather
+// writes the run. Empty slots were placed as key 0 and are taken off that record's count.
+// h_scal[SW_FAIL] set on return: a sub-bucket arrangement the path cannot take, no run.
+int count_finish_place(kc_ctx *c, Pending &p, cudaStream_t s, RunPtr *out) {
+    if (p.h_scal[SW_FAIL]) return KC_OK;
+    RunPtr r;
+    KC_TRY(super_emit(c, p.splan, p.splan, p.ws_super, p.d_scal, p.h_scal, true, 0, s, &r));
+    memcpy(c->last_scal, p.h_scal, sizeof c->last_scal);
+    if (p.h_scal[SW_FAIL]) return KC_OK;
+    if (r->n && p.h_scal[SC_INVALID]) KC_CUDA_TRY(c, place_fix_zero(c->W, r->d_keys, r->d_counts, &p.d_scal[SC_INVALID], s));
+    {
+        std::lock_guard<std::mutex> g(c->mu);
+        c->stats.launches += 4;
+    }
+    KC_TRY(strict_hide_zero(c, p, r.get(), s));
+    *out = std::move(r);
+    return KC_OK;
+}
+
+int count_finish_partition(kc_ctx *c, Pending &p, cudaStream_t s, RunPtr *out) {
     const uint64_t U = p.h_scal[SC_UNIQUE];
     const int sig = c->W == 1 ? 64 - static_zero_bits(c) : 64;
     const int target = c->cfg.table_slots ? (int)c->cfg.table_slots : 0;
     uint32_t n_sub = 0, prefix_bits = 0;
     const uint32_t *d_off = nullptr;
     if (U) partition_plan_info(p.n_slots, sig, target, p.ws_part, &n_sub, &prefix_bits, &d_off);
-    kc_run *r = nullptr;
-    bool placed = false;
-    uint64_t *pk = nullptr;
-    uint32_t *pc = nullptr, *po = nullptr;
+    RunPtr r;
     {
         std::lock_guard<std::mutex> g(c->mu);
-        if (c->place.set) {                      // one-shot, whether it fits or not
-            placed = U > 0 && U <= c->place.cap && n_sub + 1 <= c->place.cap_ranges;
-            pk = c->place.keys; pc = c->place.counts; po = c->place.offs;
-            c->place.set = false;
+        if (c->place.set && U > 0 && U <= c->place.cap && n_sub + 1 <= c->place.cap_ranges) {
+            r = RunPtr(new kc_run(), RunFree{c});
+            r->W = c->W;
+            r->n = U;
+            r->d_keys = c->place.keys;
+            r->d_counts = c->place.counts;
+            r->d_sub_off = c->place.offs;
+            r->placed = true;
         }
+        c->place.set = false;                    // one-shot, whether it fits or not
     }
-    if (placed) {
-        r = new kc_run();
-        r->W = c->W;
-        r->n = U;
-        r->d_keys = pk;
-        r->d_counts = pc;
-        r->d_sub_off = po;
-        r->placed = true;
-    } else {
-        KC_TRY(make_run(c, s, U, &r));
-    }
+    if (!r) KC_TRY(make_run(c, s, U, &r));
     if (U) {
         KC_CUDA_TRY(c, partition_gather(c->W, p.n_slots, sig, target, p.uniq, p.counts, p.ws_part, r->d_keys, r->d_counts, s));
         r->n_sub = n_sub;
         r->prefix_bits = prefix_bits;
-        if (!placed) {
+        if (!r->placed) {
             void *mem = nullptr;
             KC_TRY(dev_alloc(c, s, (uint64_t)(n_sub + 1) * 4, &mem));
             r->d_sub_off = static_cast<uint32_t *>(mem);
@@ -762,13 +767,13 @@ int count_finish_partition(kc_ctx *c, Pending &p, cudaStream_t s, kc_run **out) 
         std::lock_guard<std::mutex> g(c->mu);
         c->stats.launches += 1;
     }
-    *out = r;
+    *out = std::move(r);
     return KC_OK;
 }
 
-int count_finish_sort(kc_ctx *c, Pending &p, cudaStream_t s, kc_run **out) {
+int count_finish_sort(kc_ctx *c, Pending &p, cudaStream_t s, RunPtr *out) {
     const uint64_t U = p.h_scal[SC_UNIQUE];
-    kc_run *r = nullptr;
+    RunPtr r;
     KC_TRY(make_run(c, s, U, &r));
     if (U) {
         KC_CUDA_TRY(c, cudaMemcpyAsync(r->d_keys, p.uniq, U * c->W * 8, cudaMemcpyDeviceToDevice, s));
@@ -777,36 +782,45 @@ int count_finish_sort(kc_ctx *c, Pending &p, cudaStream_t s, kc_run **out) {
         c->stats.launches += 1;
     }
     // strict mode: empty slots were sorted in as key 0; if nothing real is left there, hide that record
-    const int rc = strict_hide_zero(c, p, r, s);
-    if (rc != KC_OK) { kc_run_free(c, r); return rc; }
-    *out = r;
+    KC_TRY(strict_hide_zero(c, p, r.get(), s));
+    *out = std::move(r);
     return KC_OK;
 }
 
-int count_finish_hash_global(kc_ctx *c, Pending &p, cudaStream_t s, kc_run **out) {
+int count_finish_hash_global(kc_ctx *c, Pending &p, cudaStream_t s, RunPtr *out) {
     const uint64_t U = p.h_scal[SC_SIDE + 3] + (p.h_scal[SC_SIDE + 0] ? 1 : 0);
-    kc_run *ra = nullptr, *rb = nullptr;
+    RunPtr ra, rb;
     KC_TRY(make_run(c, s, U, &ra));
-    int rc = make_run(c, s, U, &rb);
-    if (rc != KC_OK) { kc_run_free(c, ra); return rc; }
+    KC_TRY(make_run(c, s, U, &rb));
     int launches = 0;
     KC_CUDA_TRY(c, hash_compact(p.table, ra->d_keys, ra->d_counts, &p.d_scal[SC_HASHNUM], s, &launches));
     const uint64_t ws_bytes = sort_workspace_bytes(U, 1);
-    void *ws = nullptr;
-    KC_TRY(dev_alloc(c, s, ws_bytes, &ws));
+    DevBuf ws(s);
+    KC_TRY(ws.alloc(c, ws_bytes));
     uint64_t *sk = nullptr;
     uint32_t *sv = nullptr;
     KC_CUDA_TRY(c, radix_sort(ra->d_keys, rb->d_keys, ra->d_counts, rb->d_counts, U, 1, static_zero_bits(c),
-                              SortWorkspace{ws, ws_bytes}, s, &sk, &sv, &launches, nullptr, nullptr));
-    dev_free(s, ws);
-    kc_run *keep = (sk == ra->d_keys) ? ra : rb, *drop = (keep == ra) ? rb : ra;
-    kc_run_free(c, drop);
+                              SortWorkspace{ws.get(), ws_bytes}, s, &sk, &sv, &launches, nullptr, nullptr));
     {
         std::lock_guard<std::mutex> g(c->mu);
         c->stats.launches += launches;
     }
-    *out = keep;
+    *out = std::move(sk == ra->d_keys ? ra : rb);   // (the workspace, then the other run, go at the return)
     return KC_OK;
+}
+
+// The run of a drained chunk, built by the path it was counted by; none (and KC_OK) if that path
+// could not take the chunk.
+int count_finish_method(kc_ctx *c, Pending &p, cudaStream_t s, RunPtr *out) {
+    if (p.n_slots == 0) return make_run(c, s, 0, out);
+    const bool table_full = p.h_scal[SC_SIDE + 1] != 0;
+    switch (p.method) {
+    case KC_COUNT_SUPER: return count_finish_super(c, p, s, out);
+    case KC_COUNT_PLACE: return count_finish_place(c, p, s, out);
+    case KC_COUNT_HASH: return table_full ? KC_OK : count_finish_partition(c, p, s, out);
+    case KC_COUNT_HASH_GLOBAL: return table_full ? KC_OK : count_finish_hash_global(c, p, s, out);
+    default: return count_finish_sort(c, p, s, out);
+    }
 }
 
 int check_ctx(const kc_ctx *c) { return c ? KC_OK : KC_ERR_ARG; }
@@ -849,6 +863,7 @@ int kc_create(const kc_config *cfg, kc_ctx **out) {
     if (c0.flags & KC_CANONICAL) c->cfg.flags |= KC_COMPAT_STRICT;
     c->strict = (c->cfg.flags & KC_COMPAT_STRICT) != 0;
     c->key_flags = c->cfg.flags & (KC_COMPAT_STRICT | KC_CANONICAL);
+    if (const char *v = getenv("KC_TEST_FAIL_ALLOC")) c->fail_alloc_at = strtoull(v, nullptr, 10);
     cudaDeviceGetAttribute(&c->n_sms, cudaDevAttrMultiProcessorCount, c0.device);
     if (c->n_sms <= 0) c->n_sms = 148;
     // keep freed blocks in the stream-ordered pool: chunk after chunk reuses the same arena
@@ -965,28 +980,18 @@ void accum_free(kc_ctx *c) {
     if (a.h_sc) cudaFreeHost(a.h_sc);
     for (auto &e : a.ev) if (e) cudaEventDestroy(e);
     for (auto &e : a.sc_ev) if (e) cudaEventDestroy(e);
-    for (kc_run *r : a.parts) kc_run_free(c, r);
-    a = kc_ctx::Accum();
+    a = kc_ctx::Accum();                     // (frees the parts)
 }
 
 // Counts what the bins hold into one run (S2 .. S3c) and empties them. All slot streams are
-// drained first. An empty accumulator gives an empty run.
-int accum_finish(kc_ctx *c, bool force_dup, kc_run **out, kc_run *pre_run = nullptr, bool dup_known = false);
+// drained first. An empty accumulator gives an empty run. *run: the run already allocated, if
+// any (its arrays were the second record buffer); dup_known: force_dup is the decision; ext_e:
+// see super_emit.
+int accum_finish(kc_ctx *c, bool force_dup, RunPtr *run, bool dup_known = false, DevBuf *ext_e = nullptr);
 
-// non-exchange accumulators keep the second record buffer (E) outside the workspace: this undoes
-// what accum_count attached for one flush
-void accum_detach_e(kc_ctx *c, cudaStream_t s, kc_run *pre_run) {
-    kc_ctx::Accum &a = c->acc;
-    if (!a.pl.ext_e) return;
-    if (!pre_run) { dev_free(s, a.pl.ext_ek); dev_free(s, a.pl.ext_ec); }
-    a.pl.ext_ek = nullptr;
-    a.pl.ext_ec = nullptr;
-}
-
-int accum_count(kc_ctx *c, kc_run **out) {
+int accum_count(kc_ctx *c, RunPtr *out) {
     kc_ctx::Accum &a = c->acc;
     cudaStream_t s = c->stream;
-    *out = nullptr;
     for (auto &sl : c->slots)
         if (sl.stream) KC_CUDA_TRY(c, cudaStreamSynchronize(sl.stream));
     if (a.fresh) return make_run(c, s, 0, out);
@@ -998,7 +1003,7 @@ int accum_count(kc_ctx *c, kc_run **out) {
         return accum_finish(c, false, out);
     }
     // S2 first: once the number of distinct records is known the run is allocated with exactly that
-    // size and serves as the second record buffer of S3a/S3b before S3c sorts the records into it
+    // size and serves as the second record buffer (E) of S3a/S3b before S3c sorts the records into it
     KC_CUDA_TRY(c, super_count_bins(a.pl, !c->strict, a.ws, a.d_sc, c->n_sms, s));
     KC_CUDA_TRY(c, cudaEventRecord(a.ev[1], s));
     KC_CUDA_TRY(c, cudaMemcpyAsync(a.h_sc, a.d_sc, SC_COUNT * 8, cudaMemcpyDeviceToHost, s));
@@ -1010,43 +1015,35 @@ int accum_count(kc_ctx *c, kc_run **out) {
     const uint64_t n_d = a.h_sc[SW_D];
     const bool env_dup = env_force_dup();
     const bool dup = env_dup || a.h_sc[SW_OVF] != 0;
-    kc_run *pre = nullptr;
+    DevBuf e[2] = {DevBuf(s), DevBuf(s)};          // if records may repeat, E is this flush's own allocation
     if (!dup) {
-        KC_TRY(make_run(c, s, n_d, &pre));
-        a.pl.ext_ek = pre->d_keys;
-        a.pl.ext_ec = pre->d_counts;
+        KC_TRY(make_run(c, s, n_d, out));
+        a.pl.ext_ek = (*out)->d_keys;
+        a.pl.ext_ec = (*out)->d_counts;
     } else {
-        void *m = nullptr;
-        KC_TRY(dev_alloc(c, s, n_d * c->W * 8 + 64, &m));
-        a.pl.ext_ek = static_cast<uint64_t *>(m);
-        const int rc = dev_alloc(c, s, n_d * 4 + 64, &m);
-        if (rc != KC_OK) { dev_free(s, a.pl.ext_ek); a.pl.ext_ek = nullptr; return rc; }
-        a.pl.ext_ec = static_cast<uint32_t *>(m);
+        KC_TRY(e[0].alloc(c, n_d * c->W * 8 + 64));
+        KC_TRY(e[1].alloc(c, n_d * 4 + 64));
+        a.pl.ext_ek = e[0].get<uint64_t>();
+        a.pl.ext_ec = e[1].get<uint32_t>();
     }
-    cudaError_t e = super_place(a.pl, a.ws, a.d_sc, c->n_sms, s, &a.ev[2]);
-    if (e != cudaSuccess) {
-        accum_detach_e(c, s, pre);
-        if (pre) kc_run_free(c, pre);
-        return c->set_error(KC_ERR_CUDA, "super_place: %s", cudaGetErrorString(e));
+    const cudaError_t err = super_place(a.pl, a.ws, a.d_sc, c->n_sms, s, &a.ev[2]);
+    int rc = err == cudaSuccess ? KC_OK : c->set_error(KC_ERR_CUDA, "super_place: %s", cudaGetErrorString(err));
+    if (rc == KC_OK) {
+        if (tr.on) { cudaStreamSynchronize(s); tr.mark("flush: alloc + S3a/H2/S3b"); }
+        rc = accum_finish(c, dup, out, true, dup ? e : nullptr);
+        tr.mark("flush: S3c + emit + reset");
+        if (tr.on) fprintf(stderr, "kc trace: records D %llu, overflow %llu, big ranges %llu (%llu records), aborts %llu, dup %d\n",
+                           (unsigned long long)c->last_scal[SW_D], (unsigned long long)c->last_scal[SW_OVF], (unsigned long long)c->last_scal[SW_BIG],
+                           (unsigned long long)c->last_scal[SW_BIG_RECORDS], (unsigned long long)c->last_scal[SW_ABORTS], (int)dup);
     }
-    if (tr.on) { cudaStreamSynchronize(s); tr.mark("flush: alloc + S3a/H2/S3b"); }
-    const int rc = accum_finish(c, dup, out, pre, true);
-    tr.mark("flush: S3c + emit + reset");
-    if (tr.on) fprintf(stderr, "kc trace: records D %llu, overflow %llu, big ranges %llu (%llu records), aborts %llu, dup %d\n",
-                       (unsigned long long)c->last_scal[SW_D], (unsigned long long)c->last_scal[SW_OVF], (unsigned long long)c->last_scal[SW_BIG],
-                       (unsigned long long)c->last_scal[SW_BIG_RECORDS], (unsigned long long)c->last_scal[SW_ABORTS], (int)dup);
-    accum_detach_e(c, s, pre);
-    if (rc != KC_OK && pre) kc_run_free(c, pre);
+    a.pl.ext_ek = nullptr;                         // E is attached for this flush only
+    a.pl.ext_ec = nullptr;
     return rc;
 }
 
-// The sub-buckets are in place (S3b done or queued on the context's stream): sort them into a run
-// (folding equal keys if records may repeat), account, empty the bins. pre_run: the run, already
-// allocated (its arrays were the second record buffer); dup_known: force_dup is the decision.
-int accum_finish(kc_ctx *c, bool force_dup, kc_run **out, kc_run *pre_run, bool dup_known) {
+int accum_finish(kc_ctx *c, bool force_dup, RunPtr *run, bool dup_known, DevBuf *ext_e) {
     kc_ctx::Accum &a = c->acc;
     cudaStream_t s = c->stream;
-    *out = nullptr;
     KC_CUDA_TRY(c, cudaMemcpyAsync(a.h_sc, a.d_sc, SC_COUNT * 8, cudaMemcpyDeviceToHost, s));
     KC_CUDA_TRY(c, cudaStreamSynchronize(s));
     if (a.h_sc[SW_FAIL])
@@ -1058,64 +1055,20 @@ int accum_finish(kc_ctx *c, bool force_dup, kc_run **out, kc_run *pre_run, bool 
     const bool env_dup = env_force_dup();
     const bool dup = dup_known ? force_dup
                                : (env_dup || (a.xchg ? (force_dup && a.x_info.any_ovf != 0) : (force_dup || a.h_sc[SW_OVF] != 0)));
-    kc_run *r = pre_run;
     SuperPlan fpl = a.pl;                                   // exchange: the S3c variant is the device plan's choice
     if (a.xchg && a.x_info.fin_large) super_use_large_finish(&fpl);
-    if (!dup) {
-        if (!r) KC_TRY(make_run(c, s, n_d, &r));
-        if (n_d) KC_CUDA_TRY(c, super_finish(fpl, false, a.ws, a.d_sc, r->d_keys, r->d_counts, c->n_sms, s));
-        KC_CUDA_TRY(c, cudaMemcpyAsync(a.h_sc, a.d_sc, SC_COUNT * 8, cudaMemcpyDeviceToHost, s));
-        KC_CUDA_TRY(c, cudaStreamSynchronize(s));
-        if (!a.h_sc[SW_FAIL] && a.h_sc[SW_BIG]) {
-            const int rc = super_finish_big(c, a.pl, a.ws, a.d_sc, false, a.h_sc[SW_BIG_RECORDS], r->d_keys, r->d_counts, s);
-            if (rc != KC_OK) { if (!pre_run) kc_run_free(c, r); return rc; }
-        }
-        KC_CUDA_TRY(c, cudaEventRecord(a.ev[5], s));
-        KC_CUDA_TRY(c, cudaStreamSynchronize(s));
-    } else {
-        uint64_t *tk = nullptr;
-        uint32_t *tc = nullptr;
-        super_tmp_buffers(a.pl, a.ws, &tk, &tc);
-        KC_CUDA_TRY(c, super_finish(fpl, true, a.ws, a.d_sc, tk, tc, c->n_sms, s));
-        KC_CUDA_TRY(c, cudaMemcpyAsync(a.h_sc, a.d_sc, SC_COUNT * 8, cudaMemcpyDeviceToHost, s));
-        KC_CUDA_TRY(c, cudaStreamSynchronize(s));
-        if (!a.h_sc[SW_FAIL] && a.h_sc[SW_BIG])
-            KC_TRY(super_finish_big(c, a.pl, a.ws, a.d_sc, true, a.h_sc[SW_BIG_RECORDS], tk, tc, s));
-        KC_CUDA_TRY(c, super_fold_offsets(a.pl, a.ws, a.d_sc, s));
-        KC_CUDA_TRY(c, cudaMemcpyAsync(a.h_sc, a.d_sc, SC_COUNT * 8, cudaMemcpyDeviceToHost, s));
-        KC_CUDA_TRY(c, cudaStreamSynchronize(s));
-        if (!a.h_sc[SW_FAIL]) {
-            const uint64_t n_out = a.h_sc[SW_OUT];
-            if (a.pl.ext_e) {
-                // the temporary is this flush's own allocation: close the gaps into D (dead by now), give the
-                // temporary back, then allocate the run -- the flush never holds both next to the workspace
-                uint64_t *dk = reinterpret_cast<uint64_t *>(static_cast<uint8_t *>(a.ws) + a.pl.off_dk);
-                uint32_t *dc = reinterpret_cast<uint32_t *>(static_cast<uint8_t *>(a.ws) + a.pl.off_dc);
-                if (n_out) KC_CUDA_TRY(c, super_gather(a.pl, a.ws, tk, tc, dk, dc, c->n_sms, s));
-                accum_detach_e(c, s, nullptr);
-                KC_TRY(make_run(c, s, n_out, &r));
-                if (n_out) {
-                    KC_CUDA_TRY(c, cudaMemcpyAsync(r->d_keys, dk, n_out * c->W * 8, cudaMemcpyDeviceToDevice, s));
-                    KC_CUDA_TRY(c, cudaMemcpyAsync(r->d_counts, dc, n_out * 4, cudaMemcpyDeviceToDevice, s));
-                }
-            } else {
-                KC_TRY(make_run(c, s, n_out, &r));
-                if (r->n) KC_CUDA_TRY(c, super_gather(a.pl, a.ws, tk, tc, r->d_keys, r->d_counts, c->n_sms, s));
-            }
-        }
-        KC_CUDA_TRY(c, cudaEventRecord(a.ev[5], s));
-        KC_CUDA_TRY(c, cudaStreamSynchronize(s));
-    }
-    if (a.h_sc[SW_FAIL]) {
-        if (r && r != pre_run) kc_run_free(c, r);
+    KC_TRY(super_emit(c, a.pl, fpl, a.ws, a.d_sc, a.h_sc, dup, n_d, s, run, ext_e));
+    KC_CUDA_TRY(c, cudaEventRecord(a.ev[5], s));
+    KC_CUDA_TRY(c, cudaStreamSynchronize(s));
+    if (a.h_sc[SW_FAIL])
         return c->set_error(KC_ERR_CAPACITY, "a key range of the accumulated input does not fit shared memory (fail bits %llu)",
                             (unsigned long long)a.h_sc[SW_FAIL]);
-    }
+    const uint64_t U = (*run)->n;
     {
         std::lock_guard<std::mutex> g(c->mu);
         kc_stats &st = c->stats;
         memcpy(c->last_scal, a.h_sc, sizeof c->last_scal);
-        const uint64_t U = r->n, Kb = 8ull * c->W, ub = U * (Kb + 4), rec = a.h_sc[SW_RECORDS] * 16ull * c->W;
+        const uint64_t Kb = 8ull * c->W, ub = U * (Kb + 4), rec = a.h_sc[SW_RECORDS] * 16ull * c->W;
         st.chunks++;
         st.kmer_slots += a.windows;
         st.kmers_valid += a.windows - a.h_sc[SW_INVALID];
@@ -1123,41 +1076,28 @@ int accum_finish(kc_ctx *c, bool force_dup, kc_run **out, kc_run *pre_run, bool 
         st.distinct_last = U;
         st.method_used = KC_COUNT_SUPER;
         st.launches += dup ? 11 : 9;
-        st.n_stages = 6;
-        for (int i = 0; i < 8; i++) { st.ms_stage[i] = 0; st.stage_bytes[i] = 0; st.stage_launches[i] = 0; }
+        float ms[8] = {0};
         a.ms_scatter = 0;                                    // summed over the chunks' S1 launches (all complete by now)
         for (uint64_t i = 0; i < a.n_scatter; i++) {
-            float ms = 0;
-            if (cudaEventElapsedTime(&ms, a.sc_ev[2 * i], a.sc_ev[2 * i + 1]) == cudaSuccess) a.ms_scatter += ms;
+            float t = 0;
+            if (cudaEventElapsedTime(&t, a.sc_ev[2 * i], a.sc_ev[2 * i + 1]) == cudaSuccess) a.ms_scatter += t;
         }
         cudaGetLastError();
-        st.ms_stage[0] = a.ms_scatter;
-        for (int i = 1; i < 6; i++) cudaEventElapsedTime(&st.ms_stage[i], a.ev[i - 1], a.ev[i]);
+        ms[0] = a.ms_scatter;
+        for (int i = 1; i < 6; i++) cudaEventElapsedTime(&ms[i], a.ev[i - 1], a.ev[i]);
         st.ms_total = 0;
-        for (int i = 0; i < 6; i++) st.ms_total += st.ms_stage[i];
-        st.stage_bytes[0] = a.reads * c->cfg.read_len + rec;   st.stage_launches[0] = (uint32_t)a.n_scatter;
-        st.stage_bytes[1] = rec + ub;                           st.stage_launches[1] = 1;
-        st.stage_bytes[2] = 2 * ub;                             st.stage_launches[2] = 1;
-        st.stage_bytes[3] = U * Kb;                             st.stage_launches[3] = 1;
-        st.stage_bytes[4] = 2 * ub;                             st.stage_launches[4] = 1;
-        st.stage_bytes[5] = 2 * ub;                             st.stage_launches[5] = 1;
-        int dom = 0;
-        for (int i = 1; i < 6; i++) if (st.ms_stage[i] > st.ms_stage[dom]) dom = i;
-        st.dominant_stage = (uint32_t)dom;
-        st.ms_dominant = st.ms_stage[dom];
-        st.dominant_bytes = st.stage_bytes[dom];
-        st.dominant_launches = st.stage_launches[dom] ? st.stage_launches[dom] : 1;
-        st.ms_extract = st.ms_stage[0];
-        st.ms_emit = st.ms_stage[5];
-        st.ms_count = st.ms_total - st.ms_extract - st.ms_emit;
+        for (int i = 0; i < 6; i++) st.ms_total += ms[i];
+        const uint64_t b[8] = {a.reads * c->cfg.read_len + rec, rec + ub, 2 * ub, U * Kb, 2 * ub, 2 * ub};
+        const uint32_t l[8] = {(uint32_t)a.n_scatter, 1, 1, 1, 1, 1};
+        stage_stats(st, 6, ms, b, l, 6);
     }
     // Bins sized for the wrong redundancy cost S2 a second and third pass over most bins (too many
     // distinct keys for the table) or many nearly empty units. Now that the bins are empty and the
     // ratio is known, later flushes of this accumulator get bins of the right size (same workspace
     // if it fits, a larger one otherwise). Not with an explicit table_slots, not in exchange mode
     // (the ranks must plan alike).
-    if (!a.xchg && c->cfg.table_slots == 0 && a.windows > (1u << 20) && r && r->n) {
-        const double per_key = (double)a.windows / (double)r->n;
+    if (!a.xchg && c->cfg.table_slots == 0 && a.windows > (1u << 20) && U) {
+        const double per_key = (double)a.windows / (double)U;
         double occ = 2200.0 * per_key;
         occ = occ > 8192.0 ? 8192.0 : (occ < 1024.0 ? 1024.0 : occ);
         const uint32_t want = ((uint32_t)occ + 255u) & ~255u;
@@ -1175,7 +1115,7 @@ int accum_finish(kc_ctx *c, bool force_dup, kc_run **out, kc_run *pre_run, bool 
                     if (cudaMalloc(&nw, np.ws_bytes) != cudaSuccess) {
                         cudaGetLastError();
                         ok = cudaMalloc(&nw, a.pl.ws_bytes) == cudaSuccess;      // back to the old plan
-                        if (!ok) { kc_run_free(c, r); return c->set_error(KC_ERR_NOMEM, "accumulator workspace of %llu bytes", (unsigned long long)a.pl.ws_bytes); }
+                        if (!ok) return c->set_error(KC_ERR_NOMEM, "accumulator workspace of %llu bytes", (unsigned long long)a.pl.ws_bytes);
                         a.ws = nw;
                         a.ws_bytes = a.pl.ws_bytes;
                         ok = false;
@@ -1197,7 +1137,6 @@ int accum_finish(kc_ctx *c, bool force_dup, kc_run **out, kc_run *pre_run, bool 
     a.ovf_reserved = 0;
     a.ms_scatter = 0;
     a.n_scatter = 0;
-    *out = r;
     return KC_OK;
 }
 
@@ -1211,9 +1150,9 @@ int accum_make_room(kc_ctx *c, uint64_t n_reads) {
         return c->set_error(KC_ERR_CAPACITY, "chunk of %llu reads exceeds what the accumulator was planned for", (unsigned long long)n_reads);
     if (a.windows + w > a.max_windows) {
         if (a.xchg) return c->set_error(KC_ERR_CAPACITY, "more reads than kc_xchg_begin planned for (%llu k-mer slots)", (unsigned long long)a.max_windows);
-        kc_run *part = nullptr;
+        RunPtr part;
         KC_TRY(accum_count(c, &part));
-        a.parts.push_back(part);
+        a.parts.push_back(std::move(part));
     }
     return KC_OK;
 }
@@ -1380,17 +1319,16 @@ int kc_accum_flush(kc_ctx *c, kc_run **run) {
     if (!run) return c->set_error(KC_ERR_ARG, "null run");
     std::lock_guard<std::recursive_mutex> dg(c->direct_mu);
     if (!c->acc.on) return c->set_error(KC_ERR_STATE, "kc_accum_begin first");
+    *run = nullptr;
     cudaSetDevice(c->cfg.device);
     kc_ctx::Accum &a = c->acc;
-    kc_run *last = nullptr;
+    RunPtr last;
     KC_TRY(accum_count(c, &last));
-    if (a.parts.empty()) { *run = last; return KC_OK; }
-    a.parts.push_back(last);
-    std::vector<kc_run *> parts;
+    if (a.parts.empty()) { *run = last.release(); return KC_OK; }
+    std::vector<RunPtr> parts;
     parts.swap(a.parts);
-    const int rc = kc_merge_runs(c, parts.data(), (uint32_t)parts.size(), run);
-    for (kc_run *p : parts) kc_run_free(c, p);
-    return rc;
+    parts.push_back(std::move(last));
+    return merge_owned(c, parts, run);
 }
 
 // ------------------------------------------------------------------- multi-GPU
@@ -1514,9 +1452,13 @@ int kc_xchg_finish(kc_ctx *c, kc_run **run) {
     std::lock_guard<std::recursive_mutex> dg(c->direct_mu);
     if (!c->acc.xchg) return c->set_error(KC_ERR_STATE, "kc_xchg_begin first");
     cudaSetDevice(c->cfg.device);
+    *run = nullptr;
     KC_CUDA_TRY(c, cudaMemcpyAsync(&c->acc.x_info, super_x_info(c->acc.pl, c->acc.ws), sizeof(SuperXInfo),
                                    cudaMemcpyDeviceToHost, c->stream));
-    return accum_finish(c, true, run);        // (synchronises the stream)
+    RunPtr r;
+    KC_TRY(accum_finish(c, true, &r));        // (synchronises the stream)
+    *run = r.release();
+    return KC_OK;
 }
 
 int kc_xchg_fix_ranges(kc_ctx *c, int on) {
@@ -1585,11 +1527,15 @@ int kc_xchg_run_all(kc_ctx *const *ctxs, uint32_t n, kc_run **runs) {
     if (rc == KC_OK) barrier();                     // every rank's grouped array and sub-bucket counts are final
     for (uint32_t r = 0; r < n && rc == KC_OK; r++) rc = kc_xchg_pull(ctxs[r]);
     if (rc == KC_OK) barrier();                     // nobody reads a peer's grouped array any more
-    for (uint32_t r = 0; r < n && rc == KC_OK; r++) rc = kc_xchg_finish(ctxs[r], &runs[r]);
+    std::vector<RunPtr> got;
+    for (uint32_t r = 0; r < n && rc == KC_OK; r++) {
+        kc_run *run = nullptr;
+        rc = kc_xchg_finish(ctxs[r], &run);
+        got.emplace_back(run, RunFree{ctxs[r]});
+    }
     for (uint32_t r = 0; r < n; r++) { cudaSetDevice(ctxs[r]->cfg.device); cudaEventDestroy(ev[r]); }
-    if (rc != KC_OK)
-        for (uint32_t r = 0; r < n; r++)
-            if (runs[r]) { kc_run_free(ctxs[r], runs[r]); runs[r] = nullptr; }
+    if (rc == KC_OK)
+        for (uint32_t r = 0; r < n; r++) runs[r] = got[r].release();
     return rc;
 }
 
@@ -1602,6 +1548,7 @@ int kc_count_device(kc_ctx *c, const void *d_reads, uint64_t n_bytes, kc_run **r
     KC_TRY(check_ctx(c));
     std::lock_guard<std::recursive_mutex> dg(c->direct_mu);
     if (!run) return c->set_error(KC_ERR_ARG, "null run");
+    *run = nullptr;
     if (n_bytes && (!d_reads || (reinterpret_cast<uintptr_t>(d_reads) & 15)))
         return c->set_error(KC_ERR_ARG, "d_reads must be a 16-byte aligned device pointer");
     cudaSetDevice(c->cfg.device);
@@ -1611,23 +1558,17 @@ int kc_count_device(kc_ctx *c, const void *d_reads, uint64_t n_bytes, kc_run **r
     uint64_t n_reads = n_bytes / L;
     uint64_t max_reads = kMaxSortKeys / nk;
     max_reads -= max_reads % 16;                      // keep every piece 16-byte aligned
-    if (n_reads <= max_reads) {
-        KC_TRY(count_enqueue(c, c->direct, d_reads, n_bytes, c->stream, pick_method(c)));
-        return count_finish(c, c->direct, d_reads, n_bytes, c->stream, run);
-    }
-    std::vector<kc_run *> parts;
-    int rc = KC_OK;
-    for (uint64_t r0 = 0; r0 < n_reads && rc == KC_OK; r0 += max_reads) {
-        uint64_t nr = n_reads - r0 < max_reads ? n_reads - r0 : max_reads;
+    std::vector<RunPtr> parts;
+    for (uint64_t r0 = 0; r0 == 0 || r0 < n_reads; r0 += max_reads) {   // (an empty chunk is one piece too)
+        const uint64_t nr = std::min(max_reads, n_reads - r0);
         const uint8_t *ptr = static_cast<const uint8_t *>(d_reads) + r0 * L;
         kc_run *part = nullptr;
-        rc = count_enqueue(c, c->direct, ptr, nr * L, c->stream, pick_method(c));
-        if (rc == KC_OK) rc = count_finish(c, c->direct, ptr, nr * L, c->stream, &part);
-        if (rc == KC_OK) parts.push_back(part);
+        KC_TRY(count_enqueue(c, c->direct, ptr, nr * L, c->stream, pick_method(c)));
+        KC_TRY(count_finish(c, c->direct, ptr, nr * L, c->stream, &part));
+        parts.emplace_back(part, RunFree{c});
     }
-    if (rc == KC_OK) rc = kc_merge_runs(c, parts.data(), (uint32_t)parts.size(), run);
-    for (auto *p : parts) kc_run_free(c, p);
-    return rc;
+    if (parts.size() == 1) { *run = parts[0].release(); return KC_OK; }
+    return merge_owned(c, parts, run);
 }
 
 static int parse_fastq_impl(kc_ctx *c, Pending &ar, const void *d_text, uint64_t n_bytes, void *d_reads,
@@ -1763,17 +1704,14 @@ int kc_process_chunk(kc_ctx *c, uint32_t slot, const char *reads, uint64_t n_byt
     if (slot >= c->slots.size() || !c->slots[slot].d_in) return c->set_error(KC_ERR_ARG, "slot %u not available", slot);
     if (n_bytes && !reads) return c->set_error(KC_ERR_ARG, "null reads");
     KC_TRY(submit_from(c, slot, reads, n_bytes));
-    kc_run *run = nullptr;
-    KC_TRY(kc_wait(c, slot, &run));
-    int rc = KC_OK;
+    kc_run *h = nullptr;
+    KC_TRY(kc_wait(c, slot, &h));
+    const RunPtr run(h, RunFree{c});
     uint64_t nb = (run->n - run->skip) * (uint64_t)c->S;
     if (out_bytes) *out_bytes = nb;
-    if (records) {
-        if (nb > records_cap) rc = c->set_error(KC_ERR_CAPACITY, "run needs %llu bytes, buffer holds %llu", (unsigned long long)nb, (unsigned long long)records_cap);
-        else rc = kc_run_copy_records(c, run, records, records_cap, out_bytes);
-    }
-    kc_run_free(c, run);
-    return rc;
+    if (!records) return KC_OK;
+    if (nb > records_cap) return c->set_error(KC_ERR_CAPACITY, "run needs %llu bytes, buffer holds %llu", (unsigned long long)nb, (unsigned long long)records_cap);
+    return kc_run_copy_records(c, run.get(), records, records_cap, out_bytes);
 }
 
 // -------------------------------------------------------------------------- runs
@@ -1864,6 +1802,7 @@ int kc_merge_parts(kc_ctx *c, uint32_t n_src, const void *const *d_keys, const v
     std::lock_guard<std::recursive_mutex> dg(c->direct_mu);
     if (!out || n_src == 0 || n_src > 8 || !d_keys || !d_counts || !d_offsets || !n_records || n_sub == 0)
         return c->set_error(KC_ERR_ARG, "kc_merge_parts: bad argument");
+    *out = nullptr;
     if (c->W != 1) return c->set_error(KC_ERR_ARG, "kc_merge_parts: 64-bit keys only");
     cudaSetDevice(c->cfg.device);
     cudaStream_t s = c->stream;
@@ -1890,33 +1829,26 @@ int kc_merge_parts(kc_ctx *c, uint32_t n_src, const void *const *d_keys, const v
     unsigned long long h[2] = {0, 0};
     KC_CUDA_TRY(c, cudaMemcpyAsync(h, d_sc, 16, cudaMemcpyDeviceToHost, s));
     KC_CUDA_TRY(c, cudaStreamSynchronize(s));
-    int rc = KC_OK;
-    kc_run *r = nullptr;
     double t1 = dbg ? now() : 0;
-    if (h[1]) rc = c->set_error(KC_ERR_CAPACITY, "kc_merge_parts: a key range could not be combined in shared memory");
-    if (rc == KC_OK) rc = make_run(c, s, h[0], &r);
+    if (h[1]) return c->set_error(KC_ERR_CAPACITY, "kc_merge_parts: a key range could not be combined in shared memory");
+    RunPtr r;
+    KC_TRY(make_run(c, s, h[0], &r));
     double t2 = dbg ? now() : 0;
-    if (rc == KC_OK) {
-        void *mem = nullptr;
-        rc = dev_alloc(c, s, (uint64_t)(n_sub + 1) * 4, &mem);
-        if (rc == KC_OK) {
-            r->d_sub_off = static_cast<uint32_t *>(mem);
-            r->n_sub = n_sub;
-            r->prefix_bits = prefix_bits;
-            cudaError_t e = merge_parts_gather(n_sub, static_cast<uint64_t *>(tk), static_cast<uint32_t *>(tc), ws,
-                                               r->d_keys, r->d_counts, r->d_sub_off, s);
-            if (e == cudaSuccess) e = cudaStreamSynchronize(s);
-            if (e != cudaSuccess) rc = c->set_error(KC_ERR_CUDA, "kc_merge_parts: %s", cudaGetErrorString(e));
-        }
-    }
+    void *mem = nullptr;
+    KC_TRY(dev_alloc(c, s, (uint64_t)(n_sub + 1) * 4, &mem));
+    r->d_sub_off = static_cast<uint32_t *>(mem);
+    r->n_sub = n_sub;
+    r->prefix_bits = prefix_bits;
+    KC_CUDA_TRY(c, merge_parts_gather(n_sub, static_cast<uint64_t *>(tk), static_cast<uint32_t *>(tc), ws, r->d_keys,
+                                      r->d_counts, r->d_sub_off, s));
+    KC_CUDA_TRY(c, cudaStreamSynchronize(s));
     ar.arena_used = 0;
     if (dbg) fprintf(stderr, "kc_merge_parts: count %.2f ms, alloc %.2f ms, gather %.2f ms\n", t1 - t0, t2 - t1, now() - t2);
-    if (rc != KC_OK) { if (r) kc_run_free(c, r); return rc; }
     {
         std::lock_guard<std::mutex> g(c->mu);
         c->stats.launches += launches + 1;
     }
-    *out = r;
+    *out = r.release();
     return KC_OK;
 }
 
@@ -1971,29 +1903,19 @@ int kc_run_print(kc_ctx *c, const kc_run *r, char *dst, uint64_t cap, uint64_t *
     const uint64_t n = r->n - r->skip;
     if (out_bytes) *out_bytes = 0;
     if (n == 0) return KC_OK;
-    void *text = nullptr, *ws = nullptr, *d_bytes = nullptr;
-    int rc = dev_alloc(c, s, print_max_bytes(n, r->W), &text);
-    if (rc == KC_OK) rc = dev_alloc(c, s, print_workspace_bytes(n), &ws);
-    if (rc == KC_OK) rc = dev_alloc(c, s, 8, &d_bytes);
+    DevBuf text(s), ws(s), d_bytes(s);
+    KC_TRY(text.alloc(c, print_max_bytes(n, r->W)));
+    KC_TRY(ws.alloc(c, print_workspace_bytes(n)));
+    KC_TRY(d_bytes.alloc(c, 8));
     unsigned long long total = 0;
-    cudaError_t e = cudaSuccess;
-    if (rc == KC_OK) {
-        e = print_records_text(r->d_keys + r->skip * r->W, r->d_counts + r->skip, n, r->W, static_cast<char *>(text),
-                               static_cast<unsigned long long *>(d_bytes), ws, s);
-        if (e == cudaSuccess) e = cudaMemcpyAsync(&total, d_bytes, 8, cudaMemcpyDeviceToHost, s);
-        if (e == cudaSuccess) e = cudaStreamSynchronize(s);
-        if (e == cudaSuccess) {
-            if (out_bytes) *out_bytes = total;
-            if (total > cap || !dst) rc = c->set_error(KC_ERR_CAPACITY, "the text needs %llu bytes, buffer holds %llu", total, (unsigned long long)cap);
-            else {
-                e = cudaMemcpyAsync(dst, text, total, cudaMemcpyDeviceToHost, s);
-                if (e == cudaSuccess) e = cudaStreamSynchronize(s);
-            }
-        }
-    }
-    dev_free(s, text); dev_free(s, ws); dev_free(s, d_bytes);
-    if (rc != KC_OK) return rc;
-    if (e != cudaSuccess) return c->set_error(KC_ERR_CUDA, "kc_run_print: %s", cudaGetErrorString(e));
+    KC_CUDA_TRY(c, print_records_text(r->d_keys + r->skip * r->W, r->d_counts + r->skip, n, r->W, text.get<char>(),
+                                      d_bytes.get<unsigned long long>(), ws.get(), s));
+    KC_CUDA_TRY(c, cudaMemcpyAsync(&total, d_bytes.get(), 8, cudaMemcpyDeviceToHost, s));
+    KC_CUDA_TRY(c, cudaStreamSynchronize(s));
+    if (out_bytes) *out_bytes = total;
+    if (total > cap || !dst) return c->set_error(KC_ERR_CAPACITY, "the text needs %llu bytes, buffer holds %llu", total, (unsigned long long)cap);
+    KC_CUDA_TRY(c, cudaMemcpyAsync(dst, text.get(), total, cudaMemcpyDeviceToHost, s));
+    KC_CUDA_TRY(c, cudaStreamSynchronize(s));
     std::lock_guard<std::mutex> g(c->mu);
     c->stats.launches += 1;
     c->stats.d2h_bytes += total;
@@ -2004,14 +1926,15 @@ int kc_run_from_device(kc_ctx *c, const void *d_keys, const void *d_counts, uint
     KC_TRY(check_ctx(c));
     std::lock_guard<std::recursive_mutex> dg(c->direct_mu);
     if (!out || (n && (!d_keys || !d_counts))) return c->set_error(KC_ERR_ARG, "null argument");
+    *out = nullptr;
     cudaSetDevice(c->cfg.device);
-    kc_run *r = nullptr;
+    RunPtr r;
     KC_TRY(make_run(c, c->stream, n, &r));
     if (n) {
         KC_CUDA_TRY(c, cudaMemcpyAsync(r->d_keys, d_keys, n * c->W * 8, cudaMemcpyDeviceToDevice, c->stream));
         KC_CUDA_TRY(c, cudaMemcpyAsync(r->d_counts, d_counts, n * 4, cudaMemcpyDeviceToDevice, c->stream));
     }
-    *out = r;
+    *out = r.release();
     return KC_OK;
 }
 
@@ -2019,47 +1942,34 @@ int kc_run_upload(kc_ctx *c, const void *records, uint64_t n_bytes, kc_run **out
     KC_TRY(check_ctx(c));
     std::lock_guard<std::recursive_mutex> dg(c->direct_mu);
     if (!out || (n_bytes && !records)) return c->set_error(KC_ERR_ARG, "null argument");
+    *out = nullptr;
     const uint64_t n = n_bytes / c->S;
     if (n >= (1ull << 32)) return c->set_error(KC_ERR_CAPACITY, "run too long for one upload");
     cudaSetDevice(c->cfg.device);
     cudaStream_t s = c->stream;
-    if (n == 0) return make_run(c, s, 0, out);
-    void *d_rec = nullptr, *ws = nullptr;
-    kc_run *raw = nullptr, *folded = nullptr;
-    unsigned long long *d_num = nullptr;
-    unsigned long long U = 0;
+    if (n == 0) return kc_run_from_device(c, nullptr, nullptr, 0, out);
+    DevBuf d_rec(s), ws(s), d_num(s);
+    RunPtr raw, folded;
+    KC_TRY(d_rec.alloc(c, n * c->S));
+    KC_CUDA_TRY(c, cudaMemcpyAsync(d_rec.get(), records, n * c->S, cudaMemcpyHostToDevice, s));
+    KC_TRY(make_run(c, s, n, &raw));
+    KC_TRY(make_run(c, s, n, &folded));
     int launches = 1;
-    auto body = [&]() -> int {
-        KC_TRY(dev_alloc(c, s, n * c->S, &d_rec));
-        KC_CUDA_TRY(c, cudaMemcpyAsync(d_rec, records, n * c->S, cudaMemcpyHostToDevice, s));
-        KC_TRY(make_run(c, s, n, &raw));
-        KC_TRY(make_run(c, s, n, &folded));
-        KC_CUDA_TRY(c, unpack_records(d_rec, n, c->W, raw->d_keys, raw->d_counts, s));
-        const uint64_t ws_bytes = ((rle_workspace_bytes(n) + 255) & ~255ull) + (n + 1) * 4 + 256;
-        KC_TRY(dev_alloc(c, s, ws_bytes, &ws));
-        KC_TRY(dev_alloc(c, s, 8, (void **)&d_num));
-        KC_CUDA_TRY(c, fold_sorted_pairs(raw->d_keys, raw->d_counts, n, c->W, folded->d_keys, folded->d_counts, d_num,
-                                         ws, s, &launches));
-        KC_CUDA_TRY(c, cudaMemcpyAsync(&U, d_num, 8, cudaMemcpyDeviceToHost, s));
-        KC_CUDA_TRY(c, cudaStreamSynchronize(s));
-        return KC_OK;
-    };
-    const int brc = body();
-    if (brc != KC_OK) {                                  // nothing allocated so far outlives a failed upload
-        dev_free(s, d_rec); dev_free(s, ws); dev_free(s, d_num);
-        if (raw) kc_run_free(c, raw);
-        if (folded) kc_run_free(c, folded);
-        return brc;
-    }
+    KC_CUDA_TRY(c, unpack_records(d_rec.get(), n, c->W, raw->d_keys, raw->d_counts, s));
+    KC_TRY(ws.alloc(c, ((rle_workspace_bytes(n) + 255) & ~255ull) + (n + 1) * 4 + 256));
+    KC_TRY(d_num.alloc(c, 8));
+    KC_CUDA_TRY(c, fold_sorted_pairs(raw->d_keys, raw->d_counts, n, c->W, folded->d_keys, folded->d_counts,
+                                     d_num.get<unsigned long long>(), ws.get(), s, &launches));
+    unsigned long long U = 0;
+    KC_CUDA_TRY(c, cudaMemcpyAsync(&U, d_num.get(), 8, cudaMemcpyDeviceToHost, s));
+    KC_CUDA_TRY(c, cudaStreamSynchronize(s));
     folded->n = U;
-    dev_free(s, d_rec); dev_free(s, ws); dev_free(s, d_num);
-    kc_run_free(c, raw);
     {
         std::lock_guard<std::mutex> g(c->mu);
         c->stats.h2d_bytes += n * c->S;
         c->stats.launches += launches;
     }
-    *out = folded;
+    *out = folded.release();
     return KC_OK;
 }
 
@@ -2096,15 +2006,14 @@ int kc_run_split(kc_ctx *c, const kc_run *r, const uint64_t *splitters, uint32_t
     if (n_splitters == 0) return KC_OK;
     cudaSetDevice(c->cfg.device);
     cudaStream_t s = c->stream;
-    void *dq = nullptr, *dout = nullptr;
-    KC_TRY(dev_alloc(c, s, (uint64_t)n_splitters * c->W * 8, &dq));
-    KC_TRY(dev_alloc(c, s, (uint64_t)n_splitters * 8, &dout));
-    KC_CUDA_TRY(c, cudaMemcpyAsync(dq, splitters, (uint64_t)n_splitters * c->W * 8, cudaMemcpyHostToDevice, s));
-    KC_CUDA_TRY(c, lower_bounds(r->d_keys + r->skip * r->W, n, r->W, static_cast<uint64_t *>(dq), n_splitters,
-                                static_cast<unsigned long long *>(dout), s));
-    KC_CUDA_TRY(c, cudaMemcpyAsync(offsets + 1, dout, (uint64_t)n_splitters * 8, cudaMemcpyDeviceToHost, s));
+    DevBuf dq(s), dout(s);
+    KC_TRY(dq.alloc(c, (uint64_t)n_splitters * c->W * 8));
+    KC_TRY(dout.alloc(c, (uint64_t)n_splitters * 8));
+    KC_CUDA_TRY(c, cudaMemcpyAsync(dq.get(), splitters, (uint64_t)n_splitters * c->W * 8, cudaMemcpyHostToDevice, s));
+    KC_CUDA_TRY(c, lower_bounds(r->d_keys + r->skip * r->W, n, r->W, dq.get<uint64_t>(), n_splitters,
+                                dout.get<unsigned long long>(), s));
+    KC_CUDA_TRY(c, cudaMemcpyAsync(offsets + 1, dout.get(), (uint64_t)n_splitters * 8, cudaMemcpyDeviceToHost, s));
     KC_CUDA_TRY(c, cudaStreamSynchronize(s));
-    dev_free(s, dq); dev_free(s, dout);
     std::lock_guard<std::mutex> g(c->mu);
     c->stats.launches += 1;
     return KC_OK;
@@ -2121,15 +2030,12 @@ int kc_run_histogram(kc_ctx *c, const kc_run *r, uint64_t *hist, uint32_t n_bins
     if (n == 0) return KC_OK;
     cudaSetDevice(c->cfg.device);
     cudaStream_t s = c->stream;
-    void *d_hist = nullptr;
-    KC_TRY(dev_alloc(c, s, (uint64_t)n_bins * 8, &d_hist));
+    DevBuf d_hist(s);
+    KC_TRY(d_hist.alloc(c, (uint64_t)n_bins * 8));
     int launches = 0;
-    cudaError_t e = run_histogram(r->d_counts + r->skip, n, n_bins, static_cast<unsigned long long *>(d_hist), c->n_sms,
-                                  s, &launches);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(hist, d_hist, (uint64_t)n_bins * 8, cudaMemcpyDeviceToHost, s);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(s);
-    dev_free(s, d_hist);
-    if (e != cudaSuccess) return c->set_error(KC_ERR_CUDA, "kc_run_histogram: %s", cudaGetErrorString(e));
+    KC_CUDA_TRY(c, run_histogram(r->d_counts + r->skip, n, n_bins, d_hist.get<unsigned long long>(), c->n_sms, s, &launches));
+    KC_CUDA_TRY(c, cudaMemcpyAsync(hist, d_hist.get(), (uint64_t)n_bins * 8, cudaMemcpyDeviceToHost, s));
+    KC_CUDA_TRY(c, cudaStreamSynchronize(s));
     std::lock_guard<std::mutex> g(c->mu);
     c->stats.launches += launches;
     c->stats.d2h_bytes += (uint64_t)n_bins * 8;
@@ -2139,66 +2045,158 @@ int kc_run_histogram(kc_ctx *c, const kc_run *r, uint64_t *hist, uint32_t n_bins
 int kc_run_filter(kc_ctx *c, const kc_run *r, uint32_t min_count, uint32_t max_count, kc_run **out) {
     KC_TRY(check_ctx(c));
     if (!r || !out) return c->set_error(KC_ERR_ARG, "null argument");
+    *out = nullptr;
     if (min_count > max_count) return c->set_error(KC_ERR_ARG, "kc_run_filter: min_count %u > max_count %u", min_count, max_count);
     std::lock_guard<std::recursive_mutex> dg(c->direct_mu);
     cudaSetDevice(c->cfg.device);
     cudaStream_t s = c->stream;
     const uint64_t n = r->n - r->skip;
-    if (n == 0) return make_run(c, s, 0, out);
+    if (n == 0) return kc_run_from_device(c, nullptr, nullptr, 0, out);
     const uint64_t *keys = r->d_keys + r->skip * r->W;
     const uint32_t *counts = r->d_counts + r->skip;
-    void *ws = nullptr, *d_total = nullptr;
-    kc_run *f = nullptr;
-    unsigned long long total = 0;
+    DevBuf ws(s), d_total(s);
+    KC_TRY(ws.alloc(c, filter_workspace_bytes(n)));
+    KC_TRY(d_total.alloc(c, 8));
     int launches = 0;
-    auto body = [&]() -> int {
-        KC_TRY(dev_alloc(c, s, filter_workspace_bytes(n), &ws));
-        KC_TRY(dev_alloc(c, s, 8, &d_total));
-        KC_CUDA_TRY(c, filter_count(counts, n, min_count, max_count, ws, static_cast<unsigned long long *>(d_total), s, &launches));
-        KC_CUDA_TRY(c, cudaMemcpyAsync(&total, d_total, 8, cudaMemcpyDeviceToHost, s));
-        KC_CUDA_TRY(c, cudaStreamSynchronize(s));
-        KC_TRY(make_run(c, s, total, &f));
-        KC_CUDA_TRY(c, filter_write(keys, counts, n, r->W, min_count, max_count, ws, f->d_keys, f->d_counts, s, &launches));
-        KC_CUDA_TRY(c, cudaStreamSynchronize(s));
-        return KC_OK;
-    };
-    const int rc = body();
-    dev_free(s, ws); dev_free(s, d_total);
-    if (rc != KC_OK) {
-        if (f) kc_run_free(c, f);
-        return rc;
-    }
+    unsigned long long total = 0;
+    KC_CUDA_TRY(c, filter_count(counts, n, min_count, max_count, ws.get(), d_total.get<unsigned long long>(), s, &launches));
+    KC_CUDA_TRY(c, cudaMemcpyAsync(&total, d_total.get(), 8, cudaMemcpyDeviceToHost, s));
+    KC_CUDA_TRY(c, cudaStreamSynchronize(s));
+    RunPtr f;
+    KC_TRY(make_run(c, s, total, &f));
+    KC_CUDA_TRY(c, filter_write(keys, counts, n, r->W, min_count, max_count, ws.get(), f->d_keys, f->d_counts, s, &launches));
+    KC_CUDA_TRY(c, cudaStreamSynchronize(s));
     {
         std::lock_guard<std::mutex> g(c->mu);
         c->stats.launches += launches;
         c->stats.d2h_bytes += 8;
     }
-    *out = f;
+    *out = f.release();
     return KC_OK;
 }
 
 // ------------------------------------------------------------------------- merge
+namespace {
+// a run of one level of a merge: one of the caller's (borrowed) or one this merge made (owned)
+struct LevelRun {
+    const kc_run *run;
+    RunPtr own;
+};
+LevelRun owned(RunPtr r) {
+    const kc_run *p = r.get();
+    return {p, std::move(r)};
+}
+
+// kc_merge_runs of runs of the partitioned path with one plan: kc_merge_parts over groups of up to 8,
+// level by level
+int merge_same_plan(kc_ctx *c, std::vector<LevelRun> level, kc_run **out) {
+    while (level.size() > 1) {
+        std::vector<LevelRun> next;
+        for (size_t i = 0; i < level.size(); i += 8) {
+            const uint32_t g = (uint32_t)std::min<size_t>(8, level.size() - i);
+            if (g == 1) { next.push_back(std::move(level[i])); continue; }
+            const void *kp[8], *cp[8], *op[8];
+            uint64_t sz[8];
+            for (uint32_t j = 0; j < g; j++) {
+                const kc_run *r = level[i + j].run;
+                kp[j] = r->d_keys; cp[j] = r->d_counts; op[j] = r->d_sub_off;
+                sz[j] = r->n;
+            }
+            kc_run *m = nullptr;
+            KC_TRY(kc_merge_parts(c, g, kp, cp, op, sz, level[0].run->n_sub, level[0].run->prefix_bits, &m));
+            next.push_back(owned(RunPtr(m, RunFree{c})));
+        }
+        level.swap(next);                            // (the level before goes with next)
+    }
+    *out = level[0].own.release();
+    return KC_OK;
+}
+
+// The pairwise tree of kc_merge_runs, level by level until level[0] is the one run left. The pairs of a
+// level are queued back to back (each with its own output, sized for the no-overlap case, and its own
+// record counter); the host reads the counters once per group of pairs instead of once per pair. A
+// group closes early when its outputs would take more than a third of the free device memory.
+int merge_tree(kc_ctx *c, cudaStream_t s, std::vector<LevelRun> &level, int *launches) {
+    const uint32_t max_pairs = (uint32_t)(level.size() / 2 + 1);
+    DevBuf d_num(s);
+    KC_TRY(d_num.alloc(c, 8ull * max_pairs));
+    std::vector<unsigned long long> h_num(max_pairs, 0);
+    const bool trace = getenv("KC_TRACE") != nullptr;
+    while (level.size() > 1) {
+        std::vector<LevelRun> next;
+        struct timespec t0;
+        clock_gettime(CLOCK_MONOTONIC, &t0);
+        uint64_t level_records = 0;
+        for (size_t i = 0; i + 1 < level.size();) {
+            size_t fr = 0, tot = 0;
+            cudaMemGetInfo(&fr, &tot);
+            const uint64_t budget = fr / 3;
+            uint64_t group_bytes = 0;
+            std::vector<DevBuf> group_ws;
+            const size_t g0 = i, n0 = next.size();
+            for (; i + 1 < level.size(); i += 2) {
+                const kc_run *a = level[i].run, *b = level[i + 1].run;
+                const uint64_t na = a->n - a->skip, nb = b->n - b->skip;
+                const uint64_t bytes = (na + nb) * (8ull * c->W + 4);
+                if (i > g0 && group_bytes + bytes > budget) break;
+                RunPtr m;
+                KC_TRY(make_run(c, s, na + nb, &m));
+                group_ws.emplace_back(s);
+                KC_TRY(group_ws.back().alloc(c, merge_workspace_bytes(na, nb)));
+                const cudaError_t e = merge_pair(a->d_keys + a->skip * a->W, a->d_counts + a->skip, na,
+                                                 b->d_keys + b->skip * b->W, b->d_counts + b->skip, nb, c->W, m->d_keys,
+                                                 m->d_counts, d_num.get<unsigned long long>() + (next.size() - n0),
+                                                 group_ws.back().get(), s, launches);
+                if (e != cudaSuccess) return c->set_error(KC_ERR_CUDA, "merge failed: %s", cudaGetErrorString(e));
+                next.push_back(owned(std::move(m)));
+                group_bytes += bytes;
+                level_records += na + nb;
+            }
+            const size_t n_pairs = next.size() - n0;
+            KC_CUDA_TRY(c, cudaMemcpyAsync(h_num.data(), d_num.get(), 8 * n_pairs, cudaMemcpyDeviceToHost, s));
+            KC_CUDA_TRY(c, cudaStreamSynchronize(s));
+            for (size_t q = 0; q < n_pairs; q++) {
+                next[n0 + q].own->n = h_num[q];
+                level[g0 + 2 * q].own.reset();       // the pair's inputs, if this merge made them
+                level[g0 + 2 * q + 1].own.reset();
+            }
+        }
+        if (level.size() & 1) next.push_back(std::move(level.back()));
+        if (trace) {
+            struct timespec t1;
+            clock_gettime(CLOCK_MONOTONIC, &t1);
+            fprintf(stderr, "kc_merge_runs: level of %zu runs, %llu records in: %.2f ms\n", level.size(), (unsigned long long)level_records,
+                    (t1.tv_sec - t0.tv_sec) * 1e3 + (t1.tv_nsec - t0.tv_nsec) * 1e-6);
+        }
+        level.swap(next);
+    }
+    return KC_OK;
+}
+}  // namespace
+
+
 int kc_merge_runs(kc_ctx *c, kc_run *const *runs, uint32_t n, kc_run **out) {
     KC_TRY(check_ctx(c));
     std::lock_guard<std::recursive_mutex> dg(c->direct_mu);
     if (!out || (n && !runs)) return c->set_error(KC_ERR_ARG, "null argument");
+    *out = nullptr;
     cudaSetDevice(c->cfg.device);
     cudaStream_t s = c->stream;
     // other streams (slots) may have produced the inputs
     for (auto &sl : c->slots)
         if (sl.stream) KC_CUDA_TRY(c, cudaStreamSynchronize(sl.stream));
-    if (n == 0) return make_run(c, s, 0, out);
-    std::vector<kc_run *> level;
-    std::vector<bool> owned;
-    for (uint32_t i = 0; i < n; i++) {
+    if (n == 0) return kc_run_from_device(c, nullptr, nullptr, 0, out);   // an empty run
+    for (uint32_t i = 0; i < n; i++)
         if (!runs[i]) return c->set_error(KC_ERR_ARG, "null run in merge list");
-        level.push_back(runs[i]);
-        owned.push_back(false);
-    }
     if (n == 1) {
         const kc_run *r = runs[0];
         return kc_run_from_device(c, r->d_keys + r->skip * r->W, r->d_counts + r->skip, r->n - r->skip, out);
     }
+    auto borrow_all = [&]() {
+        std::vector<LevelRun> v;
+        for (uint32_t i = 0; i < n; i++) v.push_back({runs[i], RunPtr()});
+        return v;
+    };
     // Three or more runs of the partitioned path with the same plan (chunks of equal size): combine
     // them range by range in shared-memory tables, up to 8 at a time (kc_merge_parts: one pass over
     // the records instead of log2(n) merge-path passes; 4 runs of C2: 11.9 ms against 16.8 ms).
@@ -2208,130 +2206,18 @@ int kc_merge_runs(kc_ctx *c, kc_run *const *runs, uint32_t n, kc_run **out) {
         for (uint32_t i = 0; i < n && same; i++)
             same = runs[i]->d_sub_off && runs[i]->skip == 0 && runs[i]->n_sub == runs[0]->n_sub &&
                    runs[i]->prefix_bits == runs[0]->prefix_bits;
-        if (same) {
-            std::vector<kc_run *> cur(runs, runs + n);
-            std::vector<bool> mine(n, false);
-            int prc = KC_OK;
-            while (cur.size() > 1 && prc == KC_OK) {
-                std::vector<kc_run *> nxt;
-                std::vector<bool> nxt_mine;
-                for (size_t i = 0; i < cur.size() && prc == KC_OK; i += 8) {
-                    const uint32_t g = (uint32_t)std::min<size_t>(8, cur.size() - i);
-                    if (g == 1) { nxt.push_back(cur[i]); nxt_mine.push_back(mine[i]); mine[i] = false; continue; }
-                    const void *kp[8], *cp[8], *op[8];
-                    uint64_t sz[8];
-                    for (uint32_t j = 0; j < g; j++) {
-                        kp[j] = cur[i + j]->d_keys; cp[j] = cur[i + j]->d_counts; op[j] = cur[i + j]->d_sub_off;
-                        sz[j] = cur[i + j]->n;
-                    }
-                    kc_run *m = nullptr;
-                    prc = kc_merge_parts(c, g, kp, cp, op, sz, cur[0]->n_sub, cur[0]->prefix_bits, &m);
-                    if (prc == KC_OK) { nxt.push_back(m); nxt_mine.push_back(true); }
-                }
-                if (prc != KC_OK) {
-                    for (size_t i = 0; i < nxt.size(); i++) if (nxt_mine[i]) kc_run_free(c, nxt[i]);
-                    for (size_t i = 0; i < cur.size(); i++) if (mine[i]) kc_run_free(c, cur[i]);
-                    break;
-                }
-                for (size_t i = 0; i < cur.size(); i++) if (mine[i]) kc_run_free(c, cur[i]);
-                cur.swap(nxt);
-                mine.swap(nxt_mine);
-            }
-            if (prc == KC_OK) { *out = cur[0]; return KC_OK; }
-            // a range too large for a shared-memory table (or too many records): the tree handles anything
-        }
+        // (a range too large for a shared-memory table, or too many records: the tree handles anything)
+        if (same && merge_same_plan(c, borrow_all(), out) == KC_OK) return KC_OK;
     }
-    // Pairwise tree. The pairs of a level are queued back to back (each with its own output, sized for
-    // the no-overlap case, and its own record counter); the host reads the counters once per group of
-    // pairs instead of once per pair. A group closes early when its outputs would take more than a
-    // third of the free device memory.
-    const uint32_t max_pairs = (uint32_t)(level.size() / 2 + 1);
-    unsigned long long *d_num = nullptr;
-    KC_TRY(dev_alloc(c, s, 8ull * max_pairs, (void **)&d_num));
-    std::vector<unsigned long long> h_num(max_pairs, 0);
-    int rc = KC_OK;
+    std::vector<LevelRun> level = borrow_all();
     int launches = 0;
-    const bool trace = getenv("KC_TRACE") != nullptr;
-    while (level.size() > 1 && rc == KC_OK) {
-        std::vector<kc_run *> next;
-        std::vector<bool> next_owned;
-        struct timespec t0;
-        clock_gettime(CLOCK_MONOTONIC, &t0);
-        uint64_t level_records = 0;
-        size_t i = 0;
-        while (i + 1 < level.size() && rc == KC_OK) {
-            size_t fr = 0, tot = 0;
-            cudaMemGetInfo(&fr, &tot);
-            const uint64_t budget = fr / 3;
-            uint64_t group_bytes = 0;
-            std::vector<void *> group_ws;
-            const size_t g0 = i, n0 = next.size();
-            while (i + 1 < level.size()) {
-                kc_run *a = level[i], *b = level[i + 1];
-                const uint64_t na = a->n - a->skip, nb = b->n - b->skip;
-                const uint64_t bytes = (na + nb) * (8ull * c->W + 4);
-                if (i > g0 && group_bytes + bytes > budget) break;
-                kc_run *m = nullptr;
-                rc = make_run(c, s, na + nb, &m);
-                if (rc != KC_OK) break;
-                void *ws = nullptr;
-                rc = dev_alloc(c, s, merge_workspace_bytes(na, nb), &ws);
-                if (rc != KC_OK) { kc_run_free(c, m); break; }
-                group_ws.push_back(ws);
-                next.push_back(m);
-                next_owned.push_back(true);
-                cudaError_t e = merge_pair(a->d_keys + a->skip * a->W, a->d_counts + a->skip, na,
-                                           b->d_keys + b->skip * b->W, b->d_counts + b->skip, nb, c->W, m->d_keys,
-                                           m->d_counts, d_num + (next.size() - 1 - n0), ws, s, &launches);
-                if (e != cudaSuccess) { rc = c->set_error(KC_ERR_CUDA, "merge failed: %s", cudaGetErrorString(e)); break; }
-                group_bytes += bytes;
-                level_records += na + nb;
-                i += 2;
-            }
-            const size_t n_pairs = next.size() - n0;
-            cudaError_t e = cudaSuccess;
-            if (rc == KC_OK && n_pairs) e = cudaMemcpyAsync(h_num.data(), d_num, 8 * n_pairs, cudaMemcpyDeviceToHost, s);
-            if (e == cudaSuccess) e = cudaStreamSynchronize(s);
-            for (void *w : group_ws) dev_free(s, w);
-            if (rc == KC_OK && e != cudaSuccess) rc = c->set_error(KC_ERR_CUDA, "merge failed: %s", cudaGetErrorString(e));
-            if (rc != KC_OK) break;
-            for (size_t q = 0; q < n_pairs; q++) {
-                next[n0 + q]->n = h_num[q];
-                const size_t ia = g0 + 2 * q;
-                if (owned[ia]) kc_run_free(c, level[ia]);
-                if (owned[ia + 1]) kc_run_free(c, level[ia + 1]);
-                owned[ia] = owned[ia + 1] = false;
-            }
-        }
-        if (rc == KC_OK && (level.size() & 1)) {
-            next.push_back(level.back());
-            next_owned.push_back(owned.back());
-            owned.back() = false;
-        }
-        if (rc != KC_OK) {
-            cudaStreamSynchronize(s);
-            for (size_t q = 0; q < next.size(); q++)
-                if (next_owned[q]) kc_run_free(c, next[q]);
-            for (size_t q = 0; q < level.size(); q++)
-                if (owned[q]) kc_run_free(c, level[q]);
-            break;
-        }
-        if (trace) {
-            struct timespec t1;
-            clock_gettime(CLOCK_MONOTONIC, &t1);
-            fprintf(stderr, "kc_merge_runs: level of %zu runs, %llu records in: %.2f ms\n", level.size(), (unsigned long long)level_records,
-                    (t1.tv_sec - t0.tv_sec) * 1e3 + (t1.tv_nsec - t0.tv_nsec) * 1e-6);
-        }
-        level.swap(next);
-        owned.swap(next_owned);
-    }
-    dev_free(s, d_num);
+    const int rc = merge_tree(c, s, level, &launches);
     {
         std::lock_guard<std::mutex> g(c->mu);
         c->stats.launches += launches;
     }
     if (rc != KC_OK) return rc;
-    *out = level[0];
+    *out = level[0].own.release();
     return KC_OK;
 }
 
