@@ -347,6 +347,65 @@ template <int W> __device__ __forceinline__ uint32_t key_hash(const Key<W> &k) {
 // a second, independent hash: which of the 2^bits passes over a bin a key belongs to
 __device__ __forceinline__ uint32_t pass_hash(uint32_t h) { return (h ^ (h >> 15)) * 0x2C1B3C6Du; }
 
+// KC_SW_PROFILE (off by default; tools/s2_profile.py builds with it): every warp of sw_count_kernel
+// adds clock64() deltas per phase into g_sw_prof, plus a few counters of the insert path. Lane 0
+// takes the time at phase boundaries, most of which are barriers, so a phase's share includes the
+// warp's wait for the CTA's slowest warp in that phase. Without the switch the macros are empty.
+enum {
+    SWP_UNIT = 0,       // unit hand-over, descriptors, phantom key, first round's records
+    SWP_DEDUP,          // record table claims
+    SWP_SCAN,           // scan of the surviving records' windows, placement in shared memory, slots handed back
+    SWP_OPEN,           // next round's prefetch, opening the thread's first record
+    SWP_INSERT,         // the insert loop, drains excluded
+    SWP_DRAIN,          // draining the per-warp collision queue
+    SWP_ROUND_END,      // distinct-key count and the barrier that closes a round
+    SWP_EMIT,           // emit of the pass with its table clear, abort handling
+    SWP_PHASES,
+    SWP_QUEUED = SWP_PHASES,    // occurrences sent to the collision queue
+    SWP_DRAIN_PROBES,           // buckets probed by the drains
+    SWP_WARPS,                  // warps that ran
+    SWP_TOTAL,                  // cycles of those warps, start to end
+    SWP_SLOTS
+};
+#ifdef KC_SW_PROFILE
+__device__ unsigned long long g_sw_prof[SWP_SLOTS];
+// the sums live in shared memory (lane 0 of each warp adds), so that the timer costs S2 two registers
+// and leaves it at the default build's occupancy
+#define SWP_DECL                                                                                      \
+    __shared__ unsigned long long s_prof[THREADS / 32][SWP_SLOTS];                                    \
+    if (lane == 0)                                                                                    \
+        for (int i_ = 0; i_ < SWP_SLOTS; i_++) s_prof[warp][i_] = 0;                                  \
+    const long long swp_t0 = clock64();                                                               \
+    long long swp_t = swp_t0
+#define SWP_MARK(ph)                                                                                  \
+    do {                                                                                              \
+        const long long t_ = clock64();                                                               \
+        if (lane == 0) s_prof[warp][ph] += (unsigned long long)(t_ - swp_t);                          \
+        swp_t = t_;                                                                                   \
+    } while (0)
+#define SWP_ADD(c, v) atomicAdd(&s_prof[warp][c], (unsigned long long)(v))
+#define SWP_ADD_ACTIVE(c)                                                                             \
+    do {                                                                                              \
+        const uint32_t am_ = __activemask();                                                          \
+        if (lane == (uint32_t)__ffs(am_) - 1) SWP_ADD(c, __popc(am_));                                \
+    } while (0)
+#define SWP_FLUSH()                                                                                   \
+    do {                                                                                              \
+        __syncwarp();                                                                                 \
+        if (lane == 0) {                                                                              \
+            s_prof[warp][SWP_WARPS] = 1;                                                              \
+            s_prof[warp][SWP_TOTAL] = (unsigned long long)(clock64() - swp_t0);                       \
+            for (int i_ = 0; i_ < SWP_SLOTS; i_++) atomicAdd(&g_sw_prof[i_], s_prof[warp][i_]);       \
+        }                                                                                             \
+    } while (0)
+#else
+#define SWP_DECL do {} while (0)
+#define SWP_MARK(ph) do {} while (0)
+#define SWP_ADD(c, v) do {} while (0)
+#define SWP_ADD_ACTIVE(c) do {} while (0)
+#define SWP_FLUSH() do {} while (0)
+#endif
+
 struct SwCountParams {
     // bins [bin_begin, bin_begin + n_bins) are counted here; the records of a bin are what every
     // source put there (one source on one GPU; with several GPUs the peers' bins are read in place,
@@ -386,8 +445,8 @@ __global__ void __launch_bounds__(THREADS) sw_count_kernel(SwCountParams p) {
     Key<W> *tk = reinterpret_cast<Key<W> *>(cs_smem);                       // [TSLOTS]
     ulonglong2 *recs = reinterpret_cast<ulonglong2 *>(tk + TSLOTS);         // [RB * W]
     uint32_t *tc = reinterpret_cast<uint32_t *>(recs + RB * W);             // [TSLOTS]
-    uint32_t *pre = tc + TSLOTS;                                            // [RB + 8]
-    uint32_t *s_hist = pre + RB + 8;                                        // [kNb1Max]
+    uint32_t *s_start = tc + TSLOTS;                                        // [THREADS] thread t's first record << 8 | window in it
+    uint32_t *s_hist = s_start + THREADS;                                   // [kNb1Max]
     constexpr int kQueue = RPT > 1 ? 64 : 96;                               // collided keys a warp parks before it drains them
     Key<W> *queue = reinterpret_cast<Key<W> *>(s_hist + kNb1Max);           // [THREADS / 32][kQueue]
     uint32_t *queue_m = reinterpret_cast<uint32_t *>(queue + (THREADS / 32) * kQueue);   // their weights
@@ -397,7 +456,7 @@ __global__ void __launch_bounds__(THREADS) sw_count_kernel(SwCountParams p) {
     ulonglong2 *rt_keys = reinterpret_cast<ulonglong2 *>(queue_m + (THREADS / 32) * kQueue);   // [RT]
     uint32_t *rt_mult = reinterpret_cast<uint32_t *>(rt_keys + RT);         // [RT]
     uint32_t *rec_mult = rt_mult + RT;                                      // [RB] weight of staged record i (0: a duplicate)
-    __shared__ uint32_t s_unit, s_m, s_ones, s_abort, s_off;
+    __shared__ uint32_t s_unit, s_m, s_ones, s_abort;
     __shared__ unsigned long long s_base;
     __shared__ uint32_t s_warp[THREADS / 32];
     const uint32_t tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -410,6 +469,8 @@ __global__ void __launch_bounds__(THREADS) sw_count_kernel(SwCountParams p) {
         key_set_ones<W>(empty);
         for (uint32_t i = tid; i < (uint32_t)TSLOTS; i += THREADS) { tk[i] = empty; tc[i] = 0; }
         for (uint32_t i = tid; i < (uint32_t)p.nb1; i += THREADS) s_hist[i] = 0;
+        if constexpr (DEDUP)
+            for (uint32_t i = tid; i < (uint32_t)RT; i += THREADS) { rt_keys[i] = make_ulonglong2(~0ull, ~0ull); rt_mult[i] = 0; }
         if (tid == 0) { s_m = 0; s_ones = 0; s_abort = 0; }
     }
     unsigned long long n_ovf = p.sc[SW_OVF];
@@ -417,7 +478,8 @@ __global__ void __launch_bounds__(THREADS) sw_count_kernel(SwCountParams p) {
     const uint32_t n_ovf_units = (uint32_t)((n_ovf + p.ovf_slice - 1) / p.ovf_slice);
     const uint32_t n_units = p.n_bins + n_ovf_units;
     unsigned long long occ_local = 0;
-    uint32_t aborts_local = 0;
+    uint32_t aborts_local = 0, multi_local = 0, dedup_local = 0;
+    SWP_DECL;
     // Work units are drawn from an atomic ticket two units ahead, so that a CTA knows its next unit
     // while it counts the current one: the next unit's record counts and its first round of
     // records are fetched in the shadow of the current unit's inserts (with several GPUs those
@@ -499,6 +561,7 @@ __global__ void __launch_bounds__(THREADS) sw_count_kernel(SwCountParams p) {
                 if ((uint32_t)q < p.n_src && p.src_sc[q][SW_INVALID] != 0) phantom = true;
         }
         if (n_rec == 0 && !phantom) { __syncthreads(); continue; }
+        if (tid == 0 && n_rec > (uint32_t)RB) multi_local++;
 
         uint32_t bits = 0, val = 0;
         while (true) {                                   // passes over the unit
@@ -542,32 +605,31 @@ __global__ void __launch_bounds__(THREADS) sw_count_kernel(SwCountParams p) {
                 }
             }
             pf_id = 0xffffffffu;
+            SWP_MARK(SWP_UNIT);
             for (uint32_t r0 = 0; r0 < n_rec; r0 += RB) {
                 const uint32_t nr = min((uint32_t)RB, n_rec - r0);
                 // The round's records sit in registers (fetched with a stride of THREADS: coalesced).
                 // Equal records of the round (the same run of the same locus, seen by several reads) are
                 // counted once: the first copy claims a slot of the record table and carries the
-                // multiplicity, the others drop out.
-                uint32_t c[RPT], wt[RPT];
+                // multiplicity, the others drop out. The table is empty at the start of every round: a
+                // claimed slot is handed back by its owner once the multiplicity has been read.
+                uint32_t c[RPT], rslot[RPT];
+                bool live[RPT];
 #pragma unroll
                 for (int u2 = 0; u2 < RPT; u2++) {
                     const uint32_t i = u2 * THREADS + tid;
                     c[u2] = i < nr ? (uint32_t)(pf[u2][W - 1].y & 0xffull) : 0u;
-                    wt[u2] = i < nr ? 1u : 0u;
+                    live[u2] = i < nr;
+                    rslot[u2] = 0xffffffffu;
                 }
                 if constexpr (DEDUP) {
-                    uint32_t rslot[RPT];
-                    for (uint32_t i = tid; i < (uint32_t)RT; i += THREADS) { rt_keys[i] = make_ulonglong2(~0ull, ~0ull); rt_mult[i] = 0; }
-                    __syncthreads();
 #pragma unroll
                     for (int u2 = 0; u2 < RPT; u2++) {
-                        rslot[u2] = 0xffffffffu;
-                        const uint32_t i = u2 * THREADS + tid;
-                        if (i < nr) {
+                        if (live[u2]) {
                             const ulonglong2 rec = pf[u2][0];
                             uint32_t h = ((uint32_t)rec.x ^ (uint32_t)(rec.x >> 32) * 0x85EBCA6Bu ^ (uint32_t)(rec.y >> 8) * 0xC2B2AE35u ^
                                           (uint32_t)(rec.y >> 40)) * 0x9E3779B1u >> (32 - ILog2<(uint32_t)RT>::v);
-                            while (true) {                       // the table holds twice the records of a round: never full
+                            while (true) {                       // the table holds at least the records of a round: never full
                                 ulonglong2 cur = rt_keys[h];
                                 if (cur.x == ~0ull || cur.y == ~0ull) {        // looks empty (a record is never all ones): settled by the CAS
                                     const uint32_t a = smem_u32(&rt_keys[h]);
@@ -587,46 +649,58 @@ __global__ void __launch_bounds__(THREADS) sw_count_kernel(SwCountParams p) {
                                 if (cur.x == rec.x && cur.y == rec.y) { atomicAdd(&rt_mult[h], 1u); break; }
                                 h = (h + 1) & (RT - 1);
                             }
+                            live[u2] = rslot[u2] != 0xffffffffu;
+                            dedup_local += live[u2] ? 0u : 1u;
                         }
                     }
-                    __syncthreads();
-#pragma unroll
-                    for (int u2 = 0; u2 < RPT; u2++) wt[u2] = rslot[u2] != 0xffffffffu ? rt_mult[rslot[u2]] : 0u;
                 }
-                // One scan gives every surviving record its place in the compacted round (high half)
-                // and the index of its first window in the flattened window sequence (low half: a round
-                // has fewer than 65536 windows). Record order i = u2 * THREADS + tid, stripe after stripe.
-                uint32_t stripe_base = 0;
+                SWP_MARK(SWP_DEDUP);
+                // One block scan gives every surviving record its place in the compacted round (high
+                // half) and the index of its first window in the flattened window sequence (low half: a
+                // round has fewer than 65536 windows). A thread's records are adjacent in that order. The
+                // scan's barrier also completes the record table's multiplicities.
+                uint32_t vsum = 0;
+#pragma unroll
+                for (int u2 = 0; u2 < RPT; u2++) vsum += live[u2] ? ((1u << 16) | c[u2]) : 0u;
+                uint32_t incl = vsum;
+#pragma unroll
+                for (int o = 1; o < 32; o <<= 1) {
+                    const uint32_t t = __shfl_up_sync(0xffffffffu, incl, o);
+                    if (lane >= (uint32_t)o) incl += t;
+                }
+                if (lane == 31) s_warp[warp] = incl;
+                __syncthreads();
+                uint32_t excl = incl - vsum, all = 0;
+#pragma unroll
+                for (int wq = 0; wq < THREADS / 32; wq++) {
+                    const uint32_t t = s_warp[wq];
+                    if ((uint32_t)wq < warp) excl += t;
+                    all += t;
+                }
+                const uint32_t tot = all & 0xffffu;
+                // this thread's share of the tot windows: [f0, f1)
+                const uint32_t per = (tot + THREADS - 1) / THREADS;
 #pragma unroll
                 for (int u2 = 0; u2 < RPT; u2++) {
-                    const uint32_t v = wt[u2] ? ((1u << 16) | c[u2]) : 0u;
-                    uint32_t incl = v;
-#pragma unroll
-                    for (int o = 1; o < 32; o <<= 1) {
-                        const uint32_t t = __shfl_up_sync(0xffffffffu, incl, o);
-                        if (lane >= (uint32_t)o) incl += t;
-                    }
-                    if (lane == 31) s_warp[warp] = incl;
-                    __syncthreads();
-                    uint32_t woff = 0, tot = 0;
-#pragma unroll
-                    for (int wq = 0; wq < THREADS / 32; wq++) {
-                        const uint32_t t = s_warp[wq];
-                        if ((uint32_t)wq < warp) woff += t;
-                        tot += t;
-                    }
-                    const uint32_t excl = stripe_base + woff + incl - v;
-                    if (wt[u2]) {
-                        const uint32_t ci = excl >> 16;
+                    if (live[u2]) {
+                        const uint32_t ci = excl >> 16, w0 = excl & 0xffffu;
 #pragma unroll
                         for (int t = 0; t < W; t++) recs[ci * W + t] = pf[u2][t];
-                        pre[ci] = excl & 0xffffu;
-                        rec_mult[ci] = wt[u2];
+                        uint32_t m = 1;
+                        if constexpr (DEDUP) {
+                            m = rt_mult[rslot[u2]];
+                            rt_keys[rslot[u2]] = make_ulonglong2(~0ull, ~0ull);
+                            rt_mult[rslot[u2]] = 0;
+                        }
+                        rec_mult[ci] = m;
+                        // the threads whose first window lies in this record start here (a record has at
+                        // least one window, so per > 0; t * per < tot keeps t < THREADS)
+                        for (uint32_t t = (w0 + per - 1) / per; t * per < w0 + c[u2]; t++) s_start[t] = ci << 8 | (t * per - w0);
+                        excl += (1u << 16) | c[u2];
                     }
-                    stripe_base += tot;
-                    __syncthreads();
                 }
-                const uint32_t n_live = stripe_base >> 16, tot = stripe_base & 0xffffu;
+                __syncthreads();
+                SWP_MARK(SWP_SCAN);
                 // prefetch the next round
 #pragma unroll
                 for (int u2 = 0; u2 < RPT; u2++) {
@@ -650,8 +724,6 @@ __global__ void __launch_bounds__(THREADS) sw_count_kernel(SwCountParams p) {
                     }
                     pf_id = un;
                 }
-                // this thread's share of the tot windows: [f0, f1)
-                const uint32_t per = (tot + THREADS - 1) / THREADS;
                 const uint32_t f0 = min(tid * per, tot), f1 = min(f0 + per, tot);
                 {
                     uint32_t rem = f1 - f0;                        // windows this lane still has to fetch
@@ -663,13 +735,9 @@ __global__ void __launch_bounds__(THREADS) sw_count_kernel(SwCountParams p) {
                     uint32_t in_rec = 0;                           // windows left in the open record
                     uint32_t wgt = 1;                              // how many equal records the open one stands for
                     if (rem) {   // open the first record at window j
-                        uint32_t lo = 0, hi = n_live;              // last record whose first window is <= f0
-                        while (hi - lo > 1) {
-                            const uint32_t mid = (lo + hi) >> 1;
-                            if (pre[mid] <= f0) lo = mid; else hi = mid;
-                        }
-                        ri = lo;
-                        const uint32_t j = f0 - pre[lo];
+                        const uint32_t st = s_start[tid];
+                        ri = st >> 8;
+                        const uint32_t j = st & 0xffu;
                         wgt = rec_mult[ri];
 #pragma unroll
                         for (int t = 0; t < W; t++) { const ulonglong2 v = recs[ri * W + t]; rw[2 * t] = v.x; rw[2 * t + 1] = v.y; }
@@ -691,6 +759,7 @@ __global__ void __launch_bounds__(THREADS) sw_count_kernel(SwCountParams p) {
                         in_rec = min(rem, cnt - j);
                         ri++;
                     }
+                    SWP_MARK(SWP_OPEN);
                     // Pass 1: every lane gives each of its keys ONE probe at its home bucket (two
                     // adjacent slots, one 16-byte load for 64-bit keys) -- no loop, so no lane waits for
                     // another's probe sequence. A key whose bucket is taken by two other keys goes to
@@ -730,6 +799,7 @@ __global__ void __launch_bounds__(THREADS) sw_count_kernel(SwCountParams p) {
                         return hit;
                     };
                     auto drain = [&]() {
+                        SWP_MARK(SWP_INSERT);
                         __syncwarp();
                         for (uint32_t en = lane; en < qn; en += 32) {
                             const Key<W> k = wq[en];
@@ -739,12 +809,14 @@ __global__ void __launch_bounds__(THREADS) sw_count_kernel(SwCountParams p) {
 #pragma unroll 1
                             for (uint32_t probes = 0; probes < 64u && !done; probes++) {
                                 done = try_bucket(hb, k, kw, true);
+                                SWP_ADD_ACTIVE(SWP_DRAIN_PROBES);
                                 hb = (hb + 1) & (TSLOTS / 2 - 1);
                             }
                             if (!done) s_abort = 1;                // table (nearly) full: the pass is abandoned
                         }
                         __syncwarp();
                         qn = 0;
+                        SWP_MARK(SWP_DRAIN);
                     };
 #pragma unroll 1
                     for (uint32_t it = 0; it < per; it++) {
@@ -789,10 +861,12 @@ __global__ void __launch_bounds__(THREADS) sw_count_kernel(SwCountParams p) {
                                 wqm[qi] = wgt;
                             }
                             qn += __popc(cm);
+                            if (lane == 0) SWP_ADD(SWP_QUEUED, __popc(cm));
                             if (qn > (uint32_t)kQueue - 32u) drain();
                         }
                     }
                     if (qn) drain();
+                    SWP_MARK(SWP_INSERT);
                 }
                 // distinct keys so far
 #pragma unroll
@@ -800,9 +874,10 @@ __global__ void __launch_bounds__(THREADS) sw_count_kernel(SwCountParams p) {
                 if (lane == 0 && claims) atomicAdd(&s_m, claims);
                 claims = 0;
                 __syncthreads();
+                SWP_MARK(SWP_ROUND_END);
                 if (s_abort || s_m > kLimit) { aborted = true; break; }
             }
-            if (!aborted) {                              // (the phantom alone: no round ran)
+            if (!aborted && n_rec == 0) {                // the phantom alone: no round ran (a round's end counted the claims)
 #pragma unroll
                 for (int o = 16; o > 0; o >>= 1) claims += __shfl_xor_sync(0xffffffffu, claims, o);
                 if (lane == 0 && claims) atomicAdd(&s_m, claims);
@@ -825,43 +900,48 @@ __global__ void __launch_bounds__(THREADS) sw_count_kernel(SwCountParams p) {
                 }
                 val <<= 1;
                 __syncthreads();
+                SWP_MARK(SWP_EMIT);
                 continue;
             }
-            // ---- emit the pass: distinct (key, count) records appended to D, table cleared
+            // ---- emit the pass: distinct (key, count) records appended to D, table cleared. Warp w
+            // takes the slots [w * SPW, (w + 1) * SPW): it counts its live slots while thread 0's
+            // atomic on |D| is in flight, and one scan of the warps' counts places every record.
+            constexpr uint32_t SPW = TSLOTS / (THREADS / 32);
             const uint32_t m = s_m, ones = s_ones;
             const uint32_t m_tot = m + (ones ? 1u : 0u);
-            if (tid == 0) {
-                s_base = m_tot ? atomicAdd(&p.sc[SW_D], (unsigned long long)m_tot) : 0ull;
-                s_off = 0;
-            }
+            if (tid == 0) s_base = m_tot ? atomicAdd(&p.sc[SW_D], (unsigned long long)m_tot) : 0ull;
+            const Key<W> *wtk = tk + warp * SPW;
+            uint32_t wlive = 0;
+#pragma unroll
+            for (uint32_t i0 = 0; i0 < SPW; i0 += 32) wlive += __popc(__ballot_sync(0xffffffffu, !key_all_ones<W>(wtk[i0 + lane])));
+            if (lane == 0) s_warp[warp] = wlive;
             __syncthreads();
             const unsigned long long base = s_base;
             if (base + m_tot > p.d_cap) {
                 if (tid == 0) atomicOr(&p.sc[SW_FAIL], 2ull);
             }
+            unsigned long long o_run = base;
+#pragma unroll
+            for (int wq = 0; wq < THREADS / 32; wq++) o_run += (uint32_t)wq < warp ? s_warp[wq] : 0u;
             Key<W> empty;
             key_set_ones<W>(empty);
-            for (uint32_t i0 = 0; i0 < (uint32_t)TSLOTS; i0 += THREADS) {
-                const uint32_t i = i0 + tid;
+#pragma unroll 1
+            for (uint32_t i0 = 0; i0 < SPW; i0 += 32) {
+                const uint32_t i = warp * SPW + i0 + lane;
                 const Key<W> k = tk[i];
                 const bool live = !key_all_ones<W>(k);
                 const uint32_t bal = __ballot_sync(0xffffffffu, live);
-                if (bal) {
-                    uint32_t b = 0;
-                    const int leader = __ffs(bal) - 1;
-                    if ((int)lane == leader) b = atomicAdd(&s_off, (uint32_t)__popc(bal));
-                    b = __shfl_sync(0xffffffffu, b, leader);
-                    if (live) {
-                        const unsigned long long o = base + b + __popc(bal & lanemask_lt());
-                        if (o < p.d_cap) {
-                            st_key<W>(p.d_keys, o, k);
-                            p.d_counts[o] = tc[i];
-                        }
-                        atomicAdd(&s_hist[k.w[0] >> p.shift1], 1u);
-                        tk[i] = empty;
-                        tc[i] = 0;
+                if (live) {
+                    const unsigned long long o = o_run + __popc(bal & lanemask_lt());
+                    if (o < p.d_cap) {
+                        st_key<W>(p.d_keys, o, k);
+                        p.d_counts[o] = tc[i];
                     }
+                    atomicAdd(&s_hist[k.w[0] >> p.shift1], 1u);
+                    tk[i] = empty;
+                    tc[i] = 0;
                 }
+                o_run += __popc(bal);
             }
             if (ones && tid == 0) {
                 const unsigned long long o = base + m;
@@ -876,9 +956,10 @@ __global__ void __launch_bounds__(THREADS) sw_count_kernel(SwCountParams p) {
             // next pass: climb while this was a right half, then step to the right sibling
             // (pass ids are prefixes of the pass hash, most significant bit first)
             while (bits > 0 && (val & 1u)) { val >>= 1; bits--; }
-            if (bits == 0) { __syncthreads(); break; }
+            if (bits == 0) { SWP_MARK(SWP_EMIT); break; }      // (the next unit starts with a barrier)
             val |= 1u;
             __syncthreads();
+            SWP_MARK(SWP_EMIT);
         }
     }
     __syncthreads();
@@ -888,8 +969,12 @@ __global__ void __launch_bounds__(THREADS) sw_count_kernel(SwCountParams p) {
     }
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) occ_local += __shfl_xor_sync(0xffffffffu, occ_local, o);
+    for (int o = 16; o > 0; o >>= 1) dedup_local += __shfl_xor_sync(0xffffffffu, dedup_local, o);
     if (lane == 0 && occ_local) atomicAdd(&p.sc[SW_OCC], occ_local);
+    if (lane == 0 && dedup_local) atomicAdd(&p.sc[SW_DEDUP], (unsigned long long)dedup_local);
     if (tid == 0 && aborts_local) atomicAdd(&p.sc[SW_ABORTS], (unsigned long long)aborts_local);
+    if (tid == 0 && multi_local) atomicAdd(&p.sc[SW_MULTI], (unsigned long long)multi_local);
+    SWP_FLUSH();
 }
 
 // ============================================================ S3: ordering the records
@@ -1948,7 +2033,7 @@ cudaError_t super_scatter(const SuperPlan &pl, const void *d_reads, uint64_t n_r
 template <int W, int THREADS, int TSLOTS, int RPT = 2, bool CANON = false>
 static cudaError_t launch_count(const SwCountParams &cp, int n_sms, cudaStream_t s) {
     const uint32_t RB = THREADS * RPT, RT = W == 1 ? (RPT > 1 ? RB : 2 * RB) : 1;
-    const uint32_t smem = TSLOTS * (8 * W + 4) + RB * 16 * W + (RB + 8) * 4 + kNb1Max * 4 +
+    const uint32_t smem = TSLOTS * (8 * W + 4) + RB * 16 * W + THREADS * 4 + kNb1Max * 4 +
                           (THREADS / 32) * (RPT > 1 ? 64 : 96) * (8 * W + 4) + RT * 20 + RB * 4 + 64;
     auto kern = sw_count_kernel<W, THREADS, TSLOTS, RPT, CANON>;
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
@@ -2306,3 +2391,15 @@ uint32_t *super_hist1(const SuperPlan &pl, void *ws) { return at<uint32_t>(ws, p
 const SuperXInfo *super_x_info(const SuperPlan &pl, void *ws) { return at<XDev>(ws, pl.off_x); }
 
 }  // namespace kc
+
+#ifdef KC_SW_PROFILE
+// S2's phase timer (KC_SW_PROFILE builds only): copies the SWP_SLOTS sums out, then zeroes them when reset != 0
+extern "C" int kc_sw_profile_read(unsigned long long *out, int reset) {
+    cudaError_t e = cudaMemcpyFromSymbol(out, kc::g_sw_prof, sizeof(kc::g_sw_prof));
+    if (e == cudaSuccess && reset) {
+        static const unsigned long long zero[kc::SWP_SLOTS] = {};
+        e = cudaMemcpyToSymbol(kc::g_sw_prof, zero, sizeof(zero));
+    }
+    return e == cudaSuccess ? 0 : -1;
+}
+#endif

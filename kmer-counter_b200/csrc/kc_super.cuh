@@ -41,6 +41,8 @@ enum {
     SW_TICKET2 = 11,    // S3c work ticket
     SW_BIG = 12,        // sub-buckets too large for S3c's shared memory (sorted by the radix sorter instead)
     SW_BIG_RECORDS = 13,// records in them
+    SW_DEDUP = 14,      // records S2 counted through an equal record instead of expanding them (every pass)
+    SW_MULTI = 15,      // S2 work units whose records took more than one round
     SW_COUNT = 16
 };
 

@@ -18,7 +18,7 @@ STAGE_NAMES = {
 }
 
 SW_SCALARS = ["invalid", "overflow_records", "d_records", "fail", "ticket", "windows", "occurrences", "aborts", "folded",
-              "out_records", "records", "ticket2", "big_ranges", "big_records"]
+              "out_records", "records", "ticket2", "big_ranges", "big_records", "dedup_records", "multi_round_units"]
 
 
 def xchg_run_all(counters):
