@@ -331,6 +331,38 @@ int  kc_peer_free(kc_ctx *ctx, void *d_ptr);
  * in shared memory, up to 8 per pass (kc_merge_parts). */
 int  kc_merge_runs(kc_ctx *ctx, kc_run *const *runs, uint32_t n, kc_run **out);
 
+/* ---- set operations of two runs: what `kmc_tools simple` gives (union, intersect, kmers_subtract,
+ * counters_subtract with its -oc count modes), on the device ----
+ * For every key x with count a in run A and b in run B:
+ *
+ *   op                       x in A and B                 x only in A   x only in B
+ *   KC_SET_UNION             m(a, b)                      a             b
+ *   KC_SET_INTERSECT         m(a, b)                      -             -
+ *   KC_SET_SUBTRACT          -                            a             -
+ *   KC_SET_SUBTRACT_COUNTS   a - b if a > b, else -       a             -
+ *
+ * m is the count mode `counts`, for keys in both runs only: KC_COUNTS_SUM (a + b, uint32 wrap, as
+ * kc_merge_runs), _MIN, _MAX, _A (A's count), _B (B's count). The subtracts take no mode: they must be
+ * given KC_COUNTS_SUM (0). Keys compare as everywhere (words as unsigned 64-bit, word 0 first); a
+ * record with count 0 (the KC_COMPAT_REF phantom key-0 record) is an ordinary record; records a run
+ * hides with its strict-mode skip are not part of it. The output is a new sorted key-unique run; the
+ * inputs are unchanged. Union with KC_COUNTS_SUM is kc_merge_runs of the two runs, byte for byte.
+ * Like a merge, the output is allocated for the most records op can give (union nA + nB, intersect
+ * min(nA, nB), the subtracts nA) and has no partition structure. Never combine canonical and forward
+ * runs: a run does not say which keys it holds.
+ * KC_ERR_ARG: a null argument, an unknown op or counts, a mode given to a subtract, or runs whose key
+ * width differs from each other or from the context's. On any error *out is NULL. */
+#define KC_SET_UNION           0u
+#define KC_SET_INTERSECT       1u
+#define KC_SET_SUBTRACT        2u
+#define KC_SET_SUBTRACT_COUNTS 3u
+#define KC_COUNTS_SUM          0u
+#define KC_COUNTS_MIN          1u
+#define KC_COUNTS_MAX          2u
+#define KC_COUNTS_A            3u
+#define KC_COUNTS_B            4u
+int  kc_run_combine(kc_ctx *ctx, const kc_run *a, const kc_run *b, uint32_t op, uint32_t counts, kc_run **out);
+
 /* ---- measurement support (not a reference interface): deterministic synthetic reads
  * written straight into device memory as packed lines; bit-identical to the host
  * generator used by the tests.  genome_len == 0 -> iid bases; zipf_loci > 0 -> half of

@@ -18,6 +18,12 @@ KC_COUNT_AUTO, KC_COUNT_SORT, KC_COUNT_HASH, KC_COUNT_HASH_GLOBAL, KC_COUNT_SUPE
 METHODS = {"auto": KC_COUNT_AUTO, "sort": KC_COUNT_SORT, "hash": KC_COUNT_HASH, "hash_global": KC_COUNT_HASH_GLOBAL,
            "super": KC_COUNT_SUPER, "place": KC_COUNT_PLACE}
 METHOD_NAMES = {v: k for k, v in METHODS.items()}
+# kc_run_combine: the set operation, and how a key in both runs is counted
+KC_SET_UNION, KC_SET_INTERSECT, KC_SET_SUBTRACT, KC_SET_SUBTRACT_COUNTS = 0, 1, 2, 3
+KC_COUNTS_SUM, KC_COUNTS_MIN, KC_COUNTS_MAX, KC_COUNTS_A, KC_COUNTS_B = 0, 1, 2, 3, 4
+SET_OPS = {"union": KC_SET_UNION, "intersect": KC_SET_INTERSECT, "subtract": KC_SET_SUBTRACT,
+           "subtract_counts": KC_SET_SUBTRACT_COUNTS}
+COUNT_MODES = {"sum": KC_COUNTS_SUM, "min": KC_COUNTS_MIN, "max": KC_COUNTS_MAX, "a": KC_COUNTS_A, "b": KC_COUNTS_B}
 
 
 class KcConfig(C.Structure):
@@ -95,6 +101,7 @@ SYMBOLS = {
     "kc_run_histogram": (_i, [_vp, _vp, _pu64, _u32]),
     "kc_run_filter": (_i, [_vp, _vp, _u32, _u32, _pp]),
     "kc_merge_runs": (_i, [_vp, _pp, _u32, _pp]),
+    "kc_run_combine": (_i, [_vp, _vp, _vp, _u32, _u32, _pp]),
     "kc_place_next_run": (_i, [_vp, _vp, _vp, _vp, _u64, _u32]),
     "kc_peer_alloc": (_i, [_vp, _u64, C.POINTER(_vp), _vp]),
     "kc_peer_open": (_i, [_vp, _vp, C.POINTER(_vp)]),

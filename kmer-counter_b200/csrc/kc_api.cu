@@ -20,6 +20,10 @@
 #include "kc_internal.h"
 
 static_assert(kc::kPlanStrict == KC_COMPAT_STRICT && kc::kPlanCanonical == KC_CANONICAL, "plan flags are kc_config.flags bits");
+static_assert(kc::kSetUnion == KC_SET_UNION && kc::kSetIntersect == KC_SET_INTERSECT && kc::kSetSubtract == KC_SET_SUBTRACT &&
+                  kc::kSetSubtractCounts == KC_SET_SUBTRACT_COUNTS, "combine_pair takes the KC_SET_* values");
+static_assert(kc::kCountsSum == KC_COUNTS_SUM && kc::kCountsMin == KC_COUNTS_MIN && kc::kCountsMax == KC_COUNTS_MAX &&
+                  kc::kCountsA == KC_COUNTS_A && kc::kCountsB == KC_COUNTS_B, "combine_pair takes the KC_COUNTS_* values");
 
 using namespace kc;
 
@@ -2218,6 +2222,50 @@ int kc_merge_runs(kc_ctx *c, kc_run *const *runs, uint32_t n, kc_run **out) {
     }
     if (rc != KC_OK) return rc;
     *out = level[0].own.release();
+    return KC_OK;
+}
+
+// ------------------------------------------------------------ set operations of two runs
+// One merge-path pass (combine_pair: the merge's kernels with the op deciding what survives); the
+// output is allocated for the most records the op can give and trimmed to what it gave.
+int kc_run_combine(kc_ctx *c, const kc_run *a, const kc_run *b, uint32_t op, uint32_t counts, kc_run **out) {
+    KC_TRY(check_ctx(c));
+    if (!a || !b || !out) return c->set_error(KC_ERR_ARG, "null argument");
+    *out = nullptr;
+    if (op > KC_SET_SUBTRACT_COUNTS) return c->set_error(KC_ERR_ARG, "kc_run_combine: unknown op %u", op);
+    if (counts > KC_COUNTS_B) return c->set_error(KC_ERR_ARG, "kc_run_combine: unknown count mode %u", counts);
+    if (counts != KC_COUNTS_SUM && (op == KC_SET_SUBTRACT || op == KC_SET_SUBTRACT_COUNTS))
+        return c->set_error(KC_ERR_ARG, "kc_run_combine: a subtract takes no count mode (got %u)", counts);
+    if (a->W != c->W || b->W != c->W)
+        return c->set_error(KC_ERR_ARG, "kc_run_combine: runs of %d and %d key words, the context's keys have %d", a->W, b->W, c->W);
+    std::lock_guard<std::recursive_mutex> dg(c->direct_mu);
+    cudaSetDevice(c->cfg.device);
+    cudaStream_t s = c->stream;
+    // other streams (slots) may have produced the inputs
+    for (auto &sl : c->slots)
+        if (sl.stream) KC_CUDA_TRY(c, cudaStreamSynchronize(sl.stream));
+    const uint64_t na = a->n - a->skip, nb = b->n - b->skip;
+    const uint64_t cap = op == KC_SET_UNION ? na + nb : op == KC_SET_INTERSECT ? std::min(na, nb) : na;
+    RunPtr r;
+    DevBuf ws(s), d_num(s);
+    KC_TRY(make_run(c, s, cap, &r));
+    KC_TRY(ws.alloc(c, merge_workspace_bytes(na, nb)));
+    KC_TRY(d_num.alloc(c, 8));
+    int launches = 0;
+    const cudaError_t e = combine_pair(a->d_keys + a->skip * a->W, a->d_counts + a->skip, na, b->d_keys + b->skip * b->W,
+                                       b->d_counts + b->skip, nb, c->W, op, counts, r->d_keys, r->d_counts,
+                                       d_num.get<unsigned long long>(), ws.get(), s, &launches);
+    if (e != cudaSuccess) return c->set_error(KC_ERR_CUDA, "combine failed: %s", cudaGetErrorString(e));
+    unsigned long long n_out = 0;
+    KC_CUDA_TRY(c, cudaMemcpyAsync(&n_out, d_num.get(), 8, cudaMemcpyDeviceToHost, s));
+    KC_CUDA_TRY(c, cudaStreamSynchronize(s));
+    r->n = n_out;
+    {
+        std::lock_guard<std::mutex> g(c->mu);
+        c->stats.launches += launches;
+        c->stats.d2h_bytes += 8;
+    }
+    *out = r.release();
     return KC_OK;
 }
 

@@ -78,6 +78,15 @@ uint64_t merge_workspace_bytes(uint64_t na, uint64_t nb);
 cudaError_t merge_pair(const uint64_t *ka, const uint32_t *ca, uint64_t na, const uint64_t *kb, const uint32_t *cb,
                        uint64_t nb, int W, uint64_t *out_keys, uint32_t *out_counts,
                        unsigned long long *d_num_out, void *ws, cudaStream_t s, int *n_launches);
+// set operations of two sorted unique runs (the KC_SET_* / KC_COUNTS_* values of kc_api.h): op decides
+// which keys survive, counts how a key in both runs is counted; union with kCountsSum is merge_pair.
+// Same workspace as merge_pair; out_* hold the most records op can give (union na + nb, intersect
+// min(na, nb), the subtracts na); *d_num_out = records. A bad op or counts: cudaErrorInvalidValue
+enum : uint32_t { kSetUnion = 0, kSetIntersect = 1, kSetSubtract = 2, kSetSubtractCounts = 3 };
+enum : uint32_t { kCountsSum = 0, kCountsMin = 1, kCountsMax = 2, kCountsA = 3, kCountsB = 4 };
+cudaError_t combine_pair(const uint64_t *ka, const uint32_t *ca, uint64_t na, const uint64_t *kb, const uint32_t *cb,
+                         uint64_t nb, int W, uint32_t op, uint32_t counts, uint64_t *out_keys, uint32_t *out_counts,
+                         unsigned long long *d_num_out, void *ws, cudaStream_t s, int *n_launches);
 
 // ---- hash table (kc_hash.cu), W == 1 only
 struct HashTable {

@@ -1,5 +1,6 @@
 // kc_merge.cu -- GPU merge-path merge of two sorted key-unique runs, summing the
-// counts of equal keys.
+// counts of equal keys; and the set operations of two runs (union, intersect,
+// subtract) on the same kernels.
 //
 // Replaces KMerFileMerger::Merge (KMerFileMerger.cpp:49-96: a serial O(M) min-scan
 // per output record over file cursors) and the cursor class under it
@@ -10,12 +11,28 @@
 // loads one tile of A and B into shared memory; every thread searches its own
 // diagonal once and merges its positions serially in registers, folding the B
 // half of an equal pair into its A partner; the surviving records are written
-// in order at the offset a decoupled look-back over the tiles gives.
+// in order at the offset a decoupled look-back over the tiles gives.  Which
+// records survive, and with what count, is the tile kernel's OP.
 #include "kc_internal.h"
 
 namespace kc {
 
 namespace {
+
+// OP of the tile kernel: kTileMerge is the merge (union, counts summed); the set operations
+// kSetUnion .. kSetSubtractCounts take the count mode of keys in both runs as a kernel argument
+constexpr int kTileMerge = -1;
+
+// the count of a key present in both runs (kCounts*; the sum wraps at 2^32)
+__device__ __forceinline__ uint32_t both_count(uint32_t a, uint32_t b, uint32_t mode) {
+    switch (mode) {
+        case kCountsMin: return min(a, b);
+        case kCountsMax: return max(a, b);
+        case kCountsA: return a;
+        case kCountsB: return b;
+        default: return a + b;
+    }
+}
 
 #ifndef KC_MERGE_THREADS
 #define KC_MERGE_THREADS 512
@@ -66,12 +83,15 @@ __global__ void merge_partition_kernel(const uint64_t *__restrict__ ka, uint64_t
 // contiguous piece at the offset a decoupled look-back over the tiles gives.
 // (A tile can hold TILE + 1 records: the cut after it was moved to keep an equal pair together;
 // the extra record is that pair's B half, the last position, and needs no thread.)
-template <int W>
+// A set operation (OP != kTileMerge) decides instead whether an A record with a B partner survives
+// and with which count, whether an A record without one survives, and whether a B record without
+// one does. The B half of a pair never survives, so the extra record and the cuts stay as they are.
+template <int W, int OP>
 __global__ void __launch_bounds__(kMergeThreads) merge_tile_kernel(
     const uint64_t *__restrict__ ka, const uint32_t *__restrict__ ca, const uint64_t *__restrict__ kb,
     const uint32_t *__restrict__ cb, const uint64_t *__restrict__ cut_a, const uint64_t *__restrict__ cut_b,
     uint32_t n_tiles, uint64_t *__restrict__ out_keys, uint32_t *__restrict__ out_counts,
-    unsigned long long *__restrict__ d_num_out, unsigned long long *ticket, uint64_t *status) {
+    unsigned long long *__restrict__ d_num_out, unsigned long long *ticket, uint64_t *status, uint32_t counts) {
     constexpr int IPT = MergeCfg<W>::IPT, TILE = MergeCfg<W>::TILE;
     constexpr int CAP = TILE + 2;
     constexpr int WARPS = kMergeThreads / 32;
@@ -123,10 +143,27 @@ __global__ void __launch_bounds__(kMergeThreads) merge_tile_kernel(
             const bool take_a = bi >= nb || (ai < na && !key_lt<W>(b_head, a_head));
             if (take_a) {
                 rk[j] = a_head;
-                uint32_t c = cA[ai];
-                if (bi < nb && key_eq<W>(b_head, a_head)) c += cB[bi];
-                rc[j] = c;
-                keep |= 1u << j;
+                if constexpr (OP == kTileMerge) {
+                    uint32_t c = cA[ai];
+                    if (bi < nb && key_eq<W>(b_head, a_head)) c += cB[bi];
+                    rc[j] = c;
+                    keep |= 1u << j;
+                } else {
+                    const uint32_t c = cA[ai];
+                    if (bi < nb && key_eq<W>(b_head, a_head)) {                  // the key is in both runs
+                        const uint32_t cb_ = cB[bi];
+                        if constexpr (OP == kSetUnion || OP == kSetIntersect) {
+                            rc[j] = both_count(c, cb_, counts);
+                            keep |= 1u << j;
+                        } else if constexpr (OP == kSetSubtractCounts) {
+                            rc[j] = c - cb_;
+                            if (c > cb_) keep |= 1u << j;
+                        }
+                    } else if constexpr (OP != kSetIntersect) {                   // only in A
+                        rc[j] = c;
+                        keep |= 1u << j;
+                    }
+                }
                 a_prev = a_head;
                 have_prev = true;
                 ai++;
@@ -134,7 +171,8 @@ __global__ void __launch_bounds__(kMergeThreads) merge_tile_kernel(
             } else {
                 rk[j] = b_head;
                 rc[j] = cB[bi];
-                if (!(have_prev && key_eq<W>(a_prev, b_head))) keep |= 1u << j;
+                if constexpr (OP == kTileMerge || OP == kSetUnion)       // (only in B, or a pair's B half)
+                    if (!(have_prev && key_eq<W>(a_prev, b_head))) keep |= 1u << j;
                 bi++;
                 if (bi < nb) b_head = sB[bi];
             }
@@ -187,10 +225,10 @@ __global__ void __launch_bounds__(kMergeThreads) merge_tile_kernel(
     }
 }
 
-template <int W>
+template <int W, int OP>
 cudaError_t merge_pair_w(const uint64_t *ka, const uint32_t *ca, uint64_t na, const uint64_t *kb, const uint32_t *cb,
-                         uint64_t nb, uint64_t *out_keys, uint32_t *out_counts, unsigned long long *d_num_out,
-                         void *ws, cudaStream_t s, int *n_launches) {
+                         uint64_t nb, uint32_t counts, uint64_t *out_keys, uint32_t *out_counts,
+                         unsigned long long *d_num_out, void *ws, cudaStream_t s, int *n_launches) {
     constexpr int TILE = MergeCfg<W>::TILE;
     constexpr int CAP = TILE + 2;
     const uint64_t total = na + nb;
@@ -205,13 +243,26 @@ cudaError_t merge_pair_w(const uint64_t *ka, const uint32_t *ca, uint64_t na, co
     merge_partition_kernel<W><<<(n_tiles + 1 + 127) / 128, 128, 0, s>>>(ka, na, kb, nb, n_tiles, cut_a, cut_b);
     if ((e = cudaGetLastError()) != cudaSuccess) return e;
     const size_t smem = (size_t)CAP * (sizeof(Key<W>) + 4) + 16;
-    auto kern = merge_tile_kernel<W>;
+    auto kern = merge_tile_kernel<W, OP>;
     if ((e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)) != cudaSuccess)
         return e;
     kern<<<n_tiles, kMergeThreads, smem, s>>>(ka, ca, kb, cb, cut_a, cut_b, n_tiles, out_keys, out_counts, d_num_out,
-                                              ticket, status);
+                                              ticket, status, counts);
     if (n_launches) *n_launches += 2;
     return cudaGetLastError();
+}
+
+template <int OP>
+cudaError_t tile_pass(const uint64_t *ka, const uint32_t *ca, uint64_t na, const uint64_t *kb, const uint32_t *cb,
+                      uint64_t nb, int W, uint32_t counts, uint64_t *out_keys, uint32_t *out_counts,
+                      unsigned long long *d_num_out, void *ws, cudaStream_t s, int *n_launches) {
+    switch (W) {
+        case 1: return merge_pair_w<1, OP>(ka, ca, na, kb, cb, nb, counts, out_keys, out_counts, d_num_out, ws, s, n_launches);
+        case 2: return merge_pair_w<2, OP>(ka, ca, na, kb, cb, nb, counts, out_keys, out_counts, d_num_out, ws, s, n_launches);
+        case 3: return merge_pair_w<3, OP>(ka, ca, na, kb, cb, nb, counts, out_keys, out_counts, d_num_out, ws, s, n_launches);
+        case 4: return merge_pair_w<4, OP>(ka, ca, na, kb, cb, nb, counts, out_keys, out_counts, d_num_out, ws, s, n_launches);
+    }
+    return cudaErrorInvalidValue;
 }
 
 }  // namespace
@@ -225,11 +276,27 @@ cudaError_t merge_pair(const uint64_t *ka, const uint32_t *ca, uint64_t na, cons
                        uint64_t nb, int W, uint64_t *out_keys, uint32_t *out_counts, unsigned long long *d_num_out,
                        void *ws, cudaStream_t s, int *n_launches) {
     if (na + nb == 0) return cudaMemsetAsync(d_num_out, 0, 8, s);
-    switch (W) {
-        case 1: return merge_pair_w<1>(ka, ca, na, kb, cb, nb, out_keys, out_counts, d_num_out, ws, s, n_launches);
-        case 2: return merge_pair_w<2>(ka, ca, na, kb, cb, nb, out_keys, out_counts, d_num_out, ws, s, n_launches);
-        case 3: return merge_pair_w<3>(ka, ca, na, kb, cb, nb, out_keys, out_counts, d_num_out, ws, s, n_launches);
-        case 4: return merge_pair_w<4>(ka, ca, na, kb, cb, nb, out_keys, out_counts, d_num_out, ws, s, n_launches);
+    return tile_pass<kTileMerge>(ka, ca, na, kb, cb, nb, W, 0, out_keys, out_counts, d_num_out, ws, s, n_launches);
+}
+
+cudaError_t combine_pair(const uint64_t *ka, const uint32_t *ca, uint64_t na, const uint64_t *kb, const uint32_t *cb,
+                         uint64_t nb, int W, uint32_t op, uint32_t counts, uint64_t *out_keys, uint32_t *out_counts,
+                         unsigned long long *d_num_out, void *ws, cudaStream_t s, int *n_launches) {
+    if (counts > kCountsB || (counts != kCountsSum && (op == kSetSubtract || op == kSetSubtractCounts)))
+        return cudaErrorInvalidValue;
+    if (op == kSetUnion && counts == kCountsSum)
+        return merge_pair(ka, ca, na, kb, cb, nb, W, out_keys, out_counts, d_num_out, ws, s, n_launches);
+    if (na + nb == 0) return cudaMemsetAsync(d_num_out, 0, 8, s);
+    switch (op) {
+        case kSetUnion:
+            return tile_pass<kSetUnion>(ka, ca, na, kb, cb, nb, W, counts, out_keys, out_counts, d_num_out, ws, s, n_launches);
+        case kSetIntersect:
+            return tile_pass<kSetIntersect>(ka, ca, na, kb, cb, nb, W, counts, out_keys, out_counts, d_num_out, ws, s, n_launches);
+        case kSetSubtract:
+            return tile_pass<kSetSubtract>(ka, ca, na, kb, cb, nb, W, counts, out_keys, out_counts, d_num_out, ws, s, n_launches);
+        case kSetSubtractCounts:
+            return tile_pass<kSetSubtractCounts>(ka, ca, na, kb, cb, nb, W, counts, out_keys, out_counts, d_num_out, ws, s,
+                                                 n_launches);
     }
     return cudaErrorInvalidValue;
 }

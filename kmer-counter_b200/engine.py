@@ -125,6 +125,26 @@ class Run:
         self._c._check(self._c._lib.kc_run_filter(self._c._ctx, self._h, int(min_count), int(max_count), C.byref(h)))
         return Run(self._c, h)
 
+    # KMC's count mode when none is given: union sums, intersect takes the smaller count
+    _DEFAULT_COUNTS = {"union": "sum", "intersect": "min", "subtract": "sum", "subtract_counts": "sum"}
+
+    def combine(self, other, op, counts=None) -> "Run":
+        """A new run from this run (A) and `other` (B), computed on the device (kc_run_combine).
+        op: "union", "intersect", "subtract" (keys of A not in B) or "subtract_counts" (also keys in
+        both with a > b, counted a - b). counts: how a key in both runs is counted by union and
+        intersect -- "sum", "min", "max", "a" or "b"; None = KMC's default (sum for union, min for
+        intersect). The subtracts take no mode. Both runs must come from counters with the same k."""
+        if op not in _lib.SET_OPS:
+            raise KcError(-1, "unknown set operation %r (one of %s)" % (op, ", ".join(_lib.SET_OPS)))
+        if counts is None:
+            counts = self._DEFAULT_COUNTS[op]
+        if counts not in _lib.COUNT_MODES:
+            raise KcError(-1, "unknown count mode %r (one of %s)" % (counts, ", ".join(_lib.COUNT_MODES)))
+        h = C.c_void_p()
+        self._c._check(self._c._lib.kc_run_combine(self._c._ctx, self._h, other._h, _lib.SET_OPS[op],
+                                                   _lib.COUNT_MODES[counts], C.byref(h)))
+        return Run(self._c, h)
+
     def free(self):
         if self._h and self._c._ctx:
             self._c._lib.kc_run_free(self._c._ctx, self._h)

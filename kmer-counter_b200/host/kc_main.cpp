@@ -8,6 +8,11 @@
 //   kmer_counter_b200 print <record file> <ignored> <k>       (KMerPrinter, main.cpp:78-82)
 //   kmer_counter_b200 histo <record file> <out|-> <k> [histoMax]
 //                     the count spectrum of a record file, computed on the GPU (histoFile's format)
+//   kmer_counter_b200 combine <union|intersect|subtract|subtract_counts> <A file> <B file> <out file> <k>
+//                     [counts=sum|min|max|a|b] [minCount=N] [maxCount=N] [pieceRecords=N]
+//                     a set operation of two record files on the GPU (kc_run_combine; KMC's
+//                     `kmc_tools simple`), counts= for keys in both (default: sum for union, min for
+//                     intersect), minCount= / maxCount= on the combined counts
 //
 // minCount= / maxCount= keep only the k-mers whose final count is in range (KMC -ci/-cx, Jellyfish
 // -L/-U); histoFile= writes the spectrum of the final counts before that filter: one line "c n" per
@@ -127,6 +132,145 @@ static int histo_records(const char *path, const char *out, uint32_t k, int64_t 
     kc_destroy(ctx);
     if (rc == KC_OK) rc = write_histo(out, hist);
     return rc == KC_OK ? 0 : 1;
+}
+
+// `combine <op> <A file> <B file> <out file> <k> [counts=..] [minCount=N] [maxCount=N] [pieceRecords=N]`:
+// files of any size, piece by piece on one context. Each piece fills a buffer of up to pieceRecords
+// records from each file and is cut at the smaller of the two buffers' last keys (a file that is
+// exhausted does not bound the cut; with both exhausted everything is taken). The records at or below
+// the cut go up, are combined (and filtered) on the GPU and appended to the output; the rest of each
+// buffer opens the next piece. A key's A and B records so land in the same piece, and the buffer whose
+// last key is the cut empties, so every piece makes progress.
+struct RecordSource {
+    FILE *f = nullptr;
+    std::vector<unsigned char> buf;
+    uint64_t n = 0, read = 0;       // records in buf, records read in all
+    bool eof = false;
+    int fill(uint64_t S, uint64_t cap) {
+        if (buf.size() < cap * S) buf.resize(cap * S);
+        while (!eof && n < cap) {
+            const size_t want = (size_t)((cap - n) * S), got = fread(buf.data() + n * S, 1, want, f);
+            if (got < want) {
+                if (ferror(f)) return KC_ERR_IO;
+                eof = true;                         // (a partial record at the end is ignored)
+            }
+            n += got / S;
+            read += got / S;
+        }
+        return KC_OK;
+    }
+    const unsigned char *rec(uint64_t i, uint64_t S) const { return buf.data() + i * S; }
+};
+
+static int key_cmp(const unsigned char *a, const unsigned char *b, uint32_t W) {
+    for (uint32_t w = 0; w < W; w++) {
+        uint64_t x, y;
+        memcpy(&x, a + 8 * w, 8);
+        memcpy(&y, b + 8 * w, 8);
+        if (x != y) return x < y ? -1 : 1;
+    }
+    return 0;
+}
+
+// records of src with key <= cut (all of them when cut is null)
+static uint64_t upto(const RecordSource &src, const unsigned char *cut, uint64_t S, uint32_t W) {
+    if (!cut) return src.n;
+    uint64_t lo = 0, hi = src.n;
+    while (lo < hi) {
+        const uint64_t mid = (lo + hi) / 2;
+        if (key_cmp(src.rec(mid, S), cut, W) <= 0) lo = mid + 1;
+        else hi = mid;
+    }
+    return lo;
+}
+
+static int combine_files(int argc, char **argv) {
+    const char *usage = "usage: %s combine <union|intersect|subtract|subtract_counts> <A file> <B file> <out file> <k> "
+                        "[counts=sum|min|max|a|b] [minCount=N] [maxCount=N] [pieceRecords=N]\n";
+    if (argc < 7) { fprintf(stderr, usage, argv[0]); return 2; }
+    const std::string op_name = argv[2];
+    const char *ops[] = {"union", "intersect", "subtract", "subtract_counts"};
+    const char *modes[] = {"sum", "min", "max", "a", "b"};
+    uint32_t op = 4;
+    for (uint32_t i = 0; i < 4; i++) if (op_name == ops[i]) op = i;
+    const uint32_t k = (uint32_t)strtoul(argv[6], nullptr, 10);
+    if (op == 4 || k < 1 || k > 128) { fprintf(stderr, usage, argv[0]); return 2; }
+    uint32_t counts = op == KC_SET_INTERSECT ? KC_COUNTS_MIN : KC_COUNTS_SUM;      // KMC's defaults
+    int64_t min_count = -1, max_count = -1;
+    const uint64_t S = kc_record_size(k), W = kc_key_words(k);
+    uint64_t piece = (64ull << 20) / S;
+    for (int i = 7; i < argc; i++) {
+        const char *eq = strchr(argv[i], '=');
+        const std::string key = eq ? std::string(argv[i], eq - argv[i]) : argv[i], val = eq ? eq + 1 : "";
+        if (key == "counts") {
+            counts = 5;
+            for (uint32_t m = 0; m < 5; m++) if (val == modes[m]) counts = m;
+            if (counts == 5) { fprintf(stderr, "counts= must be sum, min, max, a or b\n"); return 2; }
+        } else if (key == "minCount") min_count = strtoll(val.c_str(), nullptr, 10);
+        else if (key == "maxCount") max_count = strtoll(val.c_str(), nullptr, 10);
+        else if (key == "pieceRecords") piece = strtoull(val.c_str(), nullptr, 10);
+        else { fprintf(stderr, usage, argv[0]); return 2; }
+    }
+    if (piece < 1 || piece > (1ull << 30)) { fprintf(stderr, "pieceRecords must be 1..%llu\n", 1ull << 30); return 2; }
+    const auto bound = [](int64_t v, uint32_t none) { return v < 0 ? none : v > 0xffffffffll ? 0xffffffffu : (uint32_t)v; };
+    const bool filtering = min_count >= 0 || max_count >= 0;
+    RecordSource src[2];
+    src[0].f = fopen(argv[3], "rb");
+    src[1].f = fopen(argv[4], "rb");
+    FILE *out = fopen(argv[5], "wb");                        // truncated here, appended to piece by piece
+    if (!src[0].f || !src[1].f || !out) {
+        fprintf(stderr, "cannot open %s\n", !src[0].f ? argv[3] : !src[1].f ? argv[4] : argv[5]);
+        for (FILE *f : {src[0].f, src[1].f, out}) if (f) fclose(f);
+        return 1;
+    }
+    fclose(out);
+    kc_config cfg = {};
+    cfg.struct_size = sizeof cfg;
+    cfg.k = k;
+    cfg.read_len = k;
+    kc_ctx *ctx = nullptr;
+    int rc = kc_create(&cfg, &ctx);
+    if (rc != KC_OK) fprintf(stderr, "kc_create: %s\n", kc_last_error(nullptr));
+    uint64_t written = 0, pieces = 0;
+    while (rc == KC_OK) {
+        if ((rc = src[0].fill(S, piece)) != KC_OK || (rc = src[1].fill(S, piece)) != KC_OK) {
+            fprintf(stderr, "read error\n");
+            break;
+        }
+        if (src[0].n == 0 && src[1].n == 0) break;
+        const unsigned char *cut = nullptr;                  // +infinity
+        for (const RecordSource &s : src)
+            if (!s.eof) {
+                const unsigned char *last = s.rec(s.n - 1, S);
+                if (!cut || key_cmp(last, cut, (uint32_t)W) < 0) cut = last;
+            }
+        const uint64_t take[2] = {upto(src[0], cut, S, (uint32_t)W), upto(src[1], cut, S, (uint32_t)W)};
+        kc_run *in[2] = {nullptr, nullptr}, *res = nullptr;
+        for (int i = 0; i < 2 && rc == KC_OK; i++) rc = kc_run_upload(ctx, src[i].buf.data(), take[i] * S, &in[i]);
+        if (rc == KC_OK) rc = kc_run_combine(ctx, in[0], in[1], op, counts, &res);
+        if (rc == KC_OK && filtering) {
+            kc_run *kept = nullptr;
+            rc = kc_run_filter(ctx, res, bound(min_count, 0), bound(max_count, 0xffffffffu), &kept);
+            kc_run_free(ctx, res);
+            res = kept;
+        }
+        if (rc == KC_OK) rc = kc_run_write(ctx, res, argv[5], 1);
+        if (rc == KC_OK) written += kc_run_records(res);
+        for (kc_run *r : {in[0], in[1], res}) if (r) kc_run_free(ctx, r);
+        if (rc != KC_OK) { fprintf(stderr, "kmer_counter_b200 combine: %s\n", kc_last_error(ctx)); break; }
+        for (int i = 0; i < 2; i++) {                        // the rest opens the next piece
+            memmove(src[i].buf.data(), src[i].rec(take[i], S), (size_t)((src[i].n - take[i]) * S));
+            src[i].n -= take[i];
+        }
+        pieces++;
+    }
+    fclose(src[0].f);
+    fclose(src[1].f);
+    if (ctx) kc_destroy(ctx);
+    if (rc != KC_OK) return 1;
+    fprintf(stderr, "combine %s counts=%s a_records=%" PRIu64 " b_records=%" PRIu64 " pieces=%" PRIu64 " records=%" PRIu64 " -> %s\n",
+            ops[op], modes[counts], src[0].read, src[1].read, pieces, written, argv[5]);
+    return 0;
 }
 
 // mode=accumulate: every chunk is only packed into super-window records (kc_accum_*); the count
@@ -289,6 +433,7 @@ int main(int argc, char **argv) {
     if (argc == 5 && strncmp(argv[1], "print", 5) == 0) return print_records(argv[2], strtoull(argv[4], nullptr, 10));
     if ((argc == 5 || argc == 6) && strcmp(argv[1], "histo") == 0)
         return histo_records(argv[2], argv[3], (uint32_t)strtoul(argv[4], nullptr, 10), argc == 6 ? strtoll(argv[5], nullptr, 10) : 10000);
+    if (argc >= 2 && strcmp(argv[1], "combine") == 0) return combine_files(argc, argv);
     Options opt = Options::parse(argc, argv);
     FinalRuns fin(opt);
     if (opt.inputFileDirectory.empty()) {
