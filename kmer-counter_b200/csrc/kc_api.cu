@@ -407,10 +407,8 @@ int count_enqueue_impl(kc_ctx *c, Pending &p, const void *d_reads, uint64_t n_by
         launches += 8;
     } else if (method == KC_COUNT_HASH) {
         // partitioned shared-memory hash counting (kc_partition.cu)
-        ExtractParams ep64;
-        static int pa_stage = -1;               // KC_PA_STAGE (development knob): bytes of reads per PA tile
-        if (pa_stage < 0) { const char *v = getenv("KC_PA_STAGE"); pa_stage = v ? atoi(v) : 6400; }
-        if (!extract_plan(d_reads, p.n_reads, L, k, c->key_flags, &p.d_scal[SC_INVALID], &ep64, (uint32_t)pa_stage))
+        ExtractParams ep64;                     // PA's tile: 6400 bytes of reads
+        if (!extract_plan(d_reads, p.n_reads, L, k, c->key_flags, &p.d_scal[SC_INVALID], &ep64, 6400))
             return c->set_error(KC_ERR_ARG, "unsupported shape k=%u read_len=%u", k, L);
         const uint64_t kb = p.n_slots * 8 * W + 64, cb = (p.n_slots + 2) * 4, wb = partition_workspace_bytes(p.n_slots);
         KC_TRY(arena_reserve(c, p, 2 * arena_round(kb) + arena_round(cb) + arena_round(wb), s));
@@ -1822,9 +1820,6 @@ int kc_merge_parts(kc_ctx *c, uint32_t n_src, const void *const *d_keys, const v
     void *ws = arena_take(ar, merge_parts_workspace_bytes(n_sub));
     unsigned long long *d_sc = static_cast<unsigned long long *>(arena_take(ar, 16));
     int launches = 0;
-    const bool dbg = getenv("KC_DEBUG_TIMING") != nullptr;
-    auto now = [&]() { cudaStreamSynchronize(s); timespec ts; clock_gettime(CLOCK_MONOTONIC, &ts); return ts.tv_sec * 1e3 + ts.tv_nsec * 1e-6; };
-    double t0 = dbg ? now() : 0;
     KC_CUDA_TRY(c, merge_parts_count(n_src, reinterpret_cast<const uint64_t *const *>(d_keys),
                                      reinterpret_cast<const uint32_t *const *>(d_counts),
                                      reinterpret_cast<const uint32_t *const *>(d_offsets), n_sub, (int)prefix_bits,
@@ -1833,11 +1828,9 @@ int kc_merge_parts(kc_ctx *c, uint32_t n_src, const void *const *d_keys, const v
     unsigned long long h[2] = {0, 0};
     KC_CUDA_TRY(c, cudaMemcpyAsync(h, d_sc, 16, cudaMemcpyDeviceToHost, s));
     KC_CUDA_TRY(c, cudaStreamSynchronize(s));
-    double t1 = dbg ? now() : 0;
     if (h[1]) return c->set_error(KC_ERR_CAPACITY, "kc_merge_parts: a key range could not be combined in shared memory");
     RunPtr r;
     KC_TRY(make_run(c, s, h[0], &r));
-    double t2 = dbg ? now() : 0;
     void *mem = nullptr;
     KC_TRY(dev_alloc(c, s, (uint64_t)(n_sub + 1) * 4, &mem));
     r->d_sub_off = static_cast<uint32_t *>(mem);
@@ -1847,7 +1840,6 @@ int kc_merge_parts(kc_ctx *c, uint32_t n_src, const void *const *d_keys, const v
                                       r->d_counts, r->d_sub_off, s));
     KC_CUDA_TRY(c, cudaStreamSynchronize(s));
     ar.arena_used = 0;
-    if (dbg) fprintf(stderr, "kc_merge_parts: count %.2f ms, alloc %.2f ms, gather %.2f ms\n", t1 - t0, t2 - t1, now() - t2);
     {
         std::lock_guard<std::mutex> g(c->mu);
         c->stats.launches += launches + 1;

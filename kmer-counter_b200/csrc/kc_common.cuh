@@ -135,40 +135,11 @@ __device__ __forceinline__ void st_release_u32(uint32_t *p, uint32_t v) {
     asm volatile("st.release.gpu.global.u32 [%0], %1;" ::"l"(p), "r"(v) : "memory");
 }
 
-// Called by ONE thread of the tile. Publishes `aggregate`, returns the exclusive
-// prefix over all earlier tiles, then publishes the inclusive value.
-__device__ __forceinline__ uint64_t lookback_exclusive(uint64_t *status, uint32_t tile, uint64_t aggregate) {
-    if (tile == 0) {
-        st_release_u64(&status[0], kLbInclusive | aggregate);
-        return 0;
-    }
-    st_release_u64(&status[tile], kLbAggregate | aggregate);
-    uint64_t excl = 0;
-    int64_t t = (int64_t)tile - 1;
-#ifdef KC_LB_WATCHDOG
-    uint32_t spins = 0;
-#endif
-    while (true) {
-        uint64_t s = ld_acquire_u64(&status[t]);
-        uint64_t st = s & ~kLbValueMask;
-        if (st == kLbEmpty) {
-#ifdef KC_LB_WATCHDOG
-            if (++spins > (1u << 22)) { printf("look-back: tile %u waits for tile %lld forever\n", tile, (long long)t); __trap(); }
-#endif
-            __nanosleep(20);
-            continue;
-        }
-        excl += s & kLbValueMask;
-        if (st == kLbInclusive) break;
-        t--;
-    }
-    st_release_u64(&status[tile], kLbInclusive | (excl + aggregate));
-    return excl;
-}
-
-// The same, called by ALL 32 lanes of one warp: a window of 32 predecessors is read per round
-// instead of one status word (a tile whose predecessors have only published their aggregates
-// walks back 32 at a time, not one L2 round trip each). Every lane returns the exclusive prefix.
+// Decoupled look-back, called by ALL 32 lanes of one warp of the tile. Publishes `aggregate`,
+// returns the exclusive prefix over all earlier tiles to every lane, then publishes the inclusive
+// value. A window of 32 predecessors is read per round instead of one status word (a tile whose
+// predecessors have only published their aggregates walks back 32 at a time, not one L2 round
+// trip each).
 __device__ __forceinline__ uint64_t lookback_exclusive_warp(uint64_t *status, uint32_t tile, uint64_t aggregate) {
     const uint32_t lane = threadIdx.x & 31;
     if (tile == 0) {

@@ -34,23 +34,14 @@ __device__ __forceinline__ uint32_t both_count(uint32_t a, uint32_t b, uint32_t 
     }
 }
 
-#ifndef KC_MERGE_THREADS
-#define KC_MERGE_THREADS 512
-#endif
-#ifndef KC_MERGE_IPT1
-#define KC_MERGE_IPT1 12
-#endif
-constexpr int kMergeThreads = KC_MERGE_THREADS;
+constexpr int kMergeThreads = 512;
 
 // items per thread of the tile kernel; a tile is kMergeThreads * IPT positions of the merged sequence.
 // Sweep on two runs of 129 M records (tools/merge_test/merge_perf.cu, profiles/r2/merge_sweep_s19.txt):
 // 256 x 8 with a one-thread look-back 3.69 ms, with the warp look-back 2.62, 512 x 12: 2.06 (W = 2: 256 x 6
 // 4.23 -> 512 x 8 3.77); 512 x 16 and 1024 x 8 are slower again (3.2 / 3.0 ms).
 template <int W> struct MergeCfg {
-#ifndef KC_MERGE_IPT2
-#define KC_MERGE_IPT2 8
-#endif
-    static constexpr int IPT = W == 1 ? KC_MERGE_IPT1 : (W == 2 ? KC_MERGE_IPT2 : 4);
+    static constexpr int IPT = W == 1 ? 12 : (W == 2 ? 8 : 4);
     static constexpr int TILE = kMergeThreads * IPT;
 };
 
@@ -202,13 +193,6 @@ __global__ void __launch_bounds__(kMergeThreads) merge_tile_kernel(
             o++;
         }
     }
-#ifdef KC_MERGE_SERIAL_LB
-    if (tid == 0) {
-        const uint64_t excl = lookback_exclusive(status, tile, total);
-        s_base = excl;
-        if (tile + 1 == n_tiles) *d_num_out = excl + total;
-    }
-#else
     if (warp == 0) {                        // the first warp looks back 32 tiles at a time
         const uint64_t excl = lookback_exclusive_warp(status, tile, total);
         if (lane == 0) {
@@ -216,7 +200,6 @@ __global__ void __launch_bounds__(kMergeThreads) merge_tile_kernel(
             if (tile + 1 == n_tiles) *d_num_out = excl + total;
         }
     }
-#endif
     __syncthreads();
     const uint64_t base = s_base;
     for (uint32_t i = tid; i < total; i += kMergeThreads) {

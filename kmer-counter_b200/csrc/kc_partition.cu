@@ -20,8 +20,6 @@
 //   PB  scatter2  keys grouped by the b1+b2 leading bits                 reads 8N, writes 8N
 //   PC  finish    per sub-bucket: shared-memory hash count, sort of the distinct keys,
 //                 ordered write via decoupled look-back                  reads 8N, writes 12U
-#include <stdlib.h>
-
 #include "kc_internal.h"
 
 namespace kc {
@@ -30,10 +28,8 @@ namespace {
 
 constexpr int kMaxBins = 1024;          // bins per level
 constexpr int kPbThreads = 256;
-#ifndef KC_PB_ITEMS
-#define KC_PB_ITEMS 16
-#endif
-template <int W> struct PbCfg { static constexpr int ITEMS = KC_PB_ITEMS / W, TILE = kPbThreads * ITEMS; };
+constexpr int kPbItems = 16;            // 64-bit keys a PB thread moves per tile (128-bit keys: half as many)
+template <int W> struct PbCfg { static constexpr int ITEMS = kPbItems / W, TILE = kPbThreads * ITEMS; };
 constexpr int kDefaultTarget = 3072;    // keys per sub-bucket the plan aims for
 
 // exclusive scan of nb (<= 1024) shared counters by THREADS threads; every thread returns the total
@@ -140,8 +136,6 @@ struct Scatter1Sink : SinkBase {
     uint32_t *g_cursor1;
     uint64_t *out;
     int shift1, nb1;
-    uint32_t *g_hist2;     // non-NULL: count the (b1+b2)-bit prefix of every key on the way out
-    int shift2;
     // shared
     uint32_t *cnt, *start, *gbase, *s_warp;
     Key<W> *staging;
@@ -192,10 +186,11 @@ struct Scatter1Sink : SinkBase {
                 if (b < nb1) gbase[b] = reserved[u] - start[b];            // dst = gbase[d] + staging index
             }
             __syncthreads();
+            // (not unrolled: unrolled by 4, this loop made PA 5 % slower on a B200, 3.18 -> 3.33 ms at C2)
+#pragma unroll 1
             for (uint32_t i = threadIdx.x; i < total; i += kExtractThreads) {
                 const Key<W> k = staging[i];
                 st_key<W>(out, gbase[k.w[0] >> shift1] + i, k);
-                if (g_hist2) atomicAdd(&g_hist2[k.w[0] >> shift2], 1u);
             }
             for (int b = threadIdx.x; b < nb1; b += kExtractThreads) cnt[b] = 0;
             __syncthreads();
@@ -389,8 +384,6 @@ struct FinishParams {
     unsigned long long *d_overflow;
     const unsigned long long *d_n_invalid;
     int add_phantom;               // KC_COMPAT_REF: key 0 exists whenever a slot was empty (SURVEY F7)
-    int cap_shift;                 // (unused)
-    float cap_factor;              // table slots per expected distinct key (first guess)
     const uint32_t *list;          // optional: only these sub-buckets (NULL = all)
     const uint32_t *list_count;
     uint32_t *tmp_start;           // [n_sub] where sub-bucket j's records start in tmp (written here, read by the gather)
@@ -402,9 +395,10 @@ struct FinishParams {
     const uint32_t *src_off[8];
 };
 
-#ifndef KC_PC_BATCH
-#define KC_PC_BATCH 4      // keys a thread loads before it starts inserting them (sweep: 16 -> 7.35 ms, 8 -> 6.41, 4 -> 6.03, 2 -> 6.04)
-#endif
+// keys a thread loads before it starts inserting them (64-bit keys, sweep: 16 -> 7.35 ms, 8 -> 6.41, 4 -> 6.03,
+// 2 -> 6.04; 128-bit keys: 4 measured better than 2)
+constexpr int kPcBatch = 4;
+constexpr float kPcLoad = 2.0f;    // table slots per expected distinct key (first guess)
 constexpr int kSortBins = 1024;    // most bins the in-table counting sort uses
 
 __device__ __forceinline__ uint32_t pow2_ceil_u32(uint32_t x) { return x <= 1 ? 1u : 1u << (32 - __clz(x - 1)); }
@@ -543,23 +537,22 @@ __global__ void __launch_bounds__(kPcThreads) finish_kernel(FinishParams p) {
                     }
                 }
             } else {
-                constexpr int kBatch = W == 1 ? KC_PC_BATCH : 4;     // 128-bit keys: 4 measured better than 2
                 // A sub-bucket far larger than the plan's target holds heavy hitters (skewed input):
                 // there the lanes of a warp that carry the same key are combined first (MATCH.ANY) and
                 // one of them adds their number, instead of 32 atomics serialising on one counter.
                 const bool hot = (end - begin) > 16384u;
                 if (!hot) {
-                    for (uint32_t i0 = begin; i0 < end; i0 += kPcThreads * kBatch) {
+                    for (uint32_t i0 = begin; i0 < end; i0 += kPcThreads * kPcBatch) {
                         if (*reinterpret_cast<volatile uint32_t *>(&s_over)) break;
-                        Key<W> kk[kBatch];
+                        Key<W> kk[kPcBatch];
 #pragma unroll
-                        for (int u = 0; u < kBatch; u++) {
+                        for (int u = 0; u < kPcBatch; u++) {
                             const uint32_t i = i0 + u * kPcThreads + tid;
                             if (i < end) kk[u] = ld_key<W>(p.keys, i);
                             else kk[u].w[0] = 0;
                         }
 #pragma unroll
-                        for (int u = 0; u < kBatch; u++) {
+                        for (int u = 0; u < kPcBatch; u++) {
                             const uint32_t i = i0 + u * kPcThreads + tid;
                             if (i >= end) continue;
                             const Key<W> k = kk[u];
@@ -732,7 +725,7 @@ __global__ void __launch_bounds__(kPcThreads) finish_kernel(FinishParams p) {
         // many distinct keys, and a wrong optimistic guess is abandoned after a couple of thousand keys)
         uint32_t round_bits = 0;
         while ((expect >> round_bits) > (uint32_t)kLcap && round_bits < 2) round_bits++;
-        uint32_t cap = pow2_ceil_u32((uint32_t)(p.cap_factor * (float)(expect >> round_bits)));
+        uint32_t cap = pow2_ceil_u32((uint32_t)(kPcLoad * (float)(expect >> round_bits)));
         cap = cap < 256 ? 256 : (cap > (uint32_t)kHcap ? (uint32_t)kHcap : cap);
         while (true) {
             const uint32_t n_rounds = 1u << round_bits;
@@ -765,8 +758,11 @@ __global__ void __launch_bounds__(kPcThreads) finish_kernel(FinishParams p) {
     }
 }
 
-template <int THREADS, int HCAP, bool MULTI = false, int W = 1>
-cudaError_t launch_finish_v(const FinishParams &fp, int n_sms, uint32_t n_sub, cudaStream_t s) {
+// PC's CTA and table shape: 256 threads and 2048 slots, the best of the sweep over CTA and table
+// sizes in profiles/r1/finish_variant_sweep.txt
+template <bool MULTI, int W>
+cudaError_t launch_finish(const FinishParams &fp, int n_sms, uint32_t n_sub, cudaStream_t s) {
+    constexpr int THREADS = 256, HCAP = 2048;
     constexpr uint32_t smem = HCAP * (8 * W + 4) + (HCAP / 2) * (8 * W + 4);
     auto kern = finish_kernel<THREADS, HCAP, MULTI, W>;
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
@@ -778,27 +774,6 @@ cudaError_t launch_finish_v(const FinishParams &fp, int n_sms, uint32_t n_sub, c
     if (grid > n_sub) grid = n_sub;
     kern<<<grid, THREADS, smem, s>>>(fp);
     return cudaGetLastError();
-}
-
-// KC_PC_VARIANT (development knob): CTA size / table size of the finish kernel
-cudaError_t launch_finish(const FinishParams &fp, int n_sms, uint32_t n_sub, cudaStream_t s) {
-    static int variant = -1;
-    if (variant < 0) {
-        const char *v = getenv("KC_PC_VARIANT");
-        variant = v ? atoi(v) : 0;
-    }
-    switch (variant) {
-        case 1: return launch_finish_v<128, 2048>(fp, n_sms, n_sub, s);
-        case 2: return launch_finish_v<128, 4096>(fp, n_sms, n_sub, s);
-        case 3: return launch_finish_v<64, 1024>(fp, n_sms, n_sub, s);
-        case 4: return launch_finish_v<256, 2048>(fp, n_sms, n_sub, s);
-        case 5: return launch_finish_v<256, 1024>(fp, n_sms, n_sub, s);
-        case 6: return launch_finish_v<512, 2048>(fp, n_sms, n_sub, s);
-        case 7: return launch_finish_v<512, 4096>(fp, n_sms, n_sub, s);
-        case 8: return launch_finish_v<384, 2048>(fp, n_sms, n_sub, s);
-        case 9: return launch_finish_v<256, 4096>(fp, n_sms, n_sub, s);
-        default: return launch_finish_v<256, 2048>(fp, n_sms, n_sub, s);   // best of the sweep in profiles/r1
-    }
 }
 
 // records of sub-bucket j: tmp[src(j) .. src(j) + m_j) -> out[off[j] ...); one warp per sub-bucket
@@ -897,12 +872,10 @@ cudaError_t merge_parts_count(uint32_t n_src, const uint64_t *const *src_keys, c
     fp.tmp_counts = tmp_counts;
     fp.m_out = m_out;
     fp.d_overflow = d_overflow;
-    fp.cap_shift = 1;
-    fp.cap_factor = 2.0f;
     fp.tmp_start = tmp_start;
     fp.n_src = n_src;
     for (uint32_t i = 0; i < n_src; i++) { fp.src_keys[i] = src_keys[i]; fp.src_counts[i] = src_counts[i]; fp.src_off[i] = src_off[i]; }
-    if ((e = launch_finish_v<256, 2048, true, 1>(fp, n_sms, n_sub, s)) != cudaSuccess) return e;
+    if ((e = launch_finish<true, 1>(fp, n_sms, n_sub, s)) != cudaSuccess) return e;
     scan2_kernel<<<(n_sub + kScan2Tile - 1) / kScan2Tile, 1024, 0, s>>>(m_out, n_sub, off, scratch);
     if ((e = cudaMemcpyAsync(d_num_out, off + n_sub, 4, cudaMemcpyDeviceToDevice, s)) != cudaSuccess) return e;
     if (n_launches) *n_launches += 2;
@@ -959,16 +932,12 @@ static cudaError_t partition_count_w(const ExtractParams &ep_in, uint64_t n_slot
     if ((e = cudaMemsetAsync(d_overflow, 0, 8, s)) != cudaSuccess) return e;
 
     const int shift1 = 64 - pl.b1, shift2 = 64 - pl.b1 - pl.b2;
-    static int fuse_h2 = -1;                // KC_FUSE_H2=1 (development knob): level-2 histogram by REDs inside PA
-    if (fuse_h2 < 0) { const char *v = getenv("KC_FUSE_H2"); fuse_h2 = (v && v[0] == '1') ? 1 : 0; }
     // P0: level-1 histogram (invalid-slot count goes to a scratch counter: PA counts it for real)
     {
-        // the histogram pass keeps nothing per tile, so it takes larger tiles than PA (fewer barriers per read)
+        // the histogram pass keeps nothing per tile, so it takes larger tiles than PA (fewer barriers
+        // per read): 12800 bytes of reads
         ExtractParams ep = ep_in;
-        static int p0_stage = -1;               // KC_P0_STAGE (development knob): bytes of reads per P0 tile
-        if (p0_stage < 0) { const char *v = getenv("KC_P0_STAGE"); p0_stage = v ? atoi(v) : 12800; }
-        if (!extract_plan(ep_in.reads, ep_in.n_reads, ep_in.L, ep_in.k, ep_in.plan_flags, d_scratch_invalid, &ep,
-                          (uint32_t)p0_stage))
+        if (!extract_plan(ep_in.reads, ep_in.n_reads, ep_in.L, ep_in.k, ep_in.plan_flags, d_scratch_invalid, &ep, 12800))
             ep = ep_in;
         ep.n_invalid = d_scratch_invalid;
         auto kern = extract_kernel_for<W, Hist1Sink<W>>(ep_in);
@@ -999,16 +968,13 @@ static cudaError_t partition_count_w(const ExtractParams &ep_in, uint64_t n_slot
         if (grid > ep_in.n_tiles) grid = ep_in.n_tiles;
         Scatter1Sink<W> sink{};
         sink.g_cursor1 = cursor1; sink.out = keys_a; sink.shift1 = shift1; sink.nb1 = (int)pl.nb1;
-        sink.g_hist2 = (fuse_h2 && pl.b2 > 0) ? hist2 : nullptr;
-        sink.shift2 = shift2;
         kern<<<grid, kExtractThreads, smem, s>>>(ep_in, sink);
         if ((e = cudaGetLastError()) != cudaSuccess) return e;
     }
     if (evs) cudaEventRecord(evs[1], s);
     // H2 + PB over the level-1 buckets
     if (pl.b2 > 0) {
-        if (!fuse_h2)
-            hist2_kernel<W><<<(uint32_t)div_up(n_slots, (uint64_t)kH2Chunk), kPbThreads, 0, s>>>(keys_a, base1 + pl.nb1, pl.b2, shift2, hist2);
+        hist2_kernel<W><<<(uint32_t)div_up(n_slots, (uint64_t)kH2Chunk), kPbThreads, 0, s>>>(keys_a, base1 + pl.nb1, pl.b2, shift2, hist2);
         scan2_kernel<<<(pl.n_sub + kScan2Tile - 1) / kScan2Tile, 1024, 0, s>>>(hist2, pl.n_sub, base2, cursor2);
         if (evs) cudaEventRecord(evs[2], s);
         scatter2_kernel<W><<<(uint32_t)div_up(n_slots, (uint64_t)PbCfg<W>::TILE), kPbThreads, 0, s>>>(
@@ -1027,14 +993,9 @@ static cudaError_t partition_count_w(const ExtractParams &ep_in, uint64_t n_slot
         FinishParams fp{};
         fp.keys = grouped; fp.base2 = base2; fp.n_sub = pl.n_sub; fp.prefix_bits = pl.b1 + pl.b2;
         fp.tmp_keys = out_keys; fp.tmp_counts = out_counts; fp.m_out = m_out; fp.d_overflow = d_overflow;
-        fp.d_n_invalid = ep_in.n_invalid; fp.add_phantom = add_phantom ? 1 : 0; fp.cap_shift = 1;
-        static float cap_factor = -1.f;             // KC_PC_LOAD (development knob): slots per expected distinct key
-        if (cap_factor < 0) { const char *v = getenv("KC_PC_LOAD"); cap_factor = v ? (float)atof(v) : 2.0f; }
-        fp.cap_factor = cap_factor;
+        fp.d_n_invalid = ep_in.n_invalid; fp.add_phantom = add_phantom ? 1 : 0;
         fp.tmp_start = status_scratch + pl.n_sub + 8;
-        if constexpr (W == 1) e = launch_finish(fp, n_sms, pl.n_sub, s);
-        else e = launch_finish_v<256, 2048, false, W>(fp, n_sms, pl.n_sub, s);
-        if (e != cudaSuccess) return e;
+        if ((e = launch_finish<false, W>(fp, n_sms, pl.n_sub, s)) != cudaSuccess) return e;
         // off[] (n_sub + 1) overwrites cursor2; its last entry is the number of records
         scan2_kernel<<<(pl.n_sub + kScan2Tile - 1) / kScan2Tile, 1024, 0, s>>>(m_out, pl.n_sub, cursor2, status_scratch);
         if ((e = cudaMemcpyAsync(d_num_out, cursor2 + pl.n_sub, 4, cudaMemcpyDeviceToDevice, s)) != cudaSuccess) return e;

@@ -428,6 +428,14 @@ struct SwCountParams {
     unsigned long long *sc;
 };
 
+// S2's CTA and table shape, the one instantiated for each key width: 512 threads and a 4096-slot
+// table, with rounds of 2 records per thread for 64-bit keys (whole bins per round: 5.06 ms at C2
+// against 6.06 ms with 1) and 1 for 128-bit keys. Picked by a sweep over CTA sizes (128 to 512),
+// table sizes (2048 to 8192 slots) and records per thread (1 to 4); see DESIGN §4.1.
+template <int W> struct SwCountCfg {
+    static constexpr int THREADS = 512, TSLOTS = 4096, RPT = W == 1 ? 2 : 1;
+};
+
 // One work unit = one bin, or one slice of the overflow list. The CTA stages RPT * THREADS records
 // at a time, splits their windows evenly over its threads (a thread takes a contiguous range of
 // the flattened window sequence, so it slides the window inside a record and every lane has the
@@ -438,7 +446,7 @@ struct SwCountParams {
 // passes, pass v counting the keys whose pass hash starts with v: the records a unit emits are
 // always key-distinct.
 // CANON: every window's key is min(forward, rc) (the records still hold forward bases).
-template <int W, int THREADS, int TSLOTS, int RPT, bool CANON = false>
+template <int W, int THREADS, int TSLOTS, int RPT, bool CANON>
 __global__ void __launch_bounds__(THREADS) sw_count_kernel(SwCountParams p) {
     constexpr int RB = THREADS * RPT;                                       // records per round
     extern __shared__ __align__(16) uint8_t cs_smem[];
@@ -452,7 +460,7 @@ __global__ void __launch_bounds__(THREADS) sw_count_kernel(SwCountParams p) {
     uint32_t *queue_m = reinterpret_cast<uint32_t *>(queue + (THREADS / 32) * kQueue);   // their weights
     // record-level table (DEDUP): equal records of a round are counted once, with a multiplicity
     constexpr bool DEDUP = (W == 1);
-    constexpr int RT = DEDUP ? (RPT > 1 ? RB : 2 * RB) : 1;               // (whole-bin rounds: records are ~40% distinct)
+    constexpr int RT = DEDUP ? RB : 1;                                      // (whole-bin rounds: records are ~40% distinct)
     ulonglong2 *rt_keys = reinterpret_cast<ulonglong2 *>(queue_m + (THREADS / 32) * kQueue);   // [RT]
     uint32_t *rt_mult = reinterpret_cast<uint32_t *>(rt_keys + RT);         // [RT]
     uint32_t *rec_mult = rt_mult + RT;                                      // [RB] weight of staged record i (0: a duplicate)
@@ -1984,10 +1992,9 @@ cudaError_t super_reset(const SuperPlan &pl, void *ws, unsigned long long *d_sc,
 template <int W>
 static cudaError_t super_scatter_w(const SuperPlan &pl, const void *d_reads, uint64_t n_reads, void *ws,
                                    unsigned long long *d_sc, int n_sms, cudaStream_t s) {
-    static int tile_bytes = -1;                 // KC_SW_STAGE (development knob): bytes of reads per S1 tile
-    if (tile_bytes < 0) { const char *v = getenv("KC_SW_STAGE"); tile_bytes = v ? atoi(v) : 4800; }   // 3200: 3.82 ms, 4800: 3.60, 6400: 4.0, 9600: 4.28 at C2
+    constexpr uint32_t kTileBytes = 4800;       // bytes of reads per S1 tile (3200: 3.82 ms, 4800: 3.60, 6400: 4.0, 9600: 4.28 at C2)
     SwScatterParams q{};
-    if (!extract_plan(d_reads, n_reads, pl.L, pl.k, pl.flags, &d_sc[SW_INVALID], &q.ep, (uint32_t)tile_bytes))
+    if (!extract_plan(d_reads, n_reads, pl.L, pl.k, pl.flags, &d_sc[SW_INVALID], &q.ep, kTileBytes))
         return cudaErrorInvalidValue;
     if (q.ep.n_tiles == 0) return cudaSuccess;
     q.m = pl.m; q.w = pl.w; q.nh = pl.nh; q.nh_stride = pl.nh_stride;
@@ -2030,9 +2037,10 @@ cudaError_t super_scatter(const SuperPlan &pl, const void *d_reads, uint64_t n_r
     return cudaErrorInvalidValue;
 }
 
-template <int W, int THREADS, int TSLOTS, int RPT = 2, bool CANON = false>
+template <int W, bool CANON>
 static cudaError_t launch_count(const SwCountParams &cp, int n_sms, cudaStream_t s) {
-    const uint32_t RB = THREADS * RPT, RT = W == 1 ? (RPT > 1 ? RB : 2 * RB) : 1;
+    constexpr uint32_t THREADS = SwCountCfg<W>::THREADS, TSLOTS = SwCountCfg<W>::TSLOTS, RPT = SwCountCfg<W>::RPT;
+    const uint32_t RB = THREADS * RPT, RT = W == 1 ? RB : 1;
     const uint32_t smem = TSLOTS * (8 * W + 4) + RB * 16 * W + THREADS * 4 + kNb1Max * 4 +
                           (THREADS / 32) * (RPT > 1 ? 64 : 96) * (8 * W + 4) + RT * 20 + RB * 4 + 64;
     auto kern = sw_count_kernel<W, THREADS, TSLOTS, RPT, CANON>;
@@ -2049,7 +2057,6 @@ template <int W>
 static cudaError_t super_count_bins_w(const SuperPlan &pl, bool add_phantom, void *ws, unsigned long long *d_sc, int n_sms,
                                       cudaStream_t s, void *const *peer_ws = nullptr, uint32_t rank = 0,
                                       uint32_t n_ranks = 1) {
-    cudaError_t e;
     SwCountParams cp{};
     const uint32_t n_src = peer_ws ? n_ranks : 1u;
     cp.n_src = n_src;
@@ -2069,34 +2076,7 @@ static cudaError_t super_count_bins_w(const SuperPlan &pl, bool add_phantom, voi
     cp.hist1 = at<uint32_t>(ws, pl.off_hist1); cp.shift1 = 64 - pl.b1; cp.nb1 = 1 << pl.b1;
     cp.add_phantom = add_phantom ? 1 : 0;
     cp.sc = d_sc;
-    // canonical keys: the default shapes only (the KC_SW_COUNT variants below are forward-only)
-    if (pl.flags & kPlanCanonical) return W == 1 ? launch_count<1, 512, 4096, 2, true>(cp, n_sms, s)
-                                                 : launch_count<2, 512, 4096, 1, true>(cp, n_sms, s);
-    static int variant = -1;                    // KC_SW_COUNT (development knob): CTA / table shape of S2
-    if (variant < 0) { const char *v = getenv("KC_SW_COUNT"); variant = v ? atoi(v) : 0; }
-    if constexpr (W == 1) {
-        switch (variant) {
-            case 1: e = launch_count<1, 256, 2048, 2>(cp, n_sms, s); break;
-            case 2: e = launch_count<1, 512, 4096, 1>(cp, n_sms, s); break;
-            case 3: e = launch_count<1, 512, 8192, 1>(cp, n_sms, s); break;
-            case 4: e = launch_count<1, 128, 4096, 2>(cp, n_sms, s); break;
-            case 5: e = launch_count<1, 128, 2048, 2>(cp, n_sms, s); break;
-            case 6: e = launch_count<1, 256, 4096, 1>(cp, n_sms, s); break;
-            case 7: e = launch_count<1, 256, 4096, 4>(cp, n_sms, s); break;
-            case 8: e = launch_count<1, 512, 4096, 1>(cp, n_sms, s); break;
-            case 9: e = launch_count<1, 384, 4096, 2>(cp, n_sms, s); break;
-            case 10: e = launch_count<1, 256, 4096, 2>(cp, n_sms, s); break;
-            default: e = launch_count<1, 512, 4096, 2>(cp, n_sms, s); break;   // whole bins per round: 5.06 ms at C2 (RPT 1: 6.06)
-        }
-    } else {
-        switch (variant) {
-            case 1: e = launch_count<2, 256, 2048, 1>(cp, n_sms, s); break;
-            case 2: e = launch_count<2, 256, 4096, 1>(cp, n_sms, s); break;
-            case 3: e = launch_count<2, 256, 4096, 2>(cp, n_sms, s); break;
-            default: e = launch_count<2, 512, 4096, 1>(cp, n_sms, s); break;
-        }
-    }
-    return e;
+    return (pl.flags & kPlanCanonical) ? launch_count<W, true>(cp, n_sms, s) : launch_count<W, false>(cp, n_sms, s);
 }
 
 cudaError_t super_count_bins(const SuperPlan &pl, bool add_phantom, void *ws, unsigned long long *d_sc, int n_sms,

@@ -1,7 +1,8 @@
 // Timing of kc::merge_pair (kc_merge.cu) on two device-generated sorted unique runs of C2's shape
-// (2 x 129 M 64-bit records, ~78 % of the keys shared), for compile-time variants of the kernel:
-//   nvcc -gencode arch=compute_100a,code=sm_100a -std=c++17 -O3 -I../../kmer-counter_b200/csrc [-DKC_MERGE_IPT1=12 ...] \
-//        merge_perf.cu ../../kmer-counter_b200/csrc/kc_merge.cu -o merge_perf_<variant>
+// (2 x 129 M 64-bit records, ~78 % of the keys shared), with the tile shape kc_merge.cu is built with
+// (the sweep of tile shapes in profiles/r2/merge_sweep_s19.txt was taken with this harness):
+//   nvcc -gencode arch=compute_100a,code=sm_100a -std=c++17 -O3 -I../../kmer-counter_b200/csrc \
+//        merge_perf.cu ../../kmer-counter_b200/csrc/kc_merge.cu -o merge_perf
 #include <cstdio>
 #include <cstdlib>
 #include "kc_internal.h"
