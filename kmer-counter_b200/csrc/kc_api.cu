@@ -327,18 +327,27 @@ int static_zero_bits(const kc_ctx *c) {
 
 constexpr uint64_t kMaxSortKeys = (1ull << 30) - 1;
 
-// the super-window path takes 64/128-bit keys whose windows span at least 22 bases
+// the super-window path takes 64/128-bit keys whose windows span at least 22 bases, from reads
+// short enough for S1's shared memory (every plan super_plan makes for the shape fits it then)
 bool super_ok(const kc_ctx *c) {
     SuperPlan pl;
-    return c->W <= 2 && super_plan(c->cfg.k, c->cfg.read_len, c->key_flags, 1, 0, &pl) && super_supported(pl);
+    return c->W <= 2 && super_plan(c->cfg.k, c->cfg.read_len, c->key_flags, 1, 0, &pl);
+}
+
+// the partitioned hash takes 64/128-bit keys from reads short enough for PA's shared-memory tile
+bool hash_ok(const kc_ctx *c) {
+    ExtractParams ep;
+    return c->W <= 2 && extract_plan(nullptr, 16, c->cfg.read_len, c->cfg.k, c->key_flags, nullptr, &ep, kPaTileBytes) &&
+           partition_fits(ep, c->W);
 }
 
 uint32_t pick_method(const kc_ctx *c) {
     uint32_t m = c->cfg.method;
-    if (m == KC_COUNT_SUPER) return super_ok(c) ? KC_COUNT_SUPER : (c->W > 2 ? KC_COUNT_SORT : KC_COUNT_HASH);
+    if (m == KC_COUNT_SUPER) return super_ok(c) ? KC_COUNT_SUPER : (hash_ok(c) ? KC_COUNT_HASH : KC_COUNT_SORT);
     if (m == KC_COUNT_AUTO && super_ok(c)) return KC_COUNT_SUPER;
     if (m == KC_COUNT_PLACE) return KC_COUNT_PLACE;
     if (c->W > 2) return m == KC_COUNT_AUTO ? KC_COUNT_PLACE : KC_COUNT_SORT;   // 192/256-bit keys: MSD placement + fold (auto), or sort + run-length
+    if ((m == KC_COUNT_AUTO || m == KC_COUNT_HASH) && !hash_ok(c)) return KC_COUNT_SORT;    // reads too long for PA
     if (c->W == 2) return (m == KC_COUNT_AUTO || m == KC_COUNT_HASH) ? KC_COUNT_HASH : KC_COUNT_SORT;
     // 64-bit keys: partitioned shared-memory hashing unless the key has too few significant
     // bits to partition on (tiny k); see DESIGN.md "method selection"
@@ -407,8 +416,8 @@ int count_enqueue_impl(kc_ctx *c, Pending &p, const void *d_reads, uint64_t n_by
         launches += 8;
     } else if (method == KC_COUNT_HASH) {
         // partitioned shared-memory hash counting (kc_partition.cu)
-        ExtractParams ep64;                     // PA's tile: 6400 bytes of reads
-        if (!extract_plan(d_reads, p.n_reads, L, k, c->key_flags, &p.d_scal[SC_INVALID], &ep64, 6400))
+        ExtractParams ep64;                     // PA's tile
+        if (!extract_plan(d_reads, p.n_reads, L, k, c->key_flags, &p.d_scal[SC_INVALID], &ep64, kPaTileBytes))
             return c->set_error(KC_ERR_ARG, "unsupported shape k=%u read_len=%u", k, L);
         const uint64_t kb = p.n_slots * 8 * W + 64, cb = (p.n_slots + 2) * 4, wb = partition_workspace_bytes(p.n_slots);
         KC_TRY(arena_reserve(c, p, 2 * arena_round(kb) + arena_round(cb) + arena_round(wb), s));
@@ -592,7 +601,7 @@ void stage_stats(kc_stats &st, int n_stages, const float *ms, const uint64_t *by
 // which sizes everything from exact histograms; a sub-bucket arrangement the placement path cannot
 // take, or a full hash table -> sort + run-length.
 uint32_t fallback(const kc_ctx *c, uint32_t m) {
-    return m == KC_COUNT_SUPER && c->W <= 2 ? KC_COUNT_HASH : KC_COUNT_SORT;
+    return m == KC_COUNT_SUPER && hash_ok(c) ? KC_COUNT_HASH : KC_COUNT_SORT;
 }
 
 int count_finish_method(kc_ctx *c, Pending &p, cudaStream_t s, RunPtr *out);
@@ -1195,7 +1204,13 @@ int kc_accum_begin(kc_ctx *c, uint64_t expected_reads) {
 static int accum_begin_impl(kc_ctx *c, uint64_t expected_reads, bool exchange, uint32_t n_ranks) {
     std::lock_guard<std::recursive_mutex> dg(c->direct_mu);
     cudaSetDevice(c->cfg.device);
-    if (!super_ok(c)) return c->set_error(KC_ERR_ARG, "accumulating mode needs k <= 64 with windows of >= 22 bases (k=%u)", c->cfg.k);
+    if (!super_ok(c)) {
+        SuperPlan pl;
+        if (c->W <= 2 && super_plan(c->cfg.k, c->cfg.k, c->key_flags, 1, 0, &pl))      // k is fine: the reads are too long
+            return c->set_error(KC_ERR_ARG, "accumulating mode: reads of %u bases are too long for the super-window path at k=%u",
+                                c->cfg.read_len, c->cfg.k);
+        return c->set_error(KC_ERR_ARG, "accumulating mode needs k <= 64 with windows of >= 22 bases (k=%u)", c->cfg.k);
+    }
     const uint64_t nk = c->cfg.read_len - c->cfg.k + 1;
     uint64_t chunk_reads = c->cfg.max_chunk_bytes / c->cfg.read_len;
     if (expected_reads < chunk_reads) expected_reads = chunk_reads;

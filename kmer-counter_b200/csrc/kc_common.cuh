@@ -214,6 +214,7 @@ __device__ __forceinline__ void tma_load_1d(void *smem_dst, const void *gmem_src
         if (_e != cudaSuccess) {                                                             \
             (ctx)->set_error(KC_ERR_CUDA, "%s failed: %s (%s:%d)", #expr, cudaGetErrorString(_e), __FILE__, \
                              __LINE__);                                                      \
+            cudaGetLastError();  /* a refused call's error must not surface at the next launch check */ \
             return KC_ERR_CUDA;                                                              \
         }                                                                                    \
     } while (0)

@@ -124,6 +124,11 @@ cudaError_t merge_parts_count(uint32_t n_src, const uint64_t *const *src_keys, c
                               void *ws, int n_sms, cudaStream_t s, int *n_launches);
 cudaError_t merge_parts_gather(uint32_t n_sub, const uint64_t *tmp_keys, const uint32_t *tmp_counts, void *ws,
                                uint64_t *out_keys, uint32_t *out_counts, uint32_t *out_offsets, cudaStream_t s);
+// PA's tile: extract_plan with kPaTileBytes of reads (16 reads from L = 201 on)
+constexpr uint32_t kPaTileBytes = 6400;
+// false when PA cannot take a tile of ep: the extraction's buffers and the tile's keys, staged by level-1
+// digit, exceed a CTA's shared memory (long reads: from about 1200 bases for 64-bit keys, 700 for 128-bit)
+bool partition_fits(const ExtractParams &ep, int W);
 cudaError_t partition_count(int W, const ExtractParams &ep, uint64_t n_slots, int sig_bits, bool add_phantom,
                             uint64_t *keys_a, uint64_t *keys_b, uint64_t *out_keys, uint32_t *out_counts,
                             unsigned long long *d_num_out, unsigned long long *d_overflow,

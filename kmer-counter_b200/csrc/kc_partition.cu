@@ -1005,6 +1005,13 @@ static cudaError_t partition_count_w(const ExtractParams &ep_in, uint64_t n_slot
     return cudaSuccess;
 }
 
+bool partition_fits(const ExtractParams &ep, int W) {
+    constexpr uint64_t kMaxSmemOptin = 227 * 1024;          // a CTA's dynamic shared memory on sm_100
+    const uint32_t keys = ep.tile_reads * ep.nk;
+    const uint64_t extra = W == 1 ? Scatter1Sink<1>::smem_bytes(keys) : Scatter1Sink<2>::smem_bytes(keys);
+    return (W == 1 || W == 2) && ep.smem_total + extra <= kMaxSmemOptin;
+}
+
 cudaError_t partition_count(int W, const ExtractParams &ep, uint64_t n_slots, int sig_bits, bool add_phantom,
                             uint64_t *keys_a, uint64_t *keys_b, uint64_t *out_keys, uint32_t *out_counts,
                             unsigned long long *d_num_out, unsigned long long *d_overflow,

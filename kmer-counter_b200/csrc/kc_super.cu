@@ -1831,6 +1831,34 @@ constexpr int kFinCapWide = 1024;                           // ... of 192/256-bi
 // ------------------------------------------------------------------------ host
 static void plan_layout(SuperPlan &pl, bool ext_e);
 
+namespace {
+constexpr uint32_t kS1TileBytes = 4800;         // bytes of reads per S1 tile (3200: 3.82 ms, 4800: 3.60, 6400: 4.0, 9600: 4.28 at C2)
+constexpr uint32_t kS1MaxSmem = 200 * 1024;     // S1's dynamic shared memory at most
+
+// S1's dynamic shared memory: the extraction's tile (ep: extract_plan with kS1TileBytes), then per
+// read of the tile the m-mer hashes, the windows' bins and two words per segment
+struct S1Smem { uint32_t h_off, bin_off, bits_off, total; };
+S1Smem s1_smem(const SuperPlan &pl, const ExtractParams &ep) {
+    S1Smem r;
+    r.h_off = (ep.smem_total + 15u) & ~15u;
+    r.bin_off = r.h_off + ep.tile_reads * pl.nh_stride * 4;
+    r.bits_off = r.bin_off + ep.tile_reads * pl.nk * 4;
+    r.total = r.bits_off + 2 * ep.tile_reads * pl.segs_per_read * 4;
+    return r;
+}
+
+// minimizer length m and what follows from it: window of w m-mers, rows of m-mer hashes, segments
+void set_minimizer(SuperPlan &pl, uint32_t m) {
+    pl.m = m;
+    pl.w = pl.span - pl.m + 1;
+    pl.nh = pl.nk + pl.w - 1;
+    pl.nh_stride = (pl.nh + 8) | 1u;                                   // odd stride: rows start in different banks
+    pl.seg_len = pl.w - 1 < (uint32_t)kSwMaxSeg - 1 ? pl.w - 1 : (uint32_t)kSwMaxSeg - 1;   // + the look-behind window
+    pl.segs_per_read = (pl.nk + pl.seg_len - 1) / pl.seg_len;
+    pl.seg_len = (pl.nk + pl.segs_per_read - 1) / pl.segs_per_read;    // even the segments out
+}
+}  // namespace
+
 bool super_plan(uint32_t k, uint32_t L, uint32_t flags, uint64_t max_windows, uint32_t occ_per_bin, SuperPlan *out,
                 double record_headroom, uint64_t distinct_hint, bool ext_e) {
     if (k == 0 || k > 64 || L < k || L > 4096) return false;
@@ -1870,14 +1898,20 @@ bool super_plan(uint32_t k, uint32_t L, uint32_t flags, uint64_t max_windows, ui
     // overflow (seen at 1e6 bins with m = 12). So m grows with the bin count: 12 up to 87k bins
     // (config 2), 13 up to 350k, 14 up to 1.4M, ... -- longer minimizers change more often
     // (2 / (w + 1) records per window), which costs a few percent more records.
-    pl.m = 12;
-    while (pl.m < 16 && pl.m + 8 < pl.span && (1ull << (2 * pl.m)) < 192ull * pl.n_bins) pl.m++;
-    pl.w = pl.span - pl.m + 1;
-    pl.nh = pl.nk + pl.w - 1;
-    pl.nh_stride = (pl.nh + 8) | 1u;                                   // odd stride: rows start in different banks
-    pl.seg_len = pl.w - 1 < (uint32_t)kSwMaxSeg - 1 ? pl.w - 1 : (uint32_t)kSwMaxSeg - 1;   // + the look-behind window
-    pl.segs_per_read = (pl.nk + pl.seg_len - 1) / pl.seg_len;
-    pl.seg_len = (pl.nk + pl.segs_per_read - 1) / pl.segs_per_read;    // even the segments out
+    // A longer minimizer also means shorter segments, so more of S1's shared memory per read: near
+    // the longest reads the path takes, m stops growing where S1 would no longer fit (uneven bins
+    // then only send more records to the overflow list). Reads too long for S1 even at m = 12 are
+    // not for this path, whatever the plan's size.
+    ExtractParams ep;
+    if (!extract_plan(nullptr, 16, L, k, pl.flags, nullptr, &ep, kS1TileBytes)) return false;
+    set_minimizer(pl, 12);
+    if (s1_smem(pl, ep).total > kS1MaxSmem) return false;
+    while (pl.m < 16 && pl.m + 8 < pl.span && (1ull << (2 * pl.m)) < 192ull * pl.n_bins) {
+        SuperPlan longer = pl;
+        set_minimizer(longer, pl.m + 1);
+        if (s1_smem(longer, ep).total > kS1MaxSmem) break;
+        pl = longer;
+    }
     // records per window: a new record whenever the minimizer changes (2 / (w + 1) of the windows for a
     // random order), at every read start, and every cmax windows
     const double rho = 2.0 / (pl.w + 1) + 1.2 / pl.nk + 1.0 / pl.cmax * 0.25;
@@ -1992,18 +2026,18 @@ cudaError_t super_reset(const SuperPlan &pl, void *ws, unsigned long long *d_sc,
 template <int W>
 static cudaError_t super_scatter_w(const SuperPlan &pl, const void *d_reads, uint64_t n_reads, void *ws,
                                    unsigned long long *d_sc, int n_sms, cudaStream_t s) {
-    constexpr uint32_t kTileBytes = 4800;       // bytes of reads per S1 tile (3200: 3.82 ms, 4800: 3.60, 6400: 4.0, 9600: 4.28 at C2)
     SwScatterParams q{};
-    if (!extract_plan(d_reads, n_reads, pl.L, pl.k, pl.flags, &d_sc[SW_INVALID], &q.ep, kTileBytes))
+    if (!extract_plan(d_reads, n_reads, pl.L, pl.k, pl.flags, &d_sc[SW_INVALID], &q.ep, kS1TileBytes))
         return cudaErrorInvalidValue;
     if (q.ep.n_tiles == 0) return cudaSuccess;
     q.m = pl.m; q.w = pl.w; q.nh = pl.nh; q.nh_stride = pl.nh_stride;
     q.seg_len = pl.seg_len; q.segs_per_read = pl.segs_per_read; q.cmax = pl.cmax; q.span = pl.span;
-    q.h_off = (q.ep.smem_total + 15u) & ~15u;
-    q.bin_off = q.h_off + q.ep.tile_reads * pl.nh_stride * 4;
-    q.bits_off = q.bin_off + q.ep.tile_reads * pl.nk * 4;
-    const uint32_t smem = q.bits_off + 2 * q.ep.tile_reads * pl.segs_per_read * 4;
-    if (smem > 200 * 1024) return cudaErrorInvalidValue;
+    const S1Smem lay = s1_smem(pl, q.ep);           // (super_plan only makes plans that fit)
+    q.h_off = lay.h_off;
+    q.bin_off = lay.bin_off;
+    q.bits_off = lay.bits_off;
+    const uint32_t smem = lay.total;
+    if (smem > kS1MaxSmem) return cudaErrorInvalidValue;
     q.n_bins = pl.n_bins; q.bin_cap = pl.bin_cap; q.ovf_cap = pl.ovf_cap;
     q.cursor = at<uint32_t>(ws, pl.off_cursor);
     q.bins = at<uint8_t>(ws, pl.off_bins);
@@ -2019,15 +2053,6 @@ static cudaError_t super_scatter_w(const SuperPlan &pl, const void *d_reads, uin
     if (grid > q.ep.n_tiles) grid = q.ep.n_tiles;
     kern<<<grid, kSwThreads, smem, s>>>(q);
     return cudaGetLastError();
-}
-
-// false when the shared-memory tile of S1 cannot hold even 16 reads of this length
-static bool super_scatter_fits(const SuperPlan &pl) {
-    ExtractParams ep;
-    if (!extract_plan(nullptr, 16, pl.L, pl.k, 0u, nullptr, &ep, 6400)) return false;
-    const uint64_t smem = ((ep.smem_total + 15u) & ~15u) + (uint64_t)ep.tile_reads * pl.nh_stride * 4 +
-                          (uint64_t)ep.tile_reads * pl.nk * 4 + 2ull * ep.tile_reads * pl.segs_per_read * 4;
-    return smem <= 200 * 1024;
 }
 
 cudaError_t super_scatter(const SuperPlan &pl, const void *d_reads, uint64_t n_reads, void *ws,
@@ -2282,8 +2307,6 @@ cudaError_t super_gather(const SuperPlan &pl, void *ws, const uint64_t *tmp_keys
     else sw_gather_kernel<4><<<(uint32_t)n_sms * 8, 256, 0, s>>>(tmp_keys, tmp_counts, src, off, plan, out_keys, out_counts);
     return cudaGetLastError();
 }
-
-bool super_supported(const SuperPlan &pl) { return super_scatter_fits(pl); }
 
 void super_use_large_finish(SuperPlan *pl) { pl->fin_cap = kFinCapLarge; }
 

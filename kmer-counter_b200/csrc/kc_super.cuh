@@ -97,7 +97,8 @@ constexpr uint32_t kSuperMaxSub = 1u << 20;
 // Plans a pipeline for up to max_windows k-mer slots (one chunk, or everything that will be
 // accumulated before the count). flags: kPlanStrict / kPlanCanonical (as extract_plan).
 // occ_per_bin = 0 -> default. Returns false for shapes the path does not take (W > 2, span < 22,
-// reads too long for the shared-memory tile).
+// reads too long for S1's shared memory). Every plan it makes fits S1: whether the path takes a
+// shape does not depend on max_windows or occ_per_bin.
 bool super_plan(uint32_t k, uint32_t L, uint32_t flags, uint64_t max_windows, uint32_t occ_per_bin, SuperPlan *out,
                 double record_headroom = 0.0, uint64_t distinct_hint = 0, bool ext_e = false);
 
@@ -165,8 +166,6 @@ cudaError_t place_init(const SuperPlan &pl, void *ws, unsigned long long *d_sc, 
 // empty slots were placed as key 0: the run's key-0 record (always first) loses *d_n_invalid occurrences
 cudaError_t place_fix_zero(int W, const uint64_t *run_keys, uint32_t *run_counts, const unsigned long long *d_n_invalid,
                            cudaStream_t s);
-// false when S1's shared-memory tile cannot hold 16 reads of this length
-bool super_supported(const SuperPlan &pl);
 // where S3c's temporary output may live in DUP mode (the level-1 buffer is dead by then)
 void super_tmp_buffers(const SuperPlan &pl, void *ws, uint64_t **tmp_keys, uint32_t **tmp_counts);
 

@@ -457,7 +457,7 @@ int main(int argc, char **argv) {
         if (r == 0 && !opt.histoFile.empty() && write_histo(opt.histoFile.c_str(), fin.hist) != KC_OK) return 1;
         if (r == 0) { fprintf(stderr, "records=%" PRIu64 " -> %s\n", n_rec, opt.outputFile.c_str()); return 0; }
         if (r < 0) return 1;
-        if (opt.gpus > 1) { fprintf(stderr, "gpus=%d needs k <= 64 with windows of at least 22 bases\n", opt.gpus); return 1; }
+        if (opt.gpus > 1) { fprintf(stderr, "gpus=%d needs the super-window path: k <= 64 with windows of at least 22 bases, reads of at most 1140 to 1191 bases by k\n", opt.gpus); return 1; }
         // not a shape for the accumulator: fall through to runs
     }
 
