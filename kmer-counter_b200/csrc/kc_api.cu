@@ -319,11 +319,7 @@ uint64_t pow2_ceil(uint64_t x) {
 
 // low bits of the last key word that are zero for every key (masked tail): the
 // radix sort skips the passes that would only see zeros
-int static_zero_bits(const kc_ctx *c) {
-    uint32_t m = c->cfg.k % 32;
-    bool masked = c->strict ? (m != 0) : (m >= 1 && m <= 28);
-    return masked ? (int)(64 - 2 * m) : 0;
-}
+int static_zero_bits(const kc_ctx *c) { return __builtin_ctzll(key_last_mask(c->cfg.k, c->strict)); }
 
 constexpr uint64_t kMaxSortKeys = (1ull << 30) - 1;
 
@@ -425,7 +421,7 @@ int count_enqueue_impl(kc_ctx *c, Pending &p, const void *d_reads, uint64_t n_by
         p.keys_b = static_cast<uint64_t *>(arena_take(p, kb));
         p.counts = static_cast<uint32_t *>(arena_take(p, cb));
         p.ws_part = arena_take(p, wb);
-        const int sig = W == 1 ? 64 - static_zero_bits(c) : 64;        // significant bits of key word 0
+        const int sig = key_sig_bits(W, key_last_mask(k, c->strict));
         const int target = c->cfg.table_slots ? (int)c->cfg.table_slots : 0;   // keys per sub-bucket (0 = default)
         p.uniq = partition_two_levels(p.n_slots, sig, target) ? p.keys_a : p.keys_b;
         KC_CUDA_TRY(c, partition_count(W, ep64, p.n_slots, sig, !c->strict, p.keys_a, p.keys_b, p.uniq, p.counts,
@@ -745,7 +741,7 @@ int count_finish_place(kc_ctx *c, Pending &p, cudaStream_t s, RunPtr *out) {
 
 int count_finish_partition(kc_ctx *c, Pending &p, cudaStream_t s, RunPtr *out) {
     const uint64_t U = p.h_scal[SC_UNIQUE];
-    const int sig = c->W == 1 ? 64 - static_zero_bits(c) : 64;
+    const int sig = key_sig_bits(c->W, key_last_mask(c->cfg.k, c->strict));
     const int target = c->cfg.table_slots ? (int)c->cfg.table_slots : 0;
     uint32_t n_sub = 0, prefix_bits = 0;
     const uint32_t *d_off = nullptr;

@@ -205,6 +205,104 @@ __device__ __forceinline__ void tma_load_1d(void *smem_dst, const void *gmem_src
         : "memory");
 }
 
+// ------------------------------------------------ shared-memory hash tables (PC, S2)
+// An empty slot holds the all-ones key (the key itself is counted on the side). 64-bit keys are
+// claimed with a 64-bit shared CAS, 128-bit keys with ATOMS.CAS.128.
+template <int W> __device__ __forceinline__ bool key_all_ones(const Key<W> &k) {
+    uint64_t a = ~0ull;
+#pragma unroll
+    for (int i = 0; i < W; i++) a &= k.w[i];
+    return a == ~0ull;
+}
+template <int W> __device__ __forceinline__ bool key_any_word_ones(const Key<W> &k) {
+    bool r = false;
+#pragma unroll
+    for (int i = 0; i < W; i++) r = r || (k.w[i] == ~0ull);
+    return r;
+}
+template <int W> __device__ __forceinline__ void key_set_ones(Key<W> &k) {
+#pragma unroll
+    for (int i = 0; i < W; i++) k.w[i] = ~0ull;
+}
+__device__ __forceinline__ Key<1> slot_claim(Key<1> *slot, const Key<1> &k) {      // returns the previous content
+    Key<1> o;
+    o.w[0] = atomicCAS(reinterpret_cast<unsigned long long *>(slot), ~0ull, (unsigned long long)k.w[0]);
+    return o;
+}
+__device__ __forceinline__ Key<2> slot_claim(Key<2> *slot, const Key<2> &k) {
+    Key<2> o;
+    const uint32_t a = smem_u32(slot);
+    asm volatile(
+        "{\n"
+        ".reg .b128 c, n, o;\n"
+        "mov.b128 c, {%3, %3};\n"
+        "mov.b128 n, {%4, %5};\n"
+        "atom.shared.cas.b128 o, [%2], c, n;\n"
+        "mov.b128 {%0, %1}, o;\n"
+        "}\n"
+        : "=l"(o.w[0]), "=l"(o.w[1])
+        : "r"(a), "l"(~0ull), "l"(k.w[0]), "l"(k.w[1])
+        : "memory");
+    return o;
+}
+template <int W> __device__ __forceinline__ uint32_t key_hash(const Key<W> &k) {
+    uint32_t x = (uint32_t)k.w[0] ^ (uint32_t)(k.w[0] >> 29);
+    if constexpr (W > 1) x ^= ((uint32_t)k.w[W - 1] ^ (uint32_t)(k.w[W - 1] >> 31)) * 0x85EBCA6Bu;
+    return x * 0x9E3779B1u;
+}
+
+__device__ __forceinline__ uint32_t pow2_ceil_u32(uint32_t x) { return x <= 1 ? 1u : 1u << (32 - __clz(x - 1)); }
+
+// ------------------------------------------------------- block scan of bin counters
+// Per-bin counters that one thread walks in runs of consecutive bins (the block scan below) can live at
+// index i + i / 32: the stride of 8 or 16 words between neighbouring threads' runs then falls on
+// different banks (unpadded it was an 8- to 16-way bank conflict: 67 % of S3c's shared wavefronts).
+__device__ __forceinline__ uint32_t pad32(uint32_t i) { return i + (i >> 5); }
+
+// exclusive scan of nb (<= MAXBINS) shared counters by THREADS threads; cnt and start are indexed
+// through pad32 when PAD is set. Every thread returns the total.
+template <int THREADS, int MAXBINS, bool PAD>
+__device__ __forceinline__ uint32_t block_scan_bins(const uint32_t *cnt, uint32_t *start, int nb, uint32_t *s_warp) {
+    constexpr int PER = MAXBINS / THREADS > 0 ? MAXBINS / THREADS : 1;
+    auto at = [](int b) {
+        if constexpr (PAD) return pad32((uint32_t)b);
+        else return b;
+    };
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    uint32_t v[PER];
+    uint32_t sum = 0;
+#pragma unroll
+    for (int i = 0; i < PER; i++) {
+        const int b = tid * PER + i;
+        v[i] = b < nb ? cnt[at(b)] : 0;
+        sum += v[i];
+    }
+    uint32_t incl = sum;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+        uint32_t t = __shfl_up_sync(0xffffffffu, incl, o);
+        if (lane >= o) incl += t;
+    }
+    if (lane == 31) s_warp[warp] = incl;
+    __syncthreads();
+    uint32_t off = 0, total = 0;
+#pragma unroll
+    for (int w = 0; w < THREADS / 32; w++) {
+        const uint32_t t = s_warp[w];
+        if (w < warp) off += t;
+        total += t;
+    }
+    uint32_t run = off + incl - sum;
+#pragma unroll
+    for (int i = 0; i < PER; i++) {
+        const int b = tid * PER + i;
+        if (b < nb) start[at(b)] = run;
+        run += v[i];
+    }
+    __syncthreads();
+    return total;
+}
+
 }  // namespace kc
 
 // ------------------------------------------------------------ host error macros

@@ -19,7 +19,6 @@ bool extract_plan(const void *d_reads, uint64_t n_reads, uint32_t L, uint32_t k,
                   unsigned long long *d_n_invalid, ExtractParams *out, uint32_t stage_bytes_target) {
     if (k == 0 || k > 128 || L < k || L > 4096) return false;
     if (flags & kPlanCanonical) flags |= kPlanStrict;      // a canonical key is exactly k bases
-    const bool strict = (flags & kPlanStrict) != 0;
     ExtractParams p{};
     p.reads = static_cast<const uint8_t *>(d_reads);
     p.n_reads = n_reads;
@@ -35,9 +34,7 @@ bool extract_plan(const void *d_reads, uint64_t n_reads, uint32_t L, uint32_t k,
     p.nb4_magic = p.nb4 == 1 ? 0xffffffffu : (uint32_t)((1ull << 32) / p.nb4 + 1);
     p.segs_per_read = (p.nk + 17) / 18;                    // ~18 positions per thread-segment (<= 32: one 64-bit lookahead word)
     p.seg_len = (p.nk + p.segs_per_read - 1) / p.segs_per_read;
-    uint32_t m = k % 32;
-    bool masked = strict ? (m != 0) : (m >= 1 && m <= 28);   // SURVEY F4
-    p.last_mask = masked ? (~0ull << (64 - 2 * m)) : ~0ull;
+    p.last_mask = key_last_mask(k, (flags & kPlanStrict) != 0);
     p.plan_flags = flags & (kPlanStrict | kPlanCanonical);
     p.n_invalid = d_n_invalid;
     extract_smem_layout(p);

@@ -9,6 +9,18 @@
 
 namespace kc {
 
+// ---- key semantics
+// The mask applied to key word W - 1 (SURVEY F4): it keeps the codes of the first k % 32 bases of that
+// word when k % 32 != 0 in strict mode, or 1 <= k % 32 <= 28 otherwise; else it is all ones (the key
+// spans 32 W bases).
+inline uint64_t key_last_mask(uint32_t k, bool strict) {
+    const uint32_t m = k % 32;
+    const bool masked = strict ? m != 0 : (m >= 1 && m <= 28);
+    return masked ? ~0ull << (64 - 2 * m) : ~0ull;
+}
+// bits of key word 0 that are not zero for every key: the bits a partition or digit plan can split on
+inline int key_sig_bits(int W, uint64_t last_mask) { return W == 1 ? 64 - __builtin_ctzll(last_mask) : 64; }
+
 // ---- extraction (kc_extract.cu)
 // Fills every field of ExtractParams for (reads, n_reads, L, k); flags: kPlanStrict selects
 // KC_COMPAT_STRICT masking, kPlanCanonical canonical keys (implies strict). Returns false for
@@ -107,6 +119,17 @@ cudaError_t hash_compact(HashTable t, uint64_t *out_keys, uint32_t *out_counts, 
 uint64_t fastq_workspace_bytes(uint64_t n_bytes);
 cudaError_t fastq_parse(const void *d_text, uint64_t n_bytes, uint32_t L, void *d_reads, uint64_t max_reads,
                         unsigned long long *d_out, void *ws, cudaStream_t s, int *n_launches);
+
+// ---- sub-bucket offsets and gather (kc_partition.cu), for the partitioned hash and the super-window path.
+// n entries: *n_ptr (device) or, when n_ptr is NULL, n; with n_ptr set, n is the most *n_ptr can be.
+// base[0 .. n] = exclusive scan of counts (base[n] = the total); cursor[0 .. n) and *total get copies when set.
+cudaError_t exclusive_scan(const uint32_t *counts, const uint32_t *n_ptr, uint32_t n, uint32_t *base, uint32_t *cursor,
+                           unsigned long long *total, cudaStream_t s);
+// records of sub-bucket j: tmp[src[j] .. src[j] + off[j + 1] - off[j]) -> out[off[j] ...), for the n sub-buckets
+// given as for exclusive_scan. W = 1 .. 4
+cudaError_t gather_records(int W, const uint64_t *tmp_keys, const uint32_t *tmp_counts, const uint32_t *src,
+                           const uint32_t *off, const uint32_t *n_ptr, uint32_t n, uint64_t *out_keys,
+                           uint32_t *out_counts, int n_sms, cudaStream_t s);
 
 // ---- partitioned shared-memory hash counting (kc_partition.cu), W = 1 or 2
 uint64_t partition_workspace_bytes(uint64_t n_slots);

@@ -32,45 +32,6 @@ constexpr int kPbItems = 16;            // 64-bit keys a PB thread moves per til
 template <int W> struct PbCfg { static constexpr int ITEMS = kPbItems / W, TILE = kPbThreads * ITEMS; };
 constexpr int kDefaultTarget = 3072;    // keys per sub-bucket the plan aims for
 
-// exclusive scan of nb (<= 1024) shared counters by THREADS threads; every thread returns the total
-template <int THREADS, int MAXBINS = kMaxBins>
-__device__ __forceinline__ uint32_t block_scan_bins(const uint32_t *cnt, uint32_t *start, int nb, uint32_t *s_warp) {
-    constexpr int PER = MAXBINS / THREADS > 0 ? MAXBINS / THREADS : 1;
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    uint32_t v[PER];
-    uint32_t sum = 0;
-#pragma unroll
-    for (int i = 0; i < PER; i++) {
-        const int b = tid * PER + i;
-        v[i] = b < nb ? cnt[b] : 0;
-        sum += v[i];
-    }
-    uint32_t incl = sum;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-        uint32_t t = __shfl_up_sync(0xffffffffu, incl, o);
-        if (lane >= o) incl += t;
-    }
-    if (lane == 31) s_warp[warp] = incl;
-    __syncthreads();
-    uint32_t off = 0, total = 0;
-#pragma unroll
-    for (int w = 0; w < THREADS / 32; w++) {
-        const uint32_t t = s_warp[w];
-        if (w < warp) off += t;
-        total += t;
-    }
-    uint32_t run = off + incl - sum;
-#pragma unroll
-    for (int i = 0; i < PER; i++) {
-        const int b = tid * PER + i;
-        if (b < nb) start[b] = run;
-        run += v[i];
-    }
-    __syncthreads();
-    return total;
-}
-
 // ------------------------------------------------------------------- P0: hist1
 template <int W>
 struct Hist1Sink : SinkBase {
@@ -166,7 +127,7 @@ struct Scatter1Sink : SinkBase {
     }
     __device__ __forceinline__ void sweep_end(int sw) {
         if (sw == 0) {
-            total = block_scan_bins<kExtractThreads>(cnt, start, nb1, s_warp);
+            total = block_scan_bins<kExtractThreads, kMaxBins, false>(cnt, start, nb1, s_warp);
             // reserve the bins' ranges now, look at the answers after the placing sweep: the
             // round trips of the global atomics are hidden behind it
 #pragma unroll
@@ -245,60 +206,6 @@ __global__ void __launch_bounds__(kPbThreads) hist2_kernel(const uint64_t *__res
     }
 }
 
-// Exclusive scan over all sub-buckets -> base2 (n+1) and the mutable cursors. One CTA per tile of
-// 4096 entries; a CTA gets its offset by summing the entries before its tile itself (at most
-// 2 MB out of L2), so there is neither a carried dependency between tiles nor scratch memory.
-// The input must not alias the outputs.
-constexpr uint32_t kScan2Tile = 4096;
-__global__ void __launch_bounds__(1024) scan2_kernel(const uint32_t *__restrict__ hist2, uint32_t n,
-                                                     uint32_t *__restrict__ base2, uint32_t *__restrict__ cursor2) {
-    __shared__ uint32_t s_w[32];
-    __shared__ uint32_t s_carry;
-    const uint32_t tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    const uint32_t t0 = blockIdx.x * kScan2Tile;
-    uint32_t acc = 0;
-#pragma unroll 8
-    for (uint32_t i = tid; i < t0; i += 1024) acc += hist2[i];
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
-    if (lane == 0) s_w[warp] = acc;
-    __syncthreads();
-    if (tid == 0) {
-        uint32_t c = 0;
-        for (int w = 0; w < 32; w++) c += s_w[w];
-        s_carry = c;
-    }
-    __syncthreads();
-    const uint32_t i0 = t0 + tid * 4;
-    uint32_t v[4];
-#pragma unroll
-    for (int u = 0; u < 4; u++) v[u] = i0 + u < n ? hist2[i0 + u] : 0;
-    const uint32_t sum = v[0] + v[1] + v[2] + v[3];
-    uint32_t incl = sum;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-        uint32_t t = __shfl_up_sync(0xffffffffu, incl, o);
-        if (lane >= (uint32_t)o) incl += t;
-    }
-    __syncthreads();                        // s_w is reused
-    if (lane == 31) s_w[warp] = incl;
-    __syncthreads();
-    uint32_t off = s_carry, tot = 0;
-#pragma unroll
-    for (uint32_t w = 0; w < 32; w++) {
-        const uint32_t x = s_w[w];
-        if (w < warp) off += x;
-        tot += x;
-    }
-    uint32_t run = off + incl - sum;
-#pragma unroll
-    for (int u = 0; u < 4; u++) {
-        if (i0 + u < n) { base2[i0 + u] = run; cursor2[i0 + u] = run; }
-        run += v[u];
-    }
-    if (tid == 0 && t0 + kScan2Tile >= n) base2[n] = s_carry + tot;    // the last tile closes the scan
-}
-
 // ---------------------------------------------------------------- PB: scatter2
 // Level-2 scatter over flat tiles of the grouped array (dense, bucket after bucket): the keys'
 // own leading bits name bucket and sub-bucket, so a CTA needs no tile map and its loads are in
@@ -344,7 +251,7 @@ __global__ void __launch_bounds__(kPbThreads) scatter2_kernel(const uint64_t *__
         }
     }
     __syncthreads();
-    const uint32_t total = block_scan_bins<kPbThreads>(cnt, start, (int)nb, s_warp);
+    const uint32_t total = block_scan_bins<kPbThreads, kMaxBins, false>(cnt, start, (int)nb, s_warp);
     // reserve the bins' ranges, stage the keys while the atomics are in flight, then look at the answers
     uint32_t reserved[kMaxBins / kPbThreads];
 #pragma unroll
@@ -400,52 +307,6 @@ struct FinishParams {
 constexpr int kPcBatch = 4;
 constexpr float kPcLoad = 2.0f;    // table slots per expected distinct key (first guess)
 constexpr int kSortBins = 1024;    // most bins the in-table counting sort uses
-
-__device__ __forceinline__ uint32_t pow2_ceil_u32(uint32_t x) { return x <= 1 ? 1u : 1u << (32 - __clz(x - 1)); }
-
-// ---- table slot primitives: 64-bit keys use a 64-bit shared CAS, 128-bit keys ATOMS.CAS.128
-template <int W> __device__ __forceinline__ bool key_all_ones(const Key<W> &k) {
-    uint64_t a = ~0ull;
-#pragma unroll
-    for (int i = 0; i < W; i++) a &= k.w[i];
-    return a == ~0ull;
-}
-template <int W> __device__ __forceinline__ bool key_any_word_ones(const Key<W> &k) {
-    bool r = false;
-#pragma unroll
-    for (int i = 0; i < W; i++) r = r || (k.w[i] == ~0ull);
-    return r;
-}
-template <int W> __device__ __forceinline__ void key_set_ones(Key<W> &k) {
-#pragma unroll
-    for (int i = 0; i < W; i++) k.w[i] = ~0ull;
-}
-__device__ __forceinline__ Key<1> slot_claim(Key<1> *slot, const Key<1> &k) {      // returns the previous content
-    Key<1> o;
-    o.w[0] = atomicCAS(reinterpret_cast<unsigned long long *>(slot), ~0ull, (unsigned long long)k.w[0]);
-    return o;
-}
-__device__ __forceinline__ Key<2> slot_claim(Key<2> *slot, const Key<2> &k) {
-    Key<2> o;
-    const uint32_t a = smem_u32(slot);
-    asm volatile(
-        "{\n"
-        ".reg .b128 c, n, o;\n"
-        "mov.b128 c, {%3, %3};\n"
-        "mov.b128 n, {%4, %5};\n"
-        "atom.shared.cas.b128 o, [%2], c, n;\n"
-        "mov.b128 {%0, %1}, o;\n"
-        "}\n"
-        : "=l"(o.w[0]), "=l"(o.w[1])
-        : "r"(a), "l"(~0ull), "l"(k.w[0]), "l"(k.w[1])
-        : "memory");
-    return o;
-}
-template <int W> __device__ __forceinline__ uint32_t key_hash(const Key<W> &k) {
-    uint32_t x = (uint32_t)k.w[0] ^ (uint32_t)(k.w[0] >> 29);
-    if constexpr (W > 1) x ^= ((uint32_t)k.w[W - 1] ^ (uint32_t)(k.w[W - 1] >> 31)) * 0x85EBCA6Bu;
-    return x * 0x9E3779B1u;
-}
 
 // One CTA per sub-bucket (round-robin over a persistent grid). Nothing here depends on
 // another CTA: a sub-bucket with n keys has at most n distinct keys, so its records are
@@ -642,7 +503,7 @@ __global__ void __launch_bounds__(kPcThreads) finish_kernel(FinishParams p) {
             uint32_t mx = 0;
             for (uint32_t i = tid; i < nb3; i += kPcThreads) mx = max(mx, c3[i]);
             if (mx > 1) atomicMax(&s_maxbin, mx);
-            block_scan_bins<kPcThreads>(c3, s3, (int)nb3, s_warp);
+            block_scan_bins<kPcThreads, kMaxBins, false>(c3, s3, (int)nb3, s_warp);
             const uint32_t maxbin = s_maxbin;
             const Key<W> *rk_keys = sk;
             const uint32_t *rk_cnts = sc;
@@ -776,19 +637,82 @@ cudaError_t launch_finish(const FinishParams &fp, int n_sms, uint32_t n_sub, cud
     return cudaGetLastError();
 }
 
-// records of sub-bucket j: tmp[src(j) .. src(j) + m_j) -> out[off[j] ...); one warp per sub-bucket
+// ---------------------------------------- sub-bucket offsets and gather (also the super-window path's)
+// Exclusive scan over n entries -> base (n+1) and the mutable cursors. One CTA per tile of 4096;
+// a CTA sums the entries before its tile itself (a few MB out of L2 at most): no carried dependency.
+// n comes from the device (n_ptr) or, when n_ptr is NULL, from n_host.
+constexpr uint32_t kScanTile = 4096;
+__global__ void __launch_bounds__(1024) exclusive_scan_kernel(const uint32_t *__restrict__ hist, const uint32_t *__restrict__ n_ptr,
+                                                              uint32_t n_host, uint32_t *__restrict__ base,
+                                                              uint32_t *__restrict__ cursor, unsigned long long *total_out) {
+    __shared__ uint32_t s_w[32];
+    __shared__ uint32_t s_carry;
+    const uint32_t n = n_ptr ? *n_ptr : n_host;
+    const uint32_t tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const uint32_t t0 = blockIdx.x * kScanTile;
+    if (t0 >= n) return;
+    uint32_t acc = 0;
+#pragma unroll 8
+    for (uint32_t i = tid; i < t0; i += 1024) acc += hist[i];
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
+    if (lane == 0) s_w[warp] = acc;
+    __syncthreads();
+    if (tid == 0) {
+        uint32_t c = 0;
+        for (int w = 0; w < 32; w++) c += s_w[w];
+        s_carry = c;
+    }
+    __syncthreads();
+    const uint32_t i0 = t0 + tid * 4;
+    uint32_t v[4];
+#pragma unroll
+    for (int u = 0; u < 4; u++) v[u] = i0 + u < n ? hist[i0 + u] : 0;
+    const uint32_t sum = v[0] + v[1] + v[2] + v[3];
+    uint32_t incl = sum;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+        uint32_t t = __shfl_up_sync(0xffffffffu, incl, o);
+        if (lane >= (uint32_t)o) incl += t;
+    }
+    __syncthreads();                        // s_w is reused
+    if (lane == 31) s_w[warp] = incl;
+    __syncthreads();
+    uint32_t off = s_carry, tot = 0;
+#pragma unroll
+    for (uint32_t w = 0; w < 32; w++) {
+        const uint32_t x = s_w[w];
+        if (w < warp) off += x;
+        tot += x;
+    }
+    uint32_t run = off + incl - sum;
+#pragma unroll
+    for (int u = 0; u < 4; u++) {
+        if (i0 + u < n) { base[i0 + u] = run; if (cursor) cursor[i0 + u] = run; }
+        run += v[u];
+    }
+    if (tid == 0 && t0 + kScanTile >= n) {       // the last tile closes the scan
+        base[n] = s_carry + tot;
+        if (total_out) *total_out = s_carry + tot;
+    }
+}
+
+// records of sub-bucket j: tmp[src[j] .. src[j] + m_j) -> out[off[j] ...); one warp per sub-bucket.
+// n_sub comes from the device (n_ptr) or, when n_ptr is NULL, from n_host.
 template <int W>
-__global__ void __launch_bounds__(256) gather_kernel(const uint64_t *__restrict__ tmp_keys,
-                                                     const uint32_t *__restrict__ tmp_counts,
-                                                     const uint32_t *__restrict__ tmp_start,
-                                                     const uint32_t *__restrict__ off, uint32_t n_sub,
-                                                     uint64_t *__restrict__ out_keys,
-                                                     uint32_t *__restrict__ out_counts) {
+__global__ void __launch_bounds__(256) gather_records_kernel(const uint64_t *__restrict__ tmp_keys,
+                                                             const uint32_t *__restrict__ tmp_counts,
+                                                             const uint32_t *__restrict__ src,
+                                                             const uint32_t *__restrict__ off,
+                                                             const uint32_t *__restrict__ n_ptr, uint32_t n_host,
+                                                             uint64_t *__restrict__ out_keys,
+                                                             uint32_t *__restrict__ out_counts) {
+    const uint32_t n_sub = n_ptr ? *n_ptr : n_host;
     const uint32_t lane = threadIdx.x & 31;
     const uint32_t warps = (gridDim.x * blockDim.x) >> 5;
     for (uint32_t j = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; j < n_sub; j += warps) {
         const uint32_t o0 = off[j], m = off[j + 1] - o0;
-        const uint64_t s0 = tmp_start[j];
+        const uint64_t s0 = src[j];
         for (uint32_t i = lane; i < m; i += 32) {
             st_key<W>(out_keys, o0 + i, ld_key<W>(tmp_keys, s0 + i));
             out_counts[o0 + i] = tmp_counts[s0 + i];
@@ -797,6 +721,26 @@ __global__ void __launch_bounds__(256) gather_kernel(const uint64_t *__restrict_
 }
 
 }  // namespace
+
+cudaError_t exclusive_scan(const uint32_t *counts, const uint32_t *n_ptr, uint32_t n, uint32_t *base, uint32_t *cursor,
+                           unsigned long long *total, cudaStream_t s) {
+    exclusive_scan_kernel<<<(n + kScanTile - 1) / kScanTile, 1024, 0, s>>>(counts, n_ptr, n, base, cursor, total);
+    return cudaGetLastError();
+}
+
+cudaError_t gather_records(int W, const uint64_t *tmp_keys, const uint32_t *tmp_counts, const uint32_t *src,
+                           const uint32_t *off, const uint32_t *n_ptr, uint32_t n, uint64_t *out_keys,
+                           uint32_t *out_counts, int n_sms, cudaStream_t s) {
+    const uint32_t grid = (uint32_t)n_sms * 8;
+    switch (W) {
+        case 1: gather_records_kernel<1><<<grid, 256, 0, s>>>(tmp_keys, tmp_counts, src, off, n_ptr, n, out_keys, out_counts); break;
+        case 2: gather_records_kernel<2><<<grid, 256, 0, s>>>(tmp_keys, tmp_counts, src, off, n_ptr, n, out_keys, out_counts); break;
+        case 3: gather_records_kernel<3><<<grid, 256, 0, s>>>(tmp_keys, tmp_counts, src, off, n_ptr, n, out_keys, out_counts); break;
+        case 4: gather_records_kernel<4><<<grid, 256, 0, s>>>(tmp_keys, tmp_counts, src, off, n_ptr, n, out_keys, out_counts); break;
+        default: return cudaErrorInvalidValue;
+    }
+    return cudaGetLastError();
+}
 
 // ------------------------------------------------------------------------ host
 struct PartitionPlan {
@@ -829,9 +773,7 @@ cudaError_t partition_gather(int W, uint64_t n_slots, int sig_bits, int target_s
     uint32_t *base2 = hist2 + pl.n_sub + 8;
     uint32_t *off = base2 + pl.n_sub + 8;
     uint32_t *tmp_start = off + pl.n_sub + 8 + pl.n_sub + 8;
-    if (W == 1) gather_kernel<1><<<(uint32_t)sm_count() * 8, 256, 0, s>>>(tmp_keys, tmp_counts, tmp_start, off, pl.n_sub, out_keys, out_counts);
-    else gather_kernel<2><<<(uint32_t)sm_count() * 8, 256, 0, s>>>(tmp_keys, tmp_counts, tmp_start, off, pl.n_sub, out_keys, out_counts);
-    return cudaGetLastError();
+    return gather_records(W, tmp_keys, tmp_counts, tmp_start, off, nullptr, pl.n_sub, out_keys, out_counts, sm_count(), s);
 }
 
 // The plan a chunk of n_slots k-mer slots is counted with, and where the per-sub-bucket
@@ -861,7 +803,6 @@ cudaError_t merge_parts_count(uint32_t n_src, const uint64_t *const *src_keys, c
     uint32_t *m_out = reinterpret_cast<uint32_t *>(ws);
     uint32_t *off = m_out + n_sub + 8;
     uint32_t *tmp_start = off + n_sub + 8;
-    uint32_t *scratch = tmp_start + n_sub + 8;
     cudaError_t e;
     if ((e = cudaMemsetAsync(d_num_out, 0, 8, s)) != cudaSuccess) return e;
     if ((e = cudaMemsetAsync(d_overflow, 0, 8, s)) != cudaSuccess) return e;
@@ -876,7 +817,7 @@ cudaError_t merge_parts_count(uint32_t n_src, const uint64_t *const *src_keys, c
     fp.n_src = n_src;
     for (uint32_t i = 0; i < n_src; i++) { fp.src_keys[i] = src_keys[i]; fp.src_counts[i] = src_counts[i]; fp.src_off[i] = src_off[i]; }
     if ((e = launch_finish<true, 1>(fp, n_sms, n_sub, s)) != cudaSuccess) return e;
-    scan2_kernel<<<(n_sub + kScan2Tile - 1) / kScan2Tile, 1024, 0, s>>>(m_out, n_sub, off, scratch);
+    if ((e = exclusive_scan(m_out, nullptr, n_sub, off, nullptr, nullptr, s)) != cudaSuccess) return e;
     if ((e = cudaMemcpyAsync(d_num_out, off + n_sub, 4, cudaMemcpyDeviceToDevice, s)) != cudaSuccess) return e;
     if (n_launches) *n_launches += 2;
     return cudaGetLastError();
@@ -887,12 +828,10 @@ cudaError_t merge_parts_gather(uint32_t n_sub, const uint64_t *tmp_keys, const u
     uint32_t *m_out = reinterpret_cast<uint32_t *>(ws);
     uint32_t *off = m_out + n_sub + 8;
     uint32_t *tmp_start = off + n_sub + 8;
-    gather_kernel<1><<<(uint32_t)sm_count() * 8, 256, 0, s>>>(tmp_keys, tmp_counts, tmp_start, off, n_sub, out_keys, out_counts);
-    if (out_offsets) {
-        cudaError_t e = cudaMemcpyAsync(out_offsets, off, (size_t)(n_sub + 1) * 4, cudaMemcpyDeviceToDevice, s);
-        if (e != cudaSuccess) return e;
-    }
-    return cudaGetLastError();
+    cudaError_t e = gather_records(1, tmp_keys, tmp_counts, tmp_start, off, nullptr, n_sub, out_keys, out_counts, sm_count(), s);
+    if (e == cudaSuccess && out_offsets)
+        e = cudaMemcpyAsync(out_offsets, off, (size_t)(n_sub + 1) * 4, cudaMemcpyDeviceToDevice, s);
+    return e;
 }
 
 bool partition_two_levels(uint64_t n_slots, int sig_bits, int target_sub) {
@@ -902,7 +841,7 @@ bool partition_two_levels(uint64_t n_slots, int sig_bits, int target_sub) {
 uint64_t partition_workspace_bytes(uint64_t n_slots) {
     (void)n_slots;
     const uint64_t nsub = 1u << 20;
-    // hist1, base1, cursor1, tile_prefix | hist2, base2, cursor2 | status | flags
+    // hist1, base1, cursor1, tile_prefix | hist2, base2, cursor2 | unused, tmp_start
     return 4 * (kMaxBins + 8) * 4 + 3 * (nsub + 8) * 4 + nsub * 8 + 256;
 }
 
@@ -924,9 +863,9 @@ static cudaError_t partition_count_w(const ExtractParams &ep_in, uint64_t n_slot
     uint32_t *hist2 = tile_prefix + kMaxBins + 8;
     uint32_t *base2 = hist2 + pl.n_sub + 8;
     uint32_t *cursor2 = base2 + pl.n_sub + 8;
-    uint32_t *status_scratch = cursor2 + pl.n_sub + 8;       // n_sub + 8 entries, scratch for the second scan
+    uint32_t *tmp_start = cursor2 + 2 * (pl.n_sub + 8);      // (the n_sub + 8 entries before it are unused)
     cudaError_t e;
-    const size_t zero_bytes = reinterpret_cast<uint8_t *>(status_scratch) - w;
+    const size_t zero_bytes = reinterpret_cast<uint8_t *>(cursor2 + pl.n_sub + 8) - w;
     if ((e = cudaMemsetAsync(ws, 0, zero_bytes, s)) != cudaSuccess) return e;
     if ((e = cudaMemsetAsync(d_num_out, 0, 8, s)) != cudaSuccess) return e;
     if ((e = cudaMemsetAsync(d_overflow, 0, 8, s)) != cudaSuccess) return e;
@@ -975,7 +914,7 @@ static cudaError_t partition_count_w(const ExtractParams &ep_in, uint64_t n_slot
     // H2 + PB over the level-1 buckets
     if (pl.b2 > 0) {
         hist2_kernel<W><<<(uint32_t)div_up(n_slots, (uint64_t)kH2Chunk), kPbThreads, 0, s>>>(keys_a, base1 + pl.nb1, pl.b2, shift2, hist2);
-        scan2_kernel<<<(pl.n_sub + kScan2Tile - 1) / kScan2Tile, 1024, 0, s>>>(hist2, pl.n_sub, base2, cursor2);
+        if ((e = exclusive_scan(hist2, nullptr, pl.n_sub, base2, cursor2, nullptr, s)) != cudaSuccess) return e;
         if (evs) cudaEventRecord(evs[2], s);
         scatter2_kernel<W><<<(uint32_t)div_up(n_slots, (uint64_t)PbCfg<W>::TILE), kPbThreads, 0, s>>>(
             keys_a, keys_b, base1 + pl.nb1, pl.b2, shift2, cursor2);
@@ -994,10 +933,10 @@ static cudaError_t partition_count_w(const ExtractParams &ep_in, uint64_t n_slot
         fp.keys = grouped; fp.base2 = base2; fp.n_sub = pl.n_sub; fp.prefix_bits = pl.b1 + pl.b2;
         fp.tmp_keys = out_keys; fp.tmp_counts = out_counts; fp.m_out = m_out; fp.d_overflow = d_overflow;
         fp.d_n_invalid = ep_in.n_invalid; fp.add_phantom = add_phantom ? 1 : 0;
-        fp.tmp_start = status_scratch + pl.n_sub + 8;
+        fp.tmp_start = tmp_start;
         if ((e = launch_finish<false, W>(fp, n_sms, pl.n_sub, s)) != cudaSuccess) return e;
         // off[] (n_sub + 1) overwrites cursor2; its last entry is the number of records
-        scan2_kernel<<<(pl.n_sub + kScan2Tile - 1) / kScan2Tile, 1024, 0, s>>>(m_out, pl.n_sub, cursor2, status_scratch);
+        if ((e = exclusive_scan(m_out, nullptr, pl.n_sub, cursor2, nullptr, nullptr, s)) != cudaSuccess) return e;
         if ((e = cudaMemcpyAsync(d_num_out, cursor2 + pl.n_sub, 4, cudaMemcpyDeviceToDevice, s)) != cudaSuccess) return e;
     }
     if (evs) cudaEventRecord(evs[4], s);

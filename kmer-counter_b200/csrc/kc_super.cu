@@ -302,48 +302,6 @@ __global__ void __launch_bounds__(kSwThreads) sw_scatter_kernel(SwScatterParams 
 }
 
 // ======================================================================= S2: count
-template <int W> __device__ __forceinline__ bool key_all_ones(const Key<W> &k) {
-    uint64_t a = ~0ull;
-#pragma unroll
-    for (int i = 0; i < W; i++) a &= k.w[i];
-    return a == ~0ull;
-}
-template <int W> __device__ __forceinline__ bool key_any_word_ones(const Key<W> &k) {
-    bool r = false;
-#pragma unroll
-    for (int i = 0; i < W; i++) r = r || (k.w[i] == ~0ull);
-    return r;
-}
-template <int W> __device__ __forceinline__ void key_set_ones(Key<W> &k) {
-#pragma unroll
-    for (int i = 0; i < W; i++) k.w[i] = ~0ull;
-}
-__device__ __forceinline__ Key<1> slot_claim(Key<1> *slot, const Key<1> &k) {      // returns the previous content
-    Key<1> o;
-    o.w[0] = atomicCAS(reinterpret_cast<unsigned long long *>(slot), ~0ull, (unsigned long long)k.w[0]);
-    return o;
-}
-__device__ __forceinline__ Key<2> slot_claim(Key<2> *slot, const Key<2> &k) {
-    Key<2> o;
-    const uint32_t a = smem_u32(slot);
-    asm volatile(
-        "{\n"
-        ".reg .b128 c, n, o;\n"
-        "mov.b128 c, {%3, %3};\n"
-        "mov.b128 n, {%4, %5};\n"
-        "atom.shared.cas.b128 o, [%2], c, n;\n"
-        "mov.b128 {%0, %1}, o;\n"
-        "}\n"
-        : "=l"(o.w[0]), "=l"(o.w[1])
-        : "r"(a), "l"(~0ull), "l"(k.w[0]), "l"(k.w[1])
-        : "memory");
-    return o;
-}
-template <int W> __device__ __forceinline__ uint32_t key_hash(const Key<W> &k) {
-    uint32_t x = (uint32_t)k.w[0] ^ (uint32_t)(k.w[0] >> 29);
-    if constexpr (W > 1) x ^= ((uint32_t)k.w[W - 1] ^ (uint32_t)(k.w[W - 1] >> 31)) * 0x85EBCA6Bu;
-    return x * 0x9E3779B1u;
-}
 // a second, independent hash: which of the 2^bits passes over a bin a key belongs to
 __device__ __forceinline__ uint32_t pass_hash(uint32_t h) { return (h ^ (h >> 15)) * 0x2C1B3C6Du; }
 
@@ -986,49 +944,8 @@ __global__ void __launch_bounds__(THREADS) sw_count_kernel(SwCountParams p) {
 }
 
 // ============================================================ S3: ordering the records
-// Per-bin counters that one thread walks in runs of consecutive bins (the block scans below) live at
-// index i + i / 32: the stride of 8 or 16 words between neighbouring threads' runs then falls on
-// different banks (unpadded it was an 8- to 16-way bank conflict: 67 % of S3c's shared wavefronts).
-__device__ __forceinline__ uint32_t pad32(uint32_t i) { return i + (i >> 5); }
+// per-bin counters of the record scatter and of S3c's counting sort are indexed through pad32
 constexpr int kRsBinsPadded = kRsBins + kRsBins / 32;
-// exclusive scan of nb (<= 1024) shared counters by THREADS threads; every thread returns the total
-template <int THREADS>
-__device__ __forceinline__ uint32_t block_scan_bins(const uint32_t *cnt, uint32_t *start, int nb, uint32_t *s_warp) {
-    constexpr int PER = kRsBins / THREADS > 0 ? kRsBins / THREADS : 1;
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    uint32_t v[PER];
-    uint32_t sum = 0;
-#pragma unroll
-    for (int i = 0; i < PER; i++) {
-        const int b = tid * PER + i;
-        v[i] = b < nb ? cnt[pad32((uint32_t)b)] : 0;
-        sum += v[i];
-    }
-    uint32_t incl = sum;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-        uint32_t t = __shfl_up_sync(0xffffffffu, incl, o);
-        if (lane >= o) incl += t;
-    }
-    if (lane == 31) s_warp[warp] = incl;
-    __syncthreads();
-    uint32_t off = 0, total = 0;
-#pragma unroll
-    for (int w = 0; w < THREADS / 32; w++) {
-        const uint32_t t = s_warp[w];
-        if (w < warp) off += t;
-        total += t;
-    }
-    uint32_t run = off + incl - sum;
-#pragma unroll
-    for (int i = 0; i < PER; i++) {
-        const int b = tid * PER + i;
-        if (b < nb) start[pad32((uint32_t)b)] = run;
-        run += v[i];
-    }
-    __syncthreads();
-    return total;
-}
 
 // One block. S2 left a histogram of the records' leading b1_max bits; the plan picks the two
 // digit widths from the number of records actually there -- B = b1 + b2 bits so that a sub-bucket
@@ -1314,7 +1231,7 @@ __global__ void __launch_bounds__(kRsThreads) rec_scatter_kernel(const uint64_t 
             }
         }
         __syncthreads();
-        const uint32_t total = block_scan_bins<kRsThreads>(cnt, start, (int)nb, s_warp);
+        const uint32_t total = block_scan_bins<kRsThreads, kRsBins, true>(cnt, start, (int)nb, s_warp);
         // reserve the bins' ranges, stage the records while the atomics are in flight, then look at the answers
         uint32_t reserved[kRsBins / kRsThreads];
 #pragma unroll
@@ -1411,67 +1328,6 @@ __global__ void __launch_bounds__(256) rec_hist2_kernel(const uint64_t *__restri
         __syncthreads();
     }
 }
-
-// Exclusive scan over n entries -> base (n+1) and the mutable cursors. One CTA per tile of 4096;
-// a CTA sums the entries before its tile itself (a few MB out of L2 at most): no carried dependency.
-// n comes from the device plan (n_ptr) or, when n_ptr is NULL, from n_host.
-constexpr uint32_t kScanTile = 4096;
-__global__ void __launch_bounds__(1024) sw_scan_kernel(const uint32_t *__restrict__ hist, const uint32_t *__restrict__ n_ptr,
-                                                       uint32_t n_host, uint32_t *__restrict__ base,
-                                                       uint32_t *__restrict__ cursor, unsigned long long *total_out) {
-    __shared__ uint32_t s_w[32];
-    __shared__ uint32_t s_carry;
-    const uint32_t n = n_ptr ? *n_ptr : n_host;
-    const uint32_t tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    const uint32_t t0 = blockIdx.x * kScanTile;
-    if (t0 >= n) return;
-    uint32_t acc = 0;
-#pragma unroll 8
-    for (uint32_t i = tid; i < t0; i += 1024) acc += hist[i];
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
-    if (lane == 0) s_w[warp] = acc;
-    __syncthreads();
-    if (tid == 0) {
-        uint32_t c = 0;
-        for (int w = 0; w < 32; w++) c += s_w[w];
-        s_carry = c;
-    }
-    __syncthreads();
-    const uint32_t i0 = t0 + tid * 4;
-    uint32_t v[4];
-#pragma unroll
-    for (int u = 0; u < 4; u++) v[u] = i0 + u < n ? hist[i0 + u] : 0;
-    const uint32_t sum = v[0] + v[1] + v[2] + v[3];
-    uint32_t incl = sum;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-        uint32_t t = __shfl_up_sync(0xffffffffu, incl, o);
-        if (lane >= (uint32_t)o) incl += t;
-    }
-    __syncthreads();                        // s_w is reused
-    if (lane == 31) s_w[warp] = incl;
-    __syncthreads();
-    uint32_t off = s_carry, tot = 0;
-#pragma unroll
-    for (uint32_t w = 0; w < 32; w++) {
-        const uint32_t x = s_w[w];
-        if (w < warp) off += x;
-        tot += x;
-    }
-    uint32_t run = off + incl - sum;
-#pragma unroll
-    for (int u = 0; u < 4; u++) {
-        if (i0 + u < n) { base[i0 + u] = run; if (cursor) cursor[i0 + u] = run; }
-        run += v[u];
-    }
-    if (tid == 0 && t0 + kScanTile >= n) {       // the last tile closes the scan
-        base[n] = s_carry + tot;
-        if (total_out) *total_out = s_carry + tot;
-    }
-}
-
-__device__ __forceinline__ uint32_t pow2_ceil_u32(uint32_t x) { return x <= 1 ? 1u : 1u << (32 - __clz(x - 1)); }
 
 struct FinishParams {
     const uint64_t *in_keys;
@@ -1705,28 +1561,6 @@ __global__ void __launch_bounds__(THREADS) rec_finish_kernel(FinishParams p) {
     if (DUP && tid == 0 && folded_local) atomicAdd(&p.sc[SW_FOLDED], folded_local);
 }
 
-// records of sub-bucket j: tmp[src[j] .. src[j] + m_j) -> out[off[j] ...); one warp per sub-bucket
-template <int W>
-__global__ void __launch_bounds__(256) sw_gather_kernel(const uint64_t *__restrict__ tmp_keys,
-                                                        const uint32_t *__restrict__ tmp_counts,
-                                                        const uint32_t *__restrict__ src,
-                                                        const uint32_t *__restrict__ off,
-                                                        const SuperPlanDev *__restrict__ plan,
-                                                        uint64_t *__restrict__ out_keys,
-                                                        uint32_t *__restrict__ out_counts) {
-    const uint32_t n_sub = plan->n_sub;
-    const uint32_t lane = threadIdx.x & 31;
-    const uint32_t warps = (gridDim.x * blockDim.x) >> 5;
-    for (uint32_t j = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; j < n_sub; j += warps) {
-        const uint32_t o0 = off[j], m = off[j + 1] - o0;
-        const uint64_t s0 = src[j];
-        for (uint32_t i = lane; i < m; i += 32) {
-            st_key<W>(out_keys, o0 + i, ld_key<W>(tmp_keys, s0 + i));
-            out_counts[o0 + i] = tmp_counts[s0 + i];
-        }
-    }
-}
-
 // ---- sub-buckets too large for S3c (see kc_super.cuh): records of sub-bucket j are
 // D[base2[j] .. base2[j] + big[j]); in the gathered / sorted array they sit at bigoff[j].
 template <int W>
@@ -1857,6 +1691,16 @@ void set_minimizer(SuperPlan &pl, uint32_t m) {
     pl.segs_per_read = (pl.nk + pl.seg_len - 1) / pl.seg_len;
     pl.seg_len = (pl.nk + pl.segs_per_read - 1) / pl.segs_per_read;    // even the segments out
 }
+
+// records per sub-bucket the device plan aims for: 70 % of S3c's capacity. KC_SW_SUB_TARGET (tests)
+// forces deep level-2 plans on small inputs.
+uint32_t plan_sub_target(uint32_t fin_cap) {
+    if (const char *v = getenv("KC_SW_SUB_TARGET")) {
+        const int t = atoi(v);
+        if (t > 0) return (uint32_t)t;
+    }
+    return fin_cap * 7 / 10;
+}
 }  // namespace
 
 bool super_plan(uint32_t k, uint32_t L, uint32_t flags, uint64_t max_windows, uint32_t occ_per_bin, SuperPlan *out,
@@ -1869,10 +1713,8 @@ bool super_plan(uint32_t k, uint32_t L, uint32_t flags, uint64_t max_windows, ui
     pl.W = (int)((k + 31) / 32);
     pl.k = k;
     pl.L = L;
-    const uint32_t mm = k % 32;
-    const bool masked = strict ? (mm != 0) : (mm >= 1 && mm <= 28);    // SURVEY F4
-    pl.span = masked ? k : 32u * pl.W;
-    pl.last_mask = masked ? (~0ull << (64 - 2 * mm)) : ~0ull;
+    pl.last_mask = key_last_mask(k, strict);
+    pl.span = pl.last_mask != ~0ull ? k : 32u * pl.W;
     if (pl.span < 22) return false;
     pl.nk = L - k + 1;
     pl.cmax = 32u * pl.W - 3;
@@ -1933,12 +1775,8 @@ bool super_plan(uint32_t k, uint32_t L, uint32_t flags, uint64_t max_windows, ui
     // S2 keeps a histogram of the leading b1 bits; the device plan picks the digits from it
     // sub-buckets of 2048 records unless the 2^20 sub-buckets two levels can cut would be too few
     pl.fin_cap = pl.d_cap > (uint64_t)kSuperMaxSub * (kFinCapSmall * 7 / 10) ? kFinCapLarge : kFinCapSmall;
-    pl.sub_target = pl.fin_cap * 7 / 10;
-    if (const char *v = getenv("KC_SW_SUB_TARGET")) {       // development / test knob: forces deep level-2 plans on small inputs
-        const int t = atoi(v);
-        if (t > 0) pl.sub_target = (uint32_t)t;
-    }
-    const int sig = pl.W == 1 ? (masked ? (int)(2 * mm) : 64) : 64;
+    pl.sub_target = plan_sub_target(pl.fin_cap);
+    const int sig = key_sig_bits(pl.W, pl.last_mask);
     pl.b1 = sig < 10 ? sig : 10;
     plan_layout(pl, ext_e);
     *out = pl;
@@ -1987,22 +1825,16 @@ bool place_plan(uint32_t k, bool strict, uint64_t n_records, SuperPlan *out) {
     SuperPlan pl{};
     pl.W = (int)((k + 31) / 32);
     pl.k = k;
-    const uint32_t mm = k % 32;
-    const bool masked = strict ? (mm != 0) : (mm >= 1 && mm <= 28);    // SURVEY F4
-    pl.span = masked ? k : 32u * pl.W;
-    pl.last_mask = masked ? (~0ull << (64 - 2 * mm)) : ~0ull;
+    pl.last_mask = key_last_mask(k, strict);
+    pl.span = pl.last_mask != ~0ull ? k : 32u * pl.W;
     pl.n_bins = 8;                                  // (unused: the arrays just exist)
     pl.d_cap = n_records < 1024 ? 1024 : n_records;
     // occurrences, not distinct keys, fill the sub-buckets; the folding S3c holds two copies of a
     // sub-bucket, so only its 2048-record variant fits shared memory for every key width
     // (192/256-bit keys: 1024-record sub-buckets keep two or three CTAs on an SM, as long as 2^20 of them are enough)
     pl.fin_cap = pl.W >= 3 && n_records <= (uint64_t)kSuperMaxSub * (kFinCapWide * 7 / 10) ? kFinCapWide : kFinCapSmall;
-    pl.sub_target = pl.fin_cap * 7 / 10;
-    if (const char *v = getenv("KC_SW_SUB_TARGET")) {
-        const int t = atoi(v);
-        if (t > 0) pl.sub_target = (uint32_t)t;
-    }
-    const int sig = pl.W == 1 ? (masked ? (int)(2 * mm) : 64) : 64;
+    pl.sub_target = plan_sub_target(pl.fin_cap);
+    const int sig = key_sig_bits(pl.W, pl.last_mask);
     pl.b1 = sig < 10 ? sig : 10;
     plan_layout(pl, false);
     *out = pl;
@@ -2112,6 +1944,24 @@ cudaError_t super_count_bins(const SuperPlan &pl, bool add_phantom, void *ws, un
     return cudaErrorInvalidValue;
 }
 
+// S3a / S3b / the exchange's pull: in -> out by the plan's level-1 or level-2 digit (range: see rec_scatter_kernel)
+template <int W, int LEVEL>
+static cudaError_t launch_rec_scatter(const SuperPlan &pl, const uint64_t *in_keys, const uint32_t *in_counts,
+                                      uint64_t *out_keys, uint32_t *out_counts, const SuperPlanDev *plan,
+                                      unsigned long long *d_sc, uint32_t *cursor, const uint32_t *range, int n_sms,
+                                      cudaStream_t s) {
+    const uint32_t smem = RsCfg<W>::TILE * (8 * W + 4) + 3 * kRsBinsPadded * 4;
+    auto kern = rec_scatter_kernel<W, LEVEL>;
+    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return e;
+    int per_sm = 1;
+    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, kRsThreads, smem);
+    if (per_sm < 1) per_sm = 1;
+    kern<<<(uint32_t)n_sms * per_sm, kRsThreads, smem, s>>>(in_keys, in_counts, out_keys, out_counts, plan, pl.b1,
+                                                           &d_sc[SW_D], pl.d_cap, cursor, range);
+    return cudaGetLastError();
+}
+
 template <int W>
 static cudaError_t super_place_w(const SuperPlan &pl, void *ws, unsigned long long *d_sc, int n_sms, cudaStream_t s,
                                  cudaEvent_t *evs) {
@@ -2124,28 +1974,16 @@ static cudaError_t super_place_w(const SuperPlan &pl, void *ws, unsigned long lo
              *base2 = at<uint32_t>(ws, pl.off_base2), *cur2 = at<uint32_t>(ws, pl.off_cur2);
     SuperPlanDev *plan = at<SuperPlanDev>(ws, pl.off_plan);
     // ---- S3a: level-1 bases + device plan, scatter D -> E
-    const int sig = pl.W == 1 ? 64 - (int)__builtin_ctzll(pl.last_mask ? pl.last_mask : 1) : 64;
-    sw_plan_kernel<<<1, 1024, 0, s>>>(hist1, pl.b1, pl.d_cap, pl.sub_target, sig, base1, cur1, plan, d_sc);
-    const uint32_t rs_smem = RsCfg<W>::TILE * (8 * W + 4) + 3 * kRsBinsPadded * 4;
-    auto k1 = rec_scatter_kernel<W, 1>;
-    auto k2 = rec_scatter_kernel<W, 2>;
-    if ((e = cudaFuncSetAttribute(k1, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)rs_smem)) != cudaSuccess) return e;
-    if ((e = cudaFuncSetAttribute(k2, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)rs_smem)) != cudaSuccess) return e;
-    int per_sm = 1;
-    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k1, kRsThreads, rs_smem);
-    if (per_sm < 1) per_sm = 1;
-    const uint32_t grid = (uint32_t)n_sms * per_sm;
-    k1<<<grid, kRsThreads, rs_smem, s>>>(dk, dc, ek, ec, plan, pl.b1, &d_sc[SW_D], pl.d_cap, cur1, nullptr);
-    if ((e = cudaGetLastError()) != cudaSuccess) return e;
+    sw_plan_kernel<<<1, 1024, 0, s>>>(hist1, pl.b1, pl.d_cap, pl.sub_target, key_sig_bits(pl.W, pl.last_mask), base1, cur1,
+                                      plan, d_sc);
+    if ((e = launch_rec_scatter<W, 1>(pl, dk, dc, ek, ec, plan, d_sc, cur1, nullptr, n_sms, s)) != cudaSuccess) return e;
     if (evs) cudaEventRecord(evs[0], s);
     // ---- level-2 histogram + scan (b2 == 0: one counter per level-1 bucket)
     rec_hist2_kernel<W><<<(uint32_t)n_sms * 8, 256, 0, s>>>(ek, plan, hist2);
-    sw_scan_kernel<<<(kSuperMaxSub + kScanTile - 1) / kScanTile, 1024, 0, s>>>(hist2, &plan->n_sub, 0, base2, cur2, nullptr);
-    if ((e = cudaGetLastError()) != cudaSuccess) return e;
+    if ((e = exclusive_scan(hist2, &plan->n_sub, kSuperMaxSub, base2, cur2, nullptr, s)) != cudaSuccess) return e;
     if (evs) cudaEventRecord(evs[1], s);
     // ---- S3b: scatter E -> D by the level-2 digit
-    k2<<<grid, kRsThreads, rs_smem, s>>>(ek, ec, dk, dc, plan, pl.b1, &d_sc[SW_D], pl.d_cap, cur2, nullptr);
-    if ((e = cudaGetLastError()) != cudaSuccess) return e;
+    if ((e = launch_rec_scatter<W, 2>(pl, ek, ec, dk, dc, plan, d_sc, cur2, nullptr, n_sms, s)) != cudaSuccess) return e;
     if (evs) cudaEventRecord(evs[2], s);
     return cudaSuccess;
 }
@@ -2258,7 +2096,8 @@ cudaError_t super_finish(const SuperPlan &pl, bool dup, void *ws, unsigned long 
 cudaError_t super_big_gather(const SuperPlan &pl, void *ws, uint64_t *tk, uint32_t *tc, int n_sms, cudaStream_t s) {
     SuperPlanDev *plan = at<SuperPlanDev>(ws, pl.off_plan);
     uint32_t *big = at<uint32_t>(ws, pl.off_big), *bigoff = at<uint32_t>(ws, pl.off_bigoff), *base2 = at<uint32_t>(ws, pl.off_base2);
-    sw_scan_kernel<<<(kSuperMaxSub + kScanTile - 1) / kScanTile, 1024, 0, s>>>(big, &plan->n_sub, 0, bigoff, nullptr, nullptr);
+    cudaError_t e = exclusive_scan(big, &plan->n_sub, kSuperMaxSub, bigoff, nullptr, nullptr, s);
+    if (e != cudaSuccess) return e;
     const uint64_t *dk = at<uint64_t>(ws, pl.off_dk);
     const uint32_t *dc = at<uint32_t>(ws, pl.off_dc);
     if (pl.W == 1) big_gather_kernel<1><<<(uint32_t)n_sms * 8, 256, 0, s>>>(dk, dc, base2, big, bigoff, plan, tk, tc);
@@ -2292,20 +2131,15 @@ cudaError_t super_big_place(const SuperPlan &pl, bool dup, void *ws, unsigned lo
 
 cudaError_t super_fold_offsets(const SuperPlan &pl, void *ws, unsigned long long *d_sc, cudaStream_t s) {
     SuperPlanDev *plan = at<SuperPlanDev>(ws, pl.off_plan);
-    sw_scan_kernel<<<(kSuperMaxSub + kScanTile - 1) / kScanTile, 1024, 0, s>>>(
-        at<uint32_t>(ws, pl.off_mout), &plan->n_sub, 0, at<uint32_t>(ws, pl.off_off), nullptr, &d_sc[SW_OUT]);
-    return cudaGetLastError();
+    return exclusive_scan(at<uint32_t>(ws, pl.off_mout), &plan->n_sub, kSuperMaxSub, at<uint32_t>(ws, pl.off_off), nullptr,
+                          &d_sc[SW_OUT], s);
 }
 
 cudaError_t super_gather(const SuperPlan &pl, void *ws, const uint64_t *tmp_keys, const uint32_t *tmp_counts,
                          uint64_t *out_keys, uint32_t *out_counts, int n_sms, cudaStream_t s) {
     const SuperPlanDev *plan = at<SuperPlanDev>(ws, pl.off_plan);
     const uint32_t *src = at<uint32_t>(ws, pl.off_base2), *off = at<uint32_t>(ws, pl.off_off);
-    if (pl.W == 1) sw_gather_kernel<1><<<(uint32_t)n_sms * 8, 256, 0, s>>>(tmp_keys, tmp_counts, src, off, plan, out_keys, out_counts);
-    else if (pl.W == 2) sw_gather_kernel<2><<<(uint32_t)n_sms * 8, 256, 0, s>>>(tmp_keys, tmp_counts, src, off, plan, out_keys, out_counts);
-    else if (pl.W == 3) sw_gather_kernel<3><<<(uint32_t)n_sms * 8, 256, 0, s>>>(tmp_keys, tmp_counts, src, off, plan, out_keys, out_counts);
-    else sw_gather_kernel<4><<<(uint32_t)n_sms * 8, 256, 0, s>>>(tmp_keys, tmp_counts, src, off, plan, out_keys, out_counts);
-    return cudaGetLastError();
+    return gather_records(pl.W, tmp_keys, tmp_counts, src, off, &plan->n_sub, kSuperMaxSub, out_keys, out_counts, n_sms, s);
 }
 
 void super_use_large_finish(SuperPlan *pl) { pl->fin_cap = kFinCapLarge; }
@@ -2316,25 +2150,18 @@ template <int W>
 static cudaError_t super_x_local_w(const SuperPlan &pl, void *ws, unsigned long long *d_sc, const uint32_t *d_all_hist,
                                    uint32_t rank, uint32_t n_ranks, bool keep_ranges, void *const *peer_ws, int n_sms,
                                    cudaStream_t s) {
-    cudaError_t e;
     if (pl.ext_e) return cudaErrorInvalidValue;      // the peers find E through the workspace mapping
     uint64_t *dk = at<uint64_t>(ws, pl.off_dk), *ek = at<uint64_t>(ws, pl.off_ek);
     uint32_t *dc = at<uint32_t>(ws, pl.off_dc), *ec = at<uint32_t>(ws, pl.off_ec);
     SuperPlanDev *plan = at<SuperPlanDev>(ws, pl.off_plan);
-    const int sig = pl.W == 1 ? 64 - (int)__builtin_ctzll(pl.last_mask ? pl.last_mask : 1) : 64;
     XScalars xs{};
     for (uint32_t i = 0; i < n_ranks; i++) xs.sc[i] = peer_ws ? at<unsigned long long>(peer_ws[i], pl.off_sc) : d_sc;
     x_plan_kernel<<<1, 1024, 0, s>>>(d_all_hist, rank, n_ranks, keep_ranges ? 1 : 0, pl.d_cap, pl.sub_target,
-                                     pl.fin_cap == kFinCapLarge ? 1 : 0, sig, at<uint32_t>(ws, pl.off_base1),
-                                     at<uint32_t>(ws, pl.off_cur1), plan, at<XDev>(ws, pl.off_x), d_sc, xs);
-    const uint32_t rs_smem = RsCfg<W>::TILE * (8 * W + 4) + 3 * kRsBinsPadded * 4;
-    auto k1 = rec_scatter_kernel<W, 1>;
-    if ((e = cudaFuncSetAttribute(k1, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)rs_smem)) != cudaSuccess) return e;
-    int per_sm = 1;
-    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k1, kRsThreads, rs_smem);
-    if (per_sm < 1) per_sm = 1;
-    k1<<<(uint32_t)n_sms * per_sm, kRsThreads, rs_smem, s>>>(dk, dc, ek, ec, plan, pl.b1, &d_sc[SW_D], pl.d_cap,
-                                                            at<uint32_t>(ws, pl.off_cur1), nullptr);
+                                     pl.fin_cap == kFinCapLarge ? 1 : 0, key_sig_bits(pl.W, pl.last_mask),
+                                     at<uint32_t>(ws, pl.off_base1), at<uint32_t>(ws, pl.off_cur1), plan,
+                                     at<XDev>(ws, pl.off_x), d_sc, xs);
+    cudaError_t e = launch_rec_scatter<W, 1>(pl, dk, dc, ek, ec, plan, d_sc, at<uint32_t>(ws, pl.off_cur1), nullptr, n_sms, s);
+    if (e != cudaSuccess) return e;
     rec_hist2_kernel<W><<<(uint32_t)n_sms * 8, 256, 0, s>>>(ek, plan, at<uint32_t>(ws, pl.off_hist2));
     return cudaGetLastError();
 }
@@ -2350,7 +2177,6 @@ cudaError_t super_x_local(const SuperPlan &pl, void *ws, unsigned long long *d_s
 template <int W>
 static cudaError_t super_x_pull_w(const SuperPlan &pl, void *ws, unsigned long long *d_sc, void *const *peer_ws,
                                   uint32_t rank, uint32_t n_ranks, int n_sms, cudaStream_t s) {
-    cudaError_t e;
     SuperPlanDev *plan = at<SuperPlanDev>(ws, pl.off_plan);
     XDev *x = at<XDev>(ws, pl.off_x);
     XPeers peers{};
@@ -2361,13 +2187,8 @@ static cudaError_t super_x_pull_w(const SuperPlan &pl, void *ws, unsigned long l
     }
     uint32_t *h2m = at<uint32_t>(ws, pl.off_h2m), *base2 = at<uint32_t>(ws, pl.off_base2), *cur2 = at<uint32_t>(ws, pl.off_cur2);
     x_merge_hist_kernel<<<(uint32_t)n_sms * 4, 256, 0, s>>>(peers, n_ranks, plan, h2m);
-    sw_scan_kernel<<<(kSuperMaxSub + kScanTile - 1) / kScanTile, 1024, 0, s>>>(h2m, &plan->n_sub, 0, base2, cur2, nullptr);
-    const uint32_t rs_smem = RsCfg<W>::TILE * (8 * W + 4) + 3 * kRsBinsPadded * 4;
-    auto k2 = rec_scatter_kernel<W, 2>;
-    if ((e = cudaFuncSetAttribute(k2, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)rs_smem)) != cudaSuccess) return e;
-    int per_sm = 1;
-    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k2, kRsThreads, rs_smem);
-    if (per_sm < 1) per_sm = 1;
+    cudaError_t e = exclusive_scan(h2m, &plan->n_sub, kSuperMaxSub, base2, cur2, nullptr, s);
+    if (e != cudaSuccess) return e;
     // the level-2 scatter reads this rank's key range straight out of every source's grouped array:
     // the exchange happens inside the kernel's loads (NVLink / NVSwitch for the peers). Rank r starts
     // with source r + 1 and ends with its own records: at any time every source is read by one peer,
@@ -2375,11 +2196,11 @@ static cudaError_t super_x_pull_w(const SuperPlan &pl, void *ws, unsigned long l
     // bottleneck of a round while the others idle.
     for (uint32_t j = 1; j <= n_ranks; j++) {
         const uint32_t i = (rank + j) % n_ranks;
-        k2<<<(uint32_t)n_sms * per_sm, kRsThreads, rs_smem, s>>>(peers.keys[i], peers.counts[i], at<uint64_t>(ws, pl.off_dk),
-                                                                at<uint32_t>(ws, pl.off_dc), plan, pl.b1, &d_sc[SW_D],
-                                                                pl.d_cap, cur2, &x->src_range[i][0]);
+        e = launch_rec_scatter<W, 2>(pl, peers.keys[i], peers.counts[i], at<uint64_t>(ws, pl.off_dk),
+                                     at<uint32_t>(ws, pl.off_dc), plan, d_sc, cur2, &x->src_range[i][0], n_sms, s);
+        if (e != cudaSuccess) return e;
     }
-    return cudaGetLastError();
+    return cudaSuccess;
 }
 
 cudaError_t super_x_pull(const SuperPlan &pl, void *ws, unsigned long long *d_sc, void *const *peer_ws, uint32_t rank,
