@@ -363,6 +363,38 @@ int  kc_merge_runs(kc_ctx *ctx, kc_run *const *runs, uint32_t n, kc_run **out);
 #define KC_COUNTS_B            4u
 int  kc_run_combine(kc_ctx *ctx, const kc_run *a, const kc_run *b, uint32_t op, uint32_t counts, kc_run **out);
 
+/* ---- lookups in a run: what `jellyfish query` and KMC's lookups give (the count of given k-mers), and
+ * the per-read view behind read filtering (`kmc_tools filter`, error-read, host or contaminant removal),
+ * on the device ----
+ * kc_run_lookup:  counts[i] = the count in `run` of key i, 0 if the run has no such record. keys: n x W
+ *   uint64, key-major, the record key layout (word 0 = most significant bases). On a KC_CANONICAL context
+ *   each key is folded to min(x, rc(x)) first, so either strand can be asked. On a KC_COMPAT_STRICT or
+ *   KC_CANONICAL context a key with bits set past its k bases is not a k-mer: its count is 0.
+ * kc_query_reads: reads = packed lines of the context's read_len L (a partial trailing read is ignored),
+ *   R = n_bytes / L reads, L - k + 1 slots each. Outputs (either may be NULL, not both):
+ *     slot_counts[r*(L-k+1) + p] = the count in `run` of the k-mer of read r at position p; 0 when that
+ *                                  window holds no k-mer (a byte other than A, C, G, T) or the k-mer is absent
+ *     read_hits[r]               = windows of read r holding a k-mer whose count c has lo <= c <= hi (an
+ *                                  absent k-mer has c = 0; a window holding no k-mer is never counted)
+ *   A slot's key is the key counting puts its occurrence under on this context (the same extraction, the
+ *   same flags): under KC_COMPAT_REF the reference's, quirks included (at k % 32 in {29, 30, 31} it spans
+ *   32 bases, positions past the read end contributing 0); under KC_CANONICAL min(x, rc(x)). So against a
+ *   run counted from exactly these reads with the same flags, every window holding a k-mer has a count >= 1.
+ * Both: records a run hides with its strict-mode skip are not found; the KC_COMPAT_REF zero-count key-0
+ * record is an ordinary record (count 0). An empty run finds nothing. The run may come from another
+ * context with the same key width; a run does not say which keys it holds, so ask a canonical run on a
+ * canonical context. Every pointer may be host memory (pageable or pinned: staged through the context's
+ * stream) or device memory of the context's device (used in place; device reads must be 16-byte aligned, as
+ * for kc_count_device; device keys of 128 or 256 bits not 16-byte aligned, and device outputs not 4-byte
+ * aligned, are staged through scratch with a device-to-device copy). Work goes in pieces of whole reads
+ * (keys), so scratch stays bounded; the call returns when the outputs are written. n == 0, n_bytes < L: success, nothing written.
+ * KC_ERR_ARG: a null ctx, run or needed pointer, both outputs NULL, lo > hi, a run whose key width is not
+ * the context's, device memory of another device, device reads not 16-byte aligned.
+ * KC_ERR_NOMEM: scratch could not be allocated; nothing is left allocated. */
+int  kc_run_lookup(kc_ctx *ctx, const kc_run *run, const uint64_t *keys, uint64_t n, uint32_t *counts);
+int  kc_query_reads(kc_ctx *ctx, const kc_run *run, const void *reads, uint64_t n_bytes,
+                    uint32_t lo, uint32_t hi, uint32_t *slot_counts, uint32_t *read_hits);
+
 /* ---- measurement support (not a reference interface): deterministic synthetic reads
  * written straight into device memory as packed lines; bit-identical to the host
  * generator used by the tests.  genome_len == 0 -> iid bases; zipf_loci > 0 -> half of

@@ -102,6 +102,8 @@ SYMBOLS = {
     "kc_run_filter": (_i, [_vp, _vp, _u32, _u32, _pp]),
     "kc_merge_runs": (_i, [_vp, _pp, _u32, _pp]),
     "kc_run_combine": (_i, [_vp, _vp, _vp, _u32, _u32, _pp]),
+    "kc_run_lookup": (_i, [_vp, _vp, _vp, _u64, _vp]),
+    "kc_query_reads": (_i, [_vp, _vp, _vp, _u64, _u32, _u32, _vp, _vp]),
     "kc_place_next_run": (_i, [_vp, _vp, _vp, _vp, _u64, _u32]),
     "kc_peer_alloc": (_i, [_vp, _u64, C.POINTER(_vp), _vp]),
     "kc_peer_open": (_i, [_vp, _vp, C.POINTER(_vp)]),

@@ -2273,3 +2273,187 @@ int kc_run_combine(kc_ctx *c, const kc_run *a, const kc_run *b, uint32_t op, uin
 }
 
 }  // extern "C"
+
+// ------------------------------------------------------------------ lookups in a run
+namespace {
+
+// Where a caller's pointer lives: device memory of the context's device (or managed) is used in place,
+// host memory (pageable or pinned) is staged; device memory of another device is refused.
+int locate(kc_ctx *c, const void *p, const char *what, bool *on_device) {
+    cudaPointerAttributes a{};
+    if (cudaPointerGetAttributes(&a, p) != cudaSuccess) {
+        cudaGetLastError();
+        a.type = cudaMemoryTypeUnregistered;
+    }
+    *on_device = a.type == cudaMemoryTypeDevice || a.type == cudaMemoryTypeManaged;
+    if (a.type == cudaMemoryTypeDevice && a.device != c->cfg.device)
+        return c->set_error(KC_ERR_ARG, "%s is memory of device %d, the context runs on device %d", what, a.device, c->cfg.device);
+    return KC_OK;
+}
+
+// Keys, reads and outputs are handled in pieces of this many keys (slots), so the scratch of a call is
+// bounded whatever its size: 8 W + 1 bytes a slot, plus 4 for staged counts.
+constexpr uint64_t kQueryPieceSlots = 1ull << 24;
+
+// The run's index (into *offsets, scratch on s) and the lookup parameters every piece shares.
+int query_prepare(kc_ctx *c, const kc_run *r, cudaStream_t s, DevBuf *offsets, QueryLookup *q, int *launches) {
+    const uint64_t n = r->n - r->skip, last_mask = key_last_mask(c->cfg.k, c->strict);
+    const int bits = query_index_bits(n, key_sig_bits(c->W, last_mask));
+    KC_TRY(offsets->alloc(c, ((1ull << bits) + 1) * 8));
+    KC_CUDA_TRY(c, query_index(r->d_keys + r->skip * r->W, c->W, n, bits, offsets->get<uint64_t>(), c->n_sms, s, launches));
+    *q = QueryLookup{};
+    q->run_keys = r->d_keys + r->skip * r->W;
+    q->run_counts = r->d_counts + r->skip;
+    q->offsets = offsets->get<uint64_t>();
+    q->shift = 64u - bits;
+    q->nk = 1;
+    return KC_OK;
+}
+
+void query_account(kc_ctx *c, int launches, uint64_t h2d, uint64_t d2h) {
+    std::lock_guard<std::mutex> g(c->mu);
+    c->stats.launches += launches;
+    c->stats.h2d_bytes += h2d;
+    c->stats.d2h_bytes += d2h;
+}
+
+bool aligned(const void *p, uintptr_t to) { return (reinterpret_cast<uintptr_t>(p) & (to - 1)) == 0; }
+
+// other streams (slots) may have produced the run
+int sync_slots(kc_ctx *c) {
+    for (auto &sl : c->slots)
+        if (sl.stream) KC_CUDA_TRY(c, cudaStreamSynchronize(sl.stream));
+    return KC_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int kc_run_lookup(kc_ctx *c, const kc_run *r, const uint64_t *keys, uint64_t n, uint32_t *counts) {
+    KC_TRY(check_ctx(c));
+    if (!r || !counts || (n && !keys)) return c->set_error(KC_ERR_ARG, "null argument");
+    if (r->W != c->W)
+        return c->set_error(KC_ERR_ARG, "kc_run_lookup: a run of %d key words, the context's keys have %d", r->W, c->W);
+    std::lock_guard<std::recursive_mutex> dg(c->direct_mu);
+    if (n == 0) return KC_OK;
+    cudaSetDevice(c->cfg.device);
+    bool keys_dev = false, counts_dev = false;
+    KC_TRY(locate(c, keys, "keys", &keys_dev));
+    KC_TRY(locate(c, counts, "counts", &counts_dev));
+    KC_TRY(sync_slots(c));
+    cudaStream_t s = c->stream;
+    const int W = c->W;
+    // device arrays the kernel cannot load in place (128- and 256-bit keys are loaded 16 bytes at a time) are
+    // staged like host memory, with a device-to-device copy
+    const bool keys_here = keys_dev && aligned(keys, W == 2 || W == 4 ? 16 : 8);
+    const bool counts_here = counts_dev && aligned(counts, 4);
+    const uint64_t piece = std::min(n, kQueryPieceSlots), last_mask = key_last_mask(c->cfg.k, c->strict);
+    DevBuf offsets(s), d_keys(s), d_counts(s);
+    QueryLookup q;
+    int launches = 0;
+    KC_TRY(query_prepare(c, r, s, &offsets, &q, &launches));
+    if (!keys_here) KC_TRY(d_keys.alloc(c, piece * W * 8));
+    if (!counts_here) KC_TRY(d_counts.alloc(c, piece * 4));
+    q.tail_bits = c->strict ? ~last_mask : 0;           // strict and canonical keys are exactly k bases
+    q.fold = (c->key_flags & KC_CANONICAL) != 0;
+    q.rc_sh = __builtin_ctzll(last_mask);
+    uint64_t h2d = 0, d2h = 0;
+    for (uint64_t i = 0; i < n; i += piece) {
+        const uint64_t m = std::min(piece, n - i);
+        q.keys = keys_here ? keys + i * W : d_keys.get<uint64_t>();
+        q.counts = counts_here ? counts + i : d_counts.get<uint32_t>();
+        q.n = m;
+        if (!keys_here) {
+            KC_CUDA_TRY(c, cudaMemcpyAsync(d_keys.get(), keys + i * W, m * W * 8, cudaMemcpyDefault, s));
+            if (!keys_dev) h2d += m * W * 8;
+        }
+        KC_CUDA_TRY(c, query_lookup(q, W, s));
+        launches++;
+        if (!counts_here) {
+            KC_CUDA_TRY(c, cudaMemcpyAsync(counts + i, d_counts.get(), m * 4, cudaMemcpyDefault, s));
+            if (!counts_dev) d2h += m * 4;
+        }
+    }
+    KC_CUDA_TRY(c, cudaStreamSynchronize(s));
+    query_account(c, launches, h2d, d2h);
+    return KC_OK;
+}
+
+int kc_query_reads(kc_ctx *c, const kc_run *r, const void *reads, uint64_t n_bytes, uint32_t lo, uint32_t hi,
+                   uint32_t *slot_counts, uint32_t *read_hits) {
+    KC_TRY(check_ctx(c));
+    if (!r || (n_bytes && !reads)) return c->set_error(KC_ERR_ARG, "null argument");
+    if (!slot_counts && !read_hits) return c->set_error(KC_ERR_ARG, "kc_query_reads: slot_counts and read_hits are both NULL");
+    if (lo > hi) return c->set_error(KC_ERR_ARG, "kc_query_reads: lo %u > hi %u", lo, hi);
+    if (r->W != c->W)
+        return c->set_error(KC_ERR_ARG, "kc_query_reads: a run of %d key words, the context's keys have %d", r->W, c->W);
+    std::lock_guard<std::recursive_mutex> dg(c->direct_mu);
+    const uint32_t L = c->cfg.read_len, k = c->cfg.k, nk = L - k + 1;
+    const uint64_t R = n_bytes / L;
+    if (R == 0) return KC_OK;
+    cudaSetDevice(c->cfg.device);
+    bool reads_dev = false, slots_dev = false, hits_dev = false;
+    KC_TRY(locate(c, reads, "reads", &reads_dev));
+    if (slot_counts) KC_TRY(locate(c, slot_counts, "slot_counts", &slots_dev));
+    if (read_hits) KC_TRY(locate(c, read_hits, "read_hits", &hits_dev));
+    if (reads_dev && !aligned(reads, 16)) return c->set_error(KC_ERR_ARG, "device reads must be 16-byte aligned");
+    // device outputs not 4-byte aligned are staged like host memory, with a device-to-device copy
+    const bool slots_here = slots_dev && aligned(slot_counts, 4), hits_here = hits_dev && aligned(read_hits, 4);
+    KC_TRY(sync_slots(c));
+    cudaStream_t s = c->stream;
+    const int W = c->W;
+    // pieces of whole reads, a multiple of 16 of them (every piece of device reads stays 16-byte aligned)
+    uint64_t piece_reads = std::max<uint64_t>(16, (kQueryPieceSlots / nk) & ~15ull);
+    if (piece_reads > R) piece_reads = R;
+    const uint64_t piece_slots = piece_reads * nk;
+    DevBuf offsets(s), d_keys(s), d_valid(s), d_inv(s), d_reads(s), d_slots(s), d_hits(s);
+    QueryLookup q;
+    int launches = 0;
+    KC_TRY(query_prepare(c, r, s, &offsets, &q, &launches));
+    KC_TRY(d_keys.alloc(c, piece_slots * W * 8));
+    KC_TRY(d_valid.alloc(c, piece_slots));
+    KC_TRY(d_inv.alloc(c, 8));
+    if (!reads_dev) KC_TRY(d_reads.alloc(c, piece_reads * L));
+    if (slot_counts && !slots_here) KC_TRY(d_slots.alloc(c, piece_slots * 4));
+    if (read_hits && !hits_here) KC_TRY(d_hits.alloc(c, piece_reads * 4));
+    if (read_hits && hits_here) KC_CUDA_TRY(c, cudaMemsetAsync(read_hits, 0, R * 4, s));
+    q.keys = d_keys.get<uint64_t>();
+    q.valid = d_valid.get<uint8_t>();
+    q.nk = nk;
+    q.lo = lo;
+    q.hi = hi;
+    uint64_t h2d = 0, d2h = 0;
+    for (uint64_t r0 = 0; r0 < R; r0 += piece_reads) {
+        const uint64_t nr = std::min(piece_reads, R - r0), ns = nr * nk;
+        const uint8_t *src = static_cast<const uint8_t *>(reads) + r0 * L;
+        if (!reads_dev) {
+            KC_CUDA_TRY(c, cudaMemcpyAsync(d_reads.get(), src, nr * L, cudaMemcpyHostToDevice, s));
+            h2d += nr * L;
+            src = d_reads.get<uint8_t>();
+        }
+        ExtractParams ep;
+        if (!extract_plan(src, nr, L, k, c->key_flags, d_inv.get<unsigned long long>(), &ep))
+            return c->set_error(KC_ERR_ARG, "unsupported shape k=%u read_len=%u", k, L);
+        KC_CUDA_TRY(c, query_extract(ep, W, d_keys.get<uint64_t>(), d_valid.get<uint8_t>(), c->n_sms, s));
+        q.n = ns;
+        q.counts = !slot_counts ? nullptr : slots_here ? slot_counts + r0 * nk : d_slots.get<uint32_t>();
+        q.hits = !read_hits ? nullptr : hits_here ? read_hits + r0 : d_hits.get<uint32_t>();
+        if (read_hits && !hits_here) KC_CUDA_TRY(c, cudaMemsetAsync(d_hits.get(), 0, nr * 4, s));
+        KC_CUDA_TRY(c, query_lookup(q, W, s));
+        launches += 2;
+        if (slot_counts && !slots_here) {
+            KC_CUDA_TRY(c, cudaMemcpyAsync(slot_counts + r0 * nk, d_slots.get(), ns * 4, cudaMemcpyDefault, s));
+            if (!slots_dev) d2h += ns * 4;
+        }
+        if (read_hits && !hits_here) {
+            KC_CUDA_TRY(c, cudaMemcpyAsync(read_hits + r0, d_hits.get(), nr * 4, cudaMemcpyDefault, s));
+            if (!hits_dev) d2h += nr * 4;
+        }
+    }
+    KC_CUDA_TRY(c, cudaStreamSynchronize(s));
+    query_account(c, launches, h2d, d2h);
+    return KC_OK;
+}
+
+}  // extern "C"

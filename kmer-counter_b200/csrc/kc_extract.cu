@@ -43,23 +43,6 @@ bool extract_plan(const void *d_reads, uint64_t n_reads, uint32_t L, uint32_t k,
     return true;
 }
 
-template <int W, class Sink>
-static cudaError_t launch_extract(const ExtractParams &p, Sink sink, int n_sms, cudaStream_t s) {
-    if (p.n_tiles == 0) return cudaSuccess;
-    auto kern = extract_kernel_for<W, Sink>(p);
-    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p.smem_total);
-    if (e != cudaSuccess) return e;
-    int per_sm = 1;
-    e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, kExtractThreads, p.smem_total);
-    if (e != cudaSuccess) return e;
-    if (per_sm < 1) per_sm = 1;
-    if (per_sm > 4) per_sm = 4;
-    uint32_t grid = (uint32_t)n_sms * per_sm;      // persistent: a whole number of CTAs per SM
-    if (grid > p.n_tiles) grid = p.n_tiles;
-    kern<<<grid, kExtractThreads, p.smem_total, s>>>(p, sink);
-    return cudaGetLastError();
-}
-
 cudaError_t launch_extract_store(const ExtractParams &p, int W, uint64_t *d_keys, int n_sms, cudaStream_t s) {
     switch (W) {
         case 1: return launch_extract<1>(p, StoreSink<1>{{}, d_keys}, n_sms, s);

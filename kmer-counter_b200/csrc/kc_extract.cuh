@@ -341,4 +341,22 @@ inline auto extract_kernel_for(const ExtractParams &p) {
     return (p.plan_flags & kPlanCanonical) ? extract_kernel<W, Sink, true> : extract_kernel<W, Sink, false>;
 }
 
+// Launch the plan's instantiation persistently: a whole number of CTAs per SM (at most 4), no more than tiles.
+template <int W, class Sink>
+inline cudaError_t launch_extract(const ExtractParams &p, Sink sink, int n_sms, cudaStream_t s) {
+    if (p.n_tiles == 0) return cudaSuccess;
+    auto kern = extract_kernel_for<W, Sink>(p);
+    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p.smem_total);
+    if (e != cudaSuccess) return e;
+    int per_sm = 1;
+    e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, kExtractThreads, p.smem_total);
+    if (e != cudaSuccess) return e;
+    if (per_sm < 1) per_sm = 1;
+    if (per_sm > 4) per_sm = 4;
+    uint32_t grid = (uint32_t)n_sms * per_sm;      // persistent: a whole number of CTAs per SM
+    if (grid > p.n_tiles) grid = p.n_tiles;
+    kern<<<grid, kExtractThreads, p.smem_total, s>>>(p, sink);
+    return cudaGetLastError();
+}
+
 }  // namespace kc

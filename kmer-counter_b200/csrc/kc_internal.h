@@ -100,6 +100,31 @@ cudaError_t combine_pair(const uint64_t *ka, const uint32_t *ca, uint64_t na, co
                          uint64_t nb, int W, uint32_t op, uint32_t counts, uint64_t *out_keys, uint32_t *out_counts,
                          unsigned long long *d_num_out, void *ws, cudaStream_t s, int *n_launches);
 
+// ---- key lookup in a run (kc_query.cu)
+// bits of word 0 that select a bucket of the run index of n records: 2^bits + 1 uint64 offsets
+int query_index_bits(uint64_t n, int sig_bits);
+// offsets[j] = first record of the sorted keys whose top `bits` bits of word 0 are >= j, j = 0 .. 2^bits
+cudaError_t query_index(const uint64_t *keys, int W, uint64_t n, int bits, uint64_t *offsets, int n_sms, cudaStream_t s,
+                        int *n_launches);
+// keys[slot] and valid[slot] (1: the window holds a k-mer) for every slot r*(L-k+1)+p of the plan
+cudaError_t query_extract(const ExtractParams &p, int W, uint64_t *d_keys, uint8_t *d_valid, int n_sms, cudaStream_t s);
+struct QueryLookup {
+    const uint64_t *run_keys;     // the run: n_run sorted unique keys, their counts, its index
+    const uint32_t *run_counts;
+    const uint64_t *offsets;
+    uint32_t shift;               // 64 - index bits
+    const uint64_t *keys;         // n query keys (key-major)
+    const uint8_t *valid;         // NULL: every key is a query; else keys with valid[i] == 0 get count 0
+    uint64_t n;
+    uint64_t tail_bits;           // bits of word W-1 a k-mer leaves zero (strict keys); a key with one set gets 0
+    bool fold;                    // look up min(x, rc(x)) (canonical context), rc_sh = rc_shift_of(last_mask)
+    uint32_t rc_sh;
+    uint32_t *counts;             // NULL or counts[i] = the key's count, 0 if absent
+    uint32_t *hits;               // NULL or hits[i / nk] += valid keys with lo <= count <= hi (n < 2^32)
+    uint32_t nk, lo, hi;
+};
+cudaError_t query_lookup(const QueryLookup &p, int W, cudaStream_t s);
+
 // ---- hash table (kc_hash.cu), W == 1 only
 struct HashTable {
     uint64_t *slots;            // capacity x {key, count|pad} as 2 x uint64

@@ -421,6 +421,38 @@ class Counter:
         self._check(self._lib.kc_merge_parts(self._ctx, n, ka, ca, oa, na, n_sub, prefix_bits, C.byref(h)))
         return Run(self, h)
 
+    # -- lookups in a run (kc_run_lookup, kc_query_reads): key semantics, L and k are this counter's; the
+    # run may come from another counter with the same k
+    def lookup(self, run, keys) -> np.ndarray:
+        """uint32 count in `run` of every key ([n, W] uint64 host array, the record key layout), 0 if absent.
+        A canonical counter looks up min(x, rc(x)), so either strand can be asked."""
+        k = np.ascontiguousarray(keys, dtype=np.uint64).reshape(-1, self.words)
+        out = np.zeros(k.shape[0], dtype=np.uint32)
+        self._check(self._lib.kc_run_lookup(self._ctx, run._h, k.ctypes.data, k.shape[0], out.ctypes.data))
+        return out
+
+    def lookup_device(self, run, d_keys, n, d_counts):
+        """kc_run_lookup with device pointers: n x W uint64 keys in, n uint32 counts out."""
+        self._check(self._lib.kc_run_lookup(self._ctx, run._h, d_keys, int(n), d_counts))
+
+    def query_reads(self, run, reads, lo=1, hi=2**32 - 1, slot_counts=True) -> tuple:
+        """Host reads (packed lines of read_len) against `run`: (slot_counts uint32[R, L-k+1] or None,
+        hits uint32[R]). slot_counts[r, p] = count of read r's k-mer at position p (0: absent, or no k-mer
+        there); hits[r] = windows of read r holding a k-mer whose count is in [lo, hi] (absent = 0)."""
+        a = np.frombuffer(reads, dtype=np.uint8) if isinstance(reads, (bytes, bytearray)) else \
+            np.ascontiguousarray(reads, dtype=np.uint8)
+        R, nk = a.size // self.read_len, self.read_len - self.k + 1
+        sc = np.zeros((R, nk), dtype=np.uint32) if slot_counts else None
+        hits = np.zeros(R, dtype=np.uint32)
+        self._check(self._lib.kc_query_reads(self._ctx, run._h, a.ctypes.data, a.size, int(lo), int(hi),
+                                             sc.ctypes.data if sc is not None else None, hits.ctypes.data))
+        return sc, hits
+
+    def query_reads_device(self, run, d_reads, n_bytes, d_slot_counts, d_hits, lo=1, hi=2**32 - 1):
+        """kc_query_reads with device pointers (d_reads 16-byte aligned); 0 for an output that is not wanted."""
+        self._check(self._lib.kc_query_reads(self._ctx, run._h, d_reads, int(n_bytes), int(lo), int(hi),
+                                             d_slot_counts or None, d_hits or None))
+
     def merge(self, runs) -> Run:
         n = len(runs)
         arr = (C.c_void_p * max(n, 1))(*[r._h for r in runs])

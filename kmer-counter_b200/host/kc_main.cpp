@@ -13,6 +13,9 @@
 //                     a set operation of two record files on the GPU (kc_run_combine; KMC's
 //                     `kmc_tools simple`), counts= for keys in both (default: sum for union, min for
 //                     intersect), minCount= / maxCount= on the combined counts
+//   kmer_counter_b200 query <record file> <k> <k-mer file|-> <out|-> [compat=ref|strict] [canonical=1]
+//                     the count of each k-mer (one per line) in a record file, looked up on the GPU
+//                     (kc_query_reads; `jellyfish query`); the flags must match how the file was counted
 //
 // minCount= / maxCount= keep only the k-mers whose final count is in range (KMC -ci/-cx, Jellyfish
 // -L/-U); histoFile= writes the spectrum of the final counts before that filter: one line "c n" per
@@ -273,6 +276,104 @@ static int combine_files(int argc, char **argv) {
     return 0;
 }
 
+// `query <record file> <k> <k-mer file|-> <out|-> [compat=ref|strict] [canonical=1]`: jellyfish query. The
+// record file goes up as one run; the k-mers, one per line of exactly k letters, are looked up on the GPU
+// in pieces of lines, each line being one read of read_len = k with one slot (kc_query_reads: the keys are
+// built by the device's extraction, with the counting's semantics). Prints "<k-mer> <count>" per line, in
+// input order. The flags must be those the file was counted with: the file does not say.
+static int query_records(int argc, char **argv) {
+    const char *usage = "usage: %s query <record file> <k> <k-mer file|-> <out|-> [compat=ref|strict] [canonical=1]\n"
+                        "  one k-mer of exactly k letters per line; prints \"<k-mer> <count>\" per line, in input order.\n"
+                        "  compat= and canonical= must be those the record file was counted with (it does not say which).\n";
+    if (argc < 6) { fprintf(stderr, usage, argv[0]); return 2; }
+    char *end = nullptr;
+    const unsigned long k = strtoul(argv[3], &end, 10);
+    if (!end || *end || k < 1 || k > 128) { fprintf(stderr, usage, argv[0]); return 2; }
+    // as kc_create has it: canonical keys are strict keys, whatever compat= says
+    bool strict = false, canonical = false;
+    for (int i = 6; i < argc; i++) {
+        if (strcmp(argv[i], "compat=ref") == 0) strict = false;
+        else if (strcmp(argv[i], "compat=strict") == 0) strict = true;
+        else if (strcmp(argv[i], "canonical=1") == 0) canonical = true;
+        else if (strcmp(argv[i], "canonical=0") == 0) canonical = false;
+        else { fprintf(stderr, usage, argv[0]); return 2; }
+    }
+    const uint32_t flags = canonical ? KC_CANONICAL | KC_COMPAT_STRICT : strict ? KC_COMPAT_STRICT : KC_COMPAT_REF;
+    if (!(flags & KC_COMPAT_STRICT) && k % 32 >= 29) {
+        fprintf(stderr, "query: compat=ref at k=%lu keys span 32 bases, so a k-mer's text does not name a record; "
+                        "use a file counted with compat=strict or canonical=1\n", k);
+        return 2;
+    }
+    FILE *rf = fopen(argv[2], "rb");
+    if (!rf) { fprintf(stderr, "cannot open %s\n", argv[2]); return 1; }
+    std::vector<unsigned char> records;
+    {
+        unsigned char tmp[1 << 16];
+        size_t got;
+        while ((got = fread(tmp, 1, sizeof tmp, rf)) > 0) records.insert(records.end(), tmp, tmp + got);
+        const bool bad = ferror(rf);
+        fclose(rf);
+        if (bad) { fprintf(stderr, "read error on %s\n", argv[2]); return 1; }
+    }
+    FILE *in = strcmp(argv[4], "-") == 0 ? stdin : fopen(argv[4], "r");
+    if (!in) { fprintf(stderr, "cannot open %s\n", argv[4]); return 1; }
+    FILE *out = strcmp(argv[5], "-") == 0 ? stdout : fopen(argv[5], "w");
+    if (!out) { fprintf(stderr, "cannot open %s\n", argv[5]); if (in != stdin) fclose(in); return 1; }
+    kc_config cfg = {};
+    cfg.struct_size = sizeof cfg;
+    cfg.k = (uint32_t)k;
+    cfg.read_len = (uint32_t)k;
+    cfg.flags = flags;
+    kc_ctx *ctx = nullptr;
+    kc_run *run = nullptr;
+    int rc = kc_create(&cfg, &ctx);
+    if (rc != KC_OK) fprintf(stderr, "kc_create: %s\n", kc_last_error(nullptr));
+    if (rc == KC_OK && (rc = kc_run_upload(ctx, records.data(), records.size(), &run)) != KC_OK)
+        fprintf(stderr, "kmer_counter_b200 query: %s\n", kc_last_error(ctx));
+    std::vector<unsigned char>().swap(records);
+    const size_t piece = 1 << 20;                            // lines per kc_query_reads call
+    std::vector<char> reads(piece * k);
+    std::vector<uint32_t> counts(piece);
+    char *line = nullptr;
+    size_t line_cap = 0;
+    uint64_t lines = 0;
+    bool done = rc != KC_OK;
+    while (!done) {
+        size_t n = 0;
+        while (n < piece) {
+            ssize_t len = getline(&line, &line_cap, in);
+            if (len < 0) { done = true; break; }
+            if (len > 0 && line[len - 1] == '\n') len--;
+            if ((size_t)len != k) {
+                fprintf(stderr, "query: line %" PRIu64 " has %zd letters, not k=%lu\n", lines + n + 1, len, k);
+                rc = KC_ERR_ARG;
+                done = true;
+                break;
+            }
+            memcpy(&reads[n * k], line, k);
+            n++;
+        }
+        if (rc != KC_OK || n == 0) break;
+        if ((rc = kc_query_reads(ctx, run, reads.data(), n * k, 1, 0xffffffffu, counts.data(), nullptr)) != KC_OK) {
+            fprintf(stderr, "kmer_counter_b200 query: %s\n", kc_last_error(ctx));
+            break;
+        }
+        for (size_t i = 0; i < n && rc == KC_OK; i++)
+            if (fprintf(out, "%.*s %u\n", (int)k, &reads[i * k], counts[i]) < 0) rc = KC_ERR_IO;
+        lines += n;
+    }
+    free(line);
+    if (run) kc_run_free(ctx, run);
+    if (ctx) kc_destroy(ctx);
+    if (in != stdin) fclose(in);
+    const bool closed = out == stdout ? fflush(out) == 0 : fclose(out) == 0;
+    if (rc == KC_OK && !closed) rc = KC_ERR_IO;
+    if (rc == KC_ERR_IO) fprintf(stderr, "short write to %s\n", argv[5]);
+    if (rc != KC_OK) return 1;
+    fprintf(stderr, "query k=%lu lines=%" PRIu64 " -> %s\n", k, lines, argv[5]);
+    return 0;
+}
+
 // mode=accumulate: every chunk is only packed into super-window records (kc_accum_*); the count
 // happens once, over everything -- on one GPU, or on gpus=N with the two exchanges fused into the
 // counting kernels (kc_xchg_*). Returns 1 if this input / shape is not for this mode (the caller
@@ -434,6 +535,7 @@ int main(int argc, char **argv) {
     if ((argc == 5 || argc == 6) && strcmp(argv[1], "histo") == 0)
         return histo_records(argv[2], argv[3], (uint32_t)strtoul(argv[4], nullptr, 10), argc == 6 ? strtoll(argv[5], nullptr, 10) : 10000);
     if (argc >= 2 && strcmp(argv[1], "combine") == 0) return combine_files(argc, argv);
+    if (argc >= 2 && strcmp(argv[1], "query") == 0) return query_records(argc, argv);
     Options opt = Options::parse(argc, argv);
     FinalRuns fin(opt);
     if (opt.inputFileDirectory.empty()) {
